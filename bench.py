@@ -9,12 +9,16 @@ transcript) of the reference's vector_mul test-circuit shape at k = 10 (BASELINE
     python bench.py --config 4                              the k = 18 lookup-heavy shape, batch 1024 (configs[3])
     python bench.py --selfcheck ...                         additionally: the (sharded) path against the C oracle on the
                                                             bench's own inputs, incl. a corrupted proof on a non-root rank
+    python bench.py --dump-outputs DIR ...                  additionally: what the last timed step returned (rank 0), as
+                                                            DIR/{status,group_verdicts,verdict}.npy (float32)
 
 A step = ONE launch set: `--fold-groups` complete, independent batch verifications (each: transcript replay,
 expression / multi-open scalars, one folded MSM, one pairing check, one verdict) of `--batch` proofs per GPU that
-share one set of kernel launches.  `value` times `--blocks` blocks of `--steps` steps on inputs already resident in
-HBM (L2 flushed between steps) and reports the median block; `e2e` times the C-ABI call a user makes
+share one set of kernel launches.  `value` times `--steps` steps on inputs already resident in HBM (L2 flushed between
+steps; `--blocks R`: R such blocks, the median block is reported); `e2e` times the C-ABI call a user makes
 (`h2v_verify_batch` at N=1, `h2v_verify_shard` at N>1) from pinned host buffers, host<->device copies included.
+Inputs are the same in every run with the same arguments: seeded proofs and, on the resident path, fold coefficients
+expanded from a fixed key.
 At N>1 the one exchange step runs device-side over NVLink inside the CUDA graph (csrc/exchange.cuh); torch.distributed
 is plumbing (barriers, start-up handle exchange).  Prints ONE JSON line on rank 0.
 """
@@ -37,6 +41,9 @@ os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 METRIC = "verified proofs/sec (BN254 SHPLONK, batch 4096)"
 UNIT = "proofs/s"
 SRS_SEED = 2  # BASELINE.md config 2: SRS secret from seed 2
+# fold-coefficient key of the resident uploads (h2v_batch_set_rlc_key: the keyed expansion that OS entropy also feeds),
+# fixed so that every run verifies the same batches with the same coefficients
+FOLD_KEY = bytes(range(1, 33))
 R_MOD = 0x30644E72E131A029B85045B68181585D2833E84879B9709143E1F593F0000001
 IMAD_SLOTS_PER_MM = 272  # 8-limb CIOS: 136 32x32->64 multiply-adds = 272 lo/hi IMAD issue slots (DESIGN.md section 5)
 
@@ -245,6 +252,7 @@ def run_ours(args):
 
     def upload(ctx, pb):
         set_groups(ctx, pb)
+        chk(ctx, lib.h2v_batch_set_rlc_key(ctx._ctx, FOLD_KEY))
         if world == 1:
             chk(ctx, lib.h2v_batch_upload(ctx._ctx, *pb.args(), NULL, 0))
         else:
@@ -348,8 +356,7 @@ def run_ours(args):
     if sampler is not None:
         sampler.start()
     lib.h2v_ctx_set_blocking_sync(bv._ctx, 0)
-    lat_steps = max(8, min(steps, 32))
-    res, dt1, _ = timed_block(lambda ctx, i: step_resident(ctx, i), lat_steps, bvs[:1])
+    res, dt1, _ = timed_block(lambda ctx, i: step_resident(ctx, i), steps, bvs[:1])
     lib.h2v_ctx_set_blocking_sync(bv._ctx, 1 if blocking else 0)
     assert all(v == 1 for v in res), "a timed batch was rejected"
     # ---------------- device-resident throughput (`value`): R timed blocks of `steps` launch sets, median block
@@ -366,6 +373,15 @@ def run_ours(args):
         assert all(v == 1 for v in res), "a timed launch set was rejected"
         launches = sum(b.launch_count() for b in bvs) - launches0
         block_dt.append(dtb)
+    if args.dump_outputs and rank == 0:  # what the last timed step's caller receives: its verdicts and per-proof statuses
+        last = bvs[plan_launch_sets(steps, n_ctx)[-1]]
+        status = np.zeros(n * G, dtype=np.uint8)
+        chk(last, lib.h2v_batch_download(last._ctx, status.ctypes.data))
+        group_verdicts = np.zeros(G, dtype=np.uint8)
+        assert lib.h2v_last_group_verdicts(last._ctx, group_verdicts.ctypes.data, G) == G
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in (("status", status), ("group_verdicts", group_verdicts), ("verdict", np.array([res[-1]]))):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a.astype(np.float32))
     clocks = sampler.summary() if sampler is not None else None
     if os.environ.get("H2V_BENCH_DIAG_TIMELINE") and rank == 0 and world == 1:  # (diagnosis only) per-block timeline of 3 sets per context
         cap = 1 << 20
@@ -414,7 +430,7 @@ def run_ours(args):
         return okk
 
     lib.h2v_ctx_set_blocking_sync(bv._ctx, 0)
-    res, _, dt_e2e1 = timed_block(lambda ctx, i: timed_e2e(ctx, i, batches), lat_steps, bvs[:1])  # e2e is what the caller sees: host clock around the calls
+    res, _, dt_e2e1 = timed_block(lambda ctx, i: timed_e2e(ctx, i, batches), steps, bvs[:1])  # e2e is what the caller sees: host clock around the calls
     lib.h2v_ctx_set_blocking_sync(bv._ctx, 1 if blocking else 0)
     assert all(res), "an end-to-end batch was rejected"
     p50 = statistics.median(lat) * 1e3
@@ -482,14 +498,14 @@ def run_ours(args):
                                  f"streams (first start -> last end), max over ranks; `value` = proofs of a block / MEDIAN block time; e2e on the host clock around the C-ABI calls",
                        "host_waits": "blocking" if blocking else "spinning",
                        "l2": "flushed before every step (256 MiB overwrite on the step's stream, inside the timed region)",
-                       "fold_randomness": "OS entropy per upload (h2v.h: no scalars, no key, seed 0)",
+                       "fold_randomness": "resident path: fixed key (h2v_batch_set_rlc_key); e2e: OS entropy per call (h2v.h: no scalars, no key, seed 0)",
                        "parallelism": (f"proof-sharded x{world}: device-side exchange (csrc/exchange.cuh) - each rank's pack kernel stores its per-window partial accumulators "
                                        f"(12,320 B per global batch) into the root's HBM window over NVLink, the root (rank i mod N for launch set i) sums them in place, runs the "
                                        f"pairing check(s) and stores the verdicts into every rank's window; all inside the CUDA graph, no host or NCCL call per step")
                        if world > 1 else "one GPU"},
             "e2e": {"value": proofs_per_step * steps / dt_e2e, "unit": UNIT, "h2d_bytes_per_step": gbatches[0].h2d_bytes, "d2h_bytes_per_step": gbatches[0].d2h_bytes,
                     "ms_per_step": dt_e2e / steps * 1e3, "block_ms": [round(x * 1e3, 3) for x in block_e2e], "p50_latency_ms_one_batch": p50},
-            "one_in_flight": {"value": n * world * lat_steps / dt1, "ms_per_batch": dt1 / lat_steps * 1e3, "e2e_value": n * world * lat_steps / dt_e2e1,
+            "one_in_flight": {"value": n * world * steps / dt1, "ms_per_batch": dt1 / steps * 1e3, "e2e_value": n * world * steps / dt_e2e1,
                               "e2e_p50_latency_ms": p50, "note": f"strictly serial single batches of {n * world} proofs on one context"},
             "gpu_launches": int(launches),
             "clocks": clocks,
@@ -788,9 +804,9 @@ def main():
     os.dup2(2, 1)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20, help="launch sets per timed block")
+    ap.add_argument("--steps", type=int, default=20, help="timed launch sets (of each timed block)")
     ap.add_argument("--warmup", type=int, default=3)
-    ap.add_argument("--blocks", type=int, default=7, help="timed blocks of --steps steps; the median block is reported")
+    ap.add_argument("--blocks", type=int, default=1, help="timed blocks of --steps steps; the median block is reported")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS), help="BASELINE.json configuration (2 = configs[1], the headline)")
     ap.add_argument("--batch", type=int, default=0)
@@ -805,7 +821,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-budget", type=float, default=12.0)
     ap.add_argument("--ref-proofs-per-core", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[args.config]
     args.batch = args.batch or cfg["batch"]
     args.shape = args.shape or cfg["shape"]

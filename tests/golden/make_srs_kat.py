@@ -1,10 +1,10 @@
 """Extracts a small known-answer set from the reference's only binary fixture,
-/root/reference/halo2_verifier/params/kzg_bn254_8.srs (33,028 B, upstream PSE RawBytes layout:
-u32le k | 2^k G1 g | 2^k G1 g_lagrange | G2 g2 | G2 s_g2, coordinates in Montgomery form).
-Run in the build container (the reference tree is not available on the GPU box); the output
+halo2_verifier/params/kzg_bn254_8.srs (33,028 B, upstream PSE RawBytes layout:
+u32le k | 2^k G1 g | 2^k G1 g_lagrange | G2 g2 | G2 s_g2, coordinates in Montgomery form),
+of which tests/golden/kzg_bn254_8.srs is a copy (make_srs_fixture.py); the output
 tests/golden/srs_kat.json is committed.  Only raw bytes are copied, no interpretation."""
 import json, os, sys
-SRC = "/root/reference/halo2_verifier/params/kzg_bn254_8.srs"
+SRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "kzg_bn254_8.srs")
 raw = open(SRC, "rb").read()
 assert len(raw) == 33028
 n = 256

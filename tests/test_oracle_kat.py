@@ -27,12 +27,18 @@ def _g1(hexs):
 
 
 def test_srs_fixture_extract_matches_live_file():
-    path = "/root/reference/halo2_verifier/params/kzg_bn254_8.srs"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present (GPU box)")
-    raw = open(path, "rb").read()
+    # the fixture file as the reference's gen_srs writes it (tests/golden/make_srs_fixture.py)
+    raw = open(os.path.join(HERE, "golden", "kzg_bn254_8.srs"), "rb").read()
+    assert len(raw) == 33028
     assert raw[:4].hex() == KAT["k_le"] and raw[4:68].hex() == KAT["g"]["0"]
-    assert raw[-128:].hex() == KAT["s_g2"]
+    assert raw[-128:].hex() == KAT["s_g2"] and raw[-256:-128].hex() == KAT["g2"]
+    off_l = 4 + 256 * 64
+    for i, v in KAT["g"].items():
+        assert raw[4 + 64 * int(i): 4 + 64 * (int(i) + 1)].hex() == v
+    for i, v in KAT["g_lagrange"].items():
+        assert raw[off_l + 64 * int(i): off_l + 64 * (int(i) + 1)].hex() == v
+    params = F.params_from_srs_fixture(raw)
+    assert params.k == 8 and params.g == bn.G1_GEN and params.s_g2 == bn.g2_mul(bn.G2_GEN, S)
 
 
 def test_srs_secret_is_chacha20_zero_key():
