@@ -15,6 +15,8 @@ Host-side mirror of the reference's verification surface (ChainSafe/halo2-verifi
     Blake2bRead | Keccak256Read (+Challenge255)        transcript="blake2b" | "keccak256"
     plonk::Error  plonk/mod.rs:19-32                   Error subclasses
     (added) verify_proofs_batch                        verify_proofs_batch(..) / BatchVerifier
+    AccumulatorStrategy over proofs of several VKs     verify_proofs_mixed(..) / MixedBatchVerifier
+      poly/kzg/strategy.rs:125-140
 
 All arithmetic runs in the CUDA library `libh2v_b200.so` behind the C ABI in include/h2v.h.
 There is NO CPU fallback: importing works anywhere, but creating a verifier without the built
@@ -149,6 +151,13 @@ def load_library():
     lib.h2v_selftest_field.argtypes = [ctypes.c_int, ctypes.c_uint32, ctypes.c_uint64]
     lib.h2v_calibrate_imad.argtypes = [ctypes.c_int]
     lib.h2v_calibrate_imad.restype = ctypes.c_double
+    lib.h2v_mix_create.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_void_p, ctypes.c_uint32]
+    lib.h2v_mix_destroy.argtypes = [ctypes.c_void_p]
+    lib.h2v_mix_destroy.restype = None
+    lib.h2v_mix_last_error.argtypes = [ctypes.c_void_p]
+    lib.h2v_mix_last_error.restype = ctypes.c_char_p
+    lib.h2v_mix_set_rlc_key.argtypes = [ctypes.c_void_p, ctypes.c_char_p]
+    lib.h2v_mix_verify.argtypes = [ctypes.c_void_p, u32p, u8p, u64p, u8p, u64p, u8p, ctypes.c_uint64, u8p, u8p, ctypes.POINTER(ctypes.c_int)]
     _lib = lib
     return lib
 
@@ -160,6 +169,7 @@ EXPORTED_SYMBOLS = (
     "h2v_last_msm_geometry", "h2v_selftest_field", "h2v_calibrate_imad",
     "h2v_attribute_shard_groups", "h2v_batch_set_rlc_key", "h2v_last_rlc_source", "h2v_comm_init", "h2v_comm_connect", "h2v_comm_set_timeout_ms",
     "h2v_batch_run_shard_exchange", "h2v_verify_shard", "h2v_comm_last_batch_accum", "h2v_ctx_cache_stats", "h2v_ctx_work_model", "h2v_ctx_vk_lint",
+    "h2v_mix_create", "h2v_mix_destroy", "h2v_mix_last_error", "h2v_mix_set_rlc_key", "h2v_mix_verify",
 )
 
 COMM_HANDLE_BYTES = 128
@@ -500,6 +510,103 @@ class BatchVerifier:
         return int(self.lib.h2v_ctx_stream(self._ctx))
 
 
+@dataclass
+class MixedBatchResult:
+    status: List[List[int]]  # one list per member, in member order
+    verdict: bool  # every proof of every member accepted
+    batch_accum: Optional[bytes] = None  # folded (L, R) of the whole mix, 2 x 64 B
+
+    def errors(self):
+        return [[None if s == 0 else STATUS_ERRORS[s]() for s in st] for st in self.status]
+
+
+class MixedBatchVerifier:
+    """Proofs of several BatchVerifiers (verifying keys, SHPLONK or GWC, Blake2b or Keccak) folded into ONE MSM and ONE
+    pairing check: the reference's AccumulatorStrategy fed proofs of different VKs under one set of KZG params
+    (include/h2v.h "mixed batches").  The members' params must agree on (g, g2, s_g2); k may differ.  The members are not
+    owned: they must stay open while the mix is used and must not run their own batches during a mixed one."""
+
+    def __init__(self, members: Sequence[BatchVerifier]):
+        self.lib = load_library()
+        self.members = list(members)
+        self._mx = ctypes.c_void_p()
+        ptrs = (ctypes.c_void_p * max(1, len(self.members)))(*[m._ctx for m in self.members])
+        if self.lib.h2v_mix_create(ctypes.byref(self._mx), ptrs if self.members else None, len(self.members)) != 0:
+            self._mx = None
+            raise BackendError(self.lib.h2v_mix_last_error(None).decode())
+
+    def close(self):
+        if getattr(self, "_mx", None):
+            self.lib.h2v_mix_destroy(self._mx)
+            self._mx = None
+
+    __del__ = close
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def _check(self, rc):
+        if rc != 0:
+            raise BackendError(self.lib.h2v_mix_last_error(self._mx).decode())
+
+    def verify_batch(self, proofs_per_member, instances_per_member, rlc_scalars: Optional[Sequence[int]] = None, seed=None, key=None,
+                     want_batch_accum=False) -> MixedBatchResult:
+        """proofs_per_member[m] / instances_per_member[m]: member m's proofs and instances as for its own verify_batch
+        (empty lists allowed).  The fold runs over the member-major concatenation: rlc_scalars has one entry per proof of
+        it.  Fold randomness as BatchVerifier.verify_batch: OS entropy unless `rlc_scalars` / `key` / `seed` say otherwise."""
+        if len(proofs_per_member) != len(self.members) or len(instances_per_member) != len(self.members):
+            raise ValueError("one proof list and one instance list per member")
+        counts = (ctypes.c_uint32 * len(self.members))()
+        pparts, iparts, poffs, ioffs, keep = [], [], [0], [0], []
+        for m, (bv, proofs, insts) in enumerate(zip(self.members, proofs_per_member, instances_per_member)):
+            if len(proofs) != len(insts):
+                raise ValueError(f"member {m}: {len(proofs)} proofs, {len(insts)} instance lists")
+            counts[m] = len(proofs)
+            if not proofs:
+                continue
+            pbytes, poff, ibytes, ioff, k = bv._pack(proofs, insts)  # (sets the member's ragged layout if needed)
+            keep += k
+            pparts.append(pbytes)
+            iparts.append(ibytes)
+            poffs += [poffs[-1] + poff[j + 1] for j in range(len(proofs))]
+            ioffs += [ioffs[-1] + ioff[j + 1] for j in range(len(proofs))]
+        n = len(poffs) - 1
+        if n == 0:
+            raise ValueError("a mixed batch needs at least one proof")
+        rlc = None
+        if rlc_scalars is not None:
+            if len(rlc_scalars) != n:
+                raise ValueError("one fold scalar per proof of the concatenation")
+            rlc = b"".join(int(r).to_bytes(32, "little") for r in rlc_scalars)
+            seed = 0
+        elif key is not None:
+            if len(key) != 32:
+                raise ValueError("the fold key is 32 bytes")
+            self._check(self.lib.h2v_mix_set_rlc_key(self._mx, bytes(key)))
+            seed = 0
+        elif seed is None:
+            seed = 0
+        elif int(seed) == 0:
+            raise ValueError("seed 0 is reserved (the C ABI reads it as 'draw from the OS'): pass seed=None for OS entropy")
+        status = (ctypes.c_uint8 * n)()
+        bacc = ctypes.create_string_buffer(128) if want_batch_accum else None
+        verdict = ctypes.c_int(0)
+        self._check(self.lib.h2v_mix_verify(self._mx, counts, b"".join(pparts), (ctypes.c_uint64 * (n + 1))(*poffs), b"".join(iparts),
+                                             (ctypes.c_uint64 * (n + 1))(*ioffs), rlc, int(seed), status, bacc, ctypes.byref(verdict)))
+        st, out = list(status), []
+        for c in counts:
+            out.append(st[:c])
+            st = st[c:]
+        return MixedBatchResult(out, bool(verdict.value), bacc.raw if bacc is not None else None)
+
+    def cache_stats(self):
+        """the lead member's caches: the mix's graph captures and prepared lines are counted there"""
+        return self.members[0].cache_stats()
+
+
 def verify_proof(params: ParamsKZG, vk: VerifyingKey, proof: bytes, instances, multiopen="shplonk", transcript="blake2b",
                  device=0) -> None:
     """verify_proof with SingleStrategy (reference lib.rs:33-46): returns None or raises a plonk Error.
@@ -519,3 +626,19 @@ def verify_proofs_batch(params: ParamsKZG, vk: VerifyingKey, proofs: Sequence[by
     non-zero test `seed` is given (parity hooks: public coefficients are not sound against an adversarial prover)."""
     with BatchVerifier(params, vk, multiopen, transcript, device) as bv:
         return bv.verify_batch(proofs, instances, rlc_scalars, seed).errors()
+
+
+def verify_proofs_mixed(circuits, device=0) -> List[List[Optional[Error]]]:
+    """Mixed batch entry point: circuits = [(params, vk, proofs, instances, multiopen, transcript), ...] whose params agree
+    on (g, g2, s_g2) (k may differ).  All proofs are folded into one MSM and one pairing check (the reference's
+    AccumulatorStrategy over proofs of several VKs), with per-proof attribution when the fold is rejected.  Returns one
+    error list per circuit, as verify_proofs_batch does; the fold coefficients come from OS entropy."""
+    bvs = []
+    try:
+        for params, vk, _proofs, _insts, multiopen, transcript in circuits:
+            bvs.append(BatchVerifier(params, vk, multiopen, transcript, device))
+        with MixedBatchVerifier(bvs) as mx:
+            return mx.verify_batch([c[2] for c in circuits], [c[3] for c in circuits]).errors()
+    finally:
+        for bv in bvs:
+            bv.close()

@@ -40,6 +40,7 @@
 #include "exchange.cuh"
 #include "transcript_quad.cuh"
 #include "glv.cuh"
+#include "mix.cuh"
 
 using namespace h2v;
 
@@ -246,38 +247,6 @@ __global__ void __launch_bounds__(256) k_shared_reduce(u32 n, u32 N, u32 Sh, con
   if (t == 0) shared_sum[grp * Sh + b] = sh[0].to_canonical();
 }
 
-// Fold groups: the N = G * n proofs of an upload may be G consecutive independent batches of n proofs (own fold
-// coefficients, own MSM, own pairing check, own verdict) that share every kernel launch: the per-proof kernels run
-// over all N proofs, the MSM kernels over G * T terms and G * nb() buckets, the pairing kernels over G blocks.
-// Everything in MsmGeom is PER GROUP except G and N (the stride of the per-proof arrays).
-struct MsmGeom {
-  u32 n, P, n_mo, Sh;  // shape of one fold group
-  u32 G, N;            // fold groups, proofs of the upload (G * n)
-  u32 T;               // terms of one group = n*P (right) + n*n_mo (left) + Sh (right, shared bases)
-  // per channel (0 = right, 1 = left): window bits, windows, buckets per window (2^(c-1)),
-  // first global window index, first global bucket index
-  u32 c[2], W[2], B[2], wbase[2], bbase[2];
-  u32 Z[2];  // scalar lift range: k'' = k + z*r, z in [0, Z), keeps every window (also the top one) uniformly filled
-  u32 Wmax;  // row stride of the digit table
-  u32 m;     // buckets per reduction chunk
-  u32 glv;   // 1: every term is split into its two GLV halves (glv.cuh), rows / entries 2 t + half; windows cover 130 bits
-             // (the attribution sub-batches: half the windows -> half the doublings of their explicit window combination)
-  __host__ __device__ u32 nb() const { return W[0] * B[0] + W[1] * B[1]; }
-  __host__ __device__ u32 channel_of_term(u32 tl) const { return (tl >= n * P && tl < n * P + n * n_mo) ? 1u : 0u; }  // tl = term inside its group
-};
-
-__device__ __forceinline__ const G1Affine& msm_point(const MsmGeom& g, u32 t, const G1Affine* pts, const G1Affine* shared_pts) {
-  const u32 grp = t / g.T, tl = t % g.T;
-  const u32 nP = g.n * g.P;
-  if (tl < nP) return pts[(size_t)(tl / g.n) * g.N + grp * g.n + tl % g.n];
-  const u32 nL = g.n * g.n_mo;
-  if (tl < nP + nL) {
-    const u32 q = (tl - nP) / g.n, jl = (tl - nP) % g.n;
-    return pts[(size_t)(g.P - g.n_mo + q) * g.N + grp * g.n + jl];  // (mo_slot + q) * N + j
-  }
-  return shared_pts[tl - nP - nL];
-}
-
 // signed c-bit digits of a little-endian magnitude kk[0..NL) (bits beyond NL limbs are zero), negated when `neg`; row of
 // the digit table + bucket histogram of the term's channel
 template <int NL>
@@ -304,9 +273,13 @@ __device__ __forceinline__ void msm_emit_digits(const MsmGeom& g, u32 ch, u32 gr
   }
 }
 
-// signed c-bit digits of every term's scalar (already multiplied by c_j) + bucket histogram
+// signed c-bit digits of every term's scalar (already multiplied by c_j) + bucket histogram.  Src = SingleVkTerms: the
+// terms of g (the pointer arguments); MixTerms: the segment table of a mixed batch (g.G = 1, g.T = every term; the pointer
+// arguments are unused)
+template <class Src>
 __global__ void __launch_bounds__(128) k_msm_digits(MsmGeom g, const Fr* right, const Fr* left, const Fr* coef, const Fr* shared_sum,
-                                                    const G1Affine* shared_pts, int16_t* dig, u32* hist, const u32* parent_verdict, u32 parent_size) {
+                                                    const G1Affine* shared_pts, int16_t* dig, u32* hist, const u32* parent_verdict, u32 parent_size,
+                                                    Src src) {
   pdl_prologue();
   TlScope tl_(4, right);
   const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -316,21 +289,28 @@ __global__ void __launch_bounds__(128) k_msm_digits(MsmGeom g, const Fr* right, 
   const u32 rows = 1 + g.glv;  // digit rows of this term
   Fr k;
   u32 ch = 0;
-  if (parent_verdict && parent_verdict[(u32)(((u64)grp * g.n) / parent_size)]) {  // sub-batch of an accepted fold group: nothing to re-check
-    ch = g.channel_of_term(tl);
-    for (u32 w = 0; w < rows * g.Wmax; w++) dig[(size_t)t * rows * g.Wmax + w] = 0;
-    return;
-  }
-  if (tl < nP) {
-    const u32 j = grp * g.n + tl % g.n;
-    k = (right[(size_t)(tl / g.n) * g.N + j] * coef[j]).to_canonical();
-  } else if (tl < nP + nL) {
-    const u32 j = grp * g.n + (tl - nP) % g.n;
-    k = (left[(size_t)((tl - nP) / g.n) * g.N + j] * coef[j]).to_canonical();
-    ch = 1;
+  if constexpr (Src::mixed) {
+    const MixSeg& sg = src.seg[mix_segment(src.seg, src.count, t)];
+    const MixTerm mt = mix_term(sg, t - sg.t0);
+    k = mix_scalar(sg, mt);
+    ch = mix_channel(mt);
   } else {
-    const G1Affine& sp = shared_pts[tl - nP - nL];
-    k = (sp.x.is_zero() && sp.y.is_zero()) ? Fr::zero() : shared_sum[grp * g.Sh + tl - nP - nL];  // identity base (all-zero fixed column)
+    if (parent_verdict && parent_verdict[(u32)(((u64)grp * g.n) / parent_size)]) {  // sub-batch of an accepted fold group: nothing to re-check
+      ch = g.channel_of_term(tl);
+      for (u32 w = 0; w < rows * g.Wmax; w++) dig[(size_t)t * rows * g.Wmax + w] = 0;
+      return;
+    }
+    if (tl < nP) {
+      const u32 j = grp * g.n + tl % g.n;
+      k = (right[(size_t)(tl / g.n) * g.N + j] * coef[j]).to_canonical();
+    } else if (tl < nP + nL) {
+      const u32 j = grp * g.n + (tl - nP) % g.n;
+      k = (left[(size_t)((tl - nP) / g.n) * g.N + j] * coef[j]).to_canonical();
+      ch = 1;
+    } else {
+      const G1Affine& sp = shared_pts[tl - nP - nL];
+      k = (sp.x.is_zero() && sp.y.is_zero()) ? Fr::zero() : shared_sum[grp * g.Sh + tl - nP - nL];  // identity base (all-zero fixed column)
+    }
   }
   if (k.is_zero()) {  // excluded proof / unused slot / identity base: no bucket entries at all
     for (u32 w = 0; w < rows * g.Wmax; w++) dig[(size_t)t * rows * g.Wmax + w] = 0;
@@ -494,14 +474,21 @@ __global__ void __launch_bounds__(SCAN_NT) k_bucket_order(u32 nb, const u32* his
   }
 }
 
-__global__ void __launch_bounds__(256) k_msm_scatter(MsmGeom g, const int16_t* dig, u32* cursor, u32* sorted) {
+template <class Src>
+__global__ void __launch_bounds__(256) k_msm_scatter(MsmGeom g, const int16_t* dig, u32* cursor, u32* sorted, Src src) {
   pdl_prologue();
   TlScope tl_(5, sorted);
   const u64 total = ((u64)g.G * g.T << g.glv) * g.Wmax;
   for (u64 idx = (u64)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (u64)gridDim.x * blockDim.x) {
     const u32 row = (u32)(idx / g.Wmax), w = (u32)(idx % g.Wmax);  // row = term, or 2 term + GLV half
     const u32 t = row >> g.glv;
-    const u32 ch = g.channel_of_term(t % g.T);
+    u32 ch;
+    if constexpr (Src::mixed) {
+      const MixSeg& sg = src.seg[mix_segment(src.seg, src.count, t)];
+      ch = mix_channel(mix_term(sg, t - sg.t0));
+    } else {
+      ch = g.channel_of_term(t % g.T);
+    }
     if (w >= g.W[ch]) continue;
     const int d = dig[idx];
     if (d == 0) continue;
@@ -528,9 +515,20 @@ __device__ __forceinline__ G1Jac shfl_down_jac(const G1Jac& p, u32 delta) {
 #ifndef GLV_BUCKET_LANES
 #define GLV_BUCKET_LANES 2
 #endif
-template <bool GLV, int LANES>
+// point of term t (the source as in k_msm_digits)
+template <class Src>
+__device__ __forceinline__ const G1Affine& term_point(const MsmGeom& g, u32 t, const G1Affine* pts, const G1Affine* shared_pts, const Src& src) {
+  if constexpr (Src::mixed) {
+    const MixSeg& sg = src.seg[mix_segment(src.seg, src.count, t)];
+    return mix_point(sg, mix_term(sg, t - sg.t0));
+  } else {
+    return msm_point(g, t, pts, shared_pts);
+  }
+}
+template <bool GLV, int LANES, class Src>
 __global__ void __launch_bounds__(128) k_msm_bucket_sum(MsmGeom g, u32 nb, const u32* off, const u32* order, const u32* sorted,
-                                                        const G1Affine* pts, const G1Affine* shared_pts, G1Jac* buckets, u32 blk_off, u32 blk_total) {
+                                                        const G1Affine* pts, const G1Affine* shared_pts, G1Jac* buckets, u32 blk_off, u32 blk_total,
+                                                        Src src) {
   pdl_prologue();
   TlScope tl_(6, pts);
   if constexpr (LANES > 1) {
@@ -546,11 +544,12 @@ __global__ void __launch_bounds__(128) k_msm_bucket_sum(MsmGeom g, u32 nb, const
         for (u32 e = off[b] + q; e < e1; e += LANES) {
           const u32 ent = sorted[e], row = ent & 0x7FFFFFFFu;
           if constexpr (GLV) {
+            static_assert(!Src::mixed, "mixed batches have no GLV split");
             G1Affine pt = msm_point(g, row >> 1, pts, shared_pts);
             if (row & 1) pt.x = Fq::mul_c(pt.x, glv_beta());
             acc = g1_add_mixed(acc, pt, (ent >> 31) != 0);
           } else {
-            acc = g1_add_mixed(acc, msm_point(g, row, pts, shared_pts), (ent >> 31) != 0);
+            acc = g1_add_mixed(acc, term_point(g, row, pts, shared_pts, src), (ent >> 31) != 0);
           }
         }
       }
@@ -566,7 +565,7 @@ __global__ void __launch_bounds__(128) k_msm_bucket_sum(MsmGeom g, u32 nb, const
       const u32 e0 = off[b], e1 = off[b + 1];
       for (u32 e = e0; e < e1; e++) {
         const u32 ent = sorted[e];
-        acc = g1_add_mixed(acc, msm_point(g, ent & 0x7FFFFFFFu, pts, shared_pts), (ent >> 31) != 0);
+        acc = g1_add_mixed(acc, term_point(g, ent & 0x7FFFFFFFu, pts, shared_pts, src), (ent >> 31) != 0);
       }
       buckets[b] = acc;
     }
@@ -1322,19 +1321,11 @@ static u32 lift_range(u32 c, u32 W) {
 
 // n_geom >= n: the window geometry is chosen as for a batch of n_geom proofs (sharded batches: every
 // rank must use the same windows so that partial window sums add up, see h2v_batch_set_shard_hint)
-static MsmGeom choose_geom(u32 n, const PlanHeader& hd, u32 n_geom, u32 groups = 1, u32 force_c = 0) {
-  MsmGeom g{};
-  g.n = n;
-  g.G = groups;
-  g.N = n * groups;
-  g.P = hd.n_points;
-  g.n_mo = hd.n_mo;
-  g.Sh = hd.n_shared;
-  g.T = n * hd.n_points + n * hd.n_mo + hd.n_shared;
-  if (n_geom < n) n_geom = n;
+// window fields of g for right_terms / left_terms terms per channel and fold group (the batch size n_geom picks the chunk)
+static void choose_windows(MsmGeom& g, u32 right_terms, u32 left_terms, u32 n_geom, u32 groups, u32 force_c) {
   const double cw = groups > 1 ? 1.0 : 2.0;
-  const double chain_right = choose_window(n_geom * hd.n_points + hd.n_shared, g.c[0], g.W[0], 0.0, cw);
-  choose_window(n_geom * hd.n_mo, g.c[1], g.W[1], chain_right, cw);
+  const double chain_right = choose_window(right_terms, g.c[0], g.W[0], 0.0, cw);
+  choose_window(left_terms, g.c[1], g.W[1], chain_right, cw);
   const char* f0 = getenv("H2V_MSM_WINDOW_RIGHT");
   const char* f1 = getenv("H2V_MSM_WINDOW_LEFT");
   for (int ch = 0; ch < 2; ch++) {
@@ -1364,6 +1355,18 @@ static MsmGeom choose_geom(u32 n, const PlanHeader& hd, u32 n_geom, u32 groups =
   }
   g.glv = force_c ? 1u : 0u;
   if (force_c) g.m = g.B[0];  // the whole window is one chunk: its weighted sum IS the window sum (enqueue_msm skips the second step)
+}
+static MsmGeom choose_geom(u32 n, const PlanHeader& hd, u32 n_geom, u32 groups = 1, u32 force_c = 0) {
+  MsmGeom g{};
+  g.n = n;
+  g.G = groups;
+  g.N = n * groups;
+  g.P = hd.n_points;
+  g.n_mo = hd.n_mo;
+  g.Sh = hd.n_shared;
+  g.T = n * hd.n_points + n * hd.n_mo + hd.n_shared;
+  if (n_geom < n) n_geom = n;
+  choose_windows(g, n_geom * hd.n_points + hd.n_shared, n_geom * hd.n_mo, n_geom, groups, force_c);
   return g;
 }
 
@@ -1430,9 +1433,9 @@ static int ensure_lines(h2v_ctx* ctx, const MsmGeom& g, int* slot_out) {
 }
 static int ensure_lines(h2v_ctx* ctx, u32 groups) { return ensure_lines(ctx, pair_geom(ctx->geom, groups), &ctx->lines_cur); }
 
-// the batch pairing check over `wsums` (W0 + W1 Jacobian window sums per group) -> d_verdict[group]
-static int launch_pairing(h2v_ctx* ctx, const G1Jac* wsums, u32 groups) {
-  const MsmGeom& g = ctx->geom;
+// the batch pairing check over `wsums` (W0 + W1 Jacobian window sums per group, window geometry g, prepared lines of
+// pair_geom(g)) -> d_verdict[group]
+static int launch_pairing(h2v_ctx* ctx, const MsmGeom& g, const G2Line* lines, const G1Jac* wsums, u32 groups) {
   const MsmGeom q = pair_geom(g, groups);
   cudaStream_t s = ctx->stream;
   const PairSkip none{nullptr, nullptr, 1, 0};
@@ -1443,7 +1446,7 @@ static int launch_pairing(h2v_ctx* ctx, const G1Jac* wsums, u32 groups) {
     KLAUNCH(k_window_group, cdiv((u64)groups * np, 64), 64, 0, s, ga, groups, wsums, ctx->d_gsums.as<G1Jac>());
     pairs = ctx->d_gsums.as<G1Jac>();
   }
-  KLAUNCH((k_lines<LINES_GROUPS>), dim3(H2V_ATE_ITERS, groups), 64 * LINES_GROUPS, k_lines_smem<LINES_GROUPS>(), s, LinesArgs{np}, pairs, ctx->d_lines(),
+  KLAUNCH((k_lines<LINES_GROUPS>), dim3(H2V_ATE_ITERS, groups), 64 * LINES_GROUPS, k_lines_smem<LINES_GROUPS>(), s, LinesArgs{np}, pairs, lines,
                                                                                        ctx->d_M.as<E12>(), none);
   // (parallel Miller segments on four blocks per group when the launch is small, pairing_cta.cuh)
   static const bool seg_off = getenv("H2V_MILLER_SEGMENTS_OFF") != nullptr;
@@ -1456,6 +1459,7 @@ static int launch_pairing(h2v_ctx* ctx, const G1Jac* wsums, u32 groups) {
   }
   return 0;
 }
+static int launch_pairing(h2v_ctx* ctx, const G1Jac* wsums, u32 groups) { return launch_pairing(ctx, ctx->geom, ctx->d_lines(), wsums, groups); }
 
 // Attribution: `count` independent 2-pair checks e(pairs[i][1], [s]G2) e(pairs[i][0], -G2) == 1 (pairs: right | left accumulator,
 // Jacobian) -> verdict[i]; groups for which sk says "skip" keep their verdict word.  M: E12[count][H2V_ATE_ITERS] scratch.
@@ -1515,15 +1519,20 @@ static cudaError_t preload_kernels() {
   H2V_PRELOAD(k_rlc_expand);
   H2V_PRELOAD(k_rlc_scan);
   H2V_PRELOAD(k_shared_reduce);
-  H2V_PRELOAD(k_msm_digits);
+  H2V_PRELOAD(k_msm_digits<SingleVkTerms>);
+  H2V_PRELOAD(k_msm_digits<MixTerms>);
   H2V_PRELOAD(k_scan_tiles);
   H2V_PRELOAD(k_scan_apply);
   H2V_PRELOAD(k_bucket_order);
-  H2V_PRELOAD(k_msm_scatter);
-  H2V_PRELOAD((k_msm_bucket_sum<false, 1>));
-  H2V_PRELOAD((k_msm_bucket_sum<false, 2>));
-  H2V_PRELOAD((k_msm_bucket_sum<false, 4>));
-  H2V_PRELOAD((k_msm_bucket_sum<true, GLV_BUCKET_LANES>));
+  H2V_PRELOAD(k_msm_scatter<SingleVkTerms>);
+  H2V_PRELOAD(k_msm_scatter<MixTerms>);
+  H2V_PRELOAD((k_msm_bucket_sum<false, 1, SingleVkTerms>));
+  H2V_PRELOAD((k_msm_bucket_sum<false, 2, SingleVkTerms>));
+  H2V_PRELOAD((k_msm_bucket_sum<false, 4, SingleVkTerms>));
+  H2V_PRELOAD((k_msm_bucket_sum<true, GLV_BUCKET_LANES, SingleVkTerms>));
+  H2V_PRELOAD((k_msm_bucket_sum<false, 1, MixTerms>));
+  H2V_PRELOAD((k_msm_bucket_sum<false, 2, MixTerms>));
+  H2V_PRELOAD((k_msm_bucket_sum<false, 4, MixTerms>));
   H2V_PRELOAD(k_msm_chunk_reduce);
   H2V_PRELOAD(k_msm_window_reduce);
   H2V_PRELOAD(k_fold_accum);
@@ -1821,35 +1830,51 @@ int h2v_batch_set_scalar_hook(h2v_ctx* ctx, uint8_t* msm_scalars) {
   return 0;
 }
 
-// The MSM of G fold groups (geometry g) over the per-proof arrays of the current upload: column sums of the shared-base
-// scalars, signed digits + histogram, bucket offsets, size-ordered buckets, counting sort, bucket sums, bucket reduction
-// -> B.wsums[G][W0 + W1].  B.coef (the fold coefficients) and a zeroed B.hist must be ready on stream s.
-// parent_verdict != null (attribution): group q of g is a sub-batch of fold group q * g.n / parent_size of the batch
-// and is skipped (no bucket entries) when that group's batch check accepted.
-static int enqueue_msm(h2v_ctx* ctx, const MsmGeom& g, h2v_ctx::MsmBufs& B, cudaStream_t s, const u32* parent_verdict, u32 parent_size) {
+// Column sums of the shared-base scalars of the current upload, shared_sum[grp][b] = sum_j c_j * shared[b][j] -> B.shared_sum.
+static int enqueue_shared_reduce(h2v_ctx* ctx, const MsmGeom& g, h2v_ctx::MsmBufs& B, cudaStream_t s) {
   const PlanHeader& hd = ctx->hd;
-  PlanView pv = ctx->pv();
-  const u32 nb = g.nb() * g.G;
   if (hd.n_shared)
     KLAUNCH(k_shared_reduce, dim3(hd.n_shared, g.G), 256, 0, s, g.n, g.N, (u32)hd.n_shared, ctx->d_shared.as<Fr>(), B.coef.as<Fr>(), B.shared_sum.as<Fr>());
-  KLAUNCH(k_msm_digits, cdiv((u64)g.G * g.T, 128), 128, 0, s, g, ctx->d_right.as<Fr>(), ctx->d_left.as<Fr>(), B.coef.as<Fr>(), B.shared_sum.as<Fr>(),
-          pv.sec<G1Affine>(hd.off_shared_pts), B.dig.as<int16_t>(), B.hist.as<u32>(), parent_verdict, parent_size);
+  return 0;
+}
+
+// where the terms of a single-VK MSM live (a mixed batch passes nulls: its segment table points to the members' arrays)
+struct TermArrays {
+  const Fr *right, *left, *coef, *shared_sum;
+  const G1Affine *pts, *shared_pts;
+};
+
+// The bucket MSM from the digits on: signed digits + histogram, bucket offsets, size-ordered buckets, counting sort,
+// bucket sums, bucket reduction -> B.wsums[G][W0 + W1].  A zeroed B.hist must be ready on stream s.
+// parent_verdict != null (attribution): group q of g is a sub-batch of fold group q * g.n / parent_size of the batch
+// and is skipped (no bucket entries) when that group's batch check accepted.
+extern "C++" {  // (inside the extern "C" block of the ABI)
+template <class Src>
+static int enqueue_buckets(h2v_ctx* ctx, const MsmGeom& g, h2v_ctx::MsmBufs& B, cudaStream_t s, const TermArrays& ta, Src src,
+                           const u32* parent_verdict, u32 parent_size) {
+  const u32 nb = g.nb() * g.G;
+  KLAUNCH(k_msm_digits<Src>, cdiv((u64)g.G * g.T, 128), 128, 0, s, g, ta.right, ta.left, ta.coef, ta.shared_sum, ta.shared_pts, B.dig.as<int16_t>(),
+          B.hist.as<u32>(), parent_verdict, parent_size, src);
   const u32 n_tiles = cdiv(nb, SCAN_TILE);
   KLAUNCH(k_scan_tiles, n_tiles, SCAN_NT, 0, s, B.hist.as<u32>(), nb, B.off.as<u32>(), B.tiles.as<u32>(), B.hist.as<u32>() + nb);
   KLAUNCH(k_scan_apply, n_tiles, SCAN_NT, 0, s, nb, n_tiles, B.tiles.as<u32>(), B.off.as<u32>(), B.cursor.as<u32>());
   KLAUNCH(k_bucket_order, n_tiles, SCAN_NT, 0, s, nb, B.hist.as<u32>(), B.hist.as<u32>() + nb, B.hist.as<u32>() + nb + SIZE_BINS, B.order.as<u32>());
-  KLAUNCH(k_msm_scatter, std::min<u32>(cdiv(((u64)g.G * g.T << g.glv) * g.Wmax, 256), 148 * 16), 256, 0, s, g, B.dig.as<int16_t>(), B.cursor.as<u32>(), B.sorted.as<u32>());
+  KLAUNCH(k_msm_scatter<Src>, std::min<u32>(cdiv(((u64)g.G * g.T << g.glv) * g.Wmax, 256), 148 * 16), 256, 0, s, g, B.dig.as<int16_t>(), B.cursor.as<u32>(),
+          B.sorted.as<u32>(), src);
   {
     set_launch_class('W');
     // lanes per bucket: 1 for launch sets of several fold groups (throughput: no shuffle additions), 2 for a single batch and
     // for the attribution sub-batches (their bucket chains are latency)
     static const int lanes_env = getenv("H2V_BUCKET_LANES") ? atoi(getenv("H2V_BUCKET_LANES")) : 0;
     const u32 lanes = g.glv ? GLV_BUCKET_LANES : (lanes_env ? (u32)lanes_env : (g.G == 1 && g.n <= 8192 ? 2u : 1u));
-    auto kern = g.glv ? k_msm_bucket_sum<true, GLV_BUCKET_LANES> : lanes == 2 ? k_msm_bucket_sum<false, 2> : lanes == 4 ? k_msm_bucket_sum<false, 4> : k_msm_bucket_sum<false, 1>;
+    void (*kern)(MsmGeom, u32, const u32*, const u32*, const u32*, const G1Affine*, const G1Affine*, G1Jac*, u32, u32, Src);
+    kern = lanes == 2 ? k_msm_bucket_sum<false, 2, Src> : lanes == 4 ? k_msm_bucket_sum<false, 4, Src> : k_msm_bucket_sum<false, 1, Src>;
+    if constexpr (!Src::mixed)  // (a mixed batch has no GLV split)
+      if (g.glv) kern = k_msm_bucket_sum<true, GLV_BUCKET_LANES, Src>;
     const u32 total = wide_grid((u64)(lanes == 2 || lanes == 4 || g.glv ? lanes : 1u) * nb, 0), K = std::min(wide_split(), total), per = cdiv(total, K);
     for (u32 off = 0; off < total; off += per)
-      KLAUNCH(kern, std::min(per, total - off), 128, 0, s, g, nb, B.off.as<u32>(), B.order.as<u32>(), B.sorted.as<u32>(), ctx->d_pts.as<G1Affine>(),
-              pv.sec<G1Affine>(hd.off_shared_pts), B.buckets.as<G1Jac>(), off, total);
+      KLAUNCH(kern, std::min(per, total - off), 128, 0, s, g, nb, B.off.as<u32>(), B.order.as<u32>(), B.sorted.as<u32>(), ta.pts, ta.shared_pts,
+              B.buckets.as<G1Jac>(), off, total, src);
   }
   set_launch_class('N');
   if (g.B[0] == g.m && g.B[1] == g.m) {
@@ -1860,6 +1885,19 @@ static int enqueue_msm(h2v_ctx* ctx, const MsmGeom& g, h2v_ctx::MsmBufs& B, cuda
     KLAUNCH(k_msm_window_reduce, (g.W[0] + g.W[1]) * g.G, 128, 0, s, g, B.partials_msm.as<G1Jac>(), B.wsums.as<G1Jac>());
   }
   return 0;
+}
+}  // extern "C++"
+
+// The MSM of G fold groups (geometry g) over the per-proof arrays of the current upload: column sums of the shared-base
+// scalars, then the bucket MSM -> B.wsums[G][W0 + W1].  B.coef (the fold coefficients) and a zeroed B.hist must be ready on
+// stream s.
+static int enqueue_msm(h2v_ctx* ctx, const MsmGeom& g, h2v_ctx::MsmBufs& B, cudaStream_t s, const u32* parent_verdict, u32 parent_size) {
+  int rc = enqueue_shared_reduce(ctx, g, B, s);
+  if (rc) return rc;
+  PlanView pv = ctx->pv();
+  const TermArrays ta{ctx->d_right.as<Fr>(), ctx->d_left.as<Fr>(), B.coef.as<Fr>(), B.shared_sum.as<Fr>(), ctx->d_pts.as<G1Affine>(),
+                      pv.sec<G1Affine>(ctx->hd.off_shared_pts)};
+  return enqueue_buckets(ctx, g, B, s, ta, SingleVkTerms{}, parent_verdict, parent_size);
 }
 
 static cudaError_t ensure_msm_bufs(const MsmGeom& g, h2v_ctx::MsmBufs& B, u32 n_shared) {
@@ -2015,17 +2053,16 @@ static int upload_impl(h2v_ctx* ctx, u32 n, const u8* proofs, const u64* proof_o
 // window combination -> affine (L, R) bytes in d_acc_bytes (parity hook); RUN_PARTIAL = pack the window
 // sums into d_partial_out (sharded batches)
 enum : int { RUN_PAIRING = 1, RUN_ACCUM = 2, RUN_PARTIAL = 4, RUN_XCHG = 8, RUN_ROOT = 16 };
-static int enqueue_batch(h2v_ctx* ctx, int mode) {
+// The per-proof stages of the current upload on the context's stream, up to the point where the MSM may start: fold
+// coefficients (auxiliary stream), instance checks, decompression, transcript replay, scalar stage, and the wait for the
+// coefficients.  Shared by a context's own batches (enqueue_batch) and the members of a mixed batch.
+static int enqueue_stages(h2v_ctx* ctx) {
   const PlanHeader& hd = ctx->hd;
   const u32 n = ctx->n;
   cudaStream_t s = ctx->stream;
   PlanView pv = ctx->pv();
   const MsmGeom& g = ctx->geom;
   const u32 nb = g.nb() * g.G;
-  if ((mode & RUN_ACCUM) && g.G != 1) {
-    ctx->err = "the folded accumulator hook is defined for a single fold group";
-    return -1;
-  }
   set_launch_class('N');
   if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[0], s));
   // c_j = prod_{i>j} r_i depends only on the coefficients: scanned on the auxiliary stream while the proofs are parsed
@@ -2082,6 +2119,20 @@ static int enqueue_batch(h2v_ctx* ctx, int mode) {
   set_launch_class('N');
   if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[3], s));
   CKC(cudaStreamWaitEvent(s, ctx->ev_join, 0));
+  return 0;
+}
+
+static int enqueue_batch(h2v_ctx* ctx, int mode) {
+  cudaStream_t s = ctx->stream;
+  const MsmGeom& g = ctx->geom;
+  if ((mode & RUN_ACCUM) && g.G != 1) {
+    ctx->err = "the folded accumulator hook is defined for a single fold group";
+    return -1;
+  }
+  {
+    int src = enqueue_stages(ctx);
+    if (src) return src;
+  }
   {
     NvtxRange nv_("h2v:msm");
     int mrc = enqueue_msm(ctx, g, ctx->mb, s, nullptr, 0);
@@ -2817,6 +2868,422 @@ double h2v_calibrate_imad(int device) {
   cudaEventDestroy(b);
   cudaFree(d);
   return cudaGetLastError() == cudaSuccess ? best : -1.0;
+}
+
+// ---- mixed batches: proofs of several contexts (verifying keys) folded into one MSM and one pairing check ----------
+// The members keep their own per-proof stages; the mix owns the joint MSM's buffers, its segment table and its graphs,
+// and runs the pairing check on the lead member (member 0), whose prepared G2 lines serve every member: all members'
+// params agree on (g, g2, s_g2).
+struct h2v_mix {
+  std::vector<h2v_ctx*> m;  // members, not owned; m[0] = lead (its stream is the mix's stream)
+  std::string err;
+  cudaEvent_t ev_fork = nullptr;
+  std::vector<cudaEvent_t> ev_join;  // per member: its stages are done
+  bool has_key = false;              // one-shot key for the next batch (h2v_mix_set_rlc_key)
+  RlcKey key{};
+  h2v_ctx::MsmBufs b;  // the joint MSM (coef / shared_sum unused: the segments point to the members')
+  DevBuf d_seg;
+  std::vector<MixSeg> segs;    // of the current batch
+  std::vector<u32> seg_member;
+  MsmGeom geom{};
+  int lines_slot = -1;  // the lead's prepared lines of the joint geometry
+  h2v_ctx::GraphSlot graphs[8];  // LRU over (member shapes, buffers), as for a context
+  u64 use_clock = 0;
+};
+
+static const G1Affine& plan_g(const h2v_ctx* c) {  // params.g: the last shared base of every plan
+  PlanView pv{c->blob.data()};
+  return pv.sec<G1Affine>(c->hd.off_shared_pts)[c->hd.n_shared - 1];
+}
+
+// joint window geometry: the single-batch choice (G = 1) over the summed terms of each channel
+static MsmGeom mix_geom(u32 N, u32 T, u32 right_terms, u32 left_terms) {
+  MsmGeom g{};
+  g.n = N;  // (picks the chunk size and bucket lanes as for a single batch of N proofs; the mixed kernels map terms through the segments)
+  g.G = 1;
+  g.N = N;
+  g.T = T;
+  choose_windows(g, right_terms, left_terms, N, 1, 0);
+  return g;
+}
+
+static std::vector<h2v_ctx*> mix_active(const h2v_mix* mx) {
+  std::vector<h2v_ctx*> v;
+  for (u32 sg : mx->seg_member) v.push_back(mx->m[sg]);
+  return v;
+}
+
+// Every kernel of a mixed batch: the members' stages forked onto their own streams, the joint MSM and the pairing on the
+// lead's stream.  *fail = the context whose call failed.
+static int mix_enqueue(h2v_mix* mx, bool accum, h2v_ctx** fail) {
+  h2v_ctx* ctx = mx->m[0];
+  *fail = ctx;
+  cudaStream_t s = ctx->stream;
+  const MsmGeom& g = mx->geom;
+  CKC(cudaMemsetAsync(mx->b.hist.p, 0, 4 * ((size_t)g.nb() + 2 * SIZE_BINS), s));
+  CKC(cudaEventRecord(mx->ev_fork, s));
+  for (u32 sg = 0; sg < mx->seg_member.size(); sg++) {
+    const u32 mi = mx->seg_member[sg];
+    h2v_ctx* mb = mx->m[mi];
+    *fail = mb;
+    if (mb != ctx) {
+      cudaError_t e = cudaStreamWaitEvent(mb->stream, mx->ev_fork, 0);
+      if (e != cudaSuccess) {
+        mb->err = std::string("cudaStreamWaitEvent: ") + cudaGetErrorString(e);
+        return -2;
+      }
+    }
+    int rc = enqueue_stages(mb);
+    if (!rc) rc = enqueue_shared_reduce(mb, mb->geom, mb->mb, mb->stream);
+    if (rc) return rc;
+    if (mb != ctx) {
+      *fail = ctx;
+      CKC(cudaEventRecord(mx->ev_join[mi], mb->stream));
+      CKC(cudaStreamWaitEvent(s, mx->ev_join[mi], 0));
+    }
+  }
+  *fail = ctx;
+  {
+    NvtxRange nv_("h2v:mix_msm");
+    const MixTerms src{mx->d_seg.as<MixSeg>(), (u32)mx->segs.size()};
+    int rc = enqueue_buckets(ctx, g, mx->b, s, TermArrays{}, src, nullptr, 0);
+    if (rc) return rc;
+  }
+  {
+    NvtxRange nv_("h2v:pairing");
+    int rc = launch_pairing(ctx, g, ctx->lines[mx->lines_slot].buf.as<G2Line>(), mx->b.wsums.as<G1Jac>(), 1);
+    if (rc) return rc;
+  }
+  if (accum) {
+    FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {g.wbase[0], g.wbase[1]}};
+    KLAUNCH(k_fold_accum, 1, 32, 0, s, fa, mx->b.wsums.as<G1Jac>(), ctx->d_acc_bytes.as<u8>());
+  }
+  return 0;
+}
+
+static u64 mix_graph_key(const h2v_mix* mx, bool accum) {
+  u64 h = 0xcbf29ce484222325ull;
+  auto mix = [&h](u64 v) {
+    h ^= v;
+    h *= 0x100000001b3ull;
+    h ^= h >> 29;
+  };
+  const h2v_ctx* lead = mx->m[0];
+  const MsmGeom& g = mx->geom;
+  mix(accum);
+  for (u32 sg = 0; sg < mx->seg_member.size(); sg++) {
+    h2v_ctx* mb = mx->m[mx->seg_member[sg]];
+    mix((u64)(size_t)mb);
+    mix(graph_key(mb, 0));  // the member's shape, options and buffers (what enqueue_stages and the segment read)
+  }
+  for (int ch = 0; ch < 2; ch++) mix((u64)g.c[ch] | (u64)g.W[ch] << 8 | (u64)g.Z[ch] << 16);
+  mix((u64)g.T | (u64)g.m << 32);
+  mix(g.N);
+  const DevBuf* bufs[] = {&mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets, &mx->b.wsums,
+                          &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &lead->d_M, &lead->d_gsums, &lead->d_verdict, &lead->d_acc_bytes,
+                          &lead->lines[mx->lines_slot].buf};
+  for (const DevBuf* b : bufs) mix((u64)(size_t)b->p);
+  mix(line_run(1));
+  return h | 1;
+}
+
+// the launch set on the lead's stream: graph replay (capture on a miss) or, with the lead's graphs off, direct launches
+static int mix_run(h2v_mix* mx, bool accum, h2v_ctx** fail) {
+  h2v_ctx* lead = mx->m[0];
+  *fail = lead;
+  h2v_ctx* ctx = lead;
+  cudaStream_t s = lead->stream;
+  const std::vector<h2v_ctx*> act = mix_active(mx);
+  // the members' uploads were queued on their own streams: the launch set (forked from the lead's stream) follows them
+  for (h2v_ctx* mb : act) {
+    if (mb == lead) continue;
+    const u32 mi = (u32)(std::find(mx->m.begin(), mx->m.end(), mb) - mx->m.begin());
+    CKC(cudaEventRecord(mx->ev_join[mi], mb->stream));
+    CKC(cudaStreamWaitEvent(s, mx->ev_join[mi], 0));
+  }
+  if (!lead->use_graphs) return mix_enqueue(mx, accum, fail);
+  const u64 key = mix_graph_key(mx, accum);
+  mx->use_clock++;
+  h2v_ctx::GraphSlot* hit = nullptr;
+  h2v_ctx::GraphSlot* victim = &mx->graphs[0];
+  for (auto& sl : mx->graphs) {
+    if (sl.exec && sl.key == key) hit = &sl;
+    if (!sl.exec ? victim->exec != nullptr : (victim->exec && sl.used < victim->used)) victim = &sl;
+  }
+  h2v_ctx::GraphSlot& gs = hit ? *hit : *victim;
+  gs.used = mx->use_clock;
+  if (!hit) {
+    if (gs.exec) cudaGraphExecDestroy(gs.exec);
+    gs.exec = nullptr;
+    gs.key = 0;
+    std::vector<u64> before;
+    for (h2v_ctx* c : mx->m) before.push_back(c->launches);
+    CKC(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+    for (h2v_ctx* mb : act) mb->capturing = true;
+    const int rc = mix_enqueue(mx, accum, fail);
+    for (h2v_ctx* mb : act) mb->capturing = false;
+    cudaGraph_t graph = nullptr;
+    const cudaError_t ce = cudaStreamEndCapture(s, &graph);
+    gs.kernels = 0;
+    for (size_t i = 0; i < mx->m.size(); i++) {
+      gs.kernels += mx->m[i]->launches - before[i];
+      mx->m[i]->launches = before[i];
+    }
+    if (rc) {
+      if (graph) cudaGraphDestroy(graph);
+      return rc;
+    }
+    *fail = lead;
+    CKC(ce);
+    const cudaError_t ie = cudaGraphInstantiate(&gs.exec, graph, 0);
+    cudaGraphDestroy(graph);
+    CKC(ie);
+    gs.key = key;
+    lead->graph_captures++;
+  }
+  CKC(cudaGraphLaunch(gs.exec, s));
+  lead->launches += gs.kernels;
+  return 0;
+}
+
+static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, const u64* proof_off, const u8* instances, const u64* inst_off,
+                           const u8* rlc, u64 seed, u8* status, u8* batch_accum, int* verdict, h2v_ctx** fail) {
+  const u32 K = (u32)mx->m.size();
+  h2v_ctx* lead = mx->m[0];
+  *fail = nullptr;
+  if (!counts || !proof_off || !inst_off || !status || !verdict) {
+    mx->err = "null argument";
+    return -1;
+  }
+  u64 N = 0;
+  for (u32 i = 0; i < K; i++) N += counts[i];
+  if (N == 0 || N > 0xFFFFFFFFull) {
+    mx->err = "a mixed batch needs between 1 and 2^32 - 1 proofs";
+    return -1;
+  }
+  // caller data: validated as upload_impl validates a context's batch
+  if (proof_off[0] != 0 || inst_off[0] != 0 || (!proofs && proof_off[N]) || (!instances && inst_off[N])) {
+    mx->err = "offset arrays must start at 0";
+    return -1;
+  }
+  for (u64 j = 0; j < N; j++) {
+    if (proof_off[j + 1] < proof_off[j] || inst_off[j + 1] < inst_off[j] || proof_off[j + 1] - proof_off[j] > 0x7FFFFFFFull ||
+        inst_off[j + 1] - inst_off[j] > 0x03FFFFFFull) {
+      mx->err = "offset arrays must be non-decreasing with per-proof sizes below 2^31 bytes / 2^26 scalars";
+      return -1;
+    }
+  }
+  u64 terms = 0;
+  for (u32 i = 0; i < K; i++) {
+    const h2v_ctx* c = mx->m[i];
+    if (c->opt_fold_groups > 1 || c->opt_shard_hint) {
+      mx->err = "member " + std::to_string(i) + " has a pending fold-group or shard-hint option: mixed batches do not combine with them";
+      return -1;
+    }
+    if (counts[i]) terms += (u64)counts[i] * (c->hd.n_points + c->hd.n_mo) + c->hd.n_shared;
+  }
+  // term ids carry the sign in bit 31 (k_msm_scatter): the limit of upload_impl, over the whole mix
+  if (terms >= (1ull << 31)) {
+    mx->err = "mixed batch too large for the 32-bit index space of the MSM (split it into several batches)";
+    return -1;
+  }
+  // fold randomness, defined over the whole concatenation (c_j = prod_{i > j} r_i for j in [0, N)): explicit scalars, the
+  // mix's key, the test seed, or one key drawn from the OS for this batch; the same key is set on every member
+  RlcKey key{};
+  bool keyed = false;
+  if (!rlc && mx->has_key) {
+    key = mx->key;
+    keyed = true;
+  } else if (!rlc && seed == 0) {
+    if (os_entropy(&key, sizeof(key)) != 0) {
+      mx->err = "no OS entropy for the fold coefficients (getrandom failed)";
+      return -2;
+    }
+    keyed = true;
+  }
+  mx->has_key = false;
+  // 1. every member's slice as a shard [off, off + count) of the global batch of N proofs
+  std::vector<u32> nm(K), Pm(K), Mm(K), Sm(K);
+  u64 off = 0;
+  for (u32 i = 0; i < K; i++) {
+    h2v_ctx* c = mx->m[i];
+    nm[i] = counts[i];
+    Pm[i] = c->hd.n_points;
+    Mm[i] = c->hd.n_mo;
+    Sm[i] = c->hd.n_shared;
+    if (!counts[i]) continue;
+    std::vector<u64> po(counts[i] + 1), io(counts[i] + 1);
+    for (u32 j = 0; j <= counts[i]; j++) {
+      po[j] = proof_off[off + j] - proof_off[off];
+      io[j] = inst_off[off + j] - inst_off[off];
+    }
+    if (keyed) {
+      c->opt_key = key;
+      c->opt_has_key = true;
+    }
+    *fail = c;
+    int rc = upload_impl(c, counts[i], proofs ? proofs + proof_off[off] : nullptr, po.data(), instances ? instances + 32 * inst_off[off] : nullptr,
+                         io.data(), rlc, keyed ? 0 : seed, off, N);
+    if (rc) return rc;
+    off += counts[i];
+  }
+  // 2. segment table, joint geometry, buffers, lines
+  mx->segs.assign(K, MixSeg{});
+  mx->seg_member.assign(K, 0);
+  unsigned long long total = 0;
+  const u32 nseg = mix_layout(K, nm.data(), Pm.data(), Mm.data(), Sm.data(), mx->segs.data(), mx->seg_member.data(), &total);
+  mx->segs.resize(nseg);
+  mx->seg_member.resize(nseg);
+  u64 right_terms = 0, left_terms = 0;
+  for (u32 sg = 0; sg < nseg; sg++) {
+    MixSeg& s = mx->segs[sg];
+    h2v_ctx* c = mx->m[mx->seg_member[sg]];
+    s.right = c->d_right.as<Fr>();
+    s.left = c->d_left.as<Fr>();
+    s.coef = c->mb.coef.as<Fr>();
+    s.shared_sum = c->mb.shared_sum.as<Fr>();
+    s.pts = c->d_pts.as<G1Affine>();
+    s.shared_pts = c->pv().sec<G1Affine>(c->hd.off_shared_pts);
+    right_terms += (u64)s.n * s.P + s.Sh;
+    left_terms += (u64)s.n * s.n_mo;
+  }
+  mx->geom = mix_geom((u32)N, (u32)total, (u32)right_terms, (u32)left_terms);
+  h2v_ctx* ctx = lead;
+  *fail = lead;
+  CKC(cudaSetDevice(lead->device));
+  CKC(ensure_msm_bufs(mx->geom, mx->b, 0));
+  CKC(mx->d_seg.ensure(sizeof(MixSeg) * nseg));
+  CKC(cudaMemcpyAsync(mx->d_seg.p, mx->segs.data(), sizeof(MixSeg) * nseg, cudaMemcpyHostToDevice, lead->stream));
+  CKC(lead->d_M.ensure(sizeof(E12) * (H2V_ATE_ITERS + MILLER_SEGS)));
+  CKC(lead->d_gsums.ensure(sizeof(G1Jac) * 128));
+  CKC(lead->d_verdict.ensure(16));
+  {
+    int lrc = ensure_lines(lead, pair_geom(mx->geom, 1), &mx->lines_slot);
+    if (lrc) return lrc;
+  }
+  // 3. stages + joint MSM + pairing (one graph)
+  {
+    int rc = mix_run(mx, batch_accum != nullptr, fail);
+    if (rc) return rc;
+  }
+  *fail = lead;
+  CKC(lead->h_verd.ensure(16));
+  u32* hv = lead->h_verd.as<u32>();
+  CKC(cudaMemcpyAsync(hv, lead->d_verdict.p, 4, cudaMemcpyDeviceToHost, lead->stream));
+  if (batch_accum) CKC(cudaMemcpyAsync(batch_accum, lead->d_acc_bytes.p, 128, cudaMemcpyDeviceToHost, lead->stream));
+  CKC(ctx_sync(lead));
+  const bool accepted = hv[0] != 0;
+  // 4. statuses; on a rejected fold every member's proofs are re-checked on their own (poly/strategy.rs:26-30)
+  const std::vector<h2v_ctx*> act = mix_active(mx);
+  for (h2v_ctx* c : act) {
+    c->verdicts_on_device = false;
+    c->ran = true;
+  }
+  bool all_ok = accepted;
+  off = 0;
+  for (u32 i = 0; i < K; i++) {
+    if (!counts[i]) continue;
+    h2v_ctx* c = mx->m[i];
+    *fail = c;
+    int rc = accepted ? 0 : attribute_impl(c);
+    if (!rc) rc = download_status(c, status + off);
+    if (rc) return rc;
+    for (u32 j = 0; j < counts[i]; j++) all_ok &= status[off + j] == ST_OK;
+    off += counts[i];
+  }
+  *verdict = all_ok ? 1 : 0;
+  return 0;
+}
+
+int h2v_mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members) {
+  if (!out) {
+    g_create_error = "null argument";
+    return -1;
+  }
+  *out = nullptr;
+  if (!members || n_members == 0 || n_members > MIX_MAX_MEMBERS) {
+    g_create_error = "a mixed batch needs between 1 and " + std::to_string(MIX_MAX_MEMBERS) + " member contexts";
+    return -1;
+  }
+  const h2v_ctx* lead = members[0];
+  for (u32 i = 0; i < n_members; i++) {
+    const h2v_ctx* c = members[i];
+    if (!c || c->device < 0) {
+      g_create_error = "member " + std::to_string(i) + " is not a context";
+      return -1;
+    }
+    for (u32 j = 0; j < i; j++)
+      if (members[j] == c) {
+        g_create_error = "member " + std::to_string(i) + " repeats member " + std::to_string(j) + " (a context holds one batch)";
+        return -1;
+      }
+    if (c->device != lead->device) {
+      g_create_error = "member " + std::to_string(i) + " is on device " + std::to_string(c->device) + ", member 0 on device " + std::to_string(lead->device);
+      return -1;
+    }
+    if (memcmp(c->info.q_left, lead->info.q_left, sizeof(lead->info.q_left)) || memcmp(c->info.q_right, lead->info.q_right, sizeof(lead->info.q_right)) ||
+        memcmp(&plan_g(c), &plan_g(lead), sizeof(G1Affine))) {
+      g_create_error = "member " + std::to_string(i) + "'s params differ from member 0's in (g, g2, s_g2): their proofs cannot share one pairing check";
+      return -1;
+    }
+  }
+  h2v_mix* mx = new h2v_mix();
+  mx->m.assign(members, members + n_members);
+  mx->ev_join.assign(n_members, nullptr);
+  h2v_ctx* l = mx->m[0];
+  for (DevBuf* d : {&mx->b.coef, &mx->b.shared_sum, &mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets,
+                    &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg})
+    d->st = &l->stream;
+  cudaError_t e = cudaSetDevice(l->device);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&mx->ev_fork, cudaEventDisableTiming);
+  for (u32 i = 0; i < n_members && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&mx->ev_join[i], cudaEventDisableTiming);
+  if (e != cudaSuccess) {
+    g_create_error = std::string("cudaEventCreate: ") + cudaGetErrorString(e);
+    h2v_mix_destroy(mx);
+    return -2;
+  }
+  *out = mx;
+  return 0;
+}
+
+void h2v_mix_destroy(h2v_mix* mx) {
+  if (!mx) return;
+  h2v_ctx* l = mx->m[0];
+  cudaSetDevice(l->device);
+  cudaStreamSynchronize(l->stream);
+  for (auto& gsl : mx->graphs)
+    if (gsl.exec) cudaGraphExecDestroy(gsl.exec);
+  for (DevBuf* d : {&mx->b.coef, &mx->b.shared_sum, &mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets,
+                    &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg})
+    d->release();
+  cudaStreamSynchronize(l->stream);  // the stream-ordered frees
+  if (mx->ev_fork) cudaEventDestroy(mx->ev_fork);
+  for (cudaEvent_t ev : mx->ev_join)
+    if (ev) cudaEventDestroy(ev);
+  delete mx;
+}
+
+const char* h2v_mix_last_error(const h2v_mix* mx) { return mx ? mx->err.c_str() : g_create_error.c_str(); }
+
+int h2v_mix_set_rlc_key(h2v_mix* mx, const uint8_t* key32) {
+  if (!mx || !key32) return -1;
+  memcpy(mx->key.w, key32, 32);
+  mx->has_key = true;
+  return 0;
+}
+
+int h2v_mix_verify(h2v_mix* mx, const uint32_t* counts, const uint8_t* proofs, const uint64_t* proof_off, const uint8_t* instances,
+                   const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint8_t* status, uint8_t* batch_accum, int* verdict) {
+  if (!mx) return -1;
+  NvtxRange nv_("h2v:mix");
+  mx->err.clear();
+  h2v_ctx* fail = nullptr;
+  const int rc = mix_verify_impl(mx, counts, proofs, proof_off, instances, inst_off, rlc_scalars, seed, status, batch_accum, verdict, &fail);
+  if (rc && fail && mx->err.empty()) {
+    const size_t i = std::find(mx->m.begin(), mx->m.end(), fail) - mx->m.begin();
+    mx->err = "member " + std::to_string(i) + ": " + fail->err;
+  }
+  return rc;
 }
 
 }  // extern "C"

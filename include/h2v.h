@@ -204,6 +204,39 @@ int h2v_verify_shard(h2v_ctx* ctx, uint32_t n, const uint8_t* proofs, const uint
                      uint64_t global_count, uint32_t root, uint8_t* status, uint8_t* group_verdicts, int* verdict);
 int h2v_comm_last_batch_accum(h2v_ctx* ctx, uint8_t* batch_accum);
 
+/* ---- mixed batches: proofs of several verifying keys in ONE fold ---------------------------------------------------
+ * The reference's AccumulatorStrategy carries only the DualMSM of the params (poly/kzg/strategy.rs:125-140): a caller may
+ * loop verify_proof(params, vk_i, strategy, instances_i, transcript_i) over proofs of different VKs, and even of
+ * VerifierSHPLONK and VerifierGWC, as long as the KZG params agree, and `finalize` then runs ONE DualMSM::check
+ * (msm.rs:185-203).  A mix is that use: it is defined over existing contexts, the "members", whose params agree on
+ * (g, g2, s_g2) (k, VK, multiopen, hash and circuit_instances may differ).  Each member runs its own per-proof stages on
+ * its slice; the fold is ONE bucket MSM over the members' terms (segmented term space, csrc/mix.cuh) and one pairing check,
+ * on member 0 ("the lead", whose stream runs the batch and whose prepared G2 lines serve every member).  The whole launch
+ * set is one CUDA graph (an LRU keyed by the members' shapes and buffers; the lead's h2v_ctx_set_graphs(0) selects direct
+ * launches, h2v_ctx_cache_stats of the lead counts the captures).
+ *   h2v_mix_create  members on ONE device, 1 .. 64 distinct contexts.  The mix keeps the pointers: members must outlive it
+ *                   and must not run their own batches while a mixed batch is in flight.  Bad member sets (none, more than
+ *                   64, repeated, on different devices, params differing in (g, g2, s_g2)) are refused before any device
+ *                   call; the text is in h2v_mix_last_error(NULL).
+ *   h2v_mix_set_rlc_key   one-shot fold key of the next batch, as h2v_batch_set_rlc_key
+ *   h2v_mix_verify  counts[m] proofs of member m (0 allowed: the member takes no part); proofs / proof_off / instances /
+ *                   inst_off as h2v_verify_batch over the concatenation, member-major (member 0's proofs first).  Fold order =
+ *                   that order: proof j of the concatenation gets c_j = prod_{i>j} r_i over all N = sum counts proofs, i.e. the
+ *                   reference's AccumulatorStrategy fed member 0's proofs, then member 1's, ...  rlc_scalars (N x 32 B) / key /
+ *                   seed / OS entropy: the precedence of h2v_verify_batch, the r_i defined over the whole concatenation.
+ *                   Ragged instances: h2v_batch_set_columns on the member before the call.  status: N bytes out;
+ *                   batch_accum: optional 2 x 64 B folded affine (L, R); verdict: 1 = every proof accepted.  On a rejected
+ *                   fold every member's proofs are re-checked on their own (poly/strategy.rs:26-30), as in h2v_verify_batch.
+ *                   A member with a pending fold-group or shard-hint option is refused: mixes do not combine with them. */
+typedef struct h2v_mix h2v_mix;
+int h2v_mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members);
+void h2v_mix_destroy(h2v_mix* mx);
+const char* h2v_mix_last_error(const h2v_mix* mx);
+int h2v_mix_set_rlc_key(h2v_mix* mx, const uint8_t* key32);
+int h2v_mix_verify(h2v_mix* mx, const uint32_t* counts, const uint8_t* proofs, const uint64_t* proof_off, const uint8_t* instances,
+                   const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint8_t* status, uint8_t* batch_accum,
+                   int* verdict);
+
 /* ---- staged execution for measurement (bench.py): upload, run (device-resident), download ---- */
 int h2v_batch_upload(h2v_ctx* ctx, uint32_t n, const uint8_t* proofs, const uint64_t* proof_off,
                      const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars,
