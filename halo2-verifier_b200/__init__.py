@@ -17,6 +17,8 @@ Host-side mirror of the reference's verification surface (ChainSafe/halo2-verifi
     (added) verify_proofs_batch                        verify_proofs_batch(..) / BatchVerifier
     AccumulatorStrategy over proofs of several VKs     verify_proofs_mixed(..) / MixedBatchVerifier
       poly/kzg/strategy.rs:125-140
+    AccumulatorStrategy across calls: process, finalize  Accumulator.{absorb, finalize, to_bytes, merge}
+      poly/kzg/strategy.rs:125-140
 
 All arithmetic runs in the CUDA library `libh2v_b200.so` behind the C ABI in include/h2v.h.
 There is NO CPU fallback: importing works anywhere, but creating a verifier without the built
@@ -158,6 +160,18 @@ def load_library():
     lib.h2v_mix_last_error.restype = ctypes.c_char_p
     lib.h2v_mix_set_rlc_key.argtypes = [ctypes.c_void_p, ctypes.c_char_p]
     lib.h2v_mix_verify.argtypes = [ctypes.c_void_p, u32p, u8p, u64p, u8p, u64p, u8p, ctypes.c_uint64, u8p, u8p, ctypes.POINTER(ctypes.c_int)]
+    lib.h2v_acc_create.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_void_p, ctypes.c_uint32]
+    lib.h2v_acc_destroy.argtypes = [ctypes.c_void_p]
+    lib.h2v_acc_destroy.restype = None
+    lib.h2v_acc_last_error.argtypes = [ctypes.c_void_p]
+    lib.h2v_acc_last_error.restype = ctypes.c_char_p
+    lib.h2v_acc_set_rlc_key.argtypes = [ctypes.c_void_p, ctypes.c_char_p]
+    lib.h2v_acc_absorb.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, u8p, u64p, u8p, u64p, u8p, ctypes.c_uint64, u8p,
+                                   ctypes.POINTER(ctypes.c_uint32)]
+    lib.h2v_acc_finalize.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int), u8p, ctypes.c_uint32]
+    lib.h2v_acc_get.argtypes = [ctypes.c_void_p, u8p]
+    lib.h2v_acc_merge.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_char_p]
+    lib.h2v_acc_reset.argtypes = [ctypes.c_void_p]
     _lib = lib
     return lib
 
@@ -170,6 +184,8 @@ EXPORTED_SYMBOLS = (
     "h2v_attribute_shard_groups", "h2v_batch_set_rlc_key", "h2v_last_rlc_source", "h2v_comm_init", "h2v_comm_connect", "h2v_comm_set_timeout_ms",
     "h2v_batch_run_shard_exchange", "h2v_verify_shard", "h2v_comm_last_batch_accum", "h2v_ctx_cache_stats", "h2v_ctx_work_model", "h2v_ctx_vk_lint",
     "h2v_mix_create", "h2v_mix_destroy", "h2v_mix_last_error", "h2v_mix_set_rlc_key", "h2v_mix_verify",
+    "h2v_acc_create", "h2v_acc_destroy", "h2v_acc_last_error", "h2v_acc_set_rlc_key", "h2v_acc_absorb", "h2v_acc_finalize", "h2v_acc_get",
+    "h2v_acc_merge", "h2v_acc_reset",
 )
 
 COMM_HANDLE_BYTES = 128
@@ -576,21 +592,9 @@ class MixedBatchVerifier:
         n = len(poffs) - 1
         if n == 0:
             raise ValueError("a mixed batch needs at least one proof")
-        rlc = None
-        if rlc_scalars is not None:
-            if len(rlc_scalars) != n:
-                raise ValueError("one fold scalar per proof of the concatenation")
-            rlc = b"".join(int(r).to_bytes(32, "little") for r in rlc_scalars)
-            seed = 0
-        elif key is not None:
-            if len(key) != 32:
-                raise ValueError("the fold key is 32 bytes")
-            self._check(self.lib.h2v_mix_set_rlc_key(self._mx, bytes(key)))
-            seed = 0
-        elif seed is None:
-            seed = 0
-        elif int(seed) == 0:
-            raise ValueError("seed 0 is reserved (the C ABI reads it as 'draw from the OS'): pass seed=None for OS entropy")
+        if rlc_scalars is not None and len(rlc_scalars) != n:
+            raise ValueError("one fold scalar per proof of the concatenation")
+        rlc, seed = _fold_args(rlc_scalars, seed, key, lambda k: self._check(self.lib.h2v_mix_set_rlc_key(self._mx, k)))
         status = (ctypes.c_uint8 * n)()
         bacc = ctypes.create_string_buffer(128) if want_batch_accum else None
         verdict = ctypes.c_int(0)
@@ -605,6 +609,113 @@ class MixedBatchVerifier:
     def cache_stats(self):
         """the lead member's caches: the mix's graph captures and prepared lines are counted there"""
         return self.members[0].cache_stats()
+
+
+@dataclass
+class AbsorbResult:
+    statuses: List[int]  # final, except that 0 means "accumulated" (a pairing failure shows at finalize)
+    index: int  # record slot of this absorb (FinalizeResult.absorb_verdicts[index])
+
+
+@dataclass
+class FinalizeResult:
+    verdict: bool  # the one pairing check on the accumulator accepts
+    absorb_verdicts: List[bool]  # one per absorb / merge since the last finalize or reset; False = fails on its own
+
+
+class Accumulator:
+    """The reference's AccumulatorStrategy (poly/kzg/strategy.rs:125-140) as a value that lives across calls (include/h2v.h
+    "persistent accumulators"): batches of any BatchVerifier whose params agree with the anchor's are absorbed into one
+    device-resident DualMSM, and `finalize` runs one pairing check.  Absorbing proofs in chunks gives the same folded
+    (L, R) as one verify_batch over their concatenation with the concatenated fold scalars.  The anchor supplies the params,
+    the device and the prepared G2 lines; it is not owned and must stay open while the accumulator is used."""
+
+    def __init__(self, anchor: BatchVerifier, max_absorbs=1024):
+        self.lib = load_library()
+        self.anchor, self.max_absorbs = anchor, int(max_absorbs)
+        self._records = 0
+        self._acc = ctypes.c_void_p()
+        if self.lib.h2v_acc_create(ctypes.byref(self._acc), anchor._ctx if anchor is not None else None, self.max_absorbs) != 0:
+            self._acc = None
+            raise BackendError(self.lib.h2v_acc_last_error(None).decode())
+
+    def close(self):
+        if getattr(self, "_acc", None):
+            self.lib.h2v_acc_destroy(self._acc)
+            self._acc = None
+
+    __del__ = close
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def _check(self, rc):
+        if rc != 0:
+            raise BackendError(self.lib.h2v_acc_last_error(self._acc).decode())
+
+    def absorb(self, verifier: BatchVerifier, proofs: Sequence[bytes], instances, rlc_scalars: Optional[Sequence[int]] = None, seed=None,
+               key=None) -> AbsorbResult:
+        """AccumulatorStrategy::process for every proof, in order: proof j gets c_j = prod_{i>j} r_i and the accumulator is
+        scaled by prod_i r_i before the batch is added.  Fold randomness as BatchVerifier.verify_batch: OS entropy unless
+        `rlc_scalars` / `key` / `seed` say otherwise."""
+        if len(proofs) != len(instances):
+            raise ValueError(f"{len(proofs)} proofs, {len(instances)} instance lists")
+        n = len(proofs)
+        pbytes, poff, ibytes, ioff, keep = verifier._pack(proofs, instances)
+        rlc, seed = _fold_args(rlc_scalars, seed, key, lambda k: self._check(self.lib.h2v_acc_set_rlc_key(self._acc, k)))
+        status = (ctypes.c_uint8 * max(1, n))()
+        index = ctypes.c_uint32(0)
+        self._check(self.lib.h2v_acc_absorb(self._acc, verifier._ctx, n, pbytes, poff, ibytes, ioff, rlc, seed, status, ctypes.byref(index)))
+        self._records = index.value + 1
+        return AbsorbResult(list(status)[:n], index.value)
+
+    def finalize(self) -> FinalizeResult:
+        """DualMSM::check on the accumulator, then reset (finalize consumes the strategy).  On a rejection every absorb is
+        checked on its own: re-verify the batches whose absorb_verdicts entry is False with verify_batch."""
+        verdict = ctypes.c_int(0)
+        av = (ctypes.c_uint8 * max(1, self._records))()
+        self._check(self.lib.h2v_acc_finalize(self._acc, ctypes.byref(verdict), av, len(av)))
+        n, self._records = self._records, 0
+        return FinalizeResult(bool(verdict.value), [bool(v) for v in av[:n]])
+
+    def to_bytes(self) -> bytes:
+        """the affine L | R, 2 x 64 B (the batch_accum layout; all-zero = identity)"""
+        out = ctypes.create_string_buffer(128)
+        self._check(self.lib.h2v_acc_get(self._acc, out))
+        return out.raw
+
+    def merge(self, data: bytes, r: Optional[int] = None):
+        """acc <- r acc + P, P = another accumulator's to_bytes() (into an empty accumulator: restore a checkpoint).  r = None
+        draws r from the OS.  Non-canonical or off-curve bytes raise BackendError and leave the accumulator unchanged."""
+        if len(data) != 128:
+            raise ValueError("an accumulator is 128 bytes")
+        rb = None if r is None else int(r).to_bytes(32, "little")
+        self._check(self.lib.h2v_acc_merge(self._acc, bytes(data), rb))
+        self._records += 1
+
+    def reset(self):
+        self._check(self.lib.h2v_acc_reset(self._acc))
+        self._records = 0
+
+
+def _fold_args(rlc_scalars, seed, key, set_key):
+    """(scalar bytes, seed) of the C call for the fold randomness precedence rlc_scalars > key > seed > OS entropy;
+    `set_key(key32)` hands a key to the library object"""
+    if rlc_scalars is not None:
+        return b"".join(int(r).to_bytes(32, "little") for r in rlc_scalars), 0
+    if key is not None:
+        if len(key) != 32:
+            raise ValueError("the fold key is 32 bytes")
+        set_key(bytes(key))
+        return None, 0
+    if seed is None:
+        return None, 0
+    if int(seed) == 0:
+        raise ValueError("seed 0 is reserved (the C ABI reads it as 'draw from the OS'): pass seed=None for OS entropy")
+    return None, int(seed)
 
 
 def verify_proof(params: ParamsKZG, vk: VerifyingKey, proof: bytes, instances, multiopen="shplonk", transcript="blake2b",

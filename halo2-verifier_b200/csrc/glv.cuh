@@ -113,4 +113,21 @@ H2V_HDN inline G1Jac g1_mul_glv_part(const G1Affine& p, const GlvHalf& h, bool e
   return acc;
 }
 
+// Same with a Jacobian base (window sums and accumulators of h2v_acc_absorb, acc.cuh): phi(X, Y, Z) = (beta X, Y, Z) holds
+// in Jacobian coordinates too (x = X / Z^2 scales with X), so no inversion is needed.  (A separate function rather than a
+// template over the base, so that the affine callers' code stays as it was.)
+H2V_HDN inline G1Jac g1_mul_glv_part(const G1Jac& p, const GlvHalf& h, bool endo, u32 lo, u32 len, u32 tail) {
+  G1Jac q = p;
+  if (endo) q.X = Fq::mul_c(p.X, glv_beta());
+  if (h.neg) q.Y = q.Y.neg();
+  G1Jac acc = G1Jac::identity();
+  for (u32 i = len; i-- > 0;) {
+    const u32 bit = lo + i;
+    acc = g1_double(acc);
+    if (bit < 160 && ((h.l[bit >> 5] >> (bit & 31)) & 1u)) acc = g1_add(acc, q);
+  }
+  for (u32 i = 0; i < tail; i++) acc = g1_double(acc);
+  return acc;
+}
+
 }  // namespace h2v

@@ -17,6 +17,7 @@
 //   k_pairing_check   product of the segments, division-free final exponentiation test   msm.rs:185-203
 //   (k_pack_partial / k_sum_partials: shards of a multi-GPU batch; k_fold_accum: explicit (L, R), parity hook only)
 //   (k_pp_*, k_window_combine: per-proof accumulators / pairings: parity hook and rejection attribution, glv.cuh)
+//   (k_acc_absorb: instead of the pairing, the window sums folded into a persistent accumulator, acc.cuh)
 #include <cuda_runtime.h>
 #include <nvtx3/nvToolsExt.h>
 #include <errno.h>
@@ -41,6 +42,7 @@
 #include "transcript_quad.cuh"
 #include "glv.cuh"
 #include "mix.cuh"
+#include "acc.cuh"
 
 using namespace h2v;
 
@@ -902,6 +904,42 @@ __global__ void __launch_bounds__(128) k_pp_status(const u32* list, const u32* c
   if (!verdict[t]) status[list[base + t]] = ST_CONSTRAINT_SYSTEM_FAILURE;
 }
 
+// ---- persistent accumulators (acc.cuh): one block folds the window sums of a batch into the accumulator.
+// acc[2] = (R, L) Jacobian; records[cap][2] = (R_b, L_b) of every absorb; *count = the next record slot, kept on the device
+// so that a captured graph stays valid from one absorb to the next.  s = *r0 * *c0 = the product of the batch's r_i
+// (r_1 times the coefficient c_1 = prod_{i>1} r_i that k_rlc_scan wrote).  Four lanes per item (acc_mul_lane), the items
+// of a channel added by a tree in shared memory.
+__global__ void __launch_bounds__(4 * ACC_MAX_ITEMS) k_acc_absorb(AccGeom ag, const G1Jac* __restrict__ wsums, const Fr* r0, const Fr* c0, G1Jac* acc,
+                                                                  G1Jac* records, u32* count, u32 cap) {
+  pdl_prologue();
+  __shared__ G1Jac items[ACC_MAX_ITEMS];
+  const u32 t = threadIdx.x, item = t >> 2, q = t & 3;
+  const u32 slot = *count;
+  const bool live = item < acc_items(ag);  // no early exit: every lane takes part in the shuffles
+  G1Jac r = G1Jac::identity();
+  if (live) {
+    const Fr s = (*r0 * *c0).to_canonical();
+    G1Jac base;
+    Fr k;
+    acc_item(ag, item, wsums, acc, s, base, k);
+    r = acc_mul_lane(base, k, q);
+  }
+  r = g1_add(r, shfl_down_jac(r, 2));
+  r = g1_add(r, shfl_down_jac(r, 1));
+  if (live && q == 0) items[item] = r;
+  __syncthreads();
+  for (u32 d = ACC_TREE_SPAN / 2; d > 0; d >>= 1) {
+    acc_tree_step(ag, items, t, d);
+    __syncthreads();
+  }
+  if (slot >= cap) return;  // (the host refuses an absorb into a full record array)
+  if (t < 2) {
+    records[2 * (size_t)slot + t] = acc_batch_sum(ag, items, t);
+    acc[t] = acc_new_value(ag, items, t);
+  }
+  if (t == 0) *count = slot + 1;
+}
+
 __global__ void k_gather_scalars(PlanView pv, u32 n, const Fr* right, const Fr* shared, const Fr* left, u8* out) {
   const PlanHeader& hd = pv.h();
   const u32 nb = hd.n_points + hd.n_shared + hd.n_mo;
@@ -1093,6 +1131,12 @@ struct h2v_ctx {
     cudaGraphExec_t exec = nullptr;
   } graphs[16];             // LRU over (entry point, batch shape, buffers): alternating shapes replay, never recapture
   u64 graph_captures = 0;   // captures so far (h2v_ctx_cache_stats)
+  // accumulator of the absorb being enqueued (RUN_ABSORB, h2v_acc_absorb): its (R, L), records and record counter
+  struct AbsorbTarget {
+    G1Jac *acc = nullptr, *records = nullptr;
+    u32* count = nullptr;
+    u32 cap = 0;
+  } absorb;
   // device-side exchange of sharded batches (exchange.cuh)
   struct Comm {
     bool ready = false;
@@ -1546,6 +1590,7 @@ static cudaError_t preload_kernels() {
   H2V_PRELOAD(k_pp_mul_list);
   H2V_PRELOAD(k_pp_reduce_list);
   H2V_PRELOAD(k_pp_status);
+  H2V_PRELOAD(k_acc_absorb);
   H2V_PRELOAD(k_lines<2>);
   H2V_PRELOAD(k_gather_scalars);
   H2V_PRELOAD(k_gather_challenges);
@@ -2051,8 +2096,8 @@ static int upload_impl(h2v_ctx* ctx, u32 n, const u8* proofs, const u64* proof_o
 
 // every kernel of the batch.  mode bits: RUN_PAIRING = batch pairing check -> d_verdict; RUN_ACCUM = explicit
 // window combination -> affine (L, R) bytes in d_acc_bytes (parity hook); RUN_PARTIAL = pack the window
-// sums into d_partial_out (sharded batches)
-enum : int { RUN_PAIRING = 1, RUN_ACCUM = 2, RUN_PARTIAL = 4, RUN_XCHG = 8, RUN_ROOT = 16 };
+// sums into d_partial_out (sharded batches); RUN_ABSORB = fold the window sums into the accumulator ctx->absorb
+enum : int { RUN_PAIRING = 1, RUN_ACCUM = 2, RUN_PARTIAL = 4, RUN_XCHG = 8, RUN_ROOT = 16, RUN_ABSORB = 32 };
 // The per-proof stages of the current upload on the context's stream, up to the point where the MSM may start: fold
 // coefficients (auxiliary stream), instance checks, decompression, transcript replay, scalar stage, and the wait for the
 // coefficients.  Shared by a context's own batches (enqueue_batch) and the members of a mixed batch.
@@ -2165,6 +2210,12 @@ static int enqueue_batch(h2v_ctx* ctx, int mode) {
     }
     KLAUNCH_P(false, k_wait_verdict, 1, 64, 0, s, cm.d_dyn, cm.window, cm.lay, g.G, vd);
   }
+  if (mode & RUN_ABSORB) {
+    const AccGeom ag{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}};
+    const h2v_ctx::AbsorbTarget& at = ctx->absorb;
+    KLAUNCH(k_acc_absorb, 1, 32 * cdiv(4 * acc_items(ag), 32), 0, s, ag, ctx->mb.wsums.as<G1Jac>(), ctx->d_r.as<Fr>(), ctx->mb.coef.as<Fr>(), at.acc, at.records,
+            at.count, at.cap);
+  }
   if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[5], s));
   if (mode & RUN_ACCUM) {
     FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {g.wbase[0], g.wbase[1]}};
@@ -2201,6 +2252,11 @@ static u64 graph_key(const h2v_ctx* ctx, int mode) {
   mix((u64)(size_t)ctx->d_lines());
   mix((u64)(size_t)ctx->d_gsums.p | (u64)line_run(ctx->geom.G ? ctx->geom.G : 1) << 56);
   mix((u64)(size_t)ctx->comm.window);
+  if (mode & RUN_ABSORB) {
+    mix((u64)(size_t)ctx->absorb.acc);
+    mix((u64)(size_t)ctx->absorb.records);
+    mix((u64)(size_t)ctx->absorb.count | (u64)ctx->absorb.cap << 48);
+  }
   return h | 1;
 }
 
@@ -2896,6 +2952,12 @@ static const G1Affine& plan_g(const h2v_ctx* c) {  // params.g: the last shared 
   return pv.sec<G1Affine>(c->hd.off_shared_pts)[c->hd.n_shared - 1];
 }
 
+// the proofs of two contexts can share one pairing check: their params agree on (g, g2, s_g2)
+static bool params_agree(const h2v_ctx* a, const h2v_ctx* b) {
+  return !memcmp(a->info.q_left, b->info.q_left, sizeof(a->info.q_left)) && !memcmp(a->info.q_right, b->info.q_right, sizeof(a->info.q_right)) &&
+         !memcmp(&plan_g(a), &plan_g(b), sizeof(G1Affine));
+}
+
 // joint window geometry: the single-batch choice (G = 1) over the summed terms of each channel
 static MsmGeom mix_geom(u32 N, u32 T, u32 right_terms, u32 left_terms) {
   MsmGeom g{};
@@ -3221,8 +3283,7 @@ int h2v_mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members) {
       g_create_error = "member " + std::to_string(i) + " is on device " + std::to_string(c->device) + ", member 0 on device " + std::to_string(lead->device);
       return -1;
     }
-    if (memcmp(c->info.q_left, lead->info.q_left, sizeof(lead->info.q_left)) || memcmp(c->info.q_right, lead->info.q_right, sizeof(lead->info.q_right)) ||
-        memcmp(&plan_g(c), &plan_g(lead), sizeof(G1Affine))) {
+    if (!params_agree(c, lead)) {
       g_create_error = "member " + std::to_string(i) + "'s params differ from member 0's in (g, g2, s_g2): their proofs cannot share one pairing check";
       return -1;
     }
@@ -3284,6 +3345,301 @@ int h2v_mix_verify(h2v_mix* mx, const uint32_t* counts, const uint8_t* proofs, c
     mx->err = "member " + std::to_string(i) + ": " + fail->err;
   }
   return rc;
+}
+
+// ---- persistent accumulators: the reference's AccumulatorStrategy as a value that lives across calls ---------------
+// The DualMSM state (R, L) and one record (R_b, L_b) per absorb or merge live in device memory of the anchor's device.
+// Absorbs from several contexts (and merges, finalize, reset) are ordered through the accumulator's event: the stream that
+// works on the state waits on it first and records it afterwards.
+struct h2v_acc {
+  h2v_ctx* anchor = nullptr;  // not owned: params, device, stream of merge / finalize, prepared unit lines
+  std::string err;
+  u32 cap = 0, count = 0;  // record array: capacity, records used (host mirror of the device counter)
+  bool has_key = false;    // one-shot fold key of the next absorb (h2v_acc_set_rlc_key)
+  RlcKey key{};
+  cudaEvent_t ev = nullptr;
+  G1Jac* d_acc = nullptr;      // (R, L)
+  G1Jac* d_records = nullptr;  // [cap][2] (R_b, L_b)
+  u32* d_words = nullptr;      // [0] record counter, [1, 1 + ACC_CHECKS) verdicts of one pass of pair checks
+  u8* d_merge = nullptr;       // merge operand: (R, L) Jacobian | r | 1 (Fr, Montgomery)
+  E12* d_M = nullptr;          // Miller scratch of one pass of pair checks
+  HostBuf h_buf;               // pinned staging of the read-backs and of the merge operand
+};
+static constexpr u32 ACC_CHECKS = 1024;  // pair checks per pass (d_M: E12[ACC_CHECKS][H2V_ATE_ITERS] = 25 MB)
+static constexpr u32 ACC_MAX_RECORDS = 1u << 20;
+static constexpr size_t ACC_MERGE_BYTES = 2 * sizeof(G1Jac) + 2 * sizeof(Fr);
+
+#define CKA(call)                                                    \
+  do {                                                               \
+    cudaError_t e_ = (call);                                         \
+    if (e_ != cudaSuccess) {                                         \
+      a->err = std::string(#call) + ": " + cudaGetErrorString(e_);   \
+      return -2;                                                     \
+    }                                                                \
+  } while (0)
+
+static int acc_fail(h2v_acc* a, const char* who, const h2v_ctx* c, int rc) {
+  a->err = std::string(who) + ": " + c->err;
+  return rc;
+}
+
+// empty accumulator and record array, on stream s (which waited on a->ev)
+static int acc_clear(h2v_acc* a, cudaStream_t s) {
+  CKA(cudaMemsetAsync(a->d_acc, 0, 2 * sizeof(G1Jac), s));  // Z = 0: the identity
+  CKA(cudaMemsetAsync(a->d_words, 0, 4, s));
+  CKA(cudaEventRecord(a->ev, s));
+  a->count = 0;
+  return 0;
+}
+
+int h2v_acc_create(h2v_acc** out, h2v_ctx* anchor, uint32_t max_absorbs) {
+  if (!out) {
+    g_create_error = "null argument";
+    return -1;
+  }
+  *out = nullptr;
+  if (!anchor || anchor->device < 0) {
+    g_create_error = "an accumulator needs an anchor context (it supplies the params, the device and the prepared G2 lines)";
+    return -1;
+  }
+  if (max_absorbs == 0 || max_absorbs > ACC_MAX_RECORDS) {
+    g_create_error = "max_absorbs must be between 1 and " + std::to_string(ACC_MAX_RECORDS);
+    return -1;
+  }
+  h2v_acc* a = new h2v_acc();
+  a->anchor = anchor;
+  a->cap = max_absorbs;
+  cudaError_t e = cudaSetDevice(anchor->device);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&a->ev, cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaMalloc(&a->d_acc, 2 * sizeof(G1Jac));
+  if (e == cudaSuccess) e = cudaMalloc(&a->d_records, 2 * sizeof(G1Jac) * (size_t)max_absorbs);
+  if (e == cudaSuccess) e = cudaMalloc(&a->d_words, 4 * (size_t)(1 + ACC_CHECKS));
+  if (e == cudaSuccess) e = cudaMalloc(&a->d_merge, ACC_MERGE_BYTES);
+  if (e == cudaSuccess) e = cudaMalloc(&a->d_M, sizeof(E12) * H2V_ATE_ITERS * (size_t)std::min(max_absorbs, ACC_CHECKS));
+  if (e == cudaSuccess) e = a->h_buf.ensure(std::max<size_t>(4 * (size_t)(1 + ACC_CHECKS), ACC_MERGE_BYTES));
+  if (e == cudaSuccess && acc_clear(a, anchor->stream) == 0) e = cudaStreamSynchronize(anchor->stream);
+  else if (e == cudaSuccess) e = cudaErrorUnknown;  // (a->err names the call)
+  if (e != cudaSuccess) {
+    g_create_error = "creating the accumulator: " + (a->err.empty() ? std::string(cudaGetErrorString(e)) : a->err);
+    h2v_acc_destroy(a);
+    return -2;
+  }
+  *out = a;
+  return 0;
+}
+
+void h2v_acc_destroy(h2v_acc* a) {
+  if (!a) return;
+  cudaSetDevice(a->anchor->device);
+  if (a->ev) cudaEventSynchronize(a->ev);
+  for (void* p : {(void*)a->d_acc, (void*)a->d_records, (void*)a->d_words, (void*)a->d_merge, (void*)a->d_M})
+    if (p) cudaFree(p);
+  a->h_buf.release();
+  if (a->ev) cudaEventDestroy(a->ev);
+  delete a;
+}
+
+const char* h2v_acc_last_error(const h2v_acc* a) { return a ? a->err.c_str() : g_create_error.c_str(); }
+
+int h2v_acc_set_rlc_key(h2v_acc* a, const uint8_t* key32) {
+  if (!a || !key32) return -1;
+  memcpy(a->key.w, key32, 32);
+  a->has_key = true;
+  return 0;
+}
+
+int h2v_acc_reset(h2v_acc* a) {
+  if (!a) return -1;
+  a->err.clear();
+  CKA(cudaSetDevice(a->anchor->device));
+  CKA(cudaStreamWaitEvent(a->anchor->stream, a->ev, 0));
+  return acc_clear(a, a->anchor->stream);
+}
+
+int h2v_acc_absorb(h2v_acc* a, h2v_ctx* ctx, uint32_t n, const uint8_t* proofs, const uint64_t* proof_off, const uint8_t* instances,
+                   const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint8_t* status, uint32_t* index) {
+  if (!a) return -1;
+  NvtxRange nv_("h2v:absorb");
+  a->err.clear();
+  // refusals before any device call: the accumulator and the context stay as they are
+  if (!ctx || ctx->device < 0 || !status) {
+    a->err = "null argument";
+    return -1;
+  }
+  if (ctx->device != a->anchor->device) {
+    a->err = "the context is on device " + std::to_string(ctx->device) + ", the accumulator's anchor on device " + std::to_string(a->anchor->device);
+    return -1;
+  }
+  if (!params_agree(ctx, a->anchor)) {
+    a->err = "the context's params differ from the anchor's in (g, g2, s_g2): its proofs cannot share the accumulator's pairing check";
+    return -1;
+  }
+  if (n == 0) {
+    a->err = "an absorb needs at least one proof";
+    return -1;
+  }
+  if (a->count >= a->cap) {
+    a->err = "the record array is full (max_absorbs = " + std::to_string(a->cap) + "): finalize or reset the accumulator first";
+    return -1;
+  }
+  if (ctx->opt_fold_groups > 1 || ctx->opt_shard_hint) {
+    a->err = "the context has a pending fold-group or shard-hint option: absorbs do not combine with them";
+    return -1;
+  }
+  const bool set_key = !rlc_scalars && a->has_key;
+  if (set_key) {
+    ctx->opt_key = a->key;
+    ctx->opt_has_key = true;
+  }
+  int rc = upload_impl(ctx, n, proofs, proof_off, instances, inst_off, rlc_scalars, seed, 0, n);
+  if (rc) {
+    if (set_key) ctx->opt_has_key = false;
+    return acc_fail(a, "context", ctx, rc);
+  }
+  a->has_key = false;
+  const MsmGeom& g = ctx->geom;
+  if (g.W[0] > ACC_TREE_SPAN || g.W[1] > ACC_TREE_SPAN) {
+    a->err = "window geometry with more than " + std::to_string(ACC_TREE_SPAN) + " windows per channel";
+    return -1;
+  }
+  CKA(cudaStreamWaitEvent(ctx->stream, a->ev, 0));  // outside any capture: the previous absorb, merge or reset first
+  ctx->absorb = h2v_ctx::AbsorbTarget{a->d_acc, a->d_records, a->d_words, a->cap};
+  rc = run_impl(ctx, RUN_ABSORB);
+  ctx->absorb = h2v_ctx::AbsorbTarget{};
+  if (rc) return acc_fail(a, "context", ctx, rc);
+  CKA(cudaEventRecord(a->ev, ctx->stream));
+  if (index) *index = a->count;
+  a->count++;
+  rc = download_status(ctx, status);
+  return rc ? acc_fail(a, "context", ctx, rc) : 0;
+}
+
+// 64 bytes x | y, little-endian canonical, all-zero = identity -> Jacobian (Montgomery); false if not a point
+static bool acc_read_point(const u8* b, G1Jac& out) {
+  bool zero = true;
+  for (int i = 0; i < 64; i++) zero &= b[i] == 0;
+  out = G1Jac::identity();
+  if (zero) return true;
+  const Fq x = Fq::load_le(b), y = Fq::load_le(b + 32);
+  if (x.geq_mod() || y.geq_mod()) return false;
+  const G1Affine p{Fq::from_canonical(x), Fq::from_canonical(y)};
+  if (!g1_on_curve(p)) return false;
+  out = G1Jac::from_affine(p);
+  return true;
+}
+
+int h2v_acc_merge(h2v_acc* a, const uint8_t* in128, const uint8_t* r32) {
+  if (!a) return -1;
+  a->err.clear();
+  if (!in128) {
+    a->err = "null argument";
+    return -1;
+  }
+  G1Jac rl[2];  // (R, L): the bytes are L | R
+  if (!acc_read_point(in128 + 64, rl[0]) || !acc_read_point(in128, rl[1])) {
+    a->err = "merge operand is not two canonical G1 points (x | y little-endian, coordinates below p, on the curve)";
+    return -1;
+  }
+  Fr sc[2] = {Fr::zero(), Fr::one()};
+  if (r32) {
+    const Fr k = Fr::load_le(r32);
+    if (k.geq_mod()) {
+      a->err = "merge scalar r is not canonical (below the group order)";
+      return -1;
+    }
+    sc[0] = Fr::from_canonical(k);
+  } else {
+    u8 wide[64];
+    if (os_entropy(wide, sizeof(wide)) != 0) {
+      a->err = "no OS entropy for the merge scalar (getrandom failed)";
+      return -1;
+    }
+    sc[0] = Fr::from_uniform(wide);
+  }
+  if (a->count >= a->cap) {
+    a->err = "the record array is full (max_absorbs = " + std::to_string(a->cap) + "): finalize or reset the accumulator first";
+    return -1;
+  }
+  h2v_ctx* ctx = a->anchor;
+  cudaStream_t s = ctx->stream;
+  CKA(cudaSetDevice(ctx->device));
+  CKA(cudaStreamWaitEvent(s, a->ev, 0));
+  u8* hb = a->h_buf.as<u8>();
+  memcpy(hb, rl, sizeof(rl));
+  memcpy(hb + sizeof(rl), sc, sizeof(sc));
+  CKA(cudaMemcpyAsync(a->d_merge, hb, ACC_MERGE_BYTES, cudaMemcpyHostToDevice, s));
+  // the absorb kernel on one window per channel of weight 2^0: acc <- r acc + P, record P
+  const AccGeom ag{{1, 1}, {0, 0}};
+  const Fr* dr = (const Fr*)(a->d_merge + sizeof(rl));
+  KLAUNCH_P(false, k_acc_absorb, 1, 32 * cdiv(4 * acc_items(ag), 32), 0, s, ag, (const G1Jac*)a->d_merge, dr, dr + 1, a->d_acc, a->d_records, a->d_words, a->cap);
+  CKA(cudaEventRecord(a->ev, s));
+  a->count++;
+  CKA(ctx_sync(ctx));  // (the staging buffer is reused by the next call)
+  return 0;
+}
+
+int h2v_acc_get(const h2v_acc* ca, uint8_t* out128) {
+  h2v_acc* a = (h2v_acc*)ca;
+  if (!a || !out128) return -1;
+  a->err.clear();
+  h2v_ctx* ctx = a->anchor;
+  CKA(cudaSetDevice(ctx->device));
+  CKA(cudaStreamWaitEvent(ctx->stream, a->ev, 0));
+  CKA(cudaMemcpyAsync(a->h_buf.p, a->d_acc, 2 * sizeof(G1Jac), cudaMemcpyDeviceToHost, ctx->stream));
+  CKA(ctx_sync(ctx));
+  const G1Jac* rl = a->h_buf.as<G1Jac>();
+  for (int ch = 0; ch < 2; ch++) {  // bytes L | R, the batch_accum layout
+    u8* o = out128 + (ch == 0 ? 64 : 0);
+    G1Affine p;
+    if (!g1_to_affine(rl[ch], p)) {
+      memset(o, 0, 64);
+      continue;
+    }
+    p.x.to_canonical().store_le(o);
+    p.y.to_canonical().store_le(o + 32);
+  }
+  return 0;
+}
+
+int h2v_acc_finalize(h2v_acc* a, int* verdict, uint8_t* absorb_verdicts, uint32_t capacity) {
+  if (!a) return -1;
+  NvtxRange nv_("h2v:acc_finalize");
+  a->err.clear();
+  if (!verdict) {
+    a->err = "null argument";
+    return -1;
+  }
+  h2v_ctx* ctx = a->anchor;
+  cudaStream_t s = ctx->stream;
+  CKA(cudaSetDevice(ctx->device));
+  MsmGeom unit{};
+  unit.c[0] = unit.c[1] = 1;
+  unit.W[0] = unit.W[1] = 1;
+  int unit_slot = -1;
+  int rc = ensure_lines(ctx, unit, &unit_slot);  // lines of -G2 (pair 0, right) and [s]G2 (pair 1, left)
+  if (rc) return acc_fail(a, "anchor", ctx, rc);
+  const G2Line* unit_lines = ctx->lines[unit_slot].buf.as<G2Line>();
+  const PairSkip none{nullptr, nullptr, 1, 0};
+  u32* hv = a->h_buf.as<u32>();
+  CKA(cudaStreamWaitEvent(s, a->ev, 0));
+  // DualMSM::check (msm.rs:185-203) on the accumulator: e(L, [s]G2) e(R, -G2) == 1
+  if ((rc = launch_pair_checks(ctx, a->d_acc, 1, unit_lines, a->d_M, a->d_words + 1, none)) != 0) return acc_fail(a, "anchor", ctx, rc);
+  CKA(cudaMemcpyAsync(hv, a->d_words + 1, 4, cudaMemcpyDeviceToHost, s));
+  CKA(ctx_sync(ctx));
+  const bool ok = hv[0] != 0;
+  if (absorb_verdicts)
+    for (u32 i = 0; i < a->count && i < capacity; i++) absorb_verdicts[i] = 1;
+  // rejected: one check per record names the absorbs (and merges) that fail; the caller re-verifies those batches
+  for (u32 base = 0; !ok && base < a->count; base += ACC_CHECKS) {
+    const u32 cnt = std::min(ACC_CHECKS, a->count - base);
+    if ((rc = launch_pair_checks(ctx, a->d_records + 2 * (size_t)base, cnt, unit_lines, a->d_M, a->d_words + 1, none)) != 0) return acc_fail(a, "anchor", ctx, rc);
+    CKA(cudaMemcpyAsync(hv, a->d_words + 1, 4 * (size_t)cnt, cudaMemcpyDeviceToHost, s));
+    CKA(ctx_sync(ctx));
+    if (absorb_verdicts)
+      for (u32 i = 0; i < cnt && base + i < capacity; i++) absorb_verdicts[base + i] = hv[i] ? 1 : 0;
+  }
+  *verdict = ok ? 1 : 0;
+  return acc_clear(a, s);  // finalize(self) consumes the strategy
 }
 
 }  // extern "C"

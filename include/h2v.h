@@ -237,6 +237,47 @@ int h2v_mix_verify(h2v_mix* mx, const uint32_t* counts, const uint8_t* proofs, c
                    const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint8_t* status, uint8_t* batch_accum,
                    int* verdict);
 
+/* ---- persistent accumulators: AccumulatorStrategy as a value that lives across calls ------------------------------------
+ * The reference's AccumulatorStrategy (poly/kzg/strategy.rs:125-140) is fed proofs through any number of verify_proof calls,
+ * possibly for different VKs, and runs ONE DualMSM::check (msm.rs:185-203) at `finalize`.  An accumulator is that value: its
+ * DualMSM (L, R) lives in device memory, batches from any context whose params agree with the anchor's are absorbed into
+ * it, and h2v_acc_finalize runs one 2-pair check.
+ *   Absorb b of n proofs with fold randomness r_1..r_n (precedence of h2v_verify_batch: rlc_scalars > h2v_acc_set_rlc_key >
+ *   seed > OS entropy): proof j gets c_j = prod_{i>j} r_i, and  acc <- s_b acc + (L_b, R_b)  with s_b = prod_i r_i.  Absorbing a
+ *   sequence in chunks therefore gives bit for bit the folded (L, R) of ONE h2v_verify_batch over the concatenation with the
+ *   concatenated r_i.  Statuses are final at absorb time, except that H2V_OK means "accumulated"; failed proofs add nothing.
+ *   Every absorb and every merge appends its own (R_b, L_b) to a record array of max_absorbs entries (index: its slot).
+ *   h2v_acc_create    anchor: supplies the params (g, g2, s_g2), the device and the prepared G2 lines; not owned, must outlive
+ *                     the accumulator.  Errors of creation: h2v_acc_last_error(NULL).
+ *   h2v_acc_absorb    ctx: any context on the anchor's device whose params agree with the anchor's in (g, g2, s_g2).  Arguments
+ *                     as h2v_verify_batch.  Refused before any device call, state unchanged: such a mismatch, n = 0, a full
+ *                     record array, a pending fold-group or shard-hint option on ctx.  The launch set is the context's batch up
+ *                     to the window sums, then one kernel that folds them into the accumulator (one CUDA graph, the context's
+ *                     LRU; h2v_ctx_set_graphs(0): direct launches).  Absorbs from different contexts are ordered through an
+ *                     event the accumulator owns.
+ *   h2v_acc_finalize  verdict: 1 = the 2-pair check on (L, R) accepts (an empty accumulator accepts).  On a rejection one check
+ *                     per record: absorb_verdicts[i] (capacity bytes) = 0 for the absorbs / merges that fail on their own, and
+ *                     the caller re-verifies those batches with h2v_verify_batch for per-proof statuses (poly/strategy.rs:26-30).
+ *                     Resets the accumulator afterwards (finalize(self) consumes the strategy).
+ *   h2v_acc_get       the affine L | R, 2 x 64 B in the batch_accum layout (all-zero = identity)
+ *   h2v_acc_merge     acc <- r acc + P with P = L | R in the same layout: the DualMSM scale followed by adding another
+ *                     accumulator (of another GPU or process; into an empty accumulator: restore from a checkpoint).  r32: 32 B
+ *                     canonical, or NULL to draw r from the OS.  Non-canonical or off-curve bytes are refused, state unchanged.
+ *                     A merge is one record.
+ *   h2v_acc_reset     empty accumulator and record array
+ * Not combinable with mixed batches, fold groups, shards or the device-side exchange. */
+typedef struct h2v_acc h2v_acc;
+int h2v_acc_create(h2v_acc** out, h2v_ctx* anchor, uint32_t max_absorbs);
+void h2v_acc_destroy(h2v_acc* acc);
+const char* h2v_acc_last_error(const h2v_acc* acc);
+int h2v_acc_set_rlc_key(h2v_acc* acc, const uint8_t* key32);
+int h2v_acc_absorb(h2v_acc* acc, h2v_ctx* ctx, uint32_t n, const uint8_t* proofs, const uint64_t* proof_off, const uint8_t* instances,
+                   const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint8_t* status, uint32_t* index);
+int h2v_acc_finalize(h2v_acc* acc, int* verdict, uint8_t* absorb_verdicts, uint32_t capacity);
+int h2v_acc_get(const h2v_acc* acc, uint8_t* out128);
+int h2v_acc_merge(h2v_acc* acc, const uint8_t* in128, const uint8_t* r32);
+int h2v_acc_reset(h2v_acc* acc);
+
 /* ---- staged execution for measurement (bench.py): upload, run (device-resident), download ---- */
 int h2v_batch_upload(h2v_ctx* ctx, uint32_t n, const uint8_t* proofs, const uint64_t* proof_off,
                      const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars,
