@@ -19,6 +19,8 @@ Host-side mirror of the reference's verification surface (ChainSafe/halo2-verifi
       poly/kzg/strategy.rs:125-140
     AccumulatorStrategy across calls: process, finalize  Accumulator.{absorb, finalize, to_bytes, merge}
       poly/kzg/strategy.rs:125-140
+    (snark-verifier) KZG accumulator in the instances    accumulator=InstanceAccumulator(limbs, bits, cells)
+      of an aggregation proof, its deferred decider
 
 All arithmetic runs in the CUDA library `libh2v_b200.so` behind the C ABI in include/h2v.h.
 There is NO CPU fallback: importing works anywhere, but creating a verifier without the built
@@ -28,7 +30,7 @@ import ctypes
 import enum
 import os
 from dataclasses import dataclass
-from typing import List, Optional, Sequence
+from typing import List, Optional, Sequence, Tuple
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libh2v_b200.so")
@@ -97,6 +99,10 @@ def load_library():
                                    ctypes.c_char_p, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int]
     lib.h2v_ctx_create_multi.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_char_p, ctypes.c_size_t, ctypes.c_int,
                                          ctypes.c_char_p, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_uint32]
+    lib.h2v_ctx_create_aggregation.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_char_p, ctypes.c_size_t, ctypes.c_int,
+                                               ctypes.c_char_p, ctypes.c_size_t, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                               ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, u32p]
+    lib.h2v_batch_set_agg_scalar.argtypes = [ctypes.c_void_p, ctypes.c_char_p]
     lib.h2v_ctx_create_from_bundle.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_char_p, ctypes.c_size_t, ctypes.c_int, ctypes.c_int,
                                                ctypes.c_int]
     lib.h2v_ctx_destroy.argtypes = [ctypes.c_void_p]
@@ -185,7 +191,7 @@ EXPORTED_SYMBOLS = (
     "h2v_batch_run_shard_exchange", "h2v_verify_shard", "h2v_comm_last_batch_accum", "h2v_ctx_cache_stats", "h2v_ctx_work_model", "h2v_ctx_vk_lint",
     "h2v_mix_create", "h2v_mix_destroy", "h2v_mix_last_error", "h2v_mix_set_rlc_key", "h2v_mix_verify",
     "h2v_acc_create", "h2v_acc_destroy", "h2v_acc_last_error", "h2v_acc_set_rlc_key", "h2v_acc_absorb", "h2v_acc_finalize", "h2v_acc_get",
-    "h2v_acc_merge", "h2v_acc_reset",
+    "h2v_acc_merge", "h2v_acc_reset", "h2v_ctx_create_aggregation", "h2v_batch_set_agg_scalar",
 )
 
 COMM_HANDLE_BYTES = 128
@@ -265,6 +271,24 @@ def pack_instances(instances) -> (bytes, List[int], Optional[List[int]], Optiona
     return bytes(out), counts, ncols, col_len
 
 
+@dataclass(frozen=True)
+class InstanceAccumulator:
+    """The KZG accumulator (lhs, rhs) an aggregation circuit (snark-verifier with halo2-lib or halo2wrong) carries in its
+    public instances, whose deferred check lhs = s * rhs the verifier must run (include/h2v.h "aggregation proofs").
+    limbs, bits: snark-verifier's LimbsEncoding<LIMBS, BITS>, (3, 88) for halo2-lib, (4, 68) for halo2wrong.  cells: 4 * limbs
+    (column, row) pairs of lhs.x, lhs.y, rhs.x, rhs.y, least significant limb first; column indexes the proof's flattened
+    instance columns (instance-major with circuit_instances > 1)."""
+
+    limbs: int
+    bits: int
+    cells: Tuple[Tuple[int, int], ...]
+
+    @classmethod
+    def rows(cls, limbs, bits, column=0, first_row=0):
+        """the common layout: the 4 * limbs values in consecutive rows of one column"""
+        return cls(int(limbs), int(bits), tuple((int(column), int(first_row) + i) for i in range(4 * int(limbs))))
+
+
 @dataclass
 class BatchResult:
     status: List[int]
@@ -282,16 +306,30 @@ class BatchResult:
 class BatchVerifier:
     """One (params, vk, multiopen, transcript, device) context: owns the device plan and buffers."""
 
-    def __init__(self, params: ParamsKZG, vk: VerifyingKey, multiopen="shplonk", transcript="blake2b", device=0, circuit_instances=1):
+    def __init__(self, params: ParamsKZG, vk: VerifyingKey, multiopen="shplonk", transcript="blake2b", device=0, circuit_instances=1,
+                 accumulator: Optional[InstanceAccumulator] = None):
         """circuit_instances = m > 1: every proof carries m circuit instances in one transcript (`instances.len()` of the
-        reference's verify_proof); the `instances` entry of a proof is then a list of m column lists."""
+        reference's verify_proof); the `instances` entry of a proof is then a list of m column lists.
+        accumulator: the proofs are aggregation proofs carrying this KZG accumulator, which is checked inside the fold
+        (a proof whose carried accumulator is false fails with ConstraintSystemFailure, a malformed encoding with
+        InvalidInstances).  A malformed spec raises BackendError here, before any device work."""
         self.lib = load_library()
         self._ctx = ctypes.c_void_p()
         self.circuit_instances = int(circuit_instances)
         self.multiopen, self.transcript = multiopen, transcript
-        rc = self.lib.h2v_ctx_create_multi(ctypes.byref(self._ctx), params.data, len(params.data), int(params.format), vk.data,
-                                           len(vk.data), int(vk.format), _MULTIOPEN[multiopen], _HASH[transcript], int(device),
-                                           self.circuit_instances)
+        self.accumulator = accumulator
+        if accumulator is None:
+            rc = self.lib.h2v_ctx_create_multi(ctypes.byref(self._ctx), params.data, len(params.data), int(params.format), vk.data,
+                                               len(vk.data), int(vk.format), _MULTIOPEN[multiopen], _HASH[transcript], int(device),
+                                               self.circuit_instances)
+        else:
+            flat = [int(v) for cell in accumulator.cells for v in cell]
+            cells = (ctypes.c_uint32 * max(1, len(flat)))(*flat) if len(flat) == 8 * int(accumulator.limbs) else None
+            if cells is None and flat:
+                raise BackendError(f"aggregation spec: {len(flat) // 2} cells given, 4 * limbs = {4 * int(accumulator.limbs)} needed")
+            rc = self.lib.h2v_ctx_create_aggregation(ctypes.byref(self._ctx), params.data, len(params.data), int(params.format), vk.data,
+                                                     len(vk.data), int(vk.format), _MULTIOPEN[multiopen], _HASH[transcript], int(device),
+                                                     self.circuit_instances, int(accumulator.limbs), int(accumulator.bits), cells)
         if rc != 0:
             self._ctx = None
             raise BackendError(self.lib.h2v_last_error(None).decode())
@@ -299,7 +337,9 @@ class BatchVerifier:
         self.lib.h2v_ctx_info(self._ctx, info)
         (self.k, self.n_points, self.n_scalars, self.n_challenges, self.proof_len, self.n_inst_cols, self.n_shared,
          self.n_mo) = list(info)
-        self.n_bases = self.n_points + self.n_shared + self.n_mo
+        # scalar hook layout: on an aggregation context the carried lhs, rhs follow the proof points in both channels
+        self.n_carry = 0 if accumulator is None else 2
+        self.n_bases = self.n_points + self.n_shared + self.n_mo + 2 * self.n_carry
 
     def close(self):
         if getattr(self, "_ctx", None):
@@ -368,17 +408,26 @@ class BatchVerifier:
             raise ValueError("seed 0 is reserved (the C ABI reads it as 'draw from the OS'): pass seed=None for OS entropy")
         return None, int(seed)
 
+    def _set_agg_scalar(self, agg_scalar):
+        """rho of the carried accumulators for the next upload (needed for bit-exact accumulators with rlc_scalars)"""
+        if agg_scalar is not None:
+            self._check(self.lib.h2v_batch_set_agg_scalar(self._ctx, int(agg_scalar).to_bytes(32, "little")))
+
     def rlc_source(self):
         """of the last upload: 'scalars' | 'seed' | 'key' | 'os'"""
         return ("scalars", "seed", "key", "os")[self.lib.h2v_last_rlc_source(self._ctx)]
 
     def verify_batch(self, proofs: Sequence[bytes], instances, rlc_scalars: Optional[Sequence[int]] = None, seed=None,
-                     want_challenges=False, want_accum=False, want_batch_accum=False, want_scalars=False, fold_groups=1, key=None) -> BatchResult:
+                     want_challenges=False, want_accum=False, want_batch_accum=False, want_scalars=False, fold_groups=1, key=None,
+                     agg_scalar=None) -> BatchResult:
         """`fold_groups` = G: the proofs are G consecutive independent batches of len(proofs) / G proofs (own fold, own
         pairing check) that share every kernel launch; `group_verdicts` holds their G batch verdicts.
-        Fold randomness: OS entropy unless `rlc_scalars` / `key` / `seed` say otherwise (_fold_randomness)."""
+        Fold randomness: OS entropy unless `rlc_scalars` / `key` / `seed` say otherwise (_fold_randomness).
+        agg_scalar (aggregation contexts, with rlc_scalars): the fold scalar rho of the carried accumulators; without it
+        rho comes from the key / seed, or from the OS next to rlc_scalars."""
         n = len(proofs)
         assert n == len(instances) and n > 0
+        self._set_agg_scalar(agg_scalar)
         if fold_groups > 1:
             self._check(self.lib.h2v_batch_set_fold_groups(self._ctx, int(fold_groups)))
         pbytes, poff, ibytes, ioff, keep = self._pack(proofs, instances)
@@ -398,12 +447,13 @@ class BatchVerifier:
                            bacc.raw if bacc else None, sc.raw if sc else None, [bool(v) for v in gv[:ng]])
 
     def accumulate_shard(self, proofs, instances, global_base, global_count, rlc_scalars=None, seed=None, shard_hint=0, fold_groups=1, key=None,
-                         partial_out=None):
+                         partial_out=None, agg_scalar=None):
         """Returns (statuses, partial): `partial` is the opaque H2V_PARTIAL_BYTES blob of this shard's
         per-window bucket sums (bytes; or None when `partial_out`, a device or host pointer, receives it).
         `shard_hint` = size of the largest shard of the global batch when the
         shards are not all of the same size (every rank must use the same window geometry)."""
         n = len(proofs)
+        self._set_agg_scalar(agg_scalar)
         pbytes, poff, ibytes, ioff, keep = self._pack(proofs, instances)
         rlc, seed = self._fold_randomness(rlc_scalars, seed, key)
         status = (ctypes.c_uint8 * n)()
@@ -569,7 +619,7 @@ class MixedBatchVerifier:
             raise BackendError(self.lib.h2v_mix_last_error(self._mx).decode())
 
     def verify_batch(self, proofs_per_member, instances_per_member, rlc_scalars: Optional[Sequence[int]] = None, seed=None, key=None,
-                     want_batch_accum=False) -> MixedBatchResult:
+                     want_batch_accum=False, agg_scalar=None) -> MixedBatchResult:
         """proofs_per_member[m] / instances_per_member[m]: member m's proofs and instances as for its own verify_batch
         (empty lists allowed).  The fold runs over the member-major concatenation: rlc_scalars has one entry per proof of
         it.  Fold randomness as BatchVerifier.verify_batch: OS entropy unless `rlc_scalars` / `key` / `seed` say otherwise."""
@@ -595,6 +645,9 @@ class MixedBatchVerifier:
         if rlc_scalars is not None and len(rlc_scalars) != n:
             raise ValueError("one fold scalar per proof of the concatenation")
         rlc, seed = _fold_args(rlc_scalars, seed, key, lambda k: self._check(self.lib.h2v_mix_set_rlc_key(self._mx, k)))
+        for bv, proofs in zip(self.members, proofs_per_member):  # one rho for every aggregation member with proofs
+            if proofs and bv.accumulator is not None:
+                bv._set_agg_scalar(agg_scalar)
         status = (ctypes.c_uint8 * n)()
         bacc = ctypes.create_string_buffer(128) if want_batch_accum else None
         verdict = ctypes.c_int(0)
@@ -657,13 +710,14 @@ class Accumulator:
             raise BackendError(self.lib.h2v_acc_last_error(self._acc).decode())
 
     def absorb(self, verifier: BatchVerifier, proofs: Sequence[bytes], instances, rlc_scalars: Optional[Sequence[int]] = None, seed=None,
-               key=None) -> AbsorbResult:
+               key=None, agg_scalar=None) -> AbsorbResult:
         """AccumulatorStrategy::process for every proof, in order: proof j gets c_j = prod_{i>j} r_i and the accumulator is
         scaled by prod_i r_i before the batch is added.  Fold randomness as BatchVerifier.verify_batch: OS entropy unless
         `rlc_scalars` / `key` / `seed` say otherwise."""
         if len(proofs) != len(instances):
             raise ValueError(f"{len(proofs)} proofs, {len(instances)} instance lists")
         n = len(proofs)
+        verifier._set_agg_scalar(agg_scalar)
         pbytes, poff, ibytes, ioff, keep = verifier._pack(proofs, instances)
         rlc, seed = _fold_args(rlc_scalars, seed, key, lambda k: self._check(self.lib.h2v_acc_set_rlc_key(self._acc, k)))
         status = (ctypes.c_uint8 * max(1, n))()
@@ -719,24 +773,27 @@ def _fold_args(rlc_scalars, seed, key, set_key):
 
 
 def verify_proof(params: ParamsKZG, vk: VerifyingKey, proof: bytes, instances, multiopen="shplonk", transcript="blake2b",
-                 device=0) -> None:
+                 device=0, accumulator: Optional[InstanceAccumulator] = None) -> None:
     """verify_proof with SingleStrategy (reference lib.rs:33-46): returns None or raises a plonk Error.
-    `instances[column][row]`: public inputs of the single circuit instance."""
-    with BatchVerifier(params, vk, multiopen, transcript, device) as bv:
+    `instances[column][row]`: public inputs of the single circuit instance.  accumulator: an aggregation proof's carried
+    KZG accumulator, checked too (InstanceAccumulator)."""
+    with BatchVerifier(params, vk, multiopen, transcript, device, accumulator=accumulator) as bv:
         res = bv.verify_batch([proof], [instances])
     if res.status[0] != 0:
         raise STATUS_ERRORS[res.status[0]]()
 
 
 def verify_proofs_batch(params: ParamsKZG, vk: VerifyingKey, proofs: Sequence[bytes], instances, multiopen="shplonk",
-                        transcript="blake2b", device=0, rlc_scalars=None, seed=None) -> List[Optional[Error]]:
+                        transcript="blake2b", device=0, rlc_scalars=None, seed=None, accumulator: Optional[InstanceAccumulator] = None,
+                        agg_scalar=None) -> List[Optional[Error]]:
     """Batch entry point: one folded pairing check for the whole batch (AccumulatorStrategy,
     strategy.rs:125-140), per-proof attribution when the fold is rejected.  Returns one entry per
     proof: None (accepted) or the plonk Error the reference's verify_proof would have returned.
     The fold coefficients come from OS entropy, as in the reference (strategy.rs:129), unless `rlc_scalars` or a
-    non-zero test `seed` is given (parity hooks: public coefficients are not sound against an adversarial prover)."""
-    with BatchVerifier(params, vk, multiopen, transcript, device) as bv:
-        return bv.verify_batch(proofs, instances, rlc_scalars, seed).errors()
+    non-zero test `seed` is given (parity hooks: public coefficients are not sound against an adversarial prover).
+    accumulator: aggregation proofs; their carried KZG accumulators are checked inside the fold (InstanceAccumulator)."""
+    with BatchVerifier(params, vk, multiopen, transcript, device, accumulator=accumulator) as bv:
+        return bv.verify_batch(proofs, instances, rlc_scalars, seed, agg_scalar=agg_scalar).errors()
 
 
 def verify_proofs_mixed(circuits, device=0) -> List[List[Optional[Error]]]:

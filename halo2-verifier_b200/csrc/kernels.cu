@@ -18,6 +18,7 @@
 //   (k_pack_partial / k_sum_partials: shards of a multi-GPU batch; k_fold_accum: explicit (L, R), parity hook only)
 //   (k_pp_*, k_window_combine: per-proof accumulators / pairings: parity hook and rejection attribution, glv.cuh)
 //   (k_acc_absorb: instead of the pairing, the window sums folded into a persistent accumulator, acc.cuh)
+//   (k_agg: aggregation contexts, after k_scalar: the KZG accumulator carried in the instances -> two more MSM terms, agg.cuh)
 #include <cuda_runtime.h>
 #include <nvtx3/nvToolsExt.h>
 #include <errno.h>
@@ -43,6 +44,7 @@
 #include "glv.cuh"
 #include "mix.cuh"
 #include "acc.cuh"
+#include "agg.cuh"
 
 using namespace h2v;
 
@@ -187,6 +189,67 @@ __global__ void __launch_bounds__(64, MINB) k_scalar(PlanView pv, u32 n, const u
       for (u32 i = 0; i < hd.n_mo; i++) left[(size_t)i * n + j] = Fr::zero();
     }
   }
+}
+
+// Aggregation contexts: the KZG accumulator (lhs, rhs) carried in every proof's instances (agg.cuh), thread per proof.  In
+// DualMSM orientation, e(L, [s]G2) e(R, -G2) = 1, the decider's lhs = s rhs is a right-channel term and rhs a left-channel
+// one: lhs goes to slot n_points with right scalar rho, rhs to slot n_points + 1 with left scalar rho (plan.h msm_points), so
+// every consumer of the per-proof terms (bucket MSM, attribution, per-proof hooks, shards, mixes) sees them.  Runs after
+// k_scalar and before the shared-base sums: a proof whose encoding is invalid gets ST_INVALID_INSTANCES whatever the later
+// stages found (the precedence of the instance check, lib.rs:51-55) and all its scalars are zeroed.  An identity point gets
+// scalar 0 (the MSM kernels take every affine point as a curve point).
+__global__ void __launch_bounds__(128) k_agg(PlanView pv, u32 n, const u8* inst, const u64* inst_off, const u32* col_len, const Fr* rho,
+                                             G1Affine* pts, Fr* right, Fr* shared, Fr* left, u32* status) {
+  pdl_prologue();
+  const u32 j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n) return;
+  const PlanHeader& hd = pv.h();
+  const u32 P0 = hd.n_points, M0 = hd.n_mo, L = hd.agg_limbs, C = hd.n_inst_cols;
+  u32 st = status[j];
+  G1Affine p[2];
+  bool id[2] = {true, true};
+  bool ok = st != ST_INVALID_INSTANCES;  // (k_init found the layout malformed: the cells cannot be located)
+  if (ok) {
+    const u64 tot = inst_off[j + 1] - inst_off[j];
+    const u8* base = inst + 32 * inst_off[j];
+    const AggCell* cells = pv.sec<AggCell>(hd.off_agg);
+    for (u32 q = 0; q < 2 && ok; q++) {
+      const u8* limb[2 * AGG_MAX_LIMBS];
+      for (u32 i = 0; i < 2 * L; i++) {
+        const AggCell c = cells[2 * L * q + i];
+        u64 start = 0, len;
+        if (col_len) {
+          for (u32 k = 0; k < c.column; k++) start += col_len[(size_t)j * C + k];
+          len = col_len[(size_t)j * C + c.column];
+        } else {
+          len = tot / C;
+          start = (u64)c.column * len;
+        }
+        if (c.row >= len) ok = false;  // a ragged column too short for the cell
+        limb[i] = base + 32 * (start + (c.row < len ? c.row : 0));
+      }
+      if (ok) ok = agg_point(limb, L, hd.agg_bits, p[q], &id[q]);
+    }
+  }
+  if (!ok) {
+    st = ST_INVALID_INSTANCES;
+    status[j] = st;
+    for (u32 i = 0; i < P0; i++) right[(size_t)i * n + j] = Fr::zero();
+    for (u32 i = 0; i < hd.n_shared; i++) shared[(size_t)i * n + j] = Fr::zero();
+    for (u32 i = 0; i < M0; i++) left[(size_t)i * n + j] = Fr::zero();
+  }
+  const bool live = st == ST_OK;
+  const Fr r = *rho;
+  for (u32 q = 0; q < 2; q++) {
+    G1Affine a;
+    a.x = ok ? p[q].x : Fq::zero();
+    a.y = ok ? p[q].y : Fq::zero();
+    pts[(size_t)(P0 + q) * n + j] = a;
+  }
+  right[(size_t)P0 * n + j] = live && !id[0] ? r : Fr::zero();
+  right[(size_t)(P0 + 1) * n + j] = Fr::zero();
+  left[(size_t)M0 * n + j] = Fr::zero();
+  left[(size_t)(M0 + 1) * n + j] = live && !id[1] ? r : Fr::zero();
 }
 
 // fold randomness r_i: caller-supplied bytes (parity hook), a 64-bit test seed (parity hook), or the secret per-batch key
@@ -746,7 +809,8 @@ __global__ void __launch_bounds__(128) k_sum_partials(u32 n_partials, u32 cbits,
 __global__ void __launch_bounds__(128) k_pp_mul(PlanView pv, u32 n, const G1Affine* pts, const Fr* right, const Fr* shared, const Fr* left,
                                                 const u32* status, G1Jac* out, const u32* gverdict, u32 gsize) {
   const PlanHeader& hd = pv.h();
-  const u32 nb = hd.n_points + hd.n_shared + hd.n_mo;
+  const u32 nP = msm_points(hd), nM = msm_mo(hd);
+  const u32 nb = nP + hd.n_shared + nM;
   const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= nb * n) return;
   const u32 j = t % n, b = t / n;
@@ -754,16 +818,16 @@ __global__ void __launch_bounds__(128) k_pp_mul(PlanView pv, u32 n, const G1Affi
   if ((status[j] == ST_OK || status[j] == ST_CONSTRAINT_SYSTEM_FAILURE) && !(gverdict && gverdict[j / gsize])) {
     Fr k;
     const G1Affine* p;
-    if (b < hd.n_points) {
+    if (b < nP) {
       k = right[(size_t)b * n + j];
       p = &pts[(size_t)b * n + j];
-    } else if (b < hd.n_points + hd.n_shared) {
-      k = shared[(size_t)(b - hd.n_points) * n + j];
-      p = &pv.sec<G1Affine>(hd.off_shared_pts)[b - hd.n_points];
+    } else if (b < nP + hd.n_shared) {
+      k = shared[(size_t)(b - nP) * n + j];
+      p = &pv.sec<G1Affine>(hd.off_shared_pts)[b - nP];
     } else {
-      const u32 q = b - hd.n_points - hd.n_shared;
+      const u32 q = b - nP - hd.n_shared;
       k = left[(size_t)q * n + j];
-      p = &pts[(size_t)(hd.n_points - hd.n_mo + q) * n + j];
+      p = &pts[(size_t)(nP - nM + q) * n + j];
     }
     if (!k.is_zero() && !(p->x.is_zero() && p->y.is_zero())) {
       k = k.to_canonical();
@@ -780,8 +844,8 @@ __global__ void __launch_bounds__(128) k_pp_reduce(PlanView pv, u32 n, const G1J
   if (t >= 2 * n) return;
   const u32 j = t % n, ch = t / n;  // ch 0 = left, 1 = right
   G1Jac acc = G1Jac::identity();
-  const u32 b0 = ch == 0 ? hd.n_points + hd.n_shared : 0;
-  const u32 b1 = ch == 0 ? hd.n_points + hd.n_shared + hd.n_mo : hd.n_points + hd.n_shared;
+  const u32 b0 = ch == 0 ? msm_points(hd) + hd.n_shared : 0;
+  const u32 b1 = ch == 0 ? msm_points(hd) + hd.n_shared + msm_mo(hd) : msm_points(hd) + hd.n_shared;
   for (u32 b = b0; b < b1; b++) acc = g1_add(acc, prod[(size_t)b * n + j]);
   lr[(size_t)ch * n + j] = acc;
   if (accum_bytes) {
@@ -844,7 +908,8 @@ __global__ void __launch_bounds__(128) k_pp_mul_list(PlanView pv, u32 n, const G
                                                      const u32* list, const u32* count, u32 base, u32 cap, G1Jac* out) {
   TlScope tl_(12, out);
   const PlanHeader& hd = pv.h();
-  const u32 nb = hd.n_points + hd.n_shared + hd.n_mo;
+  const u32 nP = msm_points(hd), nM = msm_mo(hd);
+  const u32 nb = nP + hd.n_shared + nM;
   const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
   const u32 cnt = chunk_count(*count, base, cap);
   const u32 item = t >> 2, q = t & 3;  // item = (base, suspect); no early exit: all lanes take part in the shuffles
@@ -857,16 +922,16 @@ __global__ void __launch_bounds__(128) k_pp_mul_list(PlanView pv, u32 n, const G
     const u32 j = list[base + slot];
     Fr k;
     const G1Affine* p;
-    if (b < hd.n_points) {
+    if (b < nP) {
       k = right[(size_t)b * n + j];
       p = &pts[(size_t)b * n + j];
-    } else if (b < hd.n_points + hd.n_shared) {
-      k = shared[(size_t)(b - hd.n_points) * n + j];
-      p = &pv.sec<G1Affine>(hd.off_shared_pts)[b - hd.n_points];
+    } else if (b < nP + hd.n_shared) {
+      k = shared[(size_t)(b - nP) * n + j];
+      p = &pv.sec<G1Affine>(hd.off_shared_pts)[b - nP];
     } else {
-      const u32 qq = b - hd.n_points - hd.n_shared;
+      const u32 qq = b - nP - hd.n_shared;
       k = left[(size_t)qq * n + j];
-      p = &pts[(size_t)(hd.n_points - hd.n_mo + qq) * n + j];
+      p = &pts[(size_t)(nP - nM + qq) * n + j];
     }
     if (!k.is_zero() && !(p->x.is_zero() && p->y.is_zero())) {
       k = k.to_canonical();
@@ -890,8 +955,8 @@ __global__ void __launch_bounds__(128) k_pp_reduce_list(PlanView pv, const u32* 
   if (t >= 2 * cnt) return;
   const u32 slot = t >> 1, ch = t & 1;  // ch 0 = right, 1 = left
   G1Jac acc = G1Jac::identity();
-  const u32 b0 = ch == 1 ? hd.n_points + hd.n_shared : 0;
-  const u32 b1 = ch == 1 ? hd.n_points + hd.n_shared + hd.n_mo : hd.n_points + hd.n_shared;
+  const u32 b0 = ch == 1 ? msm_points(hd) + hd.n_shared : 0;
+  const u32 b1 = ch == 1 ? msm_points(hd) + hd.n_shared + msm_mo(hd) : msm_points(hd) + hd.n_shared;
   for (u32 b = b0; b < b1; b++) acc = g1_add(acc, prod[(size_t)b * cap + slot]);
   pairs[t] = acc;
 }
@@ -942,13 +1007,12 @@ __global__ void __launch_bounds__(4 * ACC_MAX_ITEMS) k_acc_absorb(AccGeom ag, co
 
 __global__ void k_gather_scalars(PlanView pv, u32 n, const Fr* right, const Fr* shared, const Fr* left, u8* out) {
   const PlanHeader& hd = pv.h();
-  const u32 nb = hd.n_points + hd.n_shared + hd.n_mo;
+  const u32 nP = msm_points(hd);
+  const u32 nb = nP + hd.n_shared + msm_mo(hd);
   const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= nb * n) return;
   const u32 j = t % n, b = t / n;
-  Fr k = b < hd.n_points ? right[(size_t)b * n + j]
-                         : b < hd.n_points + hd.n_shared ? shared[(size_t)(b - hd.n_points) * n + j]
-                                                         : left[(size_t)(b - hd.n_points - hd.n_shared) * n + j];
+  Fr k = b < nP ? right[(size_t)b * n + j] : b < nP + hd.n_shared ? shared[(size_t)(b - nP) * n + j] : left[(size_t)(b - nP - hd.n_shared) * n + j];
   k.to_canonical().store_le(out + ((size_t)j * nb + b) * 32);
 }
 
@@ -1111,6 +1175,8 @@ struct h2v_ctx {
   bool opt_has_key = false;  // next upload: fold randomness expanded from this 256-bit key (h2v_batch_set_rlc_key)
   RlcKey opt_key{};
   u32 rlc_source = 0;  // of the last upload: 0 caller scalars, 1 test seed, 2 caller key, 3 key drawn from the OS
+  bool opt_has_agg_scalar = false;  // next upload of an aggregation context: rho from the caller (h2v_batch_set_agg_scalar)
+  Fr opt_agg_scalar{}, h_rho{};     // (Montgomery) the caller's rho; rho of the last upload, source of its copy to d_rho
   // prepared G2 window lines, one slot per window geometry (small LRU: a service alternating batch shapes on one
   // context must not rebuild ~5,000 lines on the host at every call)
   struct LinesSlot {
@@ -1160,12 +1226,12 @@ struct h2v_ctx {
   } mb, ab;
   DevBuf d_plan, d_proofs, d_proof_off, d_inst, d_inst_off, d_ncols, d_col_len, d_pts, d_bad, d_status, d_vals, d_scratch, d_right,
       d_shared, d_left, d_rlc_bytes, d_r, d_acc_bytes, d_verdict, d_partials, d_pp_prod, d_pp_lr, d_pp_bytes, d_hook, d_chal, d_flush, d_M, d_partial_out,
-      d_wsums_fin, d_sub_pairs, d_sub_verdict, d_sub_M, d_gsums, d_ptsc;
+      d_wsums_fin, d_sub_pairs, d_sub_verdict, d_sub_M, d_gsums, d_ptsc, d_rho;
   const G2Line* d_lines() const { return lines_cur >= 0 ? lines[lines_cur].buf.as<G2Line>() : nullptr; }
   std::vector<DevBuf*> all_bufs() {
     std::vector<DevBuf*> v = {&d_plan, &d_proofs, &d_proof_off, &d_inst, &d_inst_off, &d_ncols, &d_col_len, &d_pts, &d_bad, &d_status, &d_vals, &d_scratch,
                               &d_right, &d_shared, &d_left, &d_rlc_bytes, &d_r, &d_acc_bytes, &d_verdict, &d_partials, &d_pp_prod, &d_pp_lr, &d_pp_bytes,
-                              &d_hook, &d_chal, &d_flush, &d_M, &d_partial_out, &d_wsums_fin, &d_sub_pairs, &d_sub_verdict, &d_sub_M, &d_gsums, &d_ptsc,
+                              &d_hook, &d_chal, &d_flush, &d_M, &d_partial_out, &d_wsums_fin, &d_sub_pairs, &d_sub_verdict, &d_sub_M, &d_gsums, &d_ptsc, &d_rho,
                               &lines[0].buf, &lines[1].buf, &lines[2].buf, &lines[3].buf};
     for (MsmBufs* m : {&mb, &ab})
       for (DevBuf* d : {&m->coef, &m->shared_sum, &m->dig, &m->hist, &m->off, &m->cursor, &m->order, &m->sorted, &m->buckets, &m->wsums, &m->partials_msm, &m->tiles})
@@ -1247,6 +1313,23 @@ static u32 narrow_grid(u64 units) {
   }();
   const u32 u = (u32)std::min<u64>(units, 0x7FFFFFFFu);
   return cap ? std::min(u, cap) : u;
+}
+
+// rho of an aggregation context's upload: Blake2b-512("h2v-rla" | key[32]) mod r, or "h2v-rla" | seed_le64 for the test
+// seed (the personalisation and reduction of the r_i, stages.cuh; its own tag keeps rho independent of every r_i)
+static Fr agg_scalar(const RlcKey* key, u64 seed) {
+  Blake2b b;
+  b.init_halo2();
+  const char* tag = "h2v-rla";
+  for (int t = 0; t < 7; t++) b.update_byte((u8)tag[t]);
+  if (key) {
+    for (int t = 0; t < 32; t++) b.update_byte((u8)(key->w[t >> 2] >> (8 * (t & 3))));
+  } else {
+    for (int t = 0; t < 8; t++) b.update_byte((u8)(seed >> (8 * t)));
+  }
+  u8 d[64];
+  b.digest(d);
+  return Fr::from_uniform(d);
 }
 
 // `len` bytes from the kernel's CSPRNG; 0 on success
@@ -1405,12 +1488,12 @@ static MsmGeom choose_geom(u32 n, const PlanHeader& hd, u32 n_geom, u32 groups =
   g.n = n;
   g.G = groups;
   g.N = n * groups;
-  g.P = hd.n_points;
-  g.n_mo = hd.n_mo;
+  g.P = msm_points(hd);
+  g.n_mo = msm_mo(hd);
   g.Sh = hd.n_shared;
-  g.T = n * hd.n_points + n * hd.n_mo + hd.n_shared;
+  g.T = n * g.P + n * g.n_mo + hd.n_shared;
   if (n_geom < n) n_geom = n;
-  choose_windows(g, n_geom * hd.n_points + hd.n_shared, n_geom * hd.n_mo, n_geom, groups, force_c);
+  choose_windows(g, n_geom * g.P + hd.n_shared, n_geom * g.n_mo, n_geom, groups, force_c);
   return g;
 }
 
@@ -1591,6 +1674,7 @@ static cudaError_t preload_kernels() {
   H2V_PRELOAD(k_pp_reduce_list);
   H2V_PRELOAD(k_pp_status);
   H2V_PRELOAD(k_acc_absorb);
+  H2V_PRELOAD(k_agg);
   H2V_PRELOAD(k_lines<2>);
   H2V_PRELOAD(k_gather_scalars);
   H2V_PRELOAD(k_gather_challenges);
@@ -1639,15 +1723,17 @@ int h2v_ctx_create(h2v_ctx** out, const uint8_t* params, size_t params_len, int 
   return h2v_ctx_create_multi(out, params, params_len, params_format, vk, vk_len, vk_format, multiopen, hash, device, 1);
 }
 
-int h2v_ctx_create_multi(h2v_ctx** out, const uint8_t* params, size_t params_len, int params_format, const uint8_t* vk, size_t vk_len,
-                         int vk_format, int multiopen, int hash, int device, uint32_t circuit_instances) {
+}  // extern "C"
+
+static int ctx_create(h2v_ctx** out, const uint8_t* params, size_t params_len, int params_format, const uint8_t* vk, size_t vk_len, int vk_format,
+                      int multiopen, int hash, int device, uint32_t circuit_instances, const AggSpec* agg) {
   if (!out || !params || !vk) {
     g_create_error = "null argument";
     return -1;
   }
   h2v_ctx* ctx = new h2v_ctx();
   std::string err;
-  if (build_plan(params, params_len, params_format, vk, vk_len, vk_format, multiopen, hash, ctx->blob, ctx->info, err, circuit_instances) != 0) {
+  if (build_plan(params, params_len, params_format, vk, vk_len, vk_format, multiopen, hash, ctx->blob, ctx->info, err, circuit_instances, agg) != 0) {
     g_create_error = err;
     h2v_ctx_destroy(ctx);
     return -1;
@@ -1688,10 +1774,37 @@ int h2v_ctx_create_multi(h2v_ctx** out, const uint8_t* params, size_t params_len
       (e = cudaStreamSynchronize(ctx->stream)) != cudaSuccess)
     return fail("cudaMemcpy(plan)", e);
   if ((e = ctx->d_acc_bytes.ensure(128)) != cudaSuccess || (e = ctx->d_verdict.ensure(16)) != cudaSuccess) return fail("cudaMalloc", e);
+  if (ctx->hd.n_carry && (e = ctx->d_rho.ensure(sizeof(Fr))) != cudaSuccess) return fail("cudaMalloc", e);
   if ((e = cudaFuncSetAttribute(k_lines<LINES_GROUPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k_lines_smem<LINES_GROUPS>())) != cudaSuccess)
     return fail("cudaFuncSetAttribute(k_lines)", e);
   if ((e = preload_kernels()) != cudaSuccess) return fail("loading the kernels", e);
   *out = ctx;
+  return 0;
+}
+
+extern "C" {
+
+int h2v_ctx_create_multi(h2v_ctx** out, const uint8_t* params, size_t params_len, int params_format, const uint8_t* vk, size_t vk_len,
+                         int vk_format, int multiopen, int hash, int device, uint32_t circuit_instances) {
+  return ctx_create(out, params, params_len, params_format, vk, vk_len, vk_format, multiopen, hash, device, circuit_instances, nullptr);
+}
+
+int h2v_ctx_create_aggregation(h2v_ctx** out, const uint8_t* params, size_t params_len, int params_format, const uint8_t* vk, size_t vk_len,
+                               int vk_format, int multiopen, int hash, int device, uint32_t circuit_instances, uint32_t limbs, uint32_t bits,
+                               const uint32_t* cells) {
+  const AggSpec spec{limbs, bits, cells};
+  return ctx_create(out, params, params_len, params_format, vk, vk_len, vk_format, multiopen, hash, device, circuit_instances, &spec);
+}
+
+int h2v_batch_set_agg_scalar(h2v_ctx* ctx, const uint8_t* rho32) {
+  if (!ctx || !rho32) return -1;
+  const Fr k = Fr::load_le(rho32);
+  if (!ctx->hd.n_carry || k.geq_mod() || k.is_zero()) {
+    ctx->err = ctx->hd.n_carry ? "the aggregation scalar must be canonical and non-zero" : "not an aggregation context";
+    return -1;
+  }
+  ctx->opt_agg_scalar = Fr::from_canonical(k);
+  ctx->opt_has_agg_scalar = true;
   return 0;
 }
 
@@ -1992,8 +2105,8 @@ static int upload_impl(h2v_ctx* ctx, u32 n, const u8* proofs, const u64* proof_o
   {
     // 32-bit index spaces of the kernels: term ids carry the sign in bit 31 (k_msm_scatter), k_decompress indexes
     // (proof, point) pairs and the per-proof arrays with 32-bit products
-    const u64 terms = (u64)n * (hd.n_points + hd.n_mo) + (u64)hd.n_shared * groups;
-    const u64 widest = std::max<u64>(std::max<u64>(hd.n_points, hd.n_vals), hd.n_points + hd.n_shared + hd.n_mo);
+    const u64 terms = (u64)n * (msm_points(hd) + msm_mo(hd)) + (u64)hd.n_shared * groups;
+    const u64 widest = std::max<u64>(std::max<u64>(msm_points(hd), hd.n_vals), msm_points(hd) + hd.n_shared + msm_mo(hd));
     if (terms >= (1ull << 31) || (u64)n * widest >= (1ull << 32)) {
       ctx->err = "batch too large for the 32-bit index space of the MSM (split it into several uploads)";
       return -1;
@@ -2028,15 +2141,15 @@ static int upload_impl(h2v_ctx* ctx, u32 n, const u8* proofs, const u64* proof_o
   CKC(ctx->d_proof_off.ensure(8 * (size_t)(n + 1)));
   CKC(ctx->d_inst.ensure(32 * iscal + 64));
   CKC(ctx->d_inst_off.ensure(8 * (size_t)(n + 1)));
-  CKC(ctx->d_pts.ensure(sizeof(G1Affine) * (size_t)n * hd.n_points));
+  CKC(ctx->d_pts.ensure(sizeof(G1Affine) * (size_t)n * msm_points(hd)));
   if (hd.hash == HASH_BLAKE2B) CKC(ctx->d_ptsc.ensure(64 * (size_t)n * hd.n_points));
   CKC(ctx->d_bad.ensure(4 * (size_t)n));
   CKC(ctx->d_status.ensure(4 * (size_t)n));
   CKC(ctx->d_vals.ensure(32 * (size_t)n * hd.n_vals));
   CKC(ctx->d_scratch.ensure(32 * (size_t)n * ctx->scratch_rows));
-  CKC(ctx->d_right.ensure(32 * (size_t)n * hd.n_points));
+  CKC(ctx->d_right.ensure(32 * (size_t)n * msm_points(hd)));
   CKC(ctx->d_shared.ensure(32 * (size_t)n * hd.n_shared));
-  CKC(ctx->d_left.ensure(32 * (size_t)n * hd.n_mo));
+  CKC(ctx->d_left.ensure(32 * (size_t)n * msm_mo(hd)));
   CKC(ctx->d_r.ensure(32 * (size_t)gcount * groups));
   CKC(ctx->d_partial_out.ensure((size_t)H2V_PARTIAL_BYTES * groups));
   CKC(ctx->d_wsums_fin.ensure(sizeof(G1Jac) * 128 * (size_t)groups));
@@ -2088,6 +2201,22 @@ static int upload_impl(h2v_ctx* ctx, u32 n, const u8* proofs, const u64* proof_o
     ctx->rlc_source = 3;
   }
   ctx->opt_has_key = false;
+  if (hd.n_carry) {  // rho of the carried accumulators (k_agg): one per upload, independent of the r_i (DESIGN.md section 6.3)
+    if (!rlc) {
+      ctx->h_rho = agg_scalar(keyed ? &key : nullptr, seed);
+    } else if (ctx->opt_has_agg_scalar) {
+      ctx->h_rho = ctx->opt_agg_scalar;
+    } else {
+      u8 wide[64];
+      if (os_entropy(wide, sizeof(wide)) != 0) {
+        ctx->err = "no OS entropy for the aggregation scalar (getrandom failed)";
+        return -2;
+      }
+      ctx->h_rho = Fr::from_uniform(wide);
+    }
+    CKC(cudaMemcpyAsync(ctx->d_rho.p, &ctx->h_rho, sizeof(Fr), cudaMemcpyHostToDevice, s));
+  }
+  ctx->opt_has_agg_scalar = false;
   k_rlc_expand<<<cdiv(n_r, 128), 128, 0, s>>>(n_r, seed, rlc ? ctx->d_rlc_bytes.as<u8>() : nullptr, keyed, key, ctx->d_r.as<Fr>());
   LAUNCH_CHECK();
   trace(ctx, "upload enqueued");
@@ -2160,6 +2289,9 @@ static int enqueue_stages(h2v_ctx* ctx) {
             ctx->has_col_len ? ctx->d_col_len.as<u32>() : nullptr, ctx->d_vals.as<Fr>(), ctx->d_scratch.as<Fr>(), ctx->d_right.as<Fr>(),
             ctx->d_shared.as<Fr>(), ctx->d_left.as<Fr>(), ctx->d_status.as<u32>());
   }
+  if (hd.n_carry)
+    KLAUNCH(k_agg, cdiv(n, 128), 128, 0, s, pv, n, ctx->d_inst.as<u8>(), ctx->d_inst_off.as<u64>(), ctx->has_col_len ? ctx->d_col_len.as<u32>() : nullptr,
+            ctx->d_rho.as<Fr>(), ctx->d_pts.as<G1Affine>(), ctx->d_right.as<Fr>(), ctx->d_shared.as<Fr>(), ctx->d_left.as<Fr>(), ctx->d_status.as<u32>());
   nvtxRangePop();
   set_launch_class('N');
   if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[3], s));
@@ -2252,6 +2384,7 @@ static u64 graph_key(const h2v_ctx* ctx, int mode) {
   mix((u64)(size_t)ctx->d_lines());
   mix((u64)(size_t)ctx->d_gsums.p | (u64)line_run(ctx->geom.G ? ctx->geom.G : 1) << 56);
   mix((u64)(size_t)ctx->comm.window);
+  if (ctx->hd.n_carry) mix((u64)(size_t)ctx->d_rho.p);
   if (mode & RUN_ABSORB) {
     mix((u64)(size_t)ctx->absorb.acc);
     mix((u64)(size_t)ctx->absorb.records);
@@ -2330,7 +2463,7 @@ static int per_proof_accum(h2v_ctx* ctx, u8* accum_host) {
   const u32 n = ctx->n;
   cudaStream_t s = ctx->stream;
   PlanView pv = ctx->pv();
-  const u32 nbases = hd.n_points + hd.n_shared + hd.n_mo;
+  const u32 nbases = msm_points(hd) + hd.n_shared + msm_mo(hd);
   CKC(ctx->d_pp_prod.ensure(sizeof(G1Jac) * (size_t)n * nbases));
   CKC(ctx->d_pp_lr.ensure(sizeof(G1Jac) * (size_t)2 * n));
   CKC(ctx->d_pp_bytes.ensure(128 * (size_t)n));
@@ -2356,7 +2489,7 @@ static int attribute_impl(h2v_ctx* ctx) {
   cudaStream_t s = ctx->stream;
   PlanView pv = ctx->pv();
   const u32* gv = (ctx->verdicts_on_device && g.G > 1 && g.G * g.n == N) ? ctx->d_verdict.as<u32>() : nullptr;
-  const u32 nbases = hd.n_points + hd.n_shared + hd.n_mo;
+  const u32 nbases = msm_points(hd) + hd.n_shared + msm_mo(hd);
   static constexpr u32 CHUNK = 1024;  // checks per pass: bounds the Miller scratch (E12[CHUNK][65] = 115 MB)
   MsmGeom unit{};
   unit.c[0] = unit.c[1] = 1;
@@ -2381,7 +2514,7 @@ static int attribute_impl(h2v_ctx* ctx) {
   if (const char* e = getenv("H2V_ATTR_SUB")) msub = (u32)atoi(e);  // (tuning: 0 = no sub-batch level)
   // (level 1 needs twice the term ids of the batch pass - two GLV halves per term - inside the 31-bit id space)
   if (msub >= 2 && g.n >= 4 * msub && g.n % msub == 0 &&
-      2 * ((u64)N * (hd.n_points + hd.n_mo) + (u64)hd.n_shared * (N / msub)) < (1ull << 31)) {
+      2 * ((u64)N * (msm_points(hd) + msm_mo(hd)) + (u64)hd.n_shared * (N / msub)) < (1ull << 31)) {
     const u32 subs = g.n / msub, SG = N / msub;
     // window bits of the re-fold: dependent chain = bucket chain (2 * 14 * msub / 2^(c-1) entries) + in-window reduction
     // (2^c additions) + window combination (130 doublings + 130 / c additions); measured (B200, sub-batches of 16): MSM + combination
@@ -2460,7 +2593,7 @@ static int hooks_impl(h2v_ctx* ctx, u8* challenges) {
     CKC(cudaMemcpyAsync(challenges, ctx->d_chal.p, 32 * (size_t)n * hd.n_challenges, cudaMemcpyDeviceToHost, s));
   }
   if (ctx->opt_scalar_hook) {
-    const u32 nbases = hd.n_points + hd.n_shared + hd.n_mo;
+    const u32 nbases = msm_points(hd) + hd.n_shared + msm_mo(hd);
     CKC(ctx->d_hook.ensure(32 * (size_t)n * nbases));
     k_gather_scalars<<<cdiv((u64)n * nbases, 128), 128, 0, s>>>(ctx->pv(), n, ctx->d_right.as<Fr>(), ctx->d_shared.as<Fr>(),
                                                                  ctx->d_left.as<Fr>(), ctx->d_hook.as<u8>());
@@ -3142,7 +3275,7 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
       mx->err = "member " + std::to_string(i) + " has a pending fold-group or shard-hint option: mixed batches do not combine with them";
       return -1;
     }
-    if (counts[i]) terms += (u64)counts[i] * (c->hd.n_points + c->hd.n_mo) + c->hd.n_shared;
+    if (counts[i]) terms += (u64)counts[i] * (msm_points(c->hd) + msm_mo(c->hd)) + c->hd.n_shared;
   }
   // term ids carry the sign in bit 31 (k_msm_scatter): the limit of upload_impl, over the whole mix
   if (terms >= (1ull << 31)) {
@@ -3170,8 +3303,8 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
   for (u32 i = 0; i < K; i++) {
     h2v_ctx* c = mx->m[i];
     nm[i] = counts[i];
-    Pm[i] = c->hd.n_points;
-    Mm[i] = c->hd.n_mo;
+    Pm[i] = msm_points(c->hd);
+    Mm[i] = msm_mo(c->hd);
     Sm[i] = c->hd.n_shared;
     if (!counts[i]) continue;
     std::vector<u64> po(counts[i] + 1), io(counts[i] + 1);

@@ -97,7 +97,16 @@ struct PlanHeader {
   u32 off_tops, off_exprops, off_polys, off_terms, off_vars, off_polylist, off_permcols, off_lookups;
   u32 off_consts, off_pt_item, off_sc_item, off_rot, off_sets, off_setpts, off_setcms, off_setevals, off_diffs;
   u32 off_gwcpts, off_gwcq, off_instq, off_shared_pts, off_lines0, off_lines1;
+  // aggregation contexts (agg.cuh): the carried accumulator's two points (lhs, rhs) follow the proof points in the per-proof
+  // MSM layout; n_carry = 2 there, 0 for every other context.  off_agg: 4 * agg_limbs AggCell.
+  u32 n_carry, agg_limbs, agg_bits, off_agg;
 };
+
+// Per-proof point slots of the MSM: the proof points, then the carried lhs and rhs.  The last msm_mo() slots are the left
+// channel's points: the multi-open points, then lhs (left scalar 0) and rhs (left scalar rho); the right channel covers every
+// slot (lhs: rho, rhs: 0).  n_points / n_mo themselves count what is read from the proof.
+H2V_HD u32 msm_points(const PlanHeader& h) { return h.n_points + h.n_carry; }
+H2V_HD u32 msm_mo(const PlanHeader& h) { return h.n_mo + h.n_carry; }
 
 struct PlanView {
   const u8* base;

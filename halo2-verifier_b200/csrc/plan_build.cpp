@@ -16,6 +16,7 @@
 #include <algorithm>
 #include <map>
 
+#include "agg.cuh"
 #include "tower.cuh"
 
 namespace h2v {
@@ -213,7 +214,7 @@ u32 append(std::vector<u8>& blob, const std::vector<T>& v) {
 // advice / lookup / permutation / shuffle commitments and evaluations, the instance columns, the expressions and the
 // queries repeat per instance in the reference's interleaving; fixed columns, sigma, the random polynomial and h are shared.
 int build_plan(const u8* params, size_t params_len, int params_fmt, const u8* vkb, size_t vk_len, int vk_fmt,
-               int multiopen, int hash, std::vector<u8>& blob, PlanInfo& info, std::string& err, u32 m) {
+               int multiopen, int hash, std::vector<u8>& blob, PlanInfo& info, std::string& err, u32 m, const AggSpec* agg) {
   // write emits len() of the instance / fixed query lists but read takes exactly one query per column
   // (plonk/vk.rs:243-251 vs 310-322): with more queries than columns everything after them is read misaligned
   static const char* const query_hint =
@@ -750,6 +751,24 @@ int build_plan(const u8* params, size_t params_len, int params_fmt, const u8* vk
     ng2.y = ng2.y.neg();
     g2_prepare(ng2, lines1.data());  // e(right, -G2)
 
+    // ---------------- carried accumulator of an aggregation circuit (agg.cuh)
+    std::vector<AggCell> agg_cells;
+    if (agg) {
+      H2V_REQUIRE(agg->limbs >= AGG_MIN_LIMBS && agg->limbs <= AGG_MAX_LIMBS, "aggregation spec: limbs must be in [2, 8]");
+      H2V_REQUIRE(agg->bits >= 1 && agg->bits <= AGG_MAX_BITS, "aggregation spec: bits must be in [1, 128]");
+      H2V_REQUIRE(agg->limbs * agg->bits >= 254, "aggregation spec: limbs * bits must be >= 254 (a coordinate of q)");
+      H2V_REQUIRE(agg->cells != nullptr, "aggregation spec: cells is null");
+      for (u32 i = 0; i < 4 * agg->limbs; i++) {
+        const AggCell c{agg->cells[2 * i], agg->cells[2 * i + 1]};
+        H2V_REQUIRE(c.column < hd.n_inst_cols, "aggregation spec: cell " + std::to_string(i) + " names column " + std::to_string(c.column) +
+                                                   " of a proof with " + std::to_string(hd.n_inst_cols) + " instance columns");
+        agg_cells.push_back(c);
+      }
+      hd.n_carry = 2;
+      hd.agg_limbs = agg->limbs;
+      hd.agg_bits = agg->bits;
+    }
+
     // ---------------- assemble the blob
     hd.n_tops = (u32)tops.size();
     hd.n_exprops = (u32)eops.size();
@@ -778,6 +797,7 @@ int build_plan(const u8* params, size_t params_len, int params_fmt, const u8* vk
     hd.off_shared_pts = append(blob, shared_pts);
     hd.off_lines0 = append(blob, lines0);
     hd.off_lines1 = append(blob, lines1);
+    hd.off_agg = append(blob, agg_cells);
     while (blob.size() % 16) blob.push_back(0);
     hd.total_bytes = (u32)blob.size();
     memcpy(blob.data(), &hd, sizeof(hd));

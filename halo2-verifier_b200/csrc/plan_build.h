@@ -24,10 +24,17 @@ struct PlanInfo {
   std::vector<std::string> lint;
 };
 
+// The KZG accumulator an aggregation circuit carries in its instances (agg.cuh): LimbsEncoding<limbs, bits> and the
+// 4 * limbs (column, row) cells of lhs.x, lhs.y, rhs.x, rhs.y
+struct AggSpec {
+  u32 limbs, bits;
+  const u32* cells;
+};
+
 // circuit_instances: how many circuit instances one proof transcript carries (`instances.len()` of verify_proof; 1 in
-// every reference test)
+// every reference test).  agg != null: an aggregation context; the spec is validated here (before any device call).
 int build_plan(const u8* params, size_t params_len, int params_fmt, const u8* vk, size_t vk_len, int vk_fmt, int multiopen,
-               int hash, std::vector<u8>& blob, PlanInfo& info, std::string& err, u32 circuit_instances = 1);
+               int hash, std::vector<u8>& blob, PlanInfo& info, std::string& err, u32 circuit_instances = 1, const AggSpec* agg = nullptr);
 
 // Miller-line tables of the G2 multiples [2^(c w)] Q used by the window-decomposed pairing check
 // (pairing_cta.cuh): pairs 0..W0-1 = right channel (Q = -G2, c = c0), then W1 pairs of the left

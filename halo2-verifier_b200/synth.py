@@ -217,8 +217,9 @@ def _layout(bv):
     return ["P"] * (bv.n_points - bv.n_mo) + ["S"] * bv.n_scalars + ["P"] * bv.n_mo
 
 
-def synthesize_shplonk_batch(bv, shared_dlogs, s, n, seed, rows=10):
-    """n accepting SHPLONK proofs + public inputs for the context `bv` (a BatchVerifier).
+def synthesize_shplonk_batch(bv, shared_dlogs, s, n, seed, rows=10, instances_of=None):
+    """n accepting SHPLONK proofs + public inputs for the context `bv` (a BatchVerifier, plain: it parses the placeholders).
+    instances_of(j, rng) (optional) gives proof j's instances[column][row] as 32-byte strings instead of random ones.
     Returns (list of proof bytes, list of instances[column][row] as 32-byte strings)."""
     assert bv.n_mo == 2, "SHPLONK contexts only"
     rng = random.Random(repr(("bench-batch", seed, n)))
@@ -244,7 +245,8 @@ def synthesize_shplonk_batch(bv, shared_dlogs, s, n, seed, rows=10):
         body += b"".join(rng.randrange(R).to_bytes(32, "little") for _ in range(bv.n_scalars))
         proofs.append(bytes(body) + h1 + g_c)
         dlogs.append(dl)
-        instances.append([[rng.randrange(R).to_bytes(32, "little") for _ in range(rows)] for _ in range(bv.n_inst_cols)])
+        instances.append(instances_of(len(instances), rng) if instances_of else
+                         [[rng.randrange(R).to_bytes(32, "little") for _ in range(rows)] for _ in range(bv.n_inst_cols)])
     res = bv.verify_batch(proofs, instances, want_scalars=True)
     nb, P_, Sh = bv.n_bases, bv.n_points, bv.n_shared
     out = []

@@ -60,6 +60,37 @@ int h2v_ctx_create_multi(h2v_ctx** out, const uint8_t* params, size_t params_len
 /* Same from the `VALID_VK.bin` bundle the reference's tooling writes (serialize/examples/vector_mul.rs:374-393):
  * ParamsKZG::write (Processed form, 164 bytes) immediately followed by VerifyingKey::write(SerdeFormat::RawBytes). */
 int h2v_ctx_create_from_bundle(h2v_ctx** out, const uint8_t* bundle, size_t bundle_len, int multiopen, int hash, int device);
+/* ---- aggregation proofs: the KZG accumulator carried in the public instances ----------------------------------------
+ * An aggregation circuit (snark-verifier with halo2-lib or halo2wrong) verifies inner proofs in-circuit and defers their
+ * pairing: it exposes a KZG accumulator (lhs, rhs) as limbs of its public instances, and the proof is only sound if the
+ * verifier also checks e(lhs, g2) e(rhs, -[s]g2) = 1, i.e. lhs = s rhs.  An aggregation context checks it inside the batch
+ * fold.  The spec is a property of the circuit (snark-verifier's accumulator_indices + LimbsEncoding<limbs, bits>):
+ *   limbs, bits   2 <= limbs <= 8, 1 <= bits <= 128, limbs * bits >= 254; (3, 88) is halo2-lib, (4, 68) halo2wrong
+ *   cells         4 * limbs (column, row) pairs, 8 * limbs uint32: lhs.x, lhs.y, rhs.x, rhs.y, least significant limb
+ *                 first; `column` indexes the proof's flattened instance columns (instance-major when circuit_instances > 1,
+ *                 as h2v_ctx_create_multi lays them out)
+ * Exactly one carried accumulator per proof.  A malformed spec (limits above, a column beyond the flattened columns, NULL
+ * cells) is refused before any device call, text in h2v_last_error(NULL).
+ * Per proof, on the device: every limb must be < 2^bits, each coordinate sum_i limb_i 2^(bits i) < q, each point on
+ * y^2 = x^3 + 3 or (0, 0) (the identity, halo2curves from_xy); a cell whose row lies beyond its column's length (ragged
+ * layouts, h2v_batch_set_columns) fails too.  A failure is H2V_INVALID_INSTANCES for that proof only, whatever the later
+ * stages found (the precedence of lib.rs:51-55), and the proof adds nothing to the fold.
+ * Fold: proof j adds rho rhs to its L_j and rho lhs to its R_j (DualMSM orientation e(L, [s]G2) e(R, -G2) = 1), then (L_j, R_j)
+ * is folded with c_j as for any proof: two more MSM terms per proof, no extra pairing.  One rho per upload, independent of
+ * the r_i: from the upload's key (caller's or OS), Blake2b-512("h2v-rla" | key) mod r, or from the test seed likewise; with
+ * caller rlc_scalars from h2v_batch_set_agg_scalar (one-shot, 32 B canonical, non-zero), or drawn from the OS when that was
+ * not called (verdicts are unaffected; bit-exact accumulators need the setter).
+ * Every entry point covers the carried terms: h2v_verify_proof and every per-proof check (attribution after a rejected
+ * fold, the `accum` hook) include them, so a valid outer proof whose carried accumulator is false is
+ * H2V_CONSTRAINT_SYSTEM_FAILURE; fold groups, shards + h2v_finalize, the device-side exchange, mixed batches with
+ * aggregation members and h2v_acc_absorb fold them like any other term.
+ * h2v_ctx_info reports the proof's own counts (points and multi-open points read from the proof).  The scalar hook
+ * (h2v_batch_set_scalar_hook) has points + 2 right-channel and multi-open + 2 left-channel entries per proof: the carried
+ * lhs, rhs follow the proof points in both channels (right: rho, 0; left: 0, rho; 0 for an identity point). */
+int h2v_ctx_create_aggregation(h2v_ctx** out, const uint8_t* params, size_t params_len, int params_format, const uint8_t* vk, size_t vk_len,
+                               int vk_format, int multiopen, int hash, int device, uint32_t circuit_instances, uint32_t limbs, uint32_t bits,
+                               const uint32_t* cells);
+int h2v_batch_set_agg_scalar(h2v_ctx* ctx, const uint8_t* rho32);
 void h2v_ctx_destroy(h2v_ctx* ctx);
 /* error text of the last failing call on this context (ctx == NULL: of the last failed h2v_ctx_create) */
 const char* h2v_last_error(const h2v_ctx* ctx);
