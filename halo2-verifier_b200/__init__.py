@@ -157,6 +157,7 @@ def load_library():
     lib.h2v_debug_timeline_stop.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_uint32, u32p]
     lib.h2v_last_msm_geometry.argtypes = [ctypes.c_void_p, u32p]
     lib.h2v_selftest_field.argtypes = [ctypes.c_int, ctypes.c_uint32, ctypes.c_uint64]
+    lib.h2v_selftest_field_vectors.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_uint32, ctypes.c_char_p, ctypes.c_char_p, u8p]
     lib.h2v_calibrate_imad.argtypes = [ctypes.c_int]
     lib.h2v_calibrate_imad.restype = ctypes.c_double
     lib.h2v_mix_create.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_void_p, ctypes.c_uint32]
@@ -186,7 +187,7 @@ EXPORTED_SYMBOLS = (
     "h2v_ctx_create", "h2v_ctx_create_from_bundle", "h2v_ctx_destroy", "h2v_last_error", "h2v_ctx_info", "h2v_verify_proof", "h2v_verify_batch",
     "h2v_batch_set_columns", "h2v_batch_set_scalar_hook", "h2v_batch_set_shard_hint", "h2v_partial_bytes", "h2v_accumulate_shard", "h2v_finalize", "h2v_attribute_shard",
     "h2v_batch_upload", "h2v_batch_upload_shard", "h2v_batch_run", "h2v_batch_run_shard", "h2v_batch_run_shard_async", "h2v_flush_l2", "h2v_batch_download", "h2v_last_timings", "h2v_launch_count", "h2v_ctx_stream", "h2v_ctx_set_blocking_sync", "h2v_ctx_set_graphs", "h2v_ctx_create_multi", "h2v_batch_set_fold_groups", "h2v_last_group_verdicts", "h2v_finalize_groups", "h2v_debug_timeline_start", "h2v_debug_timeline_stop",
-    "h2v_last_msm_geometry", "h2v_selftest_field", "h2v_calibrate_imad",
+    "h2v_last_msm_geometry", "h2v_selftest_field", "h2v_selftest_field_vectors", "h2v_calibrate_imad",
     "h2v_attribute_shard_groups", "h2v_batch_set_rlc_key", "h2v_last_rlc_source", "h2v_comm_init", "h2v_comm_connect", "h2v_comm_set_timeout_ms",
     "h2v_batch_run_shard_exchange", "h2v_verify_shard", "h2v_comm_last_batch_accum", "h2v_ctx_cache_stats", "h2v_ctx_work_model", "h2v_ctx_vk_lint",
     "h2v_mix_create", "h2v_mix_destroy", "h2v_mix_last_error", "h2v_mix_set_rlc_key", "h2v_mix_verify",

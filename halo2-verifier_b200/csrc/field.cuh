@@ -424,8 +424,10 @@ struct alignas(16) Fp {  // 16-byte alignment: element loads / stores vectorise 
 #endif
   }
 
-  // Montgomery product for an UNREDUCED left operand: b < p, a < 2^256 (so a*b < 2^256 * p).  Used
-  // where raw 256-bit strings enter the field (from_uniform, from_canonical).
+  // Montgomery product for an UNREDUCED left operand: a < 2^256, b < p with no limb of b equal to 0xFFFFFFFF.  Used
+  // where raw 256-bit strings enter the field (from_uniform, from_canonical), always with b = R^2 or R^3 mod p, whose
+  // limbs are all below 0xFFFFFFFF (tests/test_field_vectors.py checks this).  With a close to 2^256 and a limb b_i =
+  // 0xFFFFFFFF, t + a * b_i can reach 2^288, whose carry out of t[8] is lost: the result is then wrong.
   static H2V_HD Fp mul_any(const Fp& a, const Fp& b) {
 #ifdef H2V_PTX
     Fp r;

@@ -1064,6 +1064,37 @@ __global__ void k_selftest_field(u32 count, u64 seed, u32* mismatches) {
   u32 bad = selftest_one<Fq>(s, t % 7 == 0) + selftest_one<Fr>(s, t % 5 == 0);
   if (bad) atomicAdd(mismatches, bad);
 }
+// Known-answer vectors of the field operations (h2v_selftest_field_vectors): raw limbs in and out, no conversion, so that a
+// test can place the operands anywhere in each operation's documented range.  op numbering: include/h2v.h.
+template <class F>
+__global__ void k_selftest_field_vectors(int op, u32 n, const u8* a, const u8* b, u8* out) {
+  const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const F x = F::load_le(a + 32 * (size_t)t), y = F::load_le(b + 32 * (size_t)t);
+  F r = F::zero();
+  switch (op) {
+    case 0: r = F::mul(x, y); break;
+    case 1: r = F::mul_c(x, y); break;
+    case 2: r = x.sqr(); break;
+    case 3: r = F::sqr_c(x); break;
+    case 4: r = F::mul_any(x, y); break;
+    case 5: r = x + y; break;
+    case 6: r = x - y; break;
+    case 7: r = x.neg(); break;
+    case 8: r = F::from_canonical(x); break;
+    case 9: r = x.to_canonical(); break;
+    case 10: r = x.inv(); break;
+    case 11: r = x.inv_bin(); break;
+    case 12: {
+      u8 w[64];
+      x.store_le(w);
+      y.store_le(w + 32);
+      r = F::from_uniform(w);
+      break;
+    }
+  }
+  r.store_le(out + 32 * (size_t)t);
+}
 __global__ void k_imad(u32 iters, u32* out) {
   u32 a0 = threadIdx.x, a1 = a0 + 1, a2 = a0 + 2, a3 = a0 + 3, a4 = a0 + 4, a5 = a0 + 5, a6 = a0 + 6, a7 = a0 + 7;
   const u32 m = blockIdx.x * 2654435761u + 12345u, k = threadIdx.x | 1u;
@@ -1796,6 +1827,18 @@ int h2v_ctx_create_aggregation(h2v_ctx** out, const uint8_t* params, size_t para
   return ctx_create(out, params, params_len, params_format, vk, vk_len, vk_format, multiopen, hash, device, circuit_instances, &spec);
 }
 
+// Caller fold scalars (rlc_scalars, the r of h2v_acc_merge) must be canonical and non-zero: a zero r_i, or one that reduces
+// to zero, makes c_j = prod_{i>j} r_i vanish for every earlier proof j, which then drops out of the batch check and out of
+// the re-fold of its attribution sub-batch (an invalid proof would be accepted, or reported H2V_OK inside a rejected batch).
+static const char* const FOLD_SCALARS_ERR = "fold scalars must be canonical and non-zero";
+static bool fold_scalars_ok(const u8* r32, u64 count) {
+  for (u64 i = 0; i < count; i++) {
+    const Fr k = Fr::load_le(r32 + 32 * i);
+    if (k.geq_mod() || k.is_zero()) return false;
+  }
+  return true;
+}
+
 int h2v_batch_set_agg_scalar(h2v_ctx* ctx, const uint8_t* rho32) {
   if (!ctx || !rho32) return -1;
   const Fr k = Fr::load_le(rho32);
@@ -2084,6 +2127,10 @@ static int upload_impl(h2v_ctx* ctx, u32 n, const u8* proofs, const u64* proof_o
   ctx->opt_fold_groups = 0;
   if (n == 0 || !proof_off || !inst_off || (!proofs && proof_off[n]) || groups > 1024 || n % groups != 0 || gcount < gbase + n / groups) {
     ctx->err = "bad batch arguments (with fold groups the batch must split into equal groups)";
+    return -1;
+  }
+  if (rlc && !fold_scalars_ok(rlc, gcount * groups)) {  // every group's whole global batch
+    ctx->err = FOLD_SCALARS_ERR;
     return -1;
   }
   CKC(cudaSetDevice(ctx->device));
@@ -3031,6 +3078,25 @@ int h2v_selftest_field(int device, uint32_t count, uint64_t seed) {
   return (int)h;
 }
 
+int h2v_selftest_field_vectors(int device, int field, int op, uint32_t n, const uint8_t* a, const uint8_t* b, uint8_t* out) {
+  if ((field != 0 && field != 1) || op < 0 || op > 12 || !a || !b || !out) return -1;
+  if (n == 0) return 0;
+  if (cudaSetDevice(device) != cudaSuccess) return -2;
+  const size_t bytes = 32 * (size_t)n;
+  u8* d = nullptr;
+  if (cudaMalloc(&d, 3 * bytes) != cudaSuccess) return -2;
+  cudaError_t e = cudaMemcpy(d, a, bytes, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) e = cudaMemcpy(d + bytes, b, bytes, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) {
+    if (field == 0) k_selftest_field_vectors<Fq><<<cdiv(n, 128), 128>>>(op, n, d, d + bytes, d + 2 * bytes);
+    else k_selftest_field_vectors<Fr><<<cdiv(n, 128), 128>>>(op, n, d, d + bytes, d + 2 * bytes);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaMemcpy(out, d + 2 * bytes, bytes, cudaMemcpyDeviceToHost);
+  cudaFree(d);
+  return e == cudaSuccess ? 0 : -2;
+}
+
 double h2v_calibrate_imad(int device) {
   if (cudaSetDevice(device) != cudaSuccess) return -1.0;
   cudaDeviceProp prop;
@@ -3254,6 +3320,10 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
   for (u32 i = 0; i < K; i++) N += counts[i];
   if (N == 0 || N > 0xFFFFFFFFull) {
     mx->err = "a mixed batch needs between 1 and 2^32 - 1 proofs";
+    return -1;
+  }
+  if (rlc && !fold_scalars_ok(rlc, N)) {  // before any member is uploaded
+    mx->err = FOLD_SCALARS_ERR;
     return -1;
   }
   // caller data: validated as upload_impl validates a context's batch
@@ -3675,12 +3745,11 @@ int h2v_acc_merge(h2v_acc* a, const uint8_t* in128, const uint8_t* r32) {
   }
   Fr sc[2] = {Fr::zero(), Fr::one()};
   if (r32) {
-    const Fr k = Fr::load_le(r32);
-    if (k.geq_mod()) {
-      a->err = "merge scalar r is not canonical (below the group order)";
+    if (!fold_scalars_ok(r32, 1)) {  // r = 0 would drop every earlier absorb out of the final check
+      a->err = FOLD_SCALARS_ERR;
       return -1;
     }
-    sc[0] = Fr::from_canonical(k);
+    sc[0] = Fr::from_canonical(Fr::load_le(r32));
   } else {
     u8 wide[64];
     if (os_entropy(wide, sizeof(wide)) != 0) {

@@ -117,8 +117,11 @@ int h2v_verify_proof(h2v_ctx* ctx, const uint8_t* proof, size_t proof_len, const
  *   proofs / proof_off    concatenated proof bytes, n+1 byte offsets
  *   instances / inst_off  concatenated 32-byte LE canonical Fr, n+1 offsets in units of scalars;
  *                         per proof: columns concatenated, equal length (see h2v_batch_set_columns)
- *   rlc_scalars           n x 32 B canonical r_i, or NULL to expand them from `seed`; proof j is folded
- *                         with c_j = prod_{i>j} r_i, the reference's convention (SURVEY.md 3.2)
+ *   rlc_scalars           n x 32 B canonical non-zero r_i, or NULL to expand them from `seed`; proof j is folded
+ *                         with c_j = prod_{i>j} r_i, the reference's convention (SURVEY.md 3.2).  A zero or
+ *                         non-canonical r_i (it would zero c_j of every earlier proof) is refused before any
+ *                         device call: -1, "fold scalars must be canonical and non-zero".  The same holds for
+ *                         every entry point that takes rlc_scalars.
  *   status                n bytes out
  *   challenges            optional out, n x C x 32 B canonical, squeeze order            (parity hook)
  *   accum                 optional out, n x 2 x 64 B per-proof affine (L_j, R_j), x|y LE canonical,
@@ -293,7 +296,8 @@ int h2v_mix_verify(h2v_mix* mx, const uint32_t* counts, const uint8_t* proofs, c
  *   h2v_acc_get       the affine L | R, 2 x 64 B in the batch_accum layout (all-zero = identity)
  *   h2v_acc_merge     acc <- r acc + P with P = L | R in the same layout: the DualMSM scale followed by adding another
  *                     accumulator (of another GPU or process; into an empty accumulator: restore from a checkpoint).  r32: 32 B
- *                     canonical, or NULL to draw r from the OS.  Non-canonical or off-curve bytes are refused, state unchanged.
+ *                     canonical and non-zero (r = 0 would drop every earlier absorb out of the check), or NULL to draw r from
+ *                     the OS.  A zero or non-canonical r, non-canonical or off-curve bytes are refused, state unchanged.
  *                     A merge is one record.
  *   h2v_acc_reset     empty accumulator and record array
  * Not combinable with mixed batches, fold groups, shards or the device-side exchange. */
@@ -364,6 +368,12 @@ int h2v_last_msm_geometry(const h2v_ctx* ctx, uint32_t* out4);
  * Runs the PTX field multiplication against the portable one on `count` pseudo-random and edge
  * operands for both fields; returns the number of mismatches (0 = pass), <0 on CUDA error. */
 int h2v_selftest_field(int device, uint32_t count, uint64_t seed);
+/* Known-answer vectors: one field operation on n operand pairs, raw 32-byte little-endian limbs in and out (no conversion:
+ * the caller places operands anywhere in the operation's documented range and compares with exact integers).
+ * field: 0 = Fq, 1 = Fr.  op: 0 mul (a < 2^255, b < p), 1 mul_c, 2 sqr, 3 sqr_c, 4 mul_any (a < 2^256), 5 a + b, 6 a - b,
+ * 7 neg, 8 from_canonical, 9 to_canonical, 10 inv (Fermat), 11 inv_bin, 12 from_uniform of the 64 bytes a | b.
+ * Returns 0, -1 on a bad argument, -2 on a CUDA error. */
+int h2v_selftest_field_vectors(int device, int field, int op, uint32_t n, const uint8_t* a, const uint8_t* b, uint8_t* out);
 /* integer multiply-add peak calibration: returns achieved 32-bit IMAD operations per second */
 double h2v_calibrate_imad(int device);
 
