@@ -17,6 +17,7 @@ Host-side mirror of the reference's verification surface (ChainSafe/halo2-verifi
     (added) verify_proofs_batch                        verify_proofs_batch(..) / BatchVerifier
     AccumulatorStrategy over proofs of several VKs     verify_proofs_mixed(..) / MixedBatchVerifier
       poly/kzg/strategy.rs:125-140
+    (added) one pairing check over several params     verify_proofs_mixed(.., multi_params=True) / MixedBatchVerifier
     AccumulatorStrategy across calls: process, finalize  Accumulator.{absorb, finalize, to_bytes, merge}
       poly/kzg/strategy.rs:125-140
     (snark-verifier) KZG accumulator in the instances    accumulator=InstanceAccumulator(limbs, bits, cells)
@@ -161,6 +162,8 @@ def load_library():
     lib.h2v_calibrate_imad.argtypes = [ctypes.c_int]
     lib.h2v_calibrate_imad.restype = ctypes.c_double
     lib.h2v_mix_create.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_void_p, ctypes.c_uint32]
+    lib.h2v_mix_create_multi_params.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_void_p, ctypes.c_uint32]
+    lib.h2v_mix_params_classes.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_uint32), ctypes.c_uint32]
     lib.h2v_mix_destroy.argtypes = [ctypes.c_void_p]
     lib.h2v_mix_destroy.restype = None
     lib.h2v_mix_last_error.argtypes = [ctypes.c_void_p]
@@ -191,6 +194,7 @@ EXPORTED_SYMBOLS = (
     "h2v_attribute_shard_groups", "h2v_batch_set_rlc_key", "h2v_last_rlc_source", "h2v_comm_init", "h2v_comm_connect", "h2v_comm_set_timeout_ms",
     "h2v_batch_run_shard_exchange", "h2v_verify_shard", "h2v_comm_last_batch_accum", "h2v_ctx_cache_stats", "h2v_ctx_work_model", "h2v_ctx_vk_lint",
     "h2v_mix_create", "h2v_mix_destroy", "h2v_mix_last_error", "h2v_mix_set_rlc_key", "h2v_mix_verify",
+    "h2v_mix_create_multi_params", "h2v_mix_params_classes",
     "h2v_acc_create", "h2v_acc_destroy", "h2v_acc_last_error", "h2v_acc_set_rlc_key", "h2v_acc_absorb", "h2v_acc_finalize", "h2v_acc_get",
     "h2v_acc_merge", "h2v_acc_reset", "h2v_ctx_create_aggregation", "h2v_batch_set_agg_scalar",
 )
@@ -581,7 +585,9 @@ class BatchVerifier:
 class MixedBatchResult:
     status: List[List[int]]  # one list per member, in member order
     verdict: bool  # every proof of every member accepted
-    batch_accum: Optional[bytes] = None  # folded (L, R) of the whole mix, 2 x 64 B
+    # folded (L, R) of the whole mix, 2 x 64 B; a multi_params mix: one (L_p, R_p) per params class in class order,
+    # classes x 128 B, all-zero for a class without proofs in the call
+    batch_accum: Optional[bytes] = None
 
     def errors(self):
         return [[None if s == 0 else STATUS_ERRORS[s]() for s in st] for st in self.status]
@@ -591,16 +597,23 @@ class MixedBatchVerifier:
     """Proofs of several BatchVerifiers (verifying keys, SHPLONK or GWC, Blake2b or Keccak) folded into ONE MSM and ONE
     pairing check: the reference's AccumulatorStrategy fed proofs of different VKs under one set of KZG params
     (include/h2v.h "mixed batches").  The members' params must agree on (g, g2, s_g2); k may differ.  The members are not
-    owned: they must stay open while the mix is used and must not run their own batches during a mixed one."""
+    owned: they must stay open while the mix is used and must not run their own batches during a mixed one.
+    multi_params=True: members may hold up to 8 different params (a different trapdoor or g2); each params class gets its
+    own bucket set and lines, and all classes still share one pairing check (`params_classes`, include/h2v.h
+    "multi-params mixes")."""
 
-    def __init__(self, members: Sequence[BatchVerifier]):
+    def __init__(self, members: Sequence[BatchVerifier], multi_params=False):
         self.lib = load_library()
         self.members = list(members)
         self._mx = ctypes.c_void_p()
         ptrs = (ctypes.c_void_p * max(1, len(self.members)))(*[m._ctx for m in self.members])
-        if self.lib.h2v_mix_create(ctypes.byref(self._mx), ptrs if self.members else None, len(self.members)) != 0:
+        create = self.lib.h2v_mix_create_multi_params if multi_params else self.lib.h2v_mix_create
+        if create(ctypes.byref(self._mx), ptrs if self.members else None, len(self.members)) != 0:
             self._mx = None
             raise BackendError(self.lib.h2v_mix_last_error(None).decode())
+        cls = (ctypes.c_uint32 * len(self.members))()
+        self.n_classes = self.lib.h2v_mix_params_classes(self._mx, cls, len(self.members))
+        self.params_classes = list(cls)  # params class of each member, numbered by first appearance
 
     def close(self):
         if getattr(self, "_mx", None):
@@ -650,7 +663,7 @@ class MixedBatchVerifier:
             if proofs and bv.accumulator is not None:
                 bv._set_agg_scalar(agg_scalar)
         status = (ctypes.c_uint8 * n)()
-        bacc = ctypes.create_string_buffer(128) if want_batch_accum else None
+        bacc = ctypes.create_string_buffer(128 * self.n_classes) if want_batch_accum else None
         verdict = ctypes.c_int(0)
         self._check(self.lib.h2v_mix_verify(self._mx, counts, b"".join(pparts), (ctypes.c_uint64 * (n + 1))(*poffs), b"".join(iparts),
                                              (ctypes.c_uint64 * (n + 1))(*ioffs), rlc, int(seed), status, bacc, ctypes.byref(verdict)))
@@ -797,16 +810,17 @@ def verify_proofs_batch(params: ParamsKZG, vk: VerifyingKey, proofs: Sequence[by
         return bv.verify_batch(proofs, instances, rlc_scalars, seed, agg_scalar=agg_scalar).errors()
 
 
-def verify_proofs_mixed(circuits, device=0) -> List[List[Optional[Error]]]:
+def verify_proofs_mixed(circuits, device=0, multi_params=False) -> List[List[Optional[Error]]]:
     """Mixed batch entry point: circuits = [(params, vk, proofs, instances, multiopen, transcript), ...] whose params agree
-    on (g, g2, s_g2) (k may differ).  All proofs are folded into one MSM and one pairing check (the reference's
-    AccumulatorStrategy over proofs of several VKs), with per-proof attribution when the fold is rejected.  Returns one
-    error list per circuit, as verify_proofs_batch does; the fold coefficients come from OS entropy."""
+    on (g, g2, s_g2) (k may differ), or, with multi_params=True, under up to 8 different params.  All proofs are folded into
+    one MSM and one pairing check (the reference's AccumulatorStrategy over proofs of several VKs), with per-proof
+    attribution when the fold is rejected.  Returns one error list per circuit, as verify_proofs_batch does; the fold
+    coefficients come from OS entropy."""
     bvs = []
     try:
         for params, vk, _proofs, _insts, multiopen, transcript in circuits:
             bvs.append(BatchVerifier(params, vk, multiopen, transcript, device))
-        with MixedBatchVerifier(bvs) as mx:
+        with MixedBatchVerifier(bvs, multi_params) as mx:
             return mx.verify_batch([c[2] for c in circuits], [c[3] for c in circuits]).errors()
     finally:
         for bv in bvs:

@@ -334,13 +334,13 @@ __device__ __forceinline__ void msm_emit_digits(const MsmGeom& g, u32 ch, u32 gr
     }
     if (neg) d = -d;
     row[w] = (int16_t)d;
-    if (d != 0) atomicAdd(&hist[grp * g.nb() + g.bbase[ch] + w * g.B[ch] + (u32)(d < 0 ? -d : d) - 1], 1u);
+    if (d != 0) atomicAdd(&hist[msm_bucket(g, grp, ch, w, (u32)(d < 0 ? -d : d))], 1u);
   }
 }
 
 // signed c-bit digits of every term's scalar (already multiplied by c_j) + bucket histogram.  Src = SingleVkTerms: the
-// terms of g (the pointer arguments); MixTerms: the segment table of a mixed batch (g.G = 1, g.T = every term; the pointer
-// arguments are unused)
+// terms of g (the pointer arguments); MixTerms: the segment table of a mixed batch (g.T = every term, g.G = bucket sets, a
+// term's set = its segment's class; the pointer arguments are unused)
 template <class Src>
 __global__ void __launch_bounds__(128) k_msm_digits(MsmGeom g, const Fr* right, const Fr* left, const Fr* coef, const Fr* shared_sum,
                                                     const G1Affine* shared_pts, int16_t* dig, u32* hist, const u32* parent_verdict, u32 parent_size,
@@ -348,8 +348,9 @@ __global__ void __launch_bounds__(128) k_msm_digits(MsmGeom g, const Fr* right, 
   pdl_prologue();
   TlScope tl_(4, right);
   const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= g.G * g.T) return;
-  const u32 grp = t / g.T, tl = t % g.T;
+  if (t >= (Src::mixed ? g.T : g.G * g.T)) return;
+  u32 grp = t / g.T;
+  const u32 tl = t % g.T;
   const u32 nP = g.n * g.P, nL = g.n * g.n_mo;
   const u32 rows = 1 + g.glv;  // digit rows of this term
   Fr k;
@@ -359,6 +360,7 @@ __global__ void __launch_bounds__(128) k_msm_digits(MsmGeom g, const Fr* right, 
     const MixTerm mt = mix_term(sg, t - sg.t0);
     k = mix_scalar(sg, mt);
     ch = mix_channel(mt);
+    grp = sg.cls;
   } else {
     if (parent_verdict && parent_verdict[(u32)(((u64)grp * g.n) / parent_size)]) {  // sub-batch of an accepted fold group: nothing to re-check
       ch = g.channel_of_term(tl);
@@ -543,21 +545,22 @@ template <class Src>
 __global__ void __launch_bounds__(256) k_msm_scatter(MsmGeom g, const int16_t* dig, u32* cursor, u32* sorted, Src src) {
   pdl_prologue();
   TlScope tl_(5, sorted);
-  const u64 total = ((u64)g.G * g.T << g.glv) * g.Wmax;
+  const u64 total = ((Src::mixed ? (u64)g.T : (u64)g.G * g.T) << g.glv) * g.Wmax;
   for (u64 idx = (u64)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (u64)gridDim.x * blockDim.x) {
     const u32 row = (u32)(idx / g.Wmax), w = (u32)(idx % g.Wmax);  // row = term, or 2 term + GLV half
     const u32 t = row >> g.glv;
-    u32 ch;
+    u32 ch, cls = 0;
     if constexpr (Src::mixed) {
       const MixSeg& sg = src.seg[mix_segment(src.seg, src.count, t)];
       ch = mix_channel(mix_term(sg, t - sg.t0));
+      cls = sg.cls;
     } else {
       ch = g.channel_of_term(t % g.T);
     }
     if (w >= g.W[ch]) continue;
     const int d = dig[idx];
     if (d == 0) continue;
-    const u32 b = (t / g.T) * g.nb() + g.bbase[ch] + w * g.B[ch] + (u32)(d < 0 ? -d : d) - 1;
+    const u32 b = msm_bucket(g, Src::mixed ? cls : t / g.T, ch, w, (u32)(d < 0 ? -d : d));
     const u32 pos = atomicAdd(&cursor[b], 1u);
     sorted[pos] = row | (d < 0 ? 0x80000000u : 0u);
   }
@@ -1541,9 +1544,8 @@ static u32 line_run(u32 groups) {
   return (u32)(v >= 1 && v <= 64 ? v : 2);
 }
 // the (channel, run) pairs the pairing check sees for the window geometry of g: c' = c * run, P = ceil(W / run)
-static MsmGeom pair_geom(const MsmGeom& g, u32 groups) {
+static MsmGeom pair_geom_run(const MsmGeom& g, u32 run) {
   MsmGeom q{};
-  const u32 run = line_run(groups);
   for (int ch = 0; ch < 2; ch++) {
     q.c[ch] = g.c[ch] * run;
     q.W[ch] = (g.W[ch] + run - 1) / run;
@@ -1551,6 +1553,7 @@ static MsmGeom pair_geom(const MsmGeom& g, u32 groups) {
   q.wbase[1] = q.W[0];
   return q;
 }
+static MsmGeom pair_geom(const MsmGeom& g, u32 groups) { return pair_geom_run(g, line_run(groups)); }
 static u64 lines_key_of(const MsmGeom& g) { return (u64)g.c[0] | (u64)g.W[0] << 12 | (u64)g.c[1] << 24 | (u64)g.W[1] << 36; }
 
 // Prepared Miller lines of [2^(c w)] Q for the current window geometry (host: G2Prepared-style
@@ -1591,20 +1594,22 @@ static int ensure_lines(h2v_ctx* ctx, const MsmGeom& g, int* slot_out) {
 }
 static int ensure_lines(h2v_ctx* ctx, u32 groups) { return ensure_lines(ctx, pair_geom(ctx->geom, groups), &ctx->lines_cur); }
 
-// the batch pairing check over `wsums` (W0 + W1 Jacobian window sums per group, window geometry g, prepared lines of
-// pair_geom(g)) -> d_verdict[group]
-static int launch_pairing(h2v_ctx* ctx, const MsmGeom& g, const G2Line* lines, const G1Jac* wsums, u32 groups) {
-  const MsmGeom q = pair_geom(g, groups);
+// the batch pairing check over `wsums` (W0 + W1 Jacobian window sums per bucket set, window geometry g) -> d_verdict[group].
+// Each of the `groups` checks pairs `sets` consecutive bucket sets (a multi-params mix: one per params class, 1 otherwise)
+// with the prepared lines of pair_geom_run(g, run), one table per set, set-major; run 0 = line_run(groups).
+static int launch_pairing(h2v_ctx* ctx, const MsmGeom& g, const G2Line* lines, const G1Jac* wsums, u32 groups, u32 run = 0, u32 sets = 1) {
+  if (!run) run = line_run(groups);
+  const MsmGeom q = pair_geom_run(g, run);
   cudaStream_t s = ctx->stream;
   const PairSkip none{nullptr, nullptr, 1, 0};
   const u32 np = q.W[0] + q.W[1];
   const G1Jac* pairs = wsums;
-  if (line_run(groups) > 1) {
-    GroupArgs ga{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {0, g.W[0]}, {q.W[0], q.W[1]}, {0, q.W[0]}, line_run(groups)};
-    KLAUNCH(k_window_group, cdiv((u64)groups * np, 64), 64, 0, s, ga, groups, wsums, ctx->d_gsums.as<G1Jac>());
+  if (run > 1) {
+    GroupArgs ga{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {0, g.W[0]}, {q.W[0], q.W[1]}, {0, q.W[0]}, run};
+    KLAUNCH(k_window_group, cdiv((u64)groups * sets * np, 64), 64, 0, s, ga, groups * sets, wsums, ctx->d_gsums.as<G1Jac>());
     pairs = ctx->d_gsums.as<G1Jac>();
   }
-  KLAUNCH((k_lines<LINES_GROUPS>), dim3(H2V_ATE_ITERS, groups), 64 * LINES_GROUPS, k_lines_smem<LINES_GROUPS>(), s, LinesArgs{np}, pairs, lines,
+  KLAUNCH((k_lines<LINES_GROUPS>), dim3(H2V_ATE_ITERS, groups), 64 * LINES_GROUPS, k_lines_smem<LINES_GROUPS>(), s, LinesArgs{sets * np}, pairs, lines,
                                                                                        ctx->d_M.as<E12>(), none);
   // (parallel Miller segments on four blocks per group when the launch is small, pairing_cta.cuh)
   static const bool seg_off = getenv("H2V_MILLER_SEGMENTS_OFF") != nullptr;
@@ -2054,13 +2059,14 @@ template <class Src>
 static int enqueue_buckets(h2v_ctx* ctx, const MsmGeom& g, h2v_ctx::MsmBufs& B, cudaStream_t s, const TermArrays& ta, Src src,
                            const u32* parent_verdict, u32 parent_size) {
   const u32 nb = g.nb() * g.G;
-  KLAUNCH(k_msm_digits<Src>, cdiv((u64)g.G * g.T, 128), 128, 0, s, g, ta.right, ta.left, ta.coef, ta.shared_sum, ta.shared_pts, B.dig.as<int16_t>(),
+  const u64 terms = Src::mixed ? g.T : (u64)g.G * g.T;  // (a mix: g.T is every term, g.G its bucket sets)
+  KLAUNCH(k_msm_digits<Src>, cdiv(terms, 128), 128, 0, s, g, ta.right, ta.left, ta.coef, ta.shared_sum, ta.shared_pts, B.dig.as<int16_t>(),
           B.hist.as<u32>(), parent_verdict, parent_size, src);
   const u32 n_tiles = cdiv(nb, SCAN_TILE);
   KLAUNCH(k_scan_tiles, n_tiles, SCAN_NT, 0, s, B.hist.as<u32>(), nb, B.off.as<u32>(), B.tiles.as<u32>(), B.hist.as<u32>() + nb);
   KLAUNCH(k_scan_apply, n_tiles, SCAN_NT, 0, s, nb, n_tiles, B.tiles.as<u32>(), B.off.as<u32>(), B.cursor.as<u32>());
   KLAUNCH(k_bucket_order, n_tiles, SCAN_NT, 0, s, nb, B.hist.as<u32>(), B.hist.as<u32>() + nb, B.hist.as<u32>() + nb + SIZE_BINS, B.order.as<u32>());
-  KLAUNCH(k_msm_scatter<Src>, std::min<u32>(cdiv(((u64)g.G * g.T << g.glv) * g.Wmax, 256), 148 * 16), 256, 0, s, g, B.dig.as<int16_t>(), B.cursor.as<u32>(),
+  KLAUNCH(k_msm_scatter<Src>, std::min<u32>(cdiv((terms << g.glv) * g.Wmax, 256), 148 * 16), 256, 0, s, g, B.dig.as<int16_t>(), B.cursor.as<u32>(),
           B.sorted.as<u32>(), src);
   {
     set_launch_class('W');
@@ -2101,18 +2107,19 @@ static int enqueue_msm(h2v_ctx* ctx, const MsmGeom& g, h2v_ctx::MsmBufs& B, cuda
   return enqueue_buckets(ctx, g, B, s, ta, SingleVkTerms{}, parent_verdict, parent_size);
 }
 
-static cudaError_t ensure_msm_bufs(const MsmGeom& g, h2v_ctx::MsmBufs& B, u32 n_shared) {
-  const size_t nb = (size_t)g.nb() * g.G;
+// mixed: g is a mix's geometry (g.T = every term of the mix, over all g.G bucket sets)
+static cudaError_t ensure_msm_bufs(const MsmGeom& g, h2v_ctx::MsmBufs& B, u32 n_shared, bool mixed = false) {
+  const size_t nb = (size_t)g.nb() * g.G, terms = mixed ? g.T : (size_t)g.G * g.T;
   cudaError_t e;
   if ((e = B.coef.ensure(32 * (size_t)g.N)) != cudaSuccess) return e;
   if ((e = B.shared_sum.ensure(32 * (size_t)n_shared * g.G + 32)) != cudaSuccess) return e;
-  if ((e = B.dig.ensure(2 * ((size_t)g.G * g.T << g.glv) * g.Wmax)) != cudaSuccess) return e;
+  if ((e = B.dig.ensure(2 * (terms << g.glv) * g.Wmax)) != cudaSuccess) return e;
   if ((e = B.hist.ensure(4 * (nb + 2 * SIZE_BINS))) != cudaSuccess) return e;
   if ((e = B.order.ensure(4 * nb)) != cudaSuccess) return e;
   if ((e = B.off.ensure(4 * (nb + 1))) != cudaSuccess) return e;
   if ((e = B.cursor.ensure(4 * nb)) != cudaSuccess) return e;
   if ((e = B.tiles.ensure(4 * (nb / 1024 + 2))) != cudaSuccess) return e;
-  if ((e = B.sorted.ensure(4 * ((size_t)g.G * g.T << g.glv) * g.Wmax)) != cudaSuccess) return e;
+  if ((e = B.sorted.ensure(4 * (terms << g.glv) * g.Wmax)) != cudaSuccess) return e;
   if ((e = B.buckets.ensure(sizeof(G1Jac) * nb)) != cudaSuccess) return e;
   if ((e = B.wsums.ensure(sizeof(G1Jac) * (size_t)(g.W[0] + g.W[1]) * g.G)) != cudaSuccess) return e;
   return B.partials_msm.ensure(sizeof(G1Jac) * (nb / g.m));
@@ -3127,8 +3134,10 @@ double h2v_calibrate_imad(int device) {
 
 // ---- mixed batches: proofs of several contexts (verifying keys) folded into one MSM and one pairing check ----------
 // The members keep their own per-proof stages; the mix owns the joint MSM's buffers, its segment table and its graphs,
-// and runs the pairing check on the lead member (member 0), whose prepared G2 lines serve every member: all members'
-// params agree on (g, g2, s_g2).
+// and runs the pairing check on the lead member (member 0).  In a mix of h2v_mix_create all members' params agree on
+// (g, g2, s_g2) and the lead's prepared G2 lines serve every member.  In a multi-params mix (h2v_mix_create_multi_params)
+// every params class with proofs gets its own bucket set and its own line table (owned by the mix), and the one pairing
+// check multiplies the pairs of all classes.
 struct h2v_mix {
   std::vector<h2v_ctx*> m;  // members, not owned; m[0] = lead (its stream is the mix's stream)
   std::string err;
@@ -3141,9 +3150,23 @@ struct h2v_mix {
   std::vector<MixSeg> segs;    // of the current batch
   std::vector<u32> seg_member;
   MsmGeom geom{};
-  int lines_slot = -1;  // the lead's prepared lines of the joint geometry
+  int lines_slot = -1;  // the lead's prepared lines of the joint geometry (single-params mix)
   h2v_ctx::GraphSlot graphs[8];  // LRU over (member shapes, buffers), as for a context
   u64 use_clock = 0;
+  // params classes: members whose params agree on (g, g2, s_g2), numbered by first appearance (one class unless multi)
+  bool multi = false;
+  std::vector<u32> cls_of;     // per member
+  std::vector<u32> class_rep;  // per class: its first member (whose params build the class's lines)
+  // current batch: bucket set of each class (~0u: no proofs), bucket sets, run length of the window combination
+  std::vector<u32> set_of_class;
+  u32 sets = 1, run = 0;
+  // multi-params mix: line tables of (pair geometry, classes with proofs), set-major; an LRU of its own, so that the lead's
+  // cache (keyed by geometry alone) never holds a multi-class table
+  h2v_ctx::LinesSlot mlines[4];
+  int mlines_cur = -1;
+  u64 mlines_clock = 0;
+  const G2Line* lines() const { return multi ? mlines[mlines_cur].buf.as<G2Line>() : m[0]->lines[lines_slot].buf.as<G2Line>(); }
+  const DevBuf& lines_buf() const { return multi ? mlines[mlines_cur].buf : m[0]->lines[lines_slot].buf; }
 };
 
 static const G1Affine& plan_g(const h2v_ctx* c) {  // params.g: the last shared base of every plan
@@ -3158,14 +3181,57 @@ static bool params_agree(const h2v_ctx* a, const h2v_ctx* b) {
 }
 
 // joint window geometry: the single-batch choice (G = 1) over the summed terms of each channel
-static MsmGeom mix_geom(u32 N, u32 T, u32 right_terms, u32 left_terms) {
+// joint window geometry: the single-batch choice (G = 1) over the summed terms of each channel of the largest bucket set,
+// then one bucket set per params class with proofs (G = sets; T stays every term of the mix)
+static MsmGeom mix_geom(u32 N, u32 T, u32 right_terms, u32 left_terms, u32 sets) {
   MsmGeom g{};
   g.n = N;  // (picks the chunk size and bucket lanes as for a single batch of N proofs; the mixed kernels map terms through the segments)
   g.G = 1;
   g.N = N;
   g.T = T;
   choose_windows(g, right_terms, left_terms, N, 1, 0);
+  g.G = sets;
   return g;
+}
+
+// The multi-params line table of the current batch: build_window_lines over each class with proofs (its (q_right, q_left)),
+// concatenated in class order, for the pair geometry q; cached in the mix under (geometry, classes with proofs).
+static int ensure_mix_lines(h2v_mix* mx, const MsmGeom& q) {
+  h2v_ctx* ctx = mx->m[0];
+  u64 key = lines_key_of(q);
+  for (u32 c = 0; c < mx->set_of_class.size(); c++)
+    if (mx->set_of_class[c] != ~0u) key |= 1ull << (48 + c);
+  mx->mlines_clock++;
+  int victim = 0;
+  for (int i = 0; i < 4; i++) {
+    if (mx->mlines[i].key == key) {
+      mx->mlines[i].used = mx->mlines_clock;
+      mx->mlines_cur = i;
+      return 0;
+    }
+    if (mx->mlines[i].used < mx->mlines[victim].used) victim = i;
+  }
+  if (mx->sets * (q.W[0] + q.W[1]) > 128) {
+    ctx->err = "window geometry exceeds 128 (channel, window) pairs";
+    return -1;
+  }
+  std::vector<u8> tab, one;
+  for (u32 c = 0; c < mx->set_of_class.size(); c++) {
+    if (mx->set_of_class[c] == ~0u) continue;
+    build_window_lines(mx->m[mx->class_rep[c]]->info, q.c[0], q.W[0], q.c[1], q.W[1], one);
+    tab.insert(tab.end(), one.begin(), one.end());
+  }
+  h2v_ctx::LinesSlot& sl = mx->mlines[victim];
+  CKC(ctx_sync(ctx));  // the victim's lines may still be read by queued work
+  sl.key = ~0ull;
+  CKC(sl.buf.ensure(tab.size()));
+  CKC(cudaMemcpyAsync(sl.buf.p, tab.data(), tab.size(), cudaMemcpyHostToDevice, ctx->stream));
+  CKC(ctx_sync(ctx));
+  sl.key = key;
+  sl.used = mx->mlines_clock;
+  mx->mlines_cur = victim;
+  ctx->lines_builds++;
+  return 0;
 }
 
 static std::vector<h2v_ctx*> mix_active(const h2v_mix* mx) {
@@ -3181,7 +3247,9 @@ static int mix_enqueue(h2v_mix* mx, bool accum, h2v_ctx** fail) {
   *fail = ctx;
   cudaStream_t s = ctx->stream;
   const MsmGeom& g = mx->geom;
-  CKC(cudaMemsetAsync(mx->b.hist.p, 0, 4 * ((size_t)g.nb() + 2 * SIZE_BINS), s));
+  CKC(cudaMemsetAsync(mx->b.hist.p, 0, 4 * ((size_t)g.nb() * g.G + 2 * SIZE_BINS), s));
+  const bool timed = !ctx->use_graphs;  // direct launches: the lead's events time the joint stages (h2v_last_timings)
+  if (timed) CKC(cudaEventRecord(ctx->ev[0], s));
   CKC(cudaEventRecord(mx->ev_fork, s));
   for (u32 sg = 0; sg < mx->seg_member.size(); sg++) {
     const u32 mi = mx->seg_member[sg];
@@ -3204,21 +3272,26 @@ static int mix_enqueue(h2v_mix* mx, bool accum, h2v_ctx** fail) {
     }
   }
   *fail = ctx;
+  if (timed) CKC(cudaEventRecord(ctx->ev[3], s));  // MSM = [3] -> [4], pairing = [4] -> [5]
   {
     NvtxRange nv_("h2v:mix_msm");
     const MixTerms src{mx->d_seg.as<MixSeg>(), (u32)mx->segs.size()};
     int rc = enqueue_buckets(ctx, g, mx->b, s, TermArrays{}, src, nullptr, 0);
     if (rc) return rc;
   }
+  if (timed) CKC(cudaEventRecord(ctx->ev[4], s));
   {
     NvtxRange nv_("h2v:pairing");
-    int rc = launch_pairing(ctx, g, ctx->lines[mx->lines_slot].buf.as<G2Line>(), mx->b.wsums.as<G1Jac>(), 1);
+    int rc = launch_pairing(ctx, g, mx->lines(), mx->b.wsums.as<G1Jac>(), 1, mx->run, mx->sets);
     if (rc) return rc;
   }
-  if (accum) {
-    FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {g.wbase[0], g.wbase[1]}};
-    KLAUNCH(k_fold_accum, 1, 32, 0, s, fa, mx->b.wsums.as<G1Jac>(), ctx->d_acc_bytes.as<u8>());
-  }
+  if (timed) CKC(cudaEventRecord(ctx->ev[5], s));
+  if (accum)  // one (L, R) per bucket set: its window sums are wsums[set][W0 + W1]
+    for (u32 st = 0; st < g.G; st++) {
+      FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {g.wbase[0], g.wbase[1]}};
+      KLAUNCH(k_fold_accum, 1, 32, 0, s, fa, mx->b.wsums.as<G1Jac>() + (size_t)st * (g.W[0] + g.W[1]), ctx->d_acc_bytes.as<u8>() + 128 * (size_t)st);
+    }
+  if (timed) CKC(cudaEventRecord(ctx->ev[6], s));
   return 0;
 }
 
@@ -3236,15 +3309,16 @@ static u64 mix_graph_key(const h2v_mix* mx, bool accum) {
     h2v_ctx* mb = mx->m[mx->seg_member[sg]];
     mix((u64)(size_t)mb);
     mix(graph_key(mb, 0));  // the member's shape, options and buffers (what enqueue_stages and the segment read)
+    mix(mx->segs[sg].cls);  // the class assignment (bucket set of the segment)
   }
   for (int ch = 0; ch < 2; ch++) mix((u64)g.c[ch] | (u64)g.W[ch] << 8 | (u64)g.Z[ch] << 16);
   mix((u64)g.T | (u64)g.m << 32);
-  mix(g.N);
+  mix((u64)g.N | (u64)g.G << 32);
   const DevBuf* bufs[] = {&mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets, &mx->b.wsums,
                           &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &lead->d_M, &lead->d_gsums, &lead->d_verdict, &lead->d_acc_bytes,
-                          &lead->lines[mx->lines_slot].buf};
+                          &mx->lines_buf()};
   for (const DevBuf* b : bufs) mix((u64)(size_t)b->p);
-  mix(line_run(1));
+  mix(mx->run);
   return h | 1;
 }
 
@@ -3262,6 +3336,7 @@ static int mix_run(h2v_mix* mx, bool accum, h2v_ctx** fail) {
     CKC(cudaEventRecord(mx->ev_join[mi], mb->stream));
     CKC(cudaStreamWaitEvent(s, mx->ev_join[mi], 0));
   }
+  lead->stages_timed = !lead->use_graphs;
   if (!lead->use_graphs) return mix_enqueue(mx, accum, fail);
   const u64 key = mix_graph_key(mx, accum);
   mx->use_clock++;
@@ -3392,14 +3467,23 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
     if (rc) return rc;
     off += counts[i];
   }
-  // 2. segment table, joint geometry, buffers, lines
+  // 2. bucket sets (one per params class with proofs, in class order), segment table, joint geometry, buffers, lines
+  const u32 C = (u32)mx->class_rep.size();
+  mx->set_of_class.assign(C, ~0u);
+  for (u32 i = 0; i < K; i++)
+    if (counts[i]) mx->set_of_class[mx->cls_of[i]] = 0;
+  mx->sets = 0;
+  for (u32 c = 0; c < C; c++)
+    if (mx->set_of_class[c] != ~0u) mx->set_of_class[c] = mx->sets++;
+  std::vector<u32> set_of_member(K);
+  for (u32 i = 0; i < K; i++) set_of_member[i] = mx->set_of_class[mx->cls_of[i]];
   mx->segs.assign(K, MixSeg{});
   mx->seg_member.assign(K, 0);
   unsigned long long total = 0;
-  const u32 nseg = mix_layout(K, nm.data(), Pm.data(), Mm.data(), Sm.data(), mx->segs.data(), mx->seg_member.data(), &total);
+  const u32 nseg = mix_layout(K, nm.data(), Pm.data(), Mm.data(), Sm.data(), mx->segs.data(), mx->seg_member.data(), &total, set_of_member.data());
   mx->segs.resize(nseg);
   mx->seg_member.resize(nseg);
-  u64 right_terms = 0, left_terms = 0;
+  std::vector<u64> right_terms(mx->sets), left_terms(mx->sets);  // per bucket set
   for (u32 sg = 0; sg < nseg; sg++) {
     MixSeg& s = mx->segs[sg];
     h2v_ctx* c = mx->m[mx->seg_member[sg]];
@@ -3409,21 +3493,25 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
     s.shared_sum = c->mb.shared_sum.as<Fr>();
     s.pts = c->d_pts.as<G1Affine>();
     s.shared_pts = c->pv().sec<G1Affine>(c->hd.off_shared_pts);
-    right_terms += (u64)s.n * s.P + s.Sh;
-    left_terms += (u64)s.n * s.n_mo;
+    right_terms[s.cls] += (u64)s.n * s.P + s.Sh;
+    left_terms[s.cls] += (u64)s.n * s.n_mo;
   }
-  mx->geom = mix_geom((u32)N, (u32)total, (u32)right_terms, (u32)left_terms);
+  const u32 big = (u32)(std::max_element(right_terms.begin(), right_terms.end()) - right_terms.begin());
+  mx->geom = mix_geom((u32)N, (u32)total, (u32)right_terms[big], (u32)left_terms[big], mx->sets);
+  mx->run = mix_line_run(mx->sets, mx->geom.W[0], mx->geom.W[1], line_run(1));
   h2v_ctx* ctx = lead;
   *fail = lead;
   CKC(cudaSetDevice(lead->device));
-  CKC(ensure_msm_bufs(mx->geom, mx->b, 0));
+  CKC(ensure_msm_bufs(mx->geom, mx->b, 0, true));
   CKC(mx->d_seg.ensure(sizeof(MixSeg) * nseg));
   CKC(cudaMemcpyAsync(mx->d_seg.p, mx->segs.data(), sizeof(MixSeg) * nseg, cudaMemcpyHostToDevice, lead->stream));
-  CKC(lead->d_M.ensure(sizeof(E12) * (H2V_ATE_ITERS + MILLER_SEGS)));
+  CKC(lead->d_M.ensure(sizeof(E12) * (H2V_ATE_ITERS + MILLER_SEGS)));  // one check of up to 128 pairs
   CKC(lead->d_gsums.ensure(sizeof(G1Jac) * 128));
   CKC(lead->d_verdict.ensure(16));
+  CKC(lead->d_acc_bytes.ensure(128 * (size_t)mx->sets));
   {
-    int lrc = ensure_lines(lead, pair_geom(mx->geom, 1), &mx->lines_slot);
+    const MsmGeom q = pair_geom_run(mx->geom, mx->run);
+    int lrc = mx->multi ? ensure_mix_lines(mx, q) : ensure_lines(lead, q, &mx->lines_slot);
     if (lrc) return lrc;
   }
   // 3. stages + joint MSM + pairing (one graph)
@@ -3435,8 +3523,14 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
   CKC(lead->h_verd.ensure(16));
   u32* hv = lead->h_verd.as<u32>();
   CKC(cudaMemcpyAsync(hv, lead->d_verdict.p, 4, cudaMemcpyDeviceToHost, lead->stream));
-  if (batch_accum) CKC(cudaMemcpyAsync(batch_accum, lead->d_acc_bytes.p, 128, cudaMemcpyDeviceToHost, lead->stream));
+  std::vector<u8> acc(batch_accum ? 128 * (size_t)mx->sets : 0);
+  if (batch_accum) CKC(cudaMemcpyAsync(acc.data(), lead->d_acc_bytes.p, acc.size(), cudaMemcpyDeviceToHost, lead->stream));
   CKC(ctx_sync(lead));
+  if (batch_accum)  // per class, in class order; a class without proofs adds nothing: all-zero bytes
+    for (u32 c = 0; c < C; c++) {
+      if (mx->set_of_class[c] == ~0u) memset(batch_accum + 128 * (size_t)c, 0, 128);
+      else memcpy(batch_accum + 128 * (size_t)c, acc.data() + 128 * (size_t)mx->set_of_class[c], 128);
+    }
   const bool accepted = hv[0] != 0;
   // 4. statuses; on a rejected fold every member's proofs are re-checked on their own (poly/strategy.rs:26-30)
   const std::vector<h2v_ctx*> act = mix_active(mx);
@@ -3460,7 +3554,7 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
   return 0;
 }
 
-int h2v_mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members) {
+static int mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members, bool multi) {
   if (!out) {
     g_create_error = "null argument";
     return -1;
@@ -3471,6 +3565,7 @@ int h2v_mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members) {
     return -1;
   }
   const h2v_ctx* lead = members[0];
+  std::vector<u32> cls_of(n_members), class_rep;
   for (u32 i = 0; i < n_members; i++) {
     const h2v_ctx* c = members[i];
     if (!c || c->device < 0) {
@@ -3486,18 +3581,33 @@ int h2v_mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members) {
       g_create_error = "member " + std::to_string(i) + " is on device " + std::to_string(c->device) + ", member 0 on device " + std::to_string(lead->device);
       return -1;
     }
-    if (!params_agree(c, lead)) {
+    if (!multi && !params_agree(c, lead)) {
       g_create_error = "member " + std::to_string(i) + "'s params differ from member 0's in (g, g2, s_g2): their proofs cannot share one pairing check";
       return -1;
     }
+    u32 k = 0;
+    while (k < class_rep.size() && !params_agree(c, members[class_rep[k]])) k++;
+    if (k == class_rep.size()) {
+      if (k == H2V_MIX_MAX_PARAMS) {
+        g_create_error = "member " + std::to_string(i) + " holds a " + std::to_string(k + 1) + "th set of KZG params: a multi-params mix takes 1 .. " +
+                         std::to_string(H2V_MIX_MAX_PARAMS) + " params classes";
+        return -1;
+      }
+      class_rep.push_back(i);
+    }
+    cls_of[i] = k;
   }
   h2v_mix* mx = new h2v_mix();
+  mx->multi = multi;
+  mx->cls_of = cls_of;
+  mx->class_rep = class_rep;
   mx->m.assign(members, members + n_members);
   mx->ev_join.assign(n_members, nullptr);
   h2v_ctx* l = mx->m[0];
   for (DevBuf* d : {&mx->b.coef, &mx->b.shared_sum, &mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets,
                     &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg})
     d->st = &l->stream;
+  for (auto& sl : mx->mlines) sl.buf.st = &l->stream;
   cudaError_t e = cudaSetDevice(l->device);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&mx->ev_fork, cudaEventDisableTiming);
   for (u32 i = 0; i < n_members && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&mx->ev_join[i], cudaEventDisableTiming);
@@ -3510,6 +3620,15 @@ int h2v_mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members) {
   return 0;
 }
 
+int h2v_mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members) { return mix_create(out, members, n_members, false); }
+int h2v_mix_create_multi_params(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members) { return mix_create(out, members, n_members, true); }
+
+int h2v_mix_params_classes(const h2v_mix* mx, uint32_t* class_of, uint32_t capacity) {
+  if (!mx || !class_of || capacity < mx->m.size()) return -1;
+  for (size_t i = 0; i < mx->m.size(); i++) class_of[i] = mx->cls_of[i];
+  return (int)mx->class_rep.size();
+}
+
 void h2v_mix_destroy(h2v_mix* mx) {
   if (!mx) return;
   h2v_ctx* l = mx->m[0];
@@ -3520,6 +3639,7 @@ void h2v_mix_destroy(h2v_mix* mx) {
   for (DevBuf* d : {&mx->b.coef, &mx->b.shared_sum, &mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets,
                     &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg})
     d->release();
+  for (auto& sl : mx->mlines) sl.buf.release();
   cudaStreamSynchronize(l->stream);  // the stream-ordered frees
   if (mx->ev_fork) cudaEventDestroy(mx->ev_fork);
   for (cudaEvent_t ev : mx->ev_join)

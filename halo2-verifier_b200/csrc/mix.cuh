@@ -4,7 +4,9 @@
 //               terms, Sh shared-base terms
 //   mixed batch (MixSeg table): one segment per member context with proofs, consecutive in term-id space; inside a segment
 //               the terms keep the single-VK order of one fold group, over the member's own arrays.  A one-segment table
-//               therefore maps every term exactly as msm_point / channel_of_term do.
+//               therefore maps every term exactly as msm_point / channel_of_term do.  The MsmGeom of a mix has T = every
+//               term of the mix and G = bucket sets: one per params class with proofs (h2v_mix_create_multi_params), 1
+//               otherwise; a segment's terms go to the bucket set of its class (MixSeg::cls).
 // Compiles on the host too (tests/hostlib/mix_harness.cpp checks the mapping without a GPU).
 #pragma once
 #include "curve.cuh"
@@ -56,6 +58,7 @@ static constexpr u32 MIX_MAX_MEMBERS = 64;
 struct MixSeg {
   u32 t0, T;            // first term id, terms (n*P + n*n_mo + Sh)
   u32 n, P, n_mo, Sh;   // the member's proofs and plan shape
+  u32 cls;              // bucket set of the member's params class (0 in a single-params mix)
   const Fr* right;      // [P][n]     right-channel scalars of the proof points
   const Fr* left;       // [n_mo][n]  left-channel scalars of the multi-open points
   const Fr* coef;       // [n]        fold coefficients c_j of the member's slice of the global batch
@@ -74,9 +77,11 @@ struct MixTerms {
   u32 count;  // 1 .. MIX_MAX_MEMBERS
 };
 
-// Segment table of `members` members with n[m] proofs each (members without proofs get no segment): t0 / T / shape
-// fields of seg[0 .. return value), member_of[s] = member of segment s; *total = terms of all segments.
-inline u32 mix_layout(u32 members, const u32* n, const u32* P, const u32* n_mo, const u32* Sh, MixSeg* seg, u32* member_of, unsigned long long* total) {
+// Segment table of `members` members with n[m] proofs each (members without proofs get no segment): t0 / T / shape / cls
+// fields of seg[0 .. return value), member_of[s] = member of segment s; *total = terms of all segments.  set[m] = bucket set
+// of member m (null: every segment in set 0).
+inline u32 mix_layout(u32 members, const u32* n, const u32* P, const u32* n_mo, const u32* Sh, MixSeg* seg, u32* member_of, unsigned long long* total,
+                      const u32* set = nullptr) {
   u32 count = 0;
   unsigned long long t = 0;
   for (u32 m = 0; m < members; m++) {
@@ -87,6 +92,7 @@ inline u32 mix_layout(u32 members, const u32* n, const u32* P, const u32* n_mo, 
     s.P = P[m];
     s.n_mo = n_mo[m];
     s.Sh = Sh[m];
+    s.cls = set ? set[m] : 0;
     s.T = s.n * s.P + s.n * s.n_mo + s.Sh;
     t += s.T;
     member_of[count] = m;
@@ -131,6 +137,19 @@ H2V_HD Fr mix_scalar(const MixSeg& s, const MixTerm& m) {
   if (m.kind == 1) return (s.left[(size_t)m.i * s.n + m.j] * s.coef[m.j]).to_canonical();
   const G1Affine& sp = s.shared_pts[m.i];
   return (sp.x.is_zero() && sp.y.is_zero()) ? Fr::zero() : s.shared_sum[m.i];
+}
+
+// bucket index of digit magnitude mag (1 .. B) of window w, channel ch, in bucket set `set` (fold group or params class)
+H2V_HD u32 msm_bucket(const MsmGeom& g, u32 set, u32 ch, u32 w, u32 mag) { return set * g.nb() + g.bbase[ch] + w * g.B[ch] + mag - 1; }
+
+// Run length of the partial window combination of a mix whose `sets` bucket sets share one pairing check: the smallest run
+// >= run0 for which sets * (ceil(W0 / run) + ceil(W1 / run)) <= 128 pairs (LinesSmem of k_lines).  With one set every
+// single-batch geometry (W <= 64 per channel) fits at run0 >= 1, so a single-params mix keeps run0; with 8 sets run = 8
+// always fits (2 x 8 pairs per set).
+inline u32 mix_line_run(u32 sets, u32 W0, u32 W1, u32 run0) {
+  u32 run = run0 ? run0 : 1;
+  while (sets * ((W0 + run - 1) / run + (W1 + run - 1) / run) > 128) run++;
+  return run;
 }
 
 }  // namespace h2v

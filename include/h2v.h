@@ -270,6 +270,24 @@ int h2v_mix_set_rlc_key(h2v_mix* mx, const uint8_t* key32);
 int h2v_mix_verify(h2v_mix* mx, const uint32_t* counts, const uint8_t* proofs, const uint64_t* proof_off, const uint8_t* instances,
                    const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint8_t* status, uint8_t* batch_accum,
                    int* verdict);
+/* Multi-params mixes: proofs under several KZG params in ONE fold.  For params classes p with G2 arguments
+ * ([s_p]g2_p, -g2_p) the check is prod_p e(L_p, [s_p]g2_p) e(R_p, -g2_p) = 1, L_p / R_p = the fold of class p's proofs with
+ * the c_j of the whole member-major concatenation: one Miller product over every class's pairs and one final
+ * exponentiation.  Each class with proofs gets its own bucket set of the joint MSM and its own prepared lines (owned by the
+ * mix); all classes together take at most 128 (channel, window-run) pairs, so more classes pair longer window runs.
+ * h2v_mix_verify keeps its signature and semantics (statuses, attribution under each member's own params, fold
+ * randomness) except batch_accum: classes x 128 B, the folded affine (L_p, R_p) of every class in class order; a class
+ * with no proofs in the call gets all-zero bytes and adds nothing to the check.  Not combinable with fold groups, shards
+ * or the device-side exchange, as for every mix. */
+#define H2V_MIX_MAX_PARAMS 8
+/* As h2v_mix_create, but members may hold different KZG params.  Members whose params agree on (g, g2, s_g2) (the comparison
+ * h2v_mix_create makes) form one params class; classes are numbered by first appearance in member order (member 0 is in
+ * class 0).  1 .. H2V_MIX_MAX_PARAMS classes; more are refused before any device call, with the text in
+ * h2v_mix_last_error(NULL).  The other refusals are those of h2v_mix_create. */
+int h2v_mix_create_multi_params(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members);
+/* class_of[m] = params class of member m (capacity >= n_members); returns the number of classes (1 for a mix of
+ * h2v_mix_create), -1 on a null argument or a short array */
+int h2v_mix_params_classes(const h2v_mix* mx, uint32_t* class_of, uint32_t capacity);
 
 /* ---- persistent accumulators: AccumulatorStrategy as a value that lives across calls ------------------------------------
  * The reference's AccumulatorStrategy (poly/kzg/strategy.rs:125-140) is fed proofs through any number of verify_proof calls,
