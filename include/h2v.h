@@ -108,7 +108,7 @@ int h2v_ctx_info(const h2v_ctx* ctx, uint32_t* out8);
 int h2v_ctx_vk_lint(const h2v_ctx* ctx, char* report, size_t capacity);
 
 /* verify_proof with SingleStrategy (lib.rs:33-46, strategy.rs:164-176) for one proof.
- * instances: n_inst 32-byte little-endian canonical Fr values, columns concatenated. */
+ * instances: n_inst 32-byte little-endian canonical Fr values, columns concatenated (a value >= r: H2V_INVALID_INSTANCES). */
 int h2v_verify_proof(h2v_ctx* ctx, const uint8_t* proof, size_t proof_len, const uint8_t* instances,
                      size_t n_inst, uint8_t* status);
 
@@ -116,7 +116,8 @@ int h2v_verify_proof(h2v_ctx* ctx, const uint8_t* proof, size_t proof_len, const
  * a failed batch the per-proof re-check the reference prescribes (poly/strategy.rs:26-30).
  *   proofs / proof_off    concatenated proof bytes, n+1 byte offsets
  *   instances / inst_off  concatenated 32-byte LE canonical Fr, n+1 offsets in units of scalars;
- *                         per proof: columns concatenated, equal length (see h2v_batch_set_columns)
+ *                         per proof: columns concatenated, equal length (see h2v_batch_set_columns).  A value >= r
+ *                         fails its proof alone with H2V_INVALID_INSTANCES, ahead of any transcript or opening error.
  *   rlc_scalars           n x 32 B canonical non-zero r_i, or NULL to expand them from `seed`; proof j is folded
  *                         with c_j = prod_{i>j} r_i, the reference's convention (SURVEY.md 3.2).  A zero or
  *                         non-canonical r_i (it would zero c_j of every earlier proof) is refused before any

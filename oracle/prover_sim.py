@@ -109,6 +109,12 @@ def make_vk(shape, k, seed=0):
         cs_degree = 5
     else:
         raise ValueError(shape)
+    return vk_from_cs(k, cs, cs_degree, rng)
+
+
+def vk_from_cs(k, cs, cs_degree, rng):
+    """(vk, dlogs) of a constraint system: random fixed / sigma commitments with known discrete logs, random selectors
+    and transcript_repr"""
     f_d = [rng.randrange(1, R) for _ in range(cs.num_fixed_columns)]
     s_d = [rng.randrange(1, R) for _ in range(len(cs.permutation_columns))]
     sel_bytes = ((1 << k) + 7) // 8

@@ -30,8 +30,9 @@ def test_field_ptx_matches_portable(pkg):
 
 
 def check_against_oracle(bv, params, vk, instances, proofs, mo, hk, rs):
-    n = len(proofs)
-    res = bv.verify_batch(proofs, [i[0] for i in instances], rlc_scalars=rs, want_challenges=True, want_accum=True,
+    """instances: the oracle's [circuit instance][column][row] per proof"""
+    api = [i[0] for i in instances] if bv.circuit_instances == 1 else instances
+    res = bv.verify_batch(proofs, api, rlc_scalars=rs, want_challenges=True, want_accum=True,
                           want_batch_accum=True, want_scalars=True)
     want = [orc.verify_proof(params, vk, inst, p, mo, hk) for inst, p in zip(instances, proofs)]
     assert res.status == [w.status for w in want]
