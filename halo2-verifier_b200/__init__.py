@@ -170,6 +170,16 @@ def load_library():
     lib.h2v_mix_last_error.restype = ctypes.c_char_p
     lib.h2v_mix_set_rlc_key.argtypes = [ctypes.c_void_p, ctypes.c_char_p]
     lib.h2v_mix_verify.argtypes = [ctypes.c_void_p, u32p, u8p, u64p, u8p, u64p, u8p, ctypes.c_uint64, u8p, u8p, ctypes.POINTER(ctypes.c_int)]
+    lib.h2v_mix_set_shard_hint.argtypes = [ctypes.c_void_p, ctypes.c_uint32]
+    lib.h2v_mix_partial_bytes.argtypes = [ctypes.c_void_p, u32p]
+    lib.h2v_mix_partial_bytes.restype = ctypes.c_size_t
+    lib.h2v_mix_accumulate_shard.argtypes = [ctypes.c_void_p, u32p, ctypes.c_uint64, ctypes.c_uint32, u8p, u64p, u8p, u64p, u8p, ctypes.c_uint64, u8p,
+                                             ctypes.c_void_p]
+    lib.h2v_mix_finalize.argtypes = [ctypes.c_void_p, u32p, ctypes.c_uint32, ctypes.c_void_p, u8p, ctypes.POINTER(ctypes.c_int)]
+    lib.h2v_mix_attribute_shard.argtypes = [ctypes.c_void_p, u8p]
+    lib.h2v_mix_verify_shard.argtypes = [ctypes.c_void_p, u32p, ctypes.c_uint64, ctypes.c_uint32, u8p, u64p, u8p, u64p, u8p, ctypes.c_uint64,
+                                         ctypes.c_uint32, u8p, ctypes.POINTER(ctypes.c_int)]
+    lib.h2v_mix_comm_last_batch_accum.argtypes = [ctypes.c_void_p, u8p]
     lib.h2v_acc_create.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_void_p, ctypes.c_uint32]
     lib.h2v_acc_destroy.argtypes = [ctypes.c_void_p]
     lib.h2v_acc_destroy.restype = None
@@ -195,6 +205,8 @@ EXPORTED_SYMBOLS = (
     "h2v_batch_run_shard_exchange", "h2v_verify_shard", "h2v_comm_last_batch_accum", "h2v_ctx_cache_stats", "h2v_ctx_work_model", "h2v_ctx_vk_lint",
     "h2v_mix_create", "h2v_mix_destroy", "h2v_mix_last_error", "h2v_mix_set_rlc_key", "h2v_mix_verify",
     "h2v_mix_create_multi_params", "h2v_mix_params_classes",
+    "h2v_mix_set_shard_hint", "h2v_mix_partial_bytes", "h2v_mix_accumulate_shard", "h2v_mix_finalize", "h2v_mix_attribute_shard",
+    "h2v_mix_verify_shard", "h2v_mix_comm_last_batch_accum",
     "h2v_acc_create", "h2v_acc_destroy", "h2v_acc_last_error", "h2v_acc_set_rlc_key", "h2v_acc_absorb", "h2v_acc_finalize", "h2v_acc_get",
     "h2v_acc_merge", "h2v_acc_reset", "h2v_ctx_create_aggregation", "h2v_batch_set_agg_scalar",
 )
@@ -637,14 +649,41 @@ class MixedBatchVerifier:
         """proofs_per_member[m] / instances_per_member[m]: member m's proofs and instances as for its own verify_batch
         (empty lists allowed).  The fold runs over the member-major concatenation: rlc_scalars has one entry per proof of
         it.  Fold randomness as BatchVerifier.verify_batch: OS entropy unless `rlc_scalars` / `key` / `seed` say otherwise."""
+        counts, packed = self._pack(proofs_per_member, instances_per_member)
+        n = sum(counts)
+        if n == 0:
+            raise ValueError("a mixed batch needs at least one proof")
+        if rlc_scalars is not None and len(rlc_scalars) != n:
+            raise ValueError("one fold scalar per proof of the concatenation")
+        rlc, seed = self._randomness(proofs_per_member, rlc_scalars, seed, key, agg_scalar)
+        status = (ctypes.c_uint8 * n)()
+        bacc = ctypes.create_string_buffer(128 * self.n_classes) if want_batch_accum else None
+        verdict = ctypes.c_int(0)
+        self._check(self.lib.h2v_mix_verify(self._mx, self._u32(counts), *packed[:4], rlc, int(seed), status, bacc, ctypes.byref(verdict)))
+        return MixedBatchResult(self._split(list(status), counts), bool(verdict.value), bacc.raw if bacc is not None else None)
+
+    @staticmethod
+    def _u32(values):
+        return (ctypes.c_uint32 * max(1, len(values)))(*values)
+
+    @staticmethod
+    def _split(statuses, counts):
+        out = []
+        for c in counts:
+            out.append(statuses[:c])
+            statuses = statuses[c:]
+        return out
+
+    def _pack(self, proofs_per_member, instances_per_member):
+        """member-major concatenation: (per-member counts, (proofs, proof offsets, instances, instance offsets, keep-alive))"""
         if len(proofs_per_member) != len(self.members) or len(instances_per_member) != len(self.members):
             raise ValueError("one proof list and one instance list per member")
-        counts = (ctypes.c_uint32 * len(self.members))()
+        counts = []
         pparts, iparts, poffs, ioffs, keep = [], [], [0], [0], []
         for m, (bv, proofs, insts) in enumerate(zip(self.members, proofs_per_member, instances_per_member)):
             if len(proofs) != len(insts):
                 raise ValueError(f"member {m}: {len(proofs)} proofs, {len(insts)} instance lists")
-            counts[m] = len(proofs)
+            counts.append(len(proofs))
             if not proofs:
                 continue
             pbytes, poff, ibytes, ioff, k = bv._pack(proofs, insts)  # (sets the member's ragged layout if needed)
@@ -654,24 +693,99 @@ class MixedBatchVerifier:
             poffs += [poffs[-1] + poff[j + 1] for j in range(len(proofs))]
             ioffs += [ioffs[-1] + ioff[j + 1] for j in range(len(proofs))]
         n = len(poffs) - 1
-        if n == 0:
-            raise ValueError("a mixed batch needs at least one proof")
-        if rlc_scalars is not None and len(rlc_scalars) != n:
-            raise ValueError("one fold scalar per proof of the concatenation")
+        return counts, (b"".join(pparts), (ctypes.c_uint64 * (n + 1))(*poffs), b"".join(iparts), (ctypes.c_uint64 * (n + 1))(*ioffs), keep)
+
+    def _randomness(self, proofs_per_member, rlc_scalars, seed, key, agg_scalar):
         rlc, seed = _fold_args(rlc_scalars, seed, key, lambda k: self._check(self.lib.h2v_mix_set_rlc_key(self._mx, k)))
         for bv, proofs in zip(self.members, proofs_per_member):  # one rho for every aggregation member with proofs
             if proofs and bv.accumulator is not None:
                 bv._set_agg_scalar(agg_scalar)
-        status = (ctypes.c_uint8 * n)()
+        return rlc, seed
+
+    # ---- sharded mixed batches (include/h2v.h "sharded mixed batches")
+    def _shard_args(self, proofs_per_member, instances_per_member, global_counts, global_base, rlc_scalars, shard_hint):
+        """this rank's portions, checked against the split the library derives (sharding.mixed_shard)"""
+        from .sharding import mixed_shard_counts
+        counts, packed = self._pack(proofs_per_member, instances_per_member)
+        if len(global_counts) != len(self.members):
+            raise ValueError("one global count per member")
+        want = mixed_shard_counts(global_counts, global_base, sum(counts))
+        if counts != want:
+            raise ValueError(f"proofs per member {counts} are not the share of proofs [{global_base}, {global_base + sum(counts)}) of the global batch: {want}")
+        if rlc_scalars is not None and len(rlc_scalars) != sum(global_counts):
+            raise ValueError("one fold scalar per proof of the global batch")
+        if shard_hint:
+            self._check(self.lib.h2v_mix_set_shard_hint(self._mx, int(shard_hint)))
+        return sum(counts), counts, packed
+
+    def partial_bytes(self, global_counts) -> int:
+        """bytes of one rank's partials for this global batch: one H2V_PARTIAL_BYTES blob per params class with proofs"""
+        return int(self.lib.h2v_mix_partial_bytes(self._mx, self._u32(global_counts)))
+
+    def accumulate_shard(self, proofs_per_member, instances_per_member, global_counts, global_base, rlc_scalars=None, seed=None, key=None,
+                         shard_hint=0, partial_out=None, agg_scalar=None):
+        """This rank's share [global_base, global_base + n) of the member-major global batch of global_counts proofs: returns
+        (statuses per member, partials), partials = bytes of partial_bytes(global_counts), or None when `partial_out` (a device
+        or host address) receives them.  shard_hint: the largest shard when the shards differ in size."""
+        n, counts, packed = self._shard_args(proofs_per_member, instances_per_member, global_counts, global_base, rlc_scalars, shard_hint)
+        rlc, seed = self._randomness(proofs_per_member, rlc_scalars, seed, key, agg_scalar)
+        status = (ctypes.c_uint8 * max(1, n))()
+        buf = ctypes.create_string_buffer(max(1, self.partial_bytes(global_counts))) if partial_out is None else None
+        self._check(self.lib.h2v_mix_accumulate_shard(self._mx, self._u32(global_counts), int(global_base), n, *packed[:4], rlc, int(seed), status,
+                                                      ctypes.cast(buf, ctypes.c_void_p) if buf is not None else ctypes.c_void_p(int(partial_out))))
+        return self._split(list(status)[:n], counts), (buf.raw if buf is not None else None)
+
+    def finalize(self, partials, global_counts, want_batch_accum=True, n_partials=None):
+        """partials: one accumulate_shard output per rank, or (with n_partials) the address of n_partials ranks' outputs in host or
+        device memory.  Returns (verdict of the one pairing check, classes x 128 B folded (L_p, R_p) or None)."""
         bacc = ctypes.create_string_buffer(128 * self.n_classes) if want_batch_accum else None
         verdict = ctypes.c_int(0)
-        self._check(self.lib.h2v_mix_verify(self._mx, counts, b"".join(pparts), (ctypes.c_uint64 * (n + 1))(*poffs), b"".join(iparts),
-                                             (ctypes.c_uint64 * (n + 1))(*ioffs), rlc, int(seed), status, bacc, ctypes.byref(verdict)))
-        st, out = list(status), []
-        for c in counts:
-            out.append(st[:c])
-            st = st[c:]
-        return MixedBatchResult(out, bool(verdict.value), bacc.raw if bacc is not None else None)
+        if n_partials is None:
+            buf = ctypes.create_string_buffer(b"".join(partials), max(1, sum(len(p) for p in partials)))
+            n_partials, addr = len(partials), ctypes.cast(buf, ctypes.c_void_p)
+        else:
+            addr = ctypes.c_void_p(int(partials))
+        self._check(self.lib.h2v_mix_finalize(self._mx, self._u32(global_counts), int(n_partials), addr, bacc, ctypes.byref(verdict)))
+        return bool(verdict.value), (bacc.raw if bacc is not None else None)
+
+    def attribute_shard(self, status):
+        """per-proof re-check of the shard last processed; `status`: its statuses per member (accumulate_shard's)"""
+        counts = [len(s) for s in status]
+        arr = (ctypes.c_uint8 * max(1, sum(counts)))(*[v for s in status for v in s])
+        self._check(self.lib.h2v_mix_attribute_shard(self._mx, arr))
+        return self._split(list(arr)[:sum(counts)], counts)
+
+    # device-side exchange over the lead member's channel
+    def comm_init(self, rank, world, max_groups=1) -> bytes:
+        """the lead's exchange window, for at least as many partials per rank as the mix has params classes (the most bucket
+        sets a batch can have; the same on every rank)"""
+        h = self.members[0].comm_init(rank, world, max(int(max_groups), self.n_classes))
+        self.comm_ready = False
+        return h
+
+    def comm_connect(self, handles):
+        self.members[0].comm_connect(handles)
+        self.comm_ready = True
+
+    comm_ready = False
+
+    def verify_shard(self, proofs_per_member, instances_per_member, global_counts, global_base, root, rlc_scalars=None, seed=None, key=None,
+                     shard_hint=0, agg_scalar=None):
+        """This rank's share through the device-side exchange: returns (verdict of the global check, statuses per member);
+        a rejection is attributed per proof inside this rank's share."""
+        n, counts, packed = self._shard_args(proofs_per_member, instances_per_member, global_counts, global_base, rlc_scalars, shard_hint)
+        rlc, seed = self._randomness(proofs_per_member, rlc_scalars, seed, key, agg_scalar)
+        status = (ctypes.c_uint8 * max(1, n))()
+        verdict = ctypes.c_int(0)
+        self._check(self.lib.h2v_mix_verify_shard(self._mx, self._u32(global_counts), int(global_base), n, *packed[:4], rlc, int(seed), int(root),
+                                                  status, ctypes.byref(verdict)))
+        return bool(verdict.value), self._split(list(status)[:n], counts)
+
+    def comm_last_batch_accum(self) -> bytes:
+        """root only: classes x 128 B folded (L_p, R_p) of the last exchange launch set"""
+        out = ctypes.create_string_buffer(128 * self.n_classes)
+        self._check(self.lib.h2v_mix_comm_last_batch_accum(self._mx, out))
+        return out.raw
 
     def cache_stats(self):
         """the lead member's caches: the mix's graph captures and prepared lines are counted there"""

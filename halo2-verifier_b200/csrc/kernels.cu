@@ -1635,8 +1635,9 @@ static int launch_pair_checks(h2v_ctx* ctx, const G1Jac* pairs, u32 count, const
 
 // verdicts of all fold groups of the last run -> ctx->h_verdicts; *all = every group accepted (waits for the stream).
 // xchg: the run went through the device-side exchange; its two error words follow the verdicts.
-static int read_verdicts(h2v_ctx* ctx, u32* all, bool xchg = false) {
-  const u32 G = ctx->geom.G ? ctx->geom.G : 1;
+// groups != 0: that many verdict words instead of the context's fold groups (a mixed batch's one check on its lead)
+static int read_verdicts(h2v_ctx* ctx, u32* all, bool xchg = false, u32 groups = 0) {
+  const u32 G = groups ? groups : ctx->geom.G ? ctx->geom.G : 1;
   CKC(ctx->h_verd.ensure(4 * (size_t)(G + 2)));
   u32* hv = ctx->h_verd.as<u32>();
   hv[G] = hv[G + 1] = 0;
@@ -2688,62 +2689,66 @@ int h2v_accumulate_shard(h2v_ctx* ctx, uint32_t n, const uint8_t* proofs, const 
   return download_status(ctx, status);
 }
 
-static int finalize_impl(h2v_ctx* ctx, u32 n_partials, u32 groups, const u8* partials, u8* batch_accum, int* verdict, u8* group_verdicts) {
-  if (!ctx || !partials || !n_partials || n_partials > 128 || !groups || groups > 1024 || (batch_accum && groups != 1)) return -1;
-  CKC(cudaSetDevice(ctx->device));
-  cudaStream_t s = ctx->stream;
-  // partials already in this device's memory (e.g. the output of a gather) are summed in place
-  const u8* d_parts = nullptr;
+// `bytes` of partials in this device's memory: in place when they already are (e.g. the output of a gather), else copied
+static int device_partials(h2v_ctx* ctx, const u8* partials, size_t bytes, const u8** d_parts) {
+  *d_parts = nullptr;
   {
     cudaPointerAttributes pa{};
-    if (cudaPointerGetAttributes(&pa, partials) == cudaSuccess && pa.type == cudaMemoryTypeDevice && pa.device == ctx->device) d_parts = partials;
+    if (cudaPointerGetAttributes(&pa, partials) == cudaSuccess && pa.type == cudaMemoryTypeDevice && pa.device == ctx->device) *d_parts = partials;
     (void)cudaGetLastError();
   }
-  if (!d_parts) {
-    CKC(ctx->d_partials.ensure((size_t)H2V_PARTIAL_BYTES * n_partials * groups));
-    CKC(cudaMemcpyAsync(ctx->d_partials.p, partials, (size_t)H2V_PARTIAL_BYTES * n_partials * groups, cudaMemcpyDefault, s));
-    d_parts = ctx->d_partials.as<u8>();
+  if (!*d_parts) {
+    CKC(ctx->d_partials.ensure(bytes));
+    CKC(cudaMemcpyAsync(ctx->d_partials.p, partials, bytes, cudaMemcpyDefault, ctx->stream));
+    *d_parts = ctx->d_partials.as<u8>();
   }
-  if (ctx->n == 0) {  // a context that has not processed a shard itself: take the geometry from the first partial
-    PartialHeader h;
-    CKC(cudaMemcpyAsync(&h, d_parts, sizeof(h), cudaMemcpyDeviceToHost, s));
-    CKC(ctx_sync(ctx));
-    MsmGeom& g = ctx->geom;
-    g = MsmGeom{};
-    g.c[0] = h.cbits & 0xFFFF;
-    g.c[1] = h.cbits >> 16;
-    g.W[0] = h.windows & 0xFFFF;
-    g.W[1] = h.windows >> 16;
-    if (h.magic != H2V_PARTIAL_MAGIC || g.c[0] < 1 || g.c[1] < 1 || g.W[0] + g.W[1] != h.n_pts || h.n_pts > 128) {
-      ctx->err = "malformed partial accumulator";
-      return -1;
-    }
-    g.wbase[1] = g.W[0];
+  return 0;
+}
+
+// window geometry (c, W per channel) of the partial at d_parts, from its header
+static int partial_geom(h2v_ctx* ctx, const u8* d_parts, MsmGeom& g) {
+  PartialHeader h;
+  CKC(cudaMemcpyAsync(&h, d_parts, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+  CKC(ctx_sync(ctx));
+  g = MsmGeom{};
+  g.c[0] = h.cbits & 0xFFFF;
+  g.c[1] = h.cbits >> 16;
+  g.W[0] = h.windows & 0xFFFF;
+  g.W[1] = h.windows >> 16;
+  if (h.magic != H2V_PARTIAL_MAGIC || g.c[0] < 1 || g.c[1] < 1 || g.W[0] + g.W[1] != h.n_pts || h.n_pts > 128) {
+    ctx->err = "malformed partial accumulator";
+    return -1;
   }
-  const int lines_of_batch = ctx->lines_cur;  // the resident batch of this context keeps its own line geometry (restored below)
-  {
-    int lrc = ensure_lines(ctx, groups);
-    if (lrc) return lrc;
-  }
-  const MsmGeom& g = ctx->geom;
-  const u32 npts = g.W[0] + g.W[1];
+  g.wbase[1] = g.W[0];
+  return 0;
+}
+
+// The final check of partials on ctx's stream: the window-wise sum of n_partials ranks' blobs ([rank][group][set], device
+// memory), then `groups` pairing checks of `sets` bucket sets each (geometry g, prepared lines `lines`, run length `run`, 0 =
+// line_run(groups)).  batch_accum (groups == 1): sets x 128 B folded affine (L, R), set order.  *all = every check accepted.
+static int sum_and_pair(h2v_ctx* ctx, const MsmGeom& g, const G2Line* lines, u32 run, u32 n_partials, u32 groups, u32 sets, const u8* d_parts,
+                        u8* batch_accum, u8* group_verdicts, u32* all) {
+  cudaStream_t s = ctx->stream;
+  const u32 npts = g.W[0] + g.W[1], blobs = groups * sets;
   CKC(ctx->d_verdict.ensure(4 * (size_t)groups + 16));
   CKC(ctx->d_M.ensure(sizeof(E12) * (H2V_ATE_ITERS + MILLER_SEGS) * (size_t)groups));
-  CKC(ctx->d_wsums_fin.ensure(sizeof(G1Jac) * 128 * (size_t)groups));
-  CKC(ctx->d_gsums.ensure(sizeof(G1Jac) * 128 * (size_t)groups));
+  CKC(ctx->d_wsums_fin.ensure(sizeof(G1Jac) * 128 * (size_t)blobs));
+  CKC(ctx->d_gsums.ensure(sizeof(G1Jac) * 128 * (size_t)blobs));
   CKC(cudaMemsetAsync(ctx->d_verdict.p, 0, 4 * (size_t)groups + 16, s));
   ctx->verdicts_on_device = false;  // d_verdict now belongs to the global batches being finalized
-  k_sum_partials<<<groups, 128, 0, s>>>(n_partials, g.c[0] | g.c[1] << 16, g.W[0] | g.W[1] << 16, npts, d_parts, (size_t)groups * H2V_PARTIAL_BYTES,
-                                        ctx->d_wsums_fin.as<G1Jac>(), ctx->d_verdict.as<u32>() + groups, nullptr, nullptr);
+  k_sum_partials<<<blobs, 128, 0, s>>>(n_partials, g.c[0] | g.c[1] << 16, g.W[0] | g.W[1] << 16, npts, d_parts, (size_t)blobs * H2V_PARTIAL_BYTES,
+                                       ctx->d_wsums_fin.as<G1Jac>(), ctx->d_verdict.as<u32>() + groups, nullptr, nullptr);
   LAUNCH_CHECK();
-  int prc = launch_pairing(ctx, ctx->d_wsums_fin.as<G1Jac>(), groups);
-  if (lines_of_batch >= 0 && ctx->n) ctx->lines_cur = lines_of_batch;
+  int prc = launch_pairing(ctx, g, lines, ctx->d_wsums_fin.as<G1Jac>(), groups, run, sets);
   if (prc) return prc;
   if (batch_accum) {
+    CKC(ctx->d_acc_bytes.ensure(128 * (size_t)sets));
     FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {0, g.W[0]}};
-    k_fold_accum<<<1, 32, 0, s>>>(fa, ctx->d_wsums_fin.as<G1Jac>(), ctx->d_acc_bytes.as<u8>());
-    LAUNCH_CHECK();
-    CKC(cudaMemcpyAsync(batch_accum, ctx->d_acc_bytes.p, 128, cudaMemcpyDeviceToHost, s));
+    for (u32 st = 0; st < sets; st++) {
+      k_fold_accum<<<1, 32, 0, s>>>(fa, ctx->d_wsums_fin.as<G1Jac>() + (size_t)st * npts, ctx->d_acc_bytes.as<u8>() + 128 * (size_t)st);
+      LAUNCH_CHECK();
+    }
+    CKC(cudaMemcpyAsync(batch_accum, ctx->d_acc_bytes.p, 128 * (size_t)sets, cudaMemcpyDeviceToHost, s));
   }
   CKC(ctx->h_verd.ensure(4 * (size_t)(groups + 2)));
   const u32* v = ctx->h_verd.as<u32>();
@@ -2753,11 +2758,30 @@ static int finalize_impl(h2v_ctx* ctx, u32 n_partials, u32 groups, const u8* par
     ctx->err = "partial accumulators were produced with different window geometries (use h2v_batch_set_shard_hint)";
     return -1;
   }
-  u32 all = 1;
+  *all = 1;
   for (u32 q = 0; q < groups; q++) {
-    all &= v[q] ? 1u : 0u;
+    *all &= v[q] ? 1u : 0u;
     if (group_verdicts) group_verdicts[q] = v[q] ? 1 : 0;
   }
+  return 0;
+}
+
+static int finalize_impl(h2v_ctx* ctx, u32 n_partials, u32 groups, const u8* partials, u8* batch_accum, int* verdict, u8* group_verdicts) {
+  if (!ctx || !partials || !n_partials || n_partials > 128 || !groups || groups > 1024 || (batch_accum && groups != 1)) return -1;
+  CKC(cudaSetDevice(ctx->device));
+  const u8* d_parts = nullptr;
+  int rc = device_partials(ctx, partials, (size_t)H2V_PARTIAL_BYTES * n_partials * groups, &d_parts);
+  if (rc) return rc;
+  if (ctx->n == 0 && (rc = partial_geom(ctx, d_parts, ctx->geom)) != 0) return rc;  // a context that has not processed a shard itself
+  const int lines_of_batch = ctx->lines_cur;  // the resident batch of this context keeps its own line geometry (restored below)
+  {
+    int lrc = ensure_lines(ctx, groups);
+    if (lrc) return lrc;
+  }
+  u32 all = 0;
+  rc = sum_and_pair(ctx, ctx->geom, ctx->d_lines(), 0, n_partials, groups, 1, d_parts, batch_accum, group_verdicts, &all);
+  if (lines_of_batch >= 0 && ctx->n) ctx->lines_cur = lines_of_batch;
+  if (rc) return rc;
   if (verdict) *verdict = (int)all;
   return 0;
 }
@@ -2885,6 +2909,17 @@ int h2v_comm_connect(h2v_ctx* ctx, const uint8_t* handles) {
   return 0;
 }
 
+// parameters of the next launch set on ctx's channel (sequence number, root), copied to the device on ctx's stream
+static cudaError_t comm_next_launch(h2v_ctx* ctx, u32 root) {
+  h2v_ctx::Comm& cm = ctx->comm;
+  XDyn* d = &cm.h_dyn[cm.ring++ % XDYN_RING];
+  d->seq = ++cm.seq;
+  d->root = root;
+  d->rsv = 0;
+  d->timeout_ns = cm.timeout_ns;
+  return cudaMemcpyAsync(cm.d_dyn, d, sizeof(XDyn), cudaMemcpyHostToDevice, ctx->stream);
+}
+
 // one launch set through the exchange; `status` != null: attribution inside rejected groups + status download
 static int exchange_run(h2v_ctx* ctx, u32 root, u8* group_verdicts, int* verdict, bool e2e, u8* status) {
   h2v_ctx::Comm& cm = ctx->comm;
@@ -2893,12 +2928,7 @@ static int exchange_run(h2v_ctx* ctx, u32 root, u8* group_verdicts, int* verdict
     return -1;
   }
   CKC(cudaSetDevice(ctx->device));
-  XDyn* d = &cm.h_dyn[cm.ring++ % XDYN_RING];
-  d->seq = ++cm.seq;
-  d->root = root;
-  d->rsv = 0;
-  d->timeout_ns = cm.timeout_ns;
-  CKC(cudaMemcpyAsync(cm.d_dyn, d, sizeof(XDyn), cudaMemcpyHostToDevice, ctx->stream));
+  CKC(comm_next_launch(ctx, root));
   int rc = run_impl(ctx, RUN_XCHG | (root == cm.lay.rank ? RUN_ROOT : 0));
   if (rc) return rc;
   u32 all = 0;
@@ -3165,6 +3195,12 @@ struct h2v_mix {
   h2v_ctx::LinesSlot mlines[4];
   int mlines_cur = -1;
   u64 mlines_clock = 0;
+  // sharded mixed batches (h2v_mix_accumulate_shard / h2v_mix_verify_shard)
+  DevBuf d_partial;          // this rank's partials: one H2V_PARTIAL_BYTES blob per bucket set (RUN_PARTIAL)
+  u32 opt_shard_hint = 0;    // one-shot: window geometry for shards of up to this many proofs (h2v_mix_set_shard_hint)
+  std::vector<u32> counts;   // proofs per member of the batch / shard last uploaded
+  bool ran = false;          // a launch set ran on that upload (h2v_mix_attribute_shard)
+  bool xchg_root = false;    // the last launch set went through the exchange with this rank as its root
   const G2Line* lines() const { return multi ? mlines[mlines_cur].buf.as<G2Line>() : m[0]->lines[lines_slot].buf.as<G2Line>(); }
   const DevBuf& lines_buf() const { return multi ? mlines[mlines_cur].buf : m[0]->lines[lines_slot].buf; }
 };
@@ -3240,9 +3276,12 @@ static std::vector<h2v_ctx*> mix_active(const h2v_mix* mx) {
   return v;
 }
 
-// Every kernel of a mixed batch: the members' stages forked onto their own streams, the joint MSM and the pairing on the
-// lead's stream.  *fail = the context whose call failed.
-static int mix_enqueue(h2v_mix* mx, bool accum, h2v_ctx** fail) {
+// Every kernel of a mixed batch: the members' stages forked onto their own streams, the joint MSM on the lead's stream, then,
+// by the RUN_* mode bits of enqueue_batch: RUN_PAIRING the pairing check over every bucket set -> the lead's d_verdict[0];
+// RUN_ACCUM (with RUN_PAIRING) one folded (L, R) per bucket set; RUN_PARTIAL one partial per bucket set -> mx->d_partial
+// (sharded mixes); RUN_XCHG (+ RUN_ROOT) the device-side exchange over the lead's channel, the root's summed window sums in
+// the lead's d_wsums_fin.  *fail = the context whose call failed.
+static int mix_enqueue(h2v_mix* mx, int mode, h2v_ctx** fail) {
   h2v_ctx* ctx = mx->m[0];
   *fail = ctx;
   cudaStream_t s = ctx->stream;
@@ -3280,13 +3319,31 @@ static int mix_enqueue(h2v_mix* mx, bool accum, h2v_ctx** fail) {
     if (rc) return rc;
   }
   if (timed) CKC(cudaEventRecord(ctx->ev[4], s));
-  {
+  if (mode & RUN_PAIRING) {
     NvtxRange nv_("h2v:pairing");
     int rc = launch_pairing(ctx, g, mx->lines(), mx->b.wsums.as<G1Jac>(), 1, mx->run, mx->sets);
     if (rc) return rc;
   }
+  const u32 cb = g.c[0] | g.c[1] << 16, wd = g.W[0] | g.W[1] << 16, npts = g.W[0] + g.W[1];
+  if (mode & RUN_PARTIAL) KLAUNCH(k_pack_partial, dim3(8, g.G), 256, 0, s, cb, wd, npts, mx->b.wsums.as<G1Jac>(), mx->d_partial.as<u8>());
+  if (mode & RUN_XCHG) {
+    NvtxRange nv_("h2v:exchange");
+    // as enqueue_batch's exchange step, with one blob per bucket set and ONE check over all sets on the root
+    h2v_ctx::Comm& cm = ctx->comm;
+    u32* vd = ctx->d_verdict.as<u32>();
+    CKC(cudaMemsetAsync(vd + 1, 0, 8, s));  // error words of this launch set
+    KLAUNCH(k_pack_partial_x, g.G, 256, 0, s, cb, wd, npts, mx->b.wsums.as<G1Jac>(), cm.d_dyn, cm.d_peers, cm.lay, cm.d_done);
+    if (mode & RUN_ROOT) {
+      KLAUNCH_P(false, k_sum_partials, g.G, 128, 0, s, cm.lay.world, cb, wd, npts, cm.window + cm.lay.partials_off(), (size_t)cm.lay.max_groups * H2V_PARTIAL_BYTES,
+                ctx->d_wsums_fin.as<G1Jac>(), vd + 1, cm.d_dyn, (const u64*)(cm.window + cm.lay.arrive_off()));
+      int prc = launch_pairing(ctx, g, mx->lines(), ctx->d_wsums_fin.as<G1Jac>(), 1, mx->run, mx->sets);
+      if (prc) return prc;
+      KLAUNCH_P(false, k_bcast_verdict, 1, 256, 0, s, cm.d_dyn, cm.d_peers, cm.lay, 1u, vd, vd + 1);
+    }
+    KLAUNCH_P(false, k_wait_verdict, 1, 64, 0, s, cm.d_dyn, cm.window, cm.lay, 1u, vd);
+  }
   if (timed) CKC(cudaEventRecord(ctx->ev[5], s));
-  if (accum)  // one (L, R) per bucket set: its window sums are wsums[set][W0 + W1]
+  if (mode & RUN_ACCUM)  // one (L, R) per bucket set: its window sums are wsums[set][W0 + W1]
     for (u32 st = 0; st < g.G; st++) {
       FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {g.wbase[0], g.wbase[1]}};
       KLAUNCH(k_fold_accum, 1, 32, 0, s, fa, mx->b.wsums.as<G1Jac>() + (size_t)st * (g.W[0] + g.W[1]), ctx->d_acc_bytes.as<u8>() + 128 * (size_t)st);
@@ -3295,7 +3352,7 @@ static int mix_enqueue(h2v_mix* mx, bool accum, h2v_ctx** fail) {
   return 0;
 }
 
-static u64 mix_graph_key(const h2v_mix* mx, bool accum) {
+static u64 mix_graph_key(const h2v_mix* mx, int mode) {
   u64 h = 0xcbf29ce484222325ull;
   auto mix = [&h](u64 v) {
     h ^= v;
@@ -3304,7 +3361,7 @@ static u64 mix_graph_key(const h2v_mix* mx, bool accum) {
   };
   const h2v_ctx* lead = mx->m[0];
   const MsmGeom& g = mx->geom;
-  mix(accum);
+  mix((mode & RUN_ACCUM) ? 1 : 0);
   for (u32 sg = 0; sg < mx->seg_member.size(); sg++) {
     h2v_ctx* mb = mx->m[mx->seg_member[sg]];
     mix((u64)(size_t)mb);
@@ -3319,11 +3376,21 @@ static u64 mix_graph_key(const h2v_mix* mx, bool accum) {
                           &mx->lines_buf()};
   for (const DevBuf* b : bufs) mix((u64)(size_t)b->p);
   mix(mx->run);
+  if (mode & (RUN_PARTIAL | RUN_XCHG)) {  // sharded launch sets: the mode (root or not), the partial buffers and the lead's channel
+    const h2v_ctx::Comm& cm = lead->comm;
+    mix((u64)mode);
+    mix((u64)(size_t)mx->d_partial.p);
+    mix((u64)(size_t)lead->d_wsums_fin.p);
+    mix((u64)(size_t)cm.window);
+    mix((u64)(size_t)cm.d_peers ^ (u64)(size_t)cm.d_dyn << 1 ^ (u64)(size_t)cm.d_done << 2);
+    mix((u64)cm.lay.rank | (u64)cm.lay.world << 32);
+    mix(cm.lay.max_groups);
+  }
   return h | 1;
 }
 
 // the launch set on the lead's stream: graph replay (capture on a miss) or, with the lead's graphs off, direct launches
-static int mix_run(h2v_mix* mx, bool accum, h2v_ctx** fail) {
+static int mix_run(h2v_mix* mx, int mode, h2v_ctx** fail) {
   h2v_ctx* lead = mx->m[0];
   *fail = lead;
   h2v_ctx* ctx = lead;
@@ -3337,8 +3404,8 @@ static int mix_run(h2v_mix* mx, bool accum, h2v_ctx** fail) {
     CKC(cudaStreamWaitEvent(s, mx->ev_join[mi], 0));
   }
   lead->stages_timed = !lead->use_graphs;
-  if (!lead->use_graphs) return mix_enqueue(mx, accum, fail);
-  const u64 key = mix_graph_key(mx, accum);
+  if (!lead->use_graphs) return mix_enqueue(mx, mode, fail);
+  const u64 key = mix_graph_key(mx, mode);
   mx->use_clock++;
   h2v_ctx::GraphSlot* hit = nullptr;
   h2v_ctx::GraphSlot* victim = &mx->graphs[0];
@@ -3356,7 +3423,7 @@ static int mix_run(h2v_mix* mx, bool accum, h2v_ctx** fail) {
     for (h2v_ctx* c : mx->m) before.push_back(c->launches);
     CKC(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
     for (h2v_ctx* mb : act) mb->capturing = true;
-    const int rc = mix_enqueue(mx, accum, fail);
+    const int rc = mix_enqueue(mx, mode, fail);
     for (h2v_ctx* mb : act) mb->capturing = false;
     cudaGraph_t graph = nullptr;
     const cudaError_t ce = cudaStreamEndCapture(s, &graph);
@@ -3382,17 +3449,46 @@ static int mix_run(h2v_mix* mx, bool accum, h2v_ctx** fail) {
   return 0;
 }
 
-static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, const u64* proof_off, const u8* instances, const u64* inst_off,
-                           const u8* rlc, u64 seed, u8* status, u8* batch_accum, int* verdict, h2v_ctx** fail) {
+// bucket sets of a batch in which member m has counts[m] proofs: one per params class with proofs, numbered in class order
+static void mix_assign_sets(h2v_mix* mx, const u32* counts) {
+  const u32 C = (u32)mx->class_rep.size();
+  mx->set_of_class.assign(C, ~0u);
+  for (u32 i = 0; i < mx->m.size(); i++)
+    if (counts[i]) mx->set_of_class[mx->cls_of[i]] = 0;
+  mx->sets = 0;
+  for (u32 c = 0; c < C; c++)
+    if (mx->set_of_class[c] != ~0u) mx->set_of_class[c] = mx->sets++;
+}
+static u32 mix_count_sets(const h2v_mix* mx, const u32* counts) {
+  std::vector<bool> used(mx->class_rep.size(), false);
+  for (u32 i = 0; i < mx->m.size(); i++)
+    if (counts[i]) used[mx->cls_of[i]] = true;
+  return (u32)std::count(used.begin(), used.end(), true);
+}
+
+// batch_accum in class order from one 128 B (L, R) per bucket set; a class without proofs adds nothing: all-zero bytes
+static void mix_class_accum(const h2v_mix* mx, const u8* acc, u8* batch_accum) {
+  for (u32 c = 0; c < mx->set_of_class.size(); c++) {
+    if (mx->set_of_class[c] == ~0u) memset(batch_accum + 128 * (size_t)c, 0, 128);
+    else memcpy(batch_accum + 128 * (size_t)c, acc + 128 * (size_t)mx->set_of_class[c], 128);
+  }
+}
+
+// Validation and upload of a mixed batch: local[m] proofs of member m, member-major in proofs / offsets, which are proofs
+// [gbase, gbase + sum local) of the member-major concatenation of gcounts[m] proofs (a whole batch: local = gcounts, gbase = 0).
+// The fold coefficients and the bucket sets are those of the global batch.  Window geometry: max_shard = 0 the mix's own choice
+// over its terms, otherwise every rank's common choice for shards of up to max_shard proofs (mix_shard_bound).  Then the
+// segment table, the joint MSM's buffers and the lines.  Everything up to the first upload_impl is host-only.
+static int mix_upload(h2v_mix* mx, const u32* local, const u32* gcounts, u64 gbase, u32 max_shard, const u8* proofs, const u64* proof_off,
+                      const u8* instances, const u64* inst_off, const u8* rlc, u64 seed, h2v_ctx** fail) {
   const u32 K = (u32)mx->m.size();
   h2v_ctx* lead = mx->m[0];
   *fail = nullptr;
-  if (!counts || !proof_off || !inst_off || !status || !verdict) {
-    mx->err = "null argument";
-    return -1;
+  u64 N = 0, n = 0;
+  for (u32 i = 0; i < K; i++) {
+    N += gcounts[i];
+    n += local[i];
   }
-  u64 N = 0;
-  for (u32 i = 0; i < K; i++) N += counts[i];
   if (N == 0 || N > 0xFFFFFFFFull) {
     mx->err = "a mixed batch needs between 1 and 2^32 - 1 proofs";
     return -1;
@@ -3402,11 +3498,11 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
     return -1;
   }
   // caller data: validated as upload_impl validates a context's batch
-  if (proof_off[0] != 0 || inst_off[0] != 0 || (!proofs && proof_off[N]) || (!instances && inst_off[N])) {
+  if (proof_off[0] != 0 || inst_off[0] != 0 || (!proofs && proof_off[n]) || (!instances && inst_off[n])) {
     mx->err = "offset arrays must start at 0";
     return -1;
   }
-  for (u64 j = 0; j < N; j++) {
+  for (u64 j = 0; j < n; j++) {
     if (proof_off[j + 1] < proof_off[j] || inst_off[j + 1] < inst_off[j] || proof_off[j + 1] - proof_off[j] > 0x7FFFFFFFull ||
         inst_off[j + 1] - inst_off[j] > 0x03FFFFFFull) {
       mx->err = "offset arrays must be non-decreasing with per-proof sizes below 2^31 bytes / 2^26 scalars";
@@ -3420,7 +3516,7 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
       mx->err = "member " + std::to_string(i) + " has a pending fold-group or shard-hint option: mixed batches do not combine with them";
       return -1;
     }
-    if (counts[i]) terms += (u64)counts[i] * (msm_points(c->hd) + msm_mo(c->hd)) + c->hd.n_shared;
+    if (local[i]) terms += (u64)local[i] * (msm_points(c->hd) + msm_mo(c->hd)) + c->hd.n_shared;
   }
   // term ids carry the sign in bit 31 (k_msm_scatter): the limit of upload_impl, over the whole mix
   if (terms >= (1ull << 31)) {
@@ -3442,18 +3538,22 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
     keyed = true;
   }
   mx->has_key = false;
-  // 1. every member's slice as a shard [off, off + count) of the global batch of N proofs
+  mx->opt_shard_hint = 0;
+  mx->ran = false;
+  mx->xchg_root = false;
+  mx->counts.assign(local, local + K);
+  // 1. every member's slice as a shard [gbase + off, gbase + off + local) of the global batch of N proofs
   std::vector<u32> nm(K), Pm(K), Mm(K), Sm(K);
   u64 off = 0;
   for (u32 i = 0; i < K; i++) {
     h2v_ctx* c = mx->m[i];
-    nm[i] = counts[i];
+    nm[i] = local[i];
     Pm[i] = msm_points(c->hd);
     Mm[i] = msm_mo(c->hd);
     Sm[i] = c->hd.n_shared;
-    if (!counts[i]) continue;
-    std::vector<u64> po(counts[i] + 1), io(counts[i] + 1);
-    for (u32 j = 0; j <= counts[i]; j++) {
+    if (!local[i]) continue;
+    std::vector<u64> po(local[i] + 1), io(local[i] + 1);
+    for (u32 j = 0; j <= local[i]; j++) {
       po[j] = proof_off[off + j] - proof_off[off];
       io[j] = inst_off[off + j] - inst_off[off];
     }
@@ -3462,19 +3562,14 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
       c->opt_has_key = true;
     }
     *fail = c;
-    int rc = upload_impl(c, counts[i], proofs ? proofs + proof_off[off] : nullptr, po.data(), instances ? instances + 32 * inst_off[off] : nullptr,
-                         io.data(), rlc, keyed ? 0 : seed, off, N);
+    int rc = upload_impl(c, local[i], proofs ? proofs + proof_off[off] : nullptr, po.data(), instances ? instances + 32 * inst_off[off] : nullptr,
+                         io.data(), rlc, keyed ? 0 : seed, gbase + off, N);
     if (rc) return rc;
-    off += counts[i];
+    off += local[i];
   }
-  // 2. bucket sets (one per params class with proofs, in class order), segment table, joint geometry, buffers, lines
-  const u32 C = (u32)mx->class_rep.size();
-  mx->set_of_class.assign(C, ~0u);
-  for (u32 i = 0; i < K; i++)
-    if (counts[i]) mx->set_of_class[mx->cls_of[i]] = 0;
-  mx->sets = 0;
-  for (u32 c = 0; c < C; c++)
-    if (mx->set_of_class[c] != ~0u) mx->set_of_class[c] = mx->sets++;
+  // 2. bucket sets (one per params class with proofs in the global batch, in class order), segment table, joint geometry,
+  // buffers, lines
+  mix_assign_sets(mx, gcounts);
   std::vector<u32> set_of_member(K);
   for (u32 i = 0; i < K; i++) set_of_member[i] = mx->set_of_class[mx->cls_of[i]];
   mx->segs.assign(K, MixSeg{});
@@ -3496,8 +3591,14 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
     right_terms[s.cls] += (u64)s.n * s.P + s.Sh;
     left_terms[s.cls] += (u64)s.n * s.n_mo;
   }
-  const u32 big = (u32)(std::max_element(right_terms.begin(), right_terms.end()) - right_terms.begin());
-  mx->geom = mix_geom((u32)N, (u32)total, (u32)right_terms[big], (u32)left_terms[big], mx->sets);
+  if (max_shard) {  // every rank the same (c, W): the partials add up window-wise
+    unsigned long long rb = 0, lb = 0;
+    mix_shard_bound(K, Pm.data(), Mm.data(), Sm.data(), gcounts, max_shard, &rb, &lb);
+    mx->geom = mix_geom(max_shard, (u32)total, (u32)std::min(rb, 0xFFFFFFFFull), (u32)std::min(lb, 0xFFFFFFFFull), mx->sets);
+  } else {
+    const u32 big = (u32)(std::max_element(right_terms.begin(), right_terms.end()) - right_terms.begin());
+    mx->geom = mix_geom((u32)N, (u32)total, (u32)right_terms[big], (u32)left_terms[big], mx->sets);
+  }
   mx->run = mix_line_run(mx->sets, mx->geom.W[0], mx->geom.W[1], line_run(1));
   h2v_ctx* ctx = lead;
   *fail = lead;
@@ -3509,16 +3610,59 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
   CKC(lead->d_gsums.ensure(sizeof(G1Jac) * 128));
   CKC(lead->d_verdict.ensure(16));
   CKC(lead->d_acc_bytes.ensure(128 * (size_t)mx->sets));
+  if (max_shard) {
+    CKC(mx->d_partial.ensure((size_t)H2V_PARTIAL_BYTES * mx->sets));
+    CKC(lead->d_wsums_fin.ensure(sizeof(G1Jac) * 128 * (size_t)mx->sets));
+  }
+  const MsmGeom q = pair_geom_run(mx->geom, mx->run);
+  return mx->multi ? ensure_mix_lines(mx, q) : ensure_lines(lead, q, &mx->lines_slot);
+}
+
+static void mix_mark_ran(h2v_mix* mx) {
+  for (h2v_ctx* c : mix_active(mx)) {
+    c->verdicts_on_device = false;
+    c->ran = true;
+  }
+  mx->ran = true;
+}
+
+// statuses of the upload's proofs, member-major; attribute: every member's proofs are re-checked on their own first
+// (poly/strategy.rs:26-30).  *all_ok = every status is H2V_OK.
+static int mix_statuses(h2v_mix* mx, bool attribute, u8* status, bool* all_ok, h2v_ctx** fail) {
+  *all_ok = true;
+  u64 off = 0;
+  for (u32 i = 0; i < mx->m.size(); i++) {
+    const u32 cnt = mx->counts[i];
+    if (!cnt) continue;
+    h2v_ctx* c = mx->m[i];
+    *fail = c;
+    int rc = attribute ? attribute_impl(c) : 0;
+    if (!rc) rc = download_status(c, status + off);
+    if (rc) return rc;
+    for (u32 j = 0; j < cnt; j++) *all_ok &= status[off + j] == ST_OK;
+    off += cnt;
+  }
+  return 0;
+}
+
+static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, const u64* proof_off, const u8* instances, const u64* inst_off,
+                           const u8* rlc, u64 seed, u8* status, u8* batch_accum, int* verdict, h2v_ctx** fail) {
+  h2v_ctx* lead = mx->m[0];
+  *fail = nullptr;
+  if (!counts || !proof_off || !inst_off || !status || !verdict) {
+    mx->err = "null argument";
+    return -1;
+  }
   {
-    const MsmGeom q = pair_geom_run(mx->geom, mx->run);
-    int lrc = mx->multi ? ensure_mix_lines(mx, q) : ensure_lines(lead, q, &mx->lines_slot);
-    if (lrc) return lrc;
+    int rc = mix_upload(mx, counts, counts, 0, 0, proofs, proof_off, instances, inst_off, rlc, seed, fail);
+    if (rc) return rc;
   }
   // 3. stages + joint MSM + pairing (one graph)
   {
-    int rc = mix_run(mx, batch_accum != nullptr, fail);
+    int rc = mix_run(mx, RUN_PAIRING | (batch_accum ? RUN_ACCUM : 0), fail);
     if (rc) return rc;
   }
+  h2v_ctx* ctx = lead;
   *fail = lead;
   CKC(lead->h_verd.ensure(16));
   u32* hv = lead->h_verd.as<u32>();
@@ -3526,31 +3670,14 @@ static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, con
   std::vector<u8> acc(batch_accum ? 128 * (size_t)mx->sets : 0);
   if (batch_accum) CKC(cudaMemcpyAsync(acc.data(), lead->d_acc_bytes.p, acc.size(), cudaMemcpyDeviceToHost, lead->stream));
   CKC(ctx_sync(lead));
-  if (batch_accum)  // per class, in class order; a class without proofs adds nothing: all-zero bytes
-    for (u32 c = 0; c < C; c++) {
-      if (mx->set_of_class[c] == ~0u) memset(batch_accum + 128 * (size_t)c, 0, 128);
-      else memcpy(batch_accum + 128 * (size_t)c, acc.data() + 128 * (size_t)mx->set_of_class[c], 128);
-    }
+  if (batch_accum) mix_class_accum(mx, acc.data(), batch_accum);
   const bool accepted = hv[0] != 0;
   // 4. statuses; on a rejected fold every member's proofs are re-checked on their own (poly/strategy.rs:26-30)
-  const std::vector<h2v_ctx*> act = mix_active(mx);
-  for (h2v_ctx* c : act) {
-    c->verdicts_on_device = false;
-    c->ran = true;
-  }
-  bool all_ok = accepted;
-  off = 0;
-  for (u32 i = 0; i < K; i++) {
-    if (!counts[i]) continue;
-    h2v_ctx* c = mx->m[i];
-    *fail = c;
-    int rc = accepted ? 0 : attribute_impl(c);
-    if (!rc) rc = download_status(c, status + off);
-    if (rc) return rc;
-    for (u32 j = 0; j < counts[i]; j++) all_ok &= status[off + j] == ST_OK;
-    off += counts[i];
-  }
-  *verdict = all_ok ? 1 : 0;
+  mix_mark_ran(mx);
+  bool all_ok = false;
+  int rc = mix_statuses(mx, !accepted, status, &all_ok, fail);
+  if (rc) return rc;
+  *verdict = accepted && all_ok ? 1 : 0;
   return 0;
 }
 
@@ -3605,7 +3732,7 @@ static int mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members
   mx->ev_join.assign(n_members, nullptr);
   h2v_ctx* l = mx->m[0];
   for (DevBuf* d : {&mx->b.coef, &mx->b.shared_sum, &mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets,
-                    &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg})
+                    &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_partial})
     d->st = &l->stream;
   for (auto& sl : mx->mlines) sl.buf.st = &l->stream;
   cudaError_t e = cudaSetDevice(l->device);
@@ -3637,7 +3764,7 @@ void h2v_mix_destroy(h2v_mix* mx) {
   for (auto& gsl : mx->graphs)
     if (gsl.exec) cudaGraphExecDestroy(gsl.exec);
   for (DevBuf* d : {&mx->b.coef, &mx->b.shared_sum, &mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets,
-                    &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg})
+                    &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_partial})
     d->release();
   for (auto& sl : mx->mlines) sl.buf.release();
   cudaStreamSynchronize(l->stream);  // the stream-ordered frees
@@ -3648,6 +3775,15 @@ void h2v_mix_destroy(h2v_mix* mx) {
 }
 
 const char* h2v_mix_last_error(const h2v_mix* mx) { return mx ? mx->err.c_str() : g_create_error.c_str(); }
+
+// rc of a mix call; a failure inside a member's call is reported as "member i: <its error>"
+static int mix_report(h2v_mix* mx, int rc, h2v_ctx* fail) {
+  if (rc && fail && mx->err.empty()) {
+    const size_t i = std::find(mx->m.begin(), mx->m.end(), fail) - mx->m.begin();
+    mx->err = "member " + std::to_string(i) + ": " + fail->err;
+  }
+  return rc;
+}
 
 int h2v_mix_set_rlc_key(h2v_mix* mx, const uint8_t* key32) {
   if (!mx || !key32) return -1;
@@ -3663,11 +3799,216 @@ int h2v_mix_verify(h2v_mix* mx, const uint32_t* counts, const uint8_t* proofs, c
   mx->err.clear();
   h2v_ctx* fail = nullptr;
   const int rc = mix_verify_impl(mx, counts, proofs, proof_off, instances, inst_off, rlc_scalars, seed, status, batch_accum, verdict, &fail);
-  if (rc && fail && mx->err.empty()) {
-    const size_t i = std::find(mx->m.begin(), mx->m.end(), fail) - mx->m.begin();
-    mx->err = "member " + std::to_string(i) + ": " + fail->err;
+  return mix_report(mx, rc, fail);
+}
+
+// ---- sharded mixed batches: one rank's share of a global mixed batch, partials per bucket set, one pairing check ----------
+int h2v_mix_set_shard_hint(h2v_mix* mx, uint32_t max_shard_proofs) {
+  if (!mx) return -1;
+  mx->opt_shard_hint = max_shard_proofs;
+  return 0;
+}
+
+size_t h2v_mix_partial_bytes(const h2v_mix* mx, const uint32_t* global_counts) {
+  if (!mx || !global_counts) return 0;
+  return (size_t)H2V_PARTIAL_BYTES * mix_count_sets(mx, global_counts);
+}
+
+// The checks of a shard call that need no device: local[m] = this rank's proofs of member m, *max_shard = the geometry's shard size
+static int mix_shard_args(h2v_mix* mx, const uint32_t* global_counts, uint64_t global_base, uint32_t n, const uint64_t* proof_off,
+                          const uint64_t* inst_off, const uint8_t* status, std::vector<u32>& local, u32* max_shard) {
+  if (!global_counts || !proof_off || !inst_off || !status) {
+    mx->err = "null argument";
+    return -1;
   }
-  return rc;
+  u64 N = 0;
+  for (u32 i = 0; i < mx->m.size(); i++) N += global_counts[i];
+  if (N == 0 || N > 0xFFFFFFFFull) {
+    mx->err = "a mixed batch needs between 1 and 2^32 - 1 proofs";
+    return -1;
+  }
+  local.assign(mx->m.size(), 0);
+  if (!mix_shard_counts((u32)mx->m.size(), global_counts, global_base, n, local.data())) {
+    mx->err = "the shard [global_base, global_base + n) must be a non-empty range inside the global batch";
+    return -1;
+  }
+  if (mx->opt_shard_hint && mx->opt_shard_hint < n) {
+    mx->err = "the shard hint (" + std::to_string(mx->opt_shard_hint) + ") is smaller than this shard (" + std::to_string(n) + " proofs)";
+    return -1;
+  }
+  *max_shard = mx->opt_shard_hint ? mx->opt_shard_hint : n;
+  return 0;
+}
+
+static int mix_accumulate_shard_impl(h2v_mix* mx, const uint32_t* global_counts, uint64_t global_base, uint32_t n, const uint8_t* proofs,
+                                     const uint64_t* proof_off, const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars,
+                                     uint64_t seed, uint8_t* status, uint8_t* partial, h2v_ctx** fail) {
+  std::vector<u32> local;
+  u32 max_shard = 0;
+  if (!partial) {
+    mx->err = "null argument";
+    return -1;
+  }
+  int rc = mix_shard_args(mx, global_counts, global_base, n, proof_off, inst_off, status, local, &max_shard);
+  if (!rc) rc = mix_upload(mx, local.data(), global_counts, global_base, max_shard, proofs, proof_off, instances, inst_off, rlc_scalars, seed, fail);
+  if (!rc) rc = mix_run(mx, RUN_PARTIAL, fail);
+  if (rc) return rc;
+  mix_mark_ran(mx);
+  h2v_ctx* ctx = mx->m[0];
+  *fail = ctx;
+  CKC(cudaMemcpyAsync(partial, mx->d_partial.p, (size_t)H2V_PARTIAL_BYTES * mx->sets, cudaMemcpyDefault, ctx->stream));
+  CKC(ctx_sync(ctx));
+  bool all_ok = false;
+  return mix_statuses(mx, false, status, &all_ok, fail);
+}
+
+int h2v_mix_accumulate_shard(h2v_mix* mx, const uint32_t* global_counts, uint64_t global_base, uint32_t n, const uint8_t* proofs,
+                             const uint64_t* proof_off, const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars,
+                             uint64_t seed, uint8_t* status, uint8_t* partial) {
+  if (!mx) return -1;
+  NvtxRange nv_("h2v:mix_shard");
+  mx->err.clear();
+  h2v_ctx* fail = nullptr;
+  const int rc = mix_accumulate_shard_impl(mx, global_counts, global_base, n, proofs, proof_off, instances, inst_off, rlc_scalars, seed, status,
+                                           partial, &fail);
+  return mix_report(mx, rc, fail);
+}
+
+static int mix_finalize_impl(h2v_mix* mx, const uint32_t* global_counts, uint32_t n_partials, const uint8_t* partials, uint8_t* batch_accum,
+                             int* verdict, h2v_ctx** fail) {
+  if (!global_counts || !partials || !verdict) {
+    mx->err = "null argument";
+    return -1;
+  }
+  if (n_partials == 0 || n_partials > 128) {
+    mx->err = "h2v_mix_finalize takes 1 .. 128 ranks' partials";
+    return -1;
+  }
+  if (!mix_count_sets(mx, global_counts)) {
+    mx->err = "a mixed batch needs between 1 and 2^32 - 1 proofs";
+    return -1;
+  }
+  h2v_ctx* ctx = mx->m[0];
+  *fail = ctx;
+  CKC(cudaSetDevice(ctx->device));
+  mix_assign_sets(mx, global_counts);
+  const u8* d_parts = nullptr;
+  MsmGeom g{};
+  int rc = device_partials(ctx, partials, (size_t)H2V_PARTIAL_BYTES * n_partials * mx->sets, &d_parts);
+  if (!rc) rc = partial_geom(ctx, d_parts, g);  // the geometry every rank packed with (k_sum_partials flags a rank that did not)
+  if (rc) return rc;
+  mx->run = mix_line_run(mx->sets, g.W[0], g.W[1], line_run(1));
+  const MsmGeom q = pair_geom_run(g, mx->run);
+  rc = mx->multi ? ensure_mix_lines(mx, q) : ensure_lines(ctx, q, &mx->lines_slot);
+  if (rc) return rc;
+  std::vector<u8> acc(batch_accum ? 128 * (size_t)mx->sets : 0);
+  u32 all = 0;
+  rc = sum_and_pair(ctx, g, mx->lines(), mx->run, n_partials, 1, mx->sets, d_parts, batch_accum ? acc.data() : nullptr, nullptr, &all);
+  if (rc) return rc;
+  if (batch_accum) mix_class_accum(mx, acc.data(), batch_accum);
+  *verdict = (int)all;
+  return 0;
+}
+
+int h2v_mix_finalize(h2v_mix* mx, const uint32_t* global_counts, uint32_t n_partials, const uint8_t* partials, uint8_t* batch_accum, int* verdict) {
+  if (!mx) return -1;
+  NvtxRange nv_("h2v:mix_finalize");
+  mx->err.clear();
+  h2v_ctx* fail = nullptr;
+  const int rc = mix_finalize_impl(mx, global_counts, n_partials, partials, batch_accum, verdict, &fail);  // (before fail is read)
+  return mix_report(mx, rc, fail);
+}
+
+int h2v_mix_attribute_shard(h2v_mix* mx, uint8_t* status) {
+  if (!mx) return -1;
+  mx->err.clear();
+  if (!status || !mx->ran) {
+    mx->err = status ? "no shard was processed by this mix" : "null argument";
+    return -1;
+  }
+  h2v_ctx* fail = nullptr;
+  bool all_ok = false;
+  const int rc = mix_statuses(mx, true, status, &all_ok, &fail);  // (before fail is read)
+  return mix_report(mx, rc, fail);
+}
+
+static int mix_verify_shard_impl(h2v_mix* mx, const uint32_t* global_counts, uint64_t global_base, uint32_t n, const uint8_t* proofs,
+                                 const uint64_t* proof_off, const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars,
+                                 uint64_t seed, uint32_t root, uint8_t* status, int* verdict, h2v_ctx** fail) {
+  h2v_ctx* ctx = mx->m[0];
+  const h2v_ctx::Comm& cm = ctx->comm;
+  std::vector<u32> local;
+  u32 max_shard = 0;
+  if (!verdict) {
+    mx->err = "null argument";
+    return -1;
+  }
+  int rc = mix_shard_args(mx, global_counts, global_base, n, proof_off, inst_off, status, local, &max_shard);
+  if (rc) return rc;
+  if (!cm.ready || root >= cm.lay.world) {
+    mx->err = "sharded exchange: the lead member (member 0) needs h2v_comm_init + h2v_comm_connect, and root < world";
+    return -1;
+  }
+  const u32 sets = mix_count_sets(mx, global_counts);
+  if (sets > cm.lay.max_groups) {
+    mx->err = "sharded exchange: the lead's channel takes " + std::to_string(cm.lay.max_groups) + " partials per rank, this batch has " +
+              std::to_string(sets) + " bucket sets (h2v_comm_init with max_groups >= the params classes with proofs)";
+    return -1;
+  }
+  rc = mix_upload(mx, local.data(), global_counts, global_base, max_shard, proofs, proof_off, instances, inst_off, rlc_scalars, seed, fail);
+  if (rc) return rc;
+  *fail = ctx;
+  CKC(cudaSetDevice(ctx->device));
+  CKC(comm_next_launch(ctx, root));
+  if ((rc = mix_run(mx, RUN_XCHG | (root == cm.lay.rank ? RUN_ROOT : 0), fail)) != 0) return rc;
+  mix_mark_ran(mx);
+  *fail = ctx;
+  u32 all = 0;
+  if ((rc = read_verdicts(ctx, &all, true, 1)) != 0) return rc;
+  mx->xchg_root = root == cm.lay.rank;
+  bool all_ok = false;
+  if ((rc = mix_statuses(mx, !all, status, &all_ok, fail)) != 0) return rc;
+  *verdict = (int)all;
+  return 0;
+}
+
+int h2v_mix_verify_shard(h2v_mix* mx, const uint32_t* global_counts, uint64_t global_base, uint32_t n, const uint8_t* proofs, const uint64_t* proof_off,
+                         const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint32_t root, uint8_t* status,
+                         int* verdict) {
+  if (!mx) return -1;
+  NvtxRange nv_("h2v:mix_shard");
+  mx->err.clear();
+  h2v_ctx* fail = nullptr;
+  const int rc = mix_verify_shard_impl(mx, global_counts, global_base, n, proofs, proof_off, instances, inst_off, rlc_scalars, seed, root, status,
+                                       verdict, &fail);
+  return mix_report(mx, rc, fail);
+}
+
+static int mix_comm_accum_impl(h2v_mix* mx, uint8_t* batch_accum) {
+  if (!batch_accum || !mx->xchg_root) {
+    mx->err = batch_accum ? "the last launch set of this mix was not an exchange with this rank as its root" : "null argument";
+    return -1;
+  }
+  h2v_ctx* ctx = mx->m[0];
+  const MsmGeom& g = mx->geom;
+  const u32 npts = g.W[0] + g.W[1];
+  std::vector<u8> acc(128 * (size_t)mx->sets);
+  CKC(cudaSetDevice(ctx->device));
+  FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {0, g.W[0]}};
+  for (u32 st = 0; st < mx->sets; st++) {  // the root's summed window sums of every bucket set (lead's d_wsums_fin)
+    k_fold_accum<<<1, 32, 0, ctx->stream>>>(fa, ctx->d_wsums_fin.as<G1Jac>() + (size_t)st * npts, ctx->d_acc_bytes.as<u8>() + 128 * (size_t)st);
+    LAUNCH_CHECK();
+  }
+  CKC(cudaMemcpyAsync(acc.data(), ctx->d_acc_bytes.p, acc.size(), cudaMemcpyDeviceToHost, ctx->stream));
+  CKC(ctx_sync(ctx));
+  mix_class_accum(mx, acc.data(), batch_accum);
+  return 0;
+}
+
+int h2v_mix_comm_last_batch_accum(h2v_mix* mx, uint8_t* batch_accum) {
+  if (!mx) return -1;
+  mx->err.clear();
+  return mix_report(mx, mix_comm_accum_impl(mx, batch_accum), mx->m[0]);
 }
 
 // ---- persistent accumulators: the reference's AccumulatorStrategy as a value that lives across calls ---------------

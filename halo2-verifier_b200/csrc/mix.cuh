@@ -102,6 +102,39 @@ inline u32 mix_layout(u32 members, const u32* n, const u32* P, const u32* n_mo, 
   return count;
 }
 
+// Sharded mixed batches: a rank owns proofs [base, base + n) of the member-major concatenation of global_counts[members]
+// proofs.  local[m] = how many of them belong to member m (a range may start or end inside a member).  False when the range
+// is empty or runs past the global batch.
+inline bool mix_shard_counts(u32 members, const u32* global_counts, unsigned long long base, u32 n, u32* local) {
+  unsigned long long N = 0, lo = 0;
+  for (u32 m = 0; m < members; m++) N += global_counts[m];
+  if (n == 0 || base + n > N) return false;
+  const unsigned long long hi = base + n;
+  for (u32 m = 0; m < members; m++) {
+    const unsigned long long a = lo, b = lo + global_counts[m];  // member m's global range [a, b)
+    const unsigned long long s = a > base ? a : base, e = b < hi ? b : hi;
+    local[m] = e > s ? (u32)(e - s) : 0u;
+    lo = b;
+  }
+  return true;
+}
+
+// Term counts per channel from which every rank of a sharded mix chooses its window geometry: a bound that depends only on
+// what all ranks share (the member shapes, global_counts and the largest shard max_shard), never on the rank's own member
+// composition.  right >= sum of n_m P_m + Sh_m over any rank's members with proofs (n_m summing to <= max_shard), left likewise.
+inline void mix_shard_bound(u32 members, const u32* P, const u32* n_mo, const u32* Sh, const u32* global_counts, u32 max_shard,
+                            unsigned long long* right, unsigned long long* left) {
+  u32 maxP = 0, maxM = 0;
+  unsigned long long shared = 0;
+  for (u32 m = 0; m < members; m++) {
+    if (P[m] > maxP) maxP = P[m];
+    if (n_mo[m] > maxM) maxM = n_mo[m];
+    if (global_counts[m]) shared += Sh[m];
+  }
+  *right = (unsigned long long)max_shard * maxP + shared;
+  *left = (unsigned long long)max_shard * maxM;
+}
+
 // segment of term t: the last one whose first term is <= t (seg[0].t0 = 0, t0 ascending)
 H2V_HD u32 mix_segment(const MixSeg* seg, u32 count, u32 t) {
   u32 lo = 0, hi = count;

@@ -174,6 +174,58 @@ def verify_batch_sharded(bv, proofs, instances, rank: int, world: int, rlc_scala
     return ok, status
 
 
+def mixed_shard_counts(global_counts, base: int, n: int) -> List[int]:
+    """proofs per member of the range [base, base + n) of the member-major concatenation of global_counts proofs"""
+    out, lo = [], 0
+    for c in global_counts:
+        out.append(max(0, min(lo + c, base + n) - max(lo, base)))
+        lo += c
+    return out
+
+
+def mixed_shard(global_counts, rank: int, world: int):
+    """`rank`'s share of a mixed batch of global_counts[m] proofs per member: (lo, hi) of the member-major concatenation
+    (shard_range over its N proofs) and, per member, the [lo_m, hi_m) indices into that member's own proof list."""
+    lo, hi = shard_range(sum(global_counts), rank, world)
+    per, start = [], 0
+    for c, k in zip(global_counts, mixed_shard_counts(global_counts, lo, hi - lo)):
+        first = min(max(lo - start, 0), c)
+        per.append((first, first + k))
+        start += c
+    return (lo, hi), per
+
+
+def verify_mixed_batch_sharded(mix, proofs_per_member, instances_per_member, rank: int, world: int, rlc_scalars=None, seed=None, key=None,
+                               root: int = 0, group=None):
+    """A mixed batch (the whole description on every rank, or at least this rank's share at the right indices) split over the
+    ranks as mixed_shard does: each rank folds its share with globally defined coefficients, `root` runs the one pairing check
+    (through the device-side exchange when mix.comm_ready, otherwise a library gather of the device-resident partials), and
+    a rejection is attributed per proof by every rank inside its share.  Returns (global verdict, this rank's statuses per member)."""
+    global_counts = [len(p) for p in proofs_per_member]
+    (lo, hi), per = mixed_shard(global_counts, rank, world)
+    hint = max(b - a for a, b in (shard_range(sum(global_counts), r, world) for r in range(world)))  # common window geometry
+    proofs = [p[a:b] for p, (a, b) in zip(proofs_per_member, per)]
+    insts = [i[a:b] for i, (a, b) in zip(instances_per_member, per)]
+    rlc_scalars, seed, key = _randomness(rlc_scalars, seed, key, world, group)
+    if getattr(mix, "comm_ready", False):
+        return mix.verify_shard(proofs, insts, global_counts, lo, root, rlc_scalars=rlc_scalars, seed=seed, key=key, shard_hint=hint)
+    dev = _pg_device(group) if world > 1 else torch.device("cuda", torch.cuda.current_device())
+    part = torch.empty(mix.partial_bytes(global_counts), dtype=torch.uint8, device=dev)
+    status, _ = mix.accumulate_shard(proofs, insts, global_counts, lo, rlc_scalars=rlc_scalars, seed=seed, key=key, shard_hint=hint,
+                                     partial_out=part.data_ptr())
+    parts = _gather_to_root(part, root, rank, world, group)
+    flag = torch.zeros(1, dtype=torch.int32, device=dev)
+    if rank == root:
+        ok, _ = mix.finalize(parts.data_ptr(), global_counts, want_batch_accum=False, n_partials=world)
+        flag[0] = 1 if ok else 0
+    if world > 1:
+        dist.broadcast(flag, src=root, group=group)
+    ok = bool(flag.item())
+    if not ok:
+        status = mix.attribute_shard(status)
+    return ok, status
+
+
 def split_group_partials(rank_blob: bytes, groups: int) -> List[bytes]:
     """One rank's output of a launch set with `groups` fold groups = `groups` consecutive partials."""
     assert len(rank_blob) % groups == 0

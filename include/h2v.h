@@ -278,8 +278,8 @@ int h2v_mix_verify(h2v_mix* mx, const uint32_t* counts, const uint8_t* proofs, c
  * mix); all classes together take at most 128 (channel, window-run) pairs, so more classes pair longer window runs.
  * h2v_mix_verify keeps its signature and semantics (statuses, attribution under each member's own params, fold
  * randomness) except batch_accum: classes x 128 B, the folded affine (L_p, R_p) of every class in class order; a class
- * with no proofs in the call gets all-zero bytes and adds nothing to the check.  Not combinable with fold groups, shards
- * or the device-side exchange, as for every mix. */
+ * with no proofs in the call gets all-zero bytes and adds nothing to the check.  Not combinable with fold groups, as for
+ * every mix; shards and the device-side exchange: see "sharded mixed batches" below. */
 #define H2V_MIX_MAX_PARAMS 8
 /* As h2v_mix_create, but members may hold different KZG params.  Members whose params agree on (g, g2, s_g2) (the comparison
  * h2v_mix_create makes) form one params class; classes are numbered by first appearance in member order (member 0 is in
@@ -289,6 +289,52 @@ int h2v_mix_create_multi_params(h2v_mix** out, h2v_ctx* const* members, uint32_t
 /* class_of[m] = params class of member m (capacity >= n_members); returns the number of classes (1 for a mix of
  * h2v_mix_create), -1 on a null argument or a short array */
 int h2v_mix_params_classes(const h2v_mix* mx, uint32_t* class_of, uint32_t capacity);
+
+/* ---- sharded mixed batches: one mixed batch split over the GPUs of a box, one pairing check -------------------------------
+ * Every rank holds a mix of its own member contexts (on its own GPU) with the SAME member list on every rank: the same VKs,
+ * options and params classes in the same order.  The global batch is what h2v_mix_verify would take: the member-major
+ * concatenation of global_counts[m] proofs, N = sum global_counts.  A rank owns the contiguous range [global_base, global_base
+ * + n) of it (a range may start or end inside a member, or lie inside one member) and passes only its proofs, member-major,
+ * as for h2v_mix_verify; the library derives its per-member counts.  Fold randomness as h2v_mix_verify over the GLOBAL
+ * indices: rlc_scalars has N entries, the mix's key (h2v_mix_set_rlc_key) and the test seed expand by global index; with
+ * neither, each rank draws its own key from the OS (sound, but the folded (L, R) then depend on the sharding).  With caller
+ * scalars or a shared key the folded (L, R) equal, bit for bit, those of one h2v_mix_verify over the concatenation, for
+ * every world size and split.
+ * Bucket sets: one per params class with proofs in global_counts, in class order.  Every rank emits one partial
+ * (H2V_PARTIAL_BYTES, as h2v_accumulate_shard's) per bucket set, also for a class without proofs on that rank (its window
+ * sums are the identity), so that partials line up [rank][set].  Window geometry: every rank chooses it from a bound all
+ * ranks share (the member shapes, global_counts and the largest shard), never from its own member composition; shards of
+ * unequal size need h2v_mix_set_shard_hint(largest shard) on every rank.
+ * Statuses (n bytes, this rank's proofs in member-major order) are final at accumulate time except that H2V_OK means
+ * "accumulated".  Refused before any device call, text in h2v_mix_last_error(mx), state unchanged: a null argument, N = 0,
+ * n = 0, global_base + n > N, a hint smaller than n, non-canonical or zero rlc_scalars, a member with a pending fold-group or
+ * shard-hint option; on the exchange also a lead without a connected channel, root >= world or max_groups < sets.  Partials
+ * of different window geometries give the "different window geometries" error of h2v_finalize.
+ *   h2v_mix_set_shard_hint      one-shot: window geometry of the next shard call as for shards of max_shard_proofs proofs
+ *   h2v_mix_partial_bytes       sets x H2V_PARTIAL_BYTES for this global batch (0 on a null argument)
+ *   h2v_mix_accumulate_shard    upload + every kernel up to the partials (host or device pointer) + statuses
+ *   h2v_mix_finalize            partials: n_partials ranks x sets blobs, [rank][set], host or device pointer; sums them and runs
+ *                               ONE multi-pairing check over all sets (one set: the plain 2-pair check).  Works on a mix that
+ *                               processed no shard itself (geometry from the partials' headers, sets from global_counts).
+ *                               verdict: 1 = the check accepts; batch_accum: optional, classes x 128 B as h2v_mix_verify's
+ *   h2v_mix_attribute_shard     after a rejection: every member's proofs of the shard this mix last processed are re-checked
+ *                               on their own (poly/strategy.rs:26-30); status (n bytes) out
+ *   h2v_mix_verify_shard        the end-to-end call of one rank through the device-side exchange over the LEAD member's
+ *                               channel (h2v_comm_init with max_groups >= sets + h2v_comm_connect on member 0): upload, the
+ *                               launch set (one CUDA graph: partials -> the root's window, the root's sum and one check,
+ *                               verdict -> every rank), attribution on rejection, statuses.  verdict: the global check
+ *   h2v_mix_comm_last_batch_accum   root only: classes x 128 B folded (L_p, R_p) of the last exchange launch set */
+int h2v_mix_set_shard_hint(h2v_mix* mx, uint32_t max_shard_proofs);
+size_t h2v_mix_partial_bytes(const h2v_mix* mx, const uint32_t* global_counts);
+int h2v_mix_accumulate_shard(h2v_mix* mx, const uint32_t* global_counts, uint64_t global_base, uint32_t n, const uint8_t* proofs,
+                             const uint64_t* proof_off, const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars,
+                             uint64_t seed, uint8_t* status, uint8_t* partial);
+int h2v_mix_finalize(h2v_mix* mx, const uint32_t* global_counts, uint32_t n_partials, const uint8_t* partials, uint8_t* batch_accum, int* verdict);
+int h2v_mix_attribute_shard(h2v_mix* mx, uint8_t* status);
+int h2v_mix_verify_shard(h2v_mix* mx, const uint32_t* global_counts, uint64_t global_base, uint32_t n, const uint8_t* proofs, const uint64_t* proof_off,
+                         const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint32_t root, uint8_t* status,
+                         int* verdict);
+int h2v_mix_comm_last_batch_accum(h2v_mix* mx, uint8_t* batch_accum);
 
 /* ---- persistent accumulators: AccumulatorStrategy as a value that lives across calls ------------------------------------
  * The reference's AccumulatorStrategy (poly/kzg/strategy.rs:125-140) is fed proofs through any number of verify_proof calls,
