@@ -265,8 +265,9 @@ static constexpr u32 RLC_NT = 256;
 // those with index in [base, base + n) to coef + b * n.
 //   fold groups (subs = 1, group_stride = count, offset = 0): block g scans the coefficients of its own global batch and
 //     writes the n of this rank's shard of it
-//   attribution (count = n = m, base = 0, subs = sub-batches per fold group, offset = gbase): block b scans the m
-//     coefficients of sub-batch b % subs of fold group b / subs: the fold restarts inside every sub-batch
+//   attribution (count = n = m, base = 0, subs = sub-batches per fold group, group_stride = proofs per group, offset = 0,
+//     r = the re-fold's own scalars, one per proof of the shard): block b scans the m coefficients of sub-batch b % subs of
+//     fold group b / subs: the fold restarts inside every sub-batch
 __global__ void __launch_bounds__(RLC_NT) k_rlc_scan(const Fr* r, u64 count, u64 base, u32 n, Fr* coef, u32 subs, u64 group_stride, u64 offset) {
   pdl_prologue();
   TlScope tl_(14, coef);
@@ -860,7 +861,8 @@ __global__ void __launch_bounds__(128) k_pp_reduce(PlanView pv, u32 n, const G1J
 
 // ---- attribution of a rejected fold (reference contract poly/strategy.rs:26-30: "re-process the proofs separately")
 // Level 1 re-folds the rejected group in sub-batches of ATTR_SUB proofs through the bucket MSM (the fold restarts inside
-// every sub-batch, so each is an AccumulatorStrategy run of its own) and checks every sub-batch with one 2-pair
+// every sub-batch, so each is an AccumulatorStrategy run of its own, with coefficients drawn for the attribution and
+// independent of the batch's r_i) and checks every sub-batch with one 2-pair
 // pairing; level 2 forms the accumulators of the proofs of rejected sub-batches only and checks each proof alone
 // (SingleStrategy semantics, strategy.rs:164-176).  With 1 % bad proofs level 2 sees ~15 % of the batch.
 static constexpr u32 ATTR_SUB = 16;
@@ -1260,13 +1262,13 @@ struct h2v_ctx {
   } mb, ab;
   DevBuf d_plan, d_proofs, d_proof_off, d_inst, d_inst_off, d_ncols, d_col_len, d_pts, d_bad, d_status, d_vals, d_scratch, d_right,
       d_shared, d_left, d_rlc_bytes, d_r, d_acc_bytes, d_verdict, d_partials, d_pp_prod, d_pp_lr, d_pp_bytes, d_hook, d_chal, d_flush, d_M, d_partial_out,
-      d_wsums_fin, d_sub_pairs, d_sub_verdict, d_sub_M, d_gsums, d_ptsc, d_rho;
+      d_wsums_fin, d_sub_pairs, d_sub_verdict, d_sub_M, d_gsums, d_ptsc, d_rho, d_attr_r;
   const G2Line* d_lines() const { return lines_cur >= 0 ? lines[lines_cur].buf.as<G2Line>() : nullptr; }
   std::vector<DevBuf*> all_bufs() {
     std::vector<DevBuf*> v = {&d_plan, &d_proofs, &d_proof_off, &d_inst, &d_inst_off, &d_ncols, &d_col_len, &d_pts, &d_bad, &d_status, &d_vals, &d_scratch,
                               &d_right, &d_shared, &d_left, &d_rlc_bytes, &d_r, &d_acc_bytes, &d_verdict, &d_partials, &d_pp_prod, &d_pp_lr, &d_pp_bytes,
                               &d_hook, &d_chal, &d_flush, &d_M, &d_partial_out, &d_wsums_fin, &d_sub_pairs, &d_sub_verdict, &d_sub_M, &d_gsums, &d_ptsc, &d_rho,
-                              &lines[0].buf, &lines[1].buf, &lines[2].buf, &lines[3].buf};
+                              &d_attr_r, &lines[0].buf, &lines[1].buf, &lines[2].buf, &lines[3].buf};
     for (MsmBufs* m : {&mb, &ab})
       for (DevBuf* d : {&m->coef, &m->shared_sum, &m->dig, &m->hist, &m->off, &m->cursor, &m->order, &m->sorted, &m->buckets, &m->wsums, &m->partials_msm, &m->tiles})
         v.push_back(d);
@@ -2583,7 +2585,17 @@ static int attribute_impl(h2v_ctx* ctx) {
     G1Jac* sub_pairs = (G1Jac*)(((size_t)(sv + SG) + 15) & ~(size_t)15);
     CKC(cudaMemsetAsync(ctx->ab.hist.p, 0, 4 * ((size_t)sg.nb() * sg.G + 2 * SIZE_BINS), s));
     CKC(cudaMemsetAsync(sv, 1, 4 * (size_t)SG, s));  // non-zero = accepted: sub-batches of accepted groups are never checked
-    KLAUNCH_P(false, k_rlc_scan, SG, RLC_NT, 0, s, ctx->d_r.as<Fr>(), (u64)msub, (u64)0, msub, ctx->ab.coef.as<Fr>(), subs, ctx->gcount, ctx->gbase);
+    // The re-fold draws its own coefficients from a fresh key.  With the batch's r_i (caller scalars or the public test seed)
+    // a cancellation the caller's scalars built into the batch fold, e.g. c_2 = -c_3 for two equal invalid proofs, would
+    // repeat inside the sub-batch, which would then accept and report both proofs H2V_OK.
+    RlcKey key{};
+    if (os_entropy(&key, sizeof(key)) != 0) {
+      ctx->err = "no OS entropy for the attribution coefficients (getrandom failed)";
+      return -2;
+    }
+    CKC(ctx->d_attr_r.ensure(sizeof(Fr) * (size_t)N));
+    KLAUNCH_P(false, k_rlc_expand, cdiv(N, 128), 128, 0, s, (u64)N, (u64)0, (const u8*)nullptr, true, key, ctx->d_attr_r.as<Fr>());
+    KLAUNCH_P(false, k_rlc_scan, SG, RLC_NT, 0, s, ctx->d_attr_r.as<Fr>(), (u64)msub, (u64)0, msub, ctx->ab.coef.as<Fr>(), subs, (u64)g.n, (u64)0);
     {
       const bool pdl = ctx->use_pdl;
       ctx->use_pdl = false;

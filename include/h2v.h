@@ -113,7 +113,10 @@ int h2v_verify_proof(h2v_ctx* ctx, const uint8_t* proof, size_t proof_len, const
                      size_t n_inst, uint8_t* status);
 
 /* verify_proofs_batch: AccumulatorStrategy::process per proof + finalize (strategy.rs:125-140), and on
- * a failed batch the per-proof re-check the reference prescribes (poly/strategy.rs:26-30).
+ * a failed batch the per-proof re-check the reference prescribes (poly/strategy.rs:26-30).  The statuses after a
+ * rejected fold are those of that separate re-check of every proof: they do not depend on the fold scalars (the
+ * re-check draws its own coefficients from the OS), so no choice of rlc_scalars can hide an invalid proof from it.
+ * The same holds for every entry point that attributes a rejection (fold groups, shards, mixed batches).
  *   proofs / proof_off    concatenated proof bytes, n+1 byte offsets
  *   instances / inst_off  concatenated 32-byte LE canonical Fr, n+1 offsets in units of scalars;
  *                         per proof: columns concatenated, equal length (see h2v_batch_set_columns).  A value >= r
@@ -122,7 +125,8 @@ int h2v_verify_proof(h2v_ctx* ctx, const uint8_t* proof, size_t proof_len, const
  *                         with c_j = prod_{i>j} r_i, the reference's convention (SURVEY.md 3.2).  A zero or
  *                         non-canonical r_i (it would zero c_j of every earlier proof) is refused before any
  *                         device call: -1, "fold scalars must be canonical and non-zero".  The same holds for
- *                         every entry point that takes rlc_scalars.
+ *                         every entry point that takes rlc_scalars.  They define the batch fold and the folded
+ *                         (L, R) only: per-proof statuses never depend on them.
  *   status                n bytes out
  *   challenges            optional out, n x C x 32 B canonical, squeeze order            (parity hook)
  *   accum                 optional out, n x 2 x 64 B per-proof affine (L_j, R_j), x|y LE canonical,
