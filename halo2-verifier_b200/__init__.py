@@ -180,6 +180,8 @@ def load_library():
     lib.h2v_mix_verify_shard.argtypes = [ctypes.c_void_p, u32p, ctypes.c_uint64, ctypes.c_uint32, u8p, u64p, u8p, u64p, u8p, ctypes.c_uint64,
                                          ctypes.c_uint32, u8p, ctypes.POINTER(ctypes.c_int)]
     lib.h2v_mix_comm_last_batch_accum.argtypes = [ctypes.c_void_p, u8p]
+    lib.h2v_mix_verify_groups.argtypes = [ctypes.c_void_p, ctypes.c_uint32, u32p, u8p, u64p, u8p, u64p, u8p, ctypes.c_uint64, u8p, u8p, u8p,
+                                          ctypes.POINTER(ctypes.c_int)]
     lib.h2v_acc_create.argtypes = [ctypes.POINTER(ctypes.c_void_p), ctypes.c_void_p, ctypes.c_uint32]
     lib.h2v_acc_destroy.argtypes = [ctypes.c_void_p]
     lib.h2v_acc_destroy.restype = None
@@ -206,7 +208,7 @@ EXPORTED_SYMBOLS = (
     "h2v_mix_create", "h2v_mix_destroy", "h2v_mix_last_error", "h2v_mix_set_rlc_key", "h2v_mix_verify",
     "h2v_mix_create_multi_params", "h2v_mix_params_classes",
     "h2v_mix_set_shard_hint", "h2v_mix_partial_bytes", "h2v_mix_accumulate_shard", "h2v_mix_finalize", "h2v_mix_attribute_shard",
-    "h2v_mix_verify_shard", "h2v_mix_comm_last_batch_accum",
+    "h2v_mix_verify_shard", "h2v_mix_comm_last_batch_accum", "h2v_mix_verify_groups",
     "h2v_acc_create", "h2v_acc_destroy", "h2v_acc_last_error", "h2v_acc_set_rlc_key", "h2v_acc_absorb", "h2v_acc_finalize", "h2v_acc_get",
     "h2v_acc_merge", "h2v_acc_reset", "h2v_ctx_create_aggregation", "h2v_batch_set_agg_scalar",
 )
@@ -605,6 +607,15 @@ class MixedBatchResult:
         return [[None if s == 0 else STATUS_ERRORS[s]() for s in st] for st in self.status]
 
 
+@dataclass
+class MixedGroupsResult:
+    status: List[List[List[int]]]  # status[q][m]: member m's proofs of group q
+    group_verdicts: List[bool]  # group q: its check accepted and every proof of it is valid
+    verdict: bool  # every group accepted
+    # per group: its classes x 128 B folded (L_p, R_p), as MixedBatchResult.batch_accum for that group alone
+    batch_accum: Optional[List[bytes]] = None
+
+
 class MixedBatchVerifier:
     """Proofs of several BatchVerifiers (verifying keys, SHPLONK or GWC, Blake2b or Keccak) folded into ONE MSM and ONE
     pairing check: the reference's AccumulatorStrategy fed proofs of different VKs under one set of KZG params
@@ -661,6 +672,65 @@ class MixedBatchVerifier:
         verdict = ctypes.c_int(0)
         self._check(self.lib.h2v_mix_verify(self._mx, self._u32(counts), *packed[:4], rlc, int(seed), status, bacc, ctypes.byref(verdict)))
         return MixedBatchResult(self._split(list(status), counts), bool(verdict.value), bacc.raw if bacc is not None else None)
+
+    def verify_groups(self, groups, rlc_scalars: Optional[Sequence[int]] = None, seed=None, key=None, want_batch_accum=False,
+                      agg_scalar=None) -> MixedGroupsResult:
+        """Independent mixed batches in one launch set (include/h2v.h "grouped mixed batches"): groups[q] = (proofs_per_member,
+        instances_per_member) as for verify_batch.  Each group is folded, checked and judged on its own; rlc_scalars has one
+        entry per proof in call order (group 0's member-major concatenation, then group 1's, ...), so group q's slice is what
+        verify_batch takes for group q alone."""
+        M = len(self.members)
+        groups = list(groups)
+        for q, (ppm, ipm) in enumerate(groups):
+            if len(ppm) != M or len(ipm) != M:
+                raise ValueError(f"group {q}: one proof list and one instance list per member")
+            for m in range(M):
+                if len(ppm[m]) != len(ipm[m]):
+                    raise ValueError(f"group {q}, member {m}: {len(ppm[m])} proofs, {len(ipm[m])} instance lists")
+        counts = [len(g[0][m]) for g in groups for m in range(M)]
+        n = sum(counts)
+        if not groups or n == 0:
+            raise ValueError("a grouped mixed batch needs at least one group with proofs")
+        if rlc_scalars is not None and len(rlc_scalars) != n:
+            raise ValueError("one fold scalar per proof of the call")
+        # one _pack per member over its proofs of every group (its ragged-column layout describes its whole upload)
+        per_member = []
+        for m, bv in enumerate(self.members):
+            proofs = [p for g in groups for p in g[0][m]]
+            insts = [i for g in groups for i in g[1][m]]
+            per_member.append(bv._pack(proofs, insts) if proofs else None)
+        pparts, iparts, poffs, ioffs, keep = [], [], [0], [0], []
+        first = [0] * M  # next proof of member m in its packed upload
+        for q in range(len(groups)):
+            for m in range(M):
+                c = counts[q * M + m]
+                if not c:
+                    continue
+                pbytes, poff, ibytes, ioff, k = per_member[m]
+                keep += k
+                a = first[m]
+                pparts.append(pbytes[poff[a]:poff[a + c]])
+                iparts.append(ibytes[32 * ioff[a]:32 * ioff[a + c]])
+                poffs += [poffs[-1] + poff[a + j + 1] - poff[a] for j in range(c)]
+                ioffs += [ioffs[-1] + ioff[a + j + 1] - ioff[a] for j in range(c)]
+                first[m] += c
+        ppm_all = [[p for g in groups for p in g[0][m]] for m in range(M)]
+        rlc, seed = self._randomness(ppm_all, rlc_scalars, seed, key, agg_scalar)
+        G = len(groups)
+        status = (ctypes.c_uint8 * n)()
+        gverd = (ctypes.c_uint8 * G)()
+        bacc = ctypes.create_string_buffer(128 * self.n_classes * G) if want_batch_accum else None
+        verdict = ctypes.c_int(0)
+        self._check(self.lib.h2v_mix_verify_groups(self._mx, G, self._u32(counts), b"".join(pparts), (ctypes.c_uint64 * (n + 1))(*poffs),
+                                                   b"".join(iparts), (ctypes.c_uint64 * (n + 1))(*ioffs), rlc, int(seed), status, gverd, bacc,
+                                                   ctypes.byref(verdict)))
+        st, out = list(status), []
+        for q in range(G):
+            out.append(self._split(st[:sum(counts[q * M:(q + 1) * M])], counts[q * M:(q + 1) * M]))
+            st = st[sum(counts[q * M:(q + 1) * M]):]
+        per = 128 * self.n_classes
+        return MixedGroupsResult(out, [bool(v) for v in gverd], bool(verdict.value),
+                                 [bacc.raw[q * per:(q + 1) * per] for q in range(G)] if bacc is not None else None)
 
     @staticmethod
     def _u32(values):

@@ -313,6 +313,55 @@ __global__ void __launch_bounds__(256) k_shared_reduce(u32 n, u32 N, u32 Sh, con
   if (t == 0) shared_sum[grp * Sh + b] = sh[0].to_canonical();
 }
 
+// Fold coefficients of a mixed batch, every group in one launch: block q runs the suffix scan of k_rlc_scan over group q's
+// call indices [grange[q], grange[q + 1]) (the fold restarts at every group boundary, c_i = prod_{i' in group q, i' > i} r_i')
+// and writes c_i into the coefficient array of the member that owns proof i: segment seg[q * members + m] holds call indices
+// [call0, call0 + n) at [j0, j0 + n) of member m's arrays.  A sharded mix is one group over the global batch whose segments
+// cover this rank's range only; the other indices are scanned, not written.
+__global__ void __launch_bounds__(RLC_NT) k_rlc_scan_groups(const Fr* r, const u32* grange, const MixSeg* seg, u32 members) {
+  pdl_prologue();
+  TlScope tl_(14, r);
+  __shared__ Fr sh[RLC_NT];
+  const u32 q = blockIdx.x, t = threadIdx.x;
+  const u64 g0 = grange[q], count = (u64)grange[q + 1] - g0;
+  seg += (size_t)q * members;
+  const u64 m = (count + RLC_NT - 1) / RLC_NT;
+  const u64 lo = (u64)t * m < count ? g0 + (u64)t * m : g0 + count, hi = lo + m < g0 + count ? lo + m : g0 + count;
+  Fr p = Fr::one();
+  for (u64 i = lo; i < hi; i++) p = p * r[i];
+  sh[t] = p;
+  __syncthreads();
+  for (u32 d = 1; d < RLC_NT; d <<= 1) {  // inclusive suffix products
+    Fr v = sh[t];
+    const bool act = t + d < RLC_NT;
+    Fr o = act ? sh[t + d] : Fr::one();
+    __syncthreads();
+    if (act) sh[t] = v * o;
+    __syncthreads();
+  }
+  mix_scan_chunk(r, lo, hi, t + 1 < RLC_NT ? sh[t + 1] : Fr::one(), seg, members);
+}
+
+// k_shared_reduce per segment of a mixed batch: block (s, b) writes seg[s].shared_sum[b] = sum over the segment's proofs of
+// c_j * shared[b][j] (zero for a segment without proofs)
+__global__ void __launch_bounds__(256) k_shared_reduce_seg(const MixSeg* seg) {
+  pdl_prologue();
+  const MixSeg& sg = seg[blockIdx.x];
+  const u32 b = blockIdx.y, t = threadIdx.x;
+  if (b >= sg.Sh) return;
+  TlScope tl_(15, sg.shared_sum);
+  __shared__ Fr sh[256];
+  Fr acc = Fr::zero();
+  for (u32 j = t; j < sg.n; j += 256) acc = acc + sg.shared[(size_t)b * sg.stride + sg.j0 + j] * sg.coef[sg.j0 + j];
+  sh[t] = acc;
+  __syncthreads();
+  for (u32 d = 128; d > 0; d >>= 1) {
+    if (t < d) sh[t] = sh[t] + sh[t + d];
+    __syncthreads();
+  }
+  if (t == 0) sg.shared_sum[b] = sh[0].to_canonical();
+}
+
 // signed c-bit digits of a little-endian magnitude kk[0..NL) (bits beyond NL limbs are zero), negated when `neg`; row of
 // the digit table + bucket histogram of the term's channel
 template <int NL>
@@ -1262,13 +1311,16 @@ struct h2v_ctx {
   } mb, ab;
   DevBuf d_plan, d_proofs, d_proof_off, d_inst, d_inst_off, d_ncols, d_col_len, d_pts, d_bad, d_status, d_vals, d_scratch, d_right,
       d_shared, d_left, d_rlc_bytes, d_r, d_acc_bytes, d_verdict, d_partials, d_pp_prod, d_pp_lr, d_pp_bytes, d_hook, d_chal, d_flush, d_M, d_partial_out,
-      d_wsums_fin, d_sub_pairs, d_sub_verdict, d_sub_M, d_gsums, d_ptsc, d_rho, d_attr_r;
+      d_wsums_fin, d_sub_pairs, d_sub_verdict, d_sub_M, d_gsums, d_ptsc, d_rho, d_attr_r, d_attr_mask;
+  // one-shot for the next attribute_impl (a grouped mixed batch): per proof of the upload, non-zero = its group accepted
+  // (not re-checked); empty = every proof is looked at
+  std::vector<u32> attr_accepted;
   const G2Line* d_lines() const { return lines_cur >= 0 ? lines[lines_cur].buf.as<G2Line>() : nullptr; }
   std::vector<DevBuf*> all_bufs() {
     std::vector<DevBuf*> v = {&d_plan, &d_proofs, &d_proof_off, &d_inst, &d_inst_off, &d_ncols, &d_col_len, &d_pts, &d_bad, &d_status, &d_vals, &d_scratch,
                               &d_right, &d_shared, &d_left, &d_rlc_bytes, &d_r, &d_acc_bytes, &d_verdict, &d_partials, &d_pp_prod, &d_pp_lr, &d_pp_bytes,
                               &d_hook, &d_chal, &d_flush, &d_M, &d_partial_out, &d_wsums_fin, &d_sub_pairs, &d_sub_verdict, &d_sub_M, &d_gsums, &d_ptsc, &d_rho,
-                              &d_attr_r, &lines[0].buf, &lines[1].buf, &lines[2].buf, &lines[3].buf};
+                              &d_attr_r, &d_attr_mask, &lines[0].buf, &lines[1].buf, &lines[2].buf, &lines[3].buf};
     for (MsmBufs* m : {&mb, &ab})
       for (DevBuf* d : {&m->coef, &m->shared_sum, &m->dig, &m->hist, &m->off, &m->cursor, &m->order, &m->sorted, &m->buckets, &m->wsums, &m->partials_msm, &m->tiles})
         v.push_back(d);
@@ -1685,6 +1737,8 @@ static cudaError_t preload_kernels() {
   H2V_PRELOAD(k_rlc_expand);
   H2V_PRELOAD(k_rlc_scan);
   H2V_PRELOAD(k_shared_reduce);
+  H2V_PRELOAD(k_rlc_scan_groups);
+  H2V_PRELOAD(k_shared_reduce_seg);
   H2V_PRELOAD(k_msm_digits<SingleVkTerms>);
   H2V_PRELOAD(k_msm_digits<MixTerms>);
   H2V_PRELOAD(k_scan_tiles);
@@ -2128,8 +2182,14 @@ static cudaError_t ensure_msm_bufs(const MsmGeom& g, h2v_ctx::MsmBufs& B, u32 n_
   return B.partials_msm.ensure(sizeof(G1Jac) * (nb / g.m));
 }
 
+// Host ranges that make up a batch's proof bytes and instance bytes, in order (a member of a grouped mixed batch: its proofs
+// of each group); null = the contiguous `proofs` / `instances`.
+struct UploadPieces {
+  std::vector<std::pair<const u8*, size_t>> proofs, instances;
+};
+
 static int upload_impl(h2v_ctx* ctx, u32 n, const u8* proofs, const u64* proof_off, const u8* instances, const u64* inst_off,
-                       const u8* rlc, u64 seed, u64 gbase, u64 gcount) {
+                       const u8* rlc, u64 seed, u64 gbase, u64 gcount, const UploadPieces* pieces = nullptr) {
   if (!ctx) return -1;
   NvtxRange nv_("h2v:upload");
   ctx->ran = false;
@@ -2215,9 +2275,22 @@ static int upload_impl(h2v_ctx* ctx, u32 n, const u8* proofs, const u64* proof_o
   CKC(ctx->d_M.ensure(sizeof(E12) * (H2V_ATE_ITERS + MILLER_SEGS) * (size_t)g.G));
   CKC(ctx->d_verdict.ensure(4 * (size_t)g.G + 16));
   cudaStream_t s = ctx->stream;
-  CKC(cudaMemcpyAsync(ctx->d_proofs.p, proofs, pbytes, cudaMemcpyHostToDevice, s));
+  if (pieces) {
+    size_t o = 0;
+    for (const auto& pc : pieces->proofs) {
+      if (pc.second) CKC(cudaMemcpyAsync(ctx->d_proofs.as<u8>() + o, pc.first, pc.second, cudaMemcpyHostToDevice, s));
+      o += pc.second;
+    }
+    o = 0;
+    for (const auto& pc : pieces->instances) {
+      if (pc.second) CKC(cudaMemcpyAsync(ctx->d_inst.as<u8>() + o, pc.first, pc.second, cudaMemcpyHostToDevice, s));
+      o += pc.second;
+    }
+  } else {
+    CKC(cudaMemcpyAsync(ctx->d_proofs.p, proofs, pbytes, cudaMemcpyHostToDevice, s));
+    if (iscal) CKC(cudaMemcpyAsync(ctx->d_inst.p, instances, 32 * iscal, cudaMemcpyHostToDevice, s));
+  }
   CKC(cudaMemcpyAsync(ctx->d_proof_off.p, proof_off, 8 * (size_t)(n + 1), cudaMemcpyHostToDevice, s));
-  if (iscal) CKC(cudaMemcpyAsync(ctx->d_inst.p, instances, 32 * iscal, cudaMemcpyHostToDevice, s));
   CKC(cudaMemcpyAsync(ctx->d_inst_off.p, inst_off, 8 * (size_t)(n + 1), cudaMemcpyHostToDevice, s));
   ctx->has_ncols = ctx->opt_ncols != nullptr;
   ctx->has_col_len = ctx->opt_col_len != nullptr && hd.n_inst_cols;
@@ -2286,8 +2359,9 @@ static int upload_impl(h2v_ctx* ctx, u32 n, const u8* proofs, const u64* proof_o
 enum : int { RUN_PAIRING = 1, RUN_ACCUM = 2, RUN_PARTIAL = 4, RUN_XCHG = 8, RUN_ROOT = 16, RUN_ABSORB = 32 };
 // The per-proof stages of the current upload on the context's stream, up to the point where the MSM may start: fold
 // coefficients (auxiliary stream), instance checks, decompression, transcript replay, scalar stage, and the wait for the
-// coefficients.  Shared by a context's own batches (enqueue_batch) and the members of a mixed batch.
-static int enqueue_stages(h2v_ctx* ctx) {
+// coefficients.  Shared by a context's own batches (enqueue_batch) and the members of a mixed batch, whose coefficients the
+// mix computes (own_coef = false: no scan and no histogram of the member's own MSM).
+static int enqueue_stages(h2v_ctx* ctx, bool own_coef = true) {
   const PlanHeader& hd = ctx->hd;
   const u32 n = ctx->n;
   cudaStream_t s = ctx->stream;
@@ -2297,11 +2371,13 @@ static int enqueue_stages(h2v_ctx* ctx) {
   set_launch_class('N');
   if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[0], s));
   // c_j = prod_{i>j} r_i depends only on the coefficients: scanned on the auxiliary stream while the proofs are parsed
-  CKC(cudaEventRecord(ctx->ev_fork, s));
-  CKC(cudaStreamWaitEvent(ctx->stream_aux, ctx->ev_fork, 0));
-  CKC(cudaMemsetAsync(ctx->mb.hist.p, 0, 4 * ((size_t)nb + 2 * SIZE_BINS), ctx->stream_aux));  // bucket histogram | size histogram | size cursors
-  KLAUNCH_P(false, k_rlc_scan, g.G, RLC_NT, 0, ctx->stream_aux, ctx->d_r.as<Fr>(), ctx->gcount, ctx->gbase, g.n, ctx->mb.coef.as<Fr>(), 1u, ctx->gcount, (u64)0);
-  CKC(cudaEventRecord(ctx->ev_join, ctx->stream_aux));
+  if (own_coef) {
+    CKC(cudaEventRecord(ctx->ev_fork, s));
+    CKC(cudaStreamWaitEvent(ctx->stream_aux, ctx->ev_fork, 0));
+    CKC(cudaMemsetAsync(ctx->mb.hist.p, 0, 4 * ((size_t)nb + 2 * SIZE_BINS), ctx->stream_aux));  // bucket histogram | size histogram | size cursors
+    KLAUNCH_P(false, k_rlc_scan, g.G, RLC_NT, 0, ctx->stream_aux, ctx->d_r.as<Fr>(), ctx->gcount, ctx->gbase, g.n, ctx->mb.coef.as<Fr>(), 1u, ctx->gcount, (u64)0);
+    CKC(cudaEventRecord(ctx->ev_join, ctx->stream_aux));
+  }
   nvtxRangePushA("h2v:decompress");
   KLAUNCH(k_init, cdiv(n, 128), 128, 0, s, pv, n, ctx->d_inst_off.as<u64>(), ctx->has_ncols ? ctx->d_ncols.as<u32>() : nullptr,
                                       ctx->has_col_len ? ctx->d_col_len.as<u32>() : nullptr, ctx->d_status.as<u32>(), ctx->d_bad.as<u32>());
@@ -2352,7 +2428,7 @@ static int enqueue_stages(h2v_ctx* ctx) {
   nvtxRangePop();
   set_launch_class('N');
   if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[3], s));
-  CKC(cudaStreamWaitEvent(s, ctx->ev_join, 0));
+  if (own_coef) CKC(cudaStreamWaitEvent(s, ctx->ev_join, 0));
   return 0;
 }
 
@@ -2546,6 +2622,22 @@ static int attribute_impl(h2v_ctx* ctx) {
   cudaStream_t s = ctx->stream;
   PlanView pv = ctx->pv();
   const u32* gv = (ctx->verdicts_on_device && g.G > 1 && g.G * g.n == N) ? ctx->d_verdict.as<u32>() : nullptr;
+  u32 gsize = g.n;  // proofs per flag of gv
+  // grouped mixed batch: the per-proof flags of attr_accepted | one flag per level-1 sub-batch (accepted = all its proofs are)
+  std::vector<u32> mask;
+  mask.swap(ctx->attr_accepted);
+  if (!mask.empty()) {
+    const u32 ms = ATTR_SUB;
+    for (u32 b = 0; b * ms < N; b++) {
+      u32 all = 1;
+      for (u32 j = b * ms; j < std::min(N, (b + 1) * ms); j++) all &= mask[j] ? 1u : 0u;
+      mask.push_back(all);
+    }
+    CKC(ctx->d_attr_mask.ensure(4 * mask.size()));
+    CKC(cudaMemcpyAsync(ctx->d_attr_mask.p, mask.data(), 4 * mask.size(), cudaMemcpyHostToDevice, s));
+    gv = ctx->d_attr_mask.as<u32>();
+    gsize = 1;
+  }
   const u32 nbases = msm_points(hd) + hd.n_shared + msm_mo(hd);
   static constexpr u32 CHUNK = 1024;  // checks per pass: bounds the Miller scratch (E12[CHUNK][65] = 115 MB)
   MsmGeom unit{};
@@ -2569,6 +2661,7 @@ static int attribute_impl(h2v_ctx* ctx) {
   // ---- level 1: sub-batches of ATTR_SUB proofs through the bucket MSM, one 2-pair check each
   u32 msub = ATTR_SUB;
   if (const char* e = getenv("H2V_ATTR_SUB")) msub = (u32)atoi(e);  // (tuning: 0 = no sub-batch level)
+  if (!mask.empty() && msub != ATTR_SUB) msub = 0;  // (the sub-batch flags are built for ATTR_SUB)
   // (level 1 needs twice the term ids of the batch pass - two GLV halves per term - inside the 31-bit id space)
   if (msub >= 2 && g.n >= 4 * msub && g.n % msub == 0 &&
       2 * ((u64)N * (msm_points(hd) + msm_mo(hd)) + (u64)hd.n_shared * (N / msub)) < (1ull << 31)) {
@@ -2599,7 +2692,7 @@ static int attribute_impl(h2v_ctx* ctx) {
     {
       const bool pdl = ctx->use_pdl;
       ctx->use_pdl = false;
-      int mrc = enqueue_msm(ctx, sg, ctx->ab, s, gv, g.n);
+      int mrc = enqueue_msm(ctx, sg, ctx->ab, s, mask.empty() ? gv : gv + N, mask.empty() ? g.n : msub);
       ctx->use_pdl = pdl;
       if (mrc) return mrc;
     }
@@ -2609,7 +2702,8 @@ static int attribute_impl(h2v_ctx* ctx) {
     if (trace_on()) { ctx_sync(ctx); trace(ctx, "attr: window combine done"); }
     for (u32 base = 0; base < SG; base += CHUNK) {
       const u32 cnt = std::min(CHUNK, SG - base);
-      int prc = launch_pair_checks(ctx, sub_pairs + 2 * (size_t)base, cnt, unit_lines, ctx->d_sub_M.as<E12>(), sv + base, PairSkip{gv, nullptr, subs, base});
+      const PairSkip sk = mask.empty() ? PairSkip{gv, nullptr, subs, base} : PairSkip{gv + N, nullptr, 1, base};
+      int prc = launch_pair_checks(ctx, sub_pairs + 2 * (size_t)base, cnt, unit_lines, ctx->d_sub_M.as<E12>(), sv + base, sk);
       if (prc) return prc;
     }
     sub_verdict = sv;
@@ -2617,7 +2711,7 @@ static int attribute_impl(h2v_ctx* ctx) {
   }
   // ---- level 2: every suspect proof alone
   CKC(cudaMemsetAsync(count, 0, 4, s));
-  KLAUNCH_P(false, k_pp_suspects, cdiv(N, 128), 128, 0, s, N, ctx->d_status.as<u32>(), sub_verdict, sub_size, gv, g.n, list, count);
+  KLAUNCH_P(false, k_pp_suspects, cdiv(N, 128), 128, 0, s, N, ctx->d_status.as<u32>(), sub_verdict, sub_size, gv, gsize, list, count);
   CKC(ctx->h_verd.ensure(4 * 1040));
   u32* h_count = ctx->h_verd.as<u32>() + 1030;
   CKC(cudaMemcpyAsync(h_count, count, 4, cudaMemcpyDeviceToHost, s));
@@ -3187,10 +3281,13 @@ struct h2v_mix {
   std::vector<cudaEvent_t> ev_join;  // per member: its stages are done
   bool has_key = false;              // one-shot key for the next batch (h2v_mix_set_rlc_key)
   RlcKey key{};
-  h2v_ctx::MsmBufs b;  // the joint MSM (coef / shared_sum unused: the segments point to the members')
-  DevBuf d_seg;
-  std::vector<MixSeg> segs;    // of the current batch
-  std::vector<u32> seg_member;
+  h2v_ctx::MsmBufs b;  // the joint MSM (coef / shared_sum unused: the segments point to the members' coefficients and d_ssum)
+  DevBuf d_seg, d_grange, d_ssum;
+  std::vector<MixSeg> segs;    // of the current batch: groups x members, group-major (mix_layout_groups)
+  std::vector<u32> active;     // members with proofs in the current batch
+  u32 groups = 1;              // fold groups of the current batch (h2v_mix_verify_groups), each with its own check
+  u64 call_base = 0;           // call index of the upload's first proof (a shard: its global base)
+  std::vector<u32> grange;     // call-index range of every group: [grange[q], grange[q + 1])
   MsmGeom geom{};
   int lines_slot = -1;  // the lead's prepared lines of the joint geometry (single-params mix)
   h2v_ctx::GraphSlot graphs[8];  // LRU over (member shapes, buffers), as for a context
@@ -3228,16 +3325,16 @@ static bool params_agree(const h2v_ctx* a, const h2v_ctx* b) {
          !memcmp(&plan_g(a), &plan_g(b), sizeof(G1Affine));
 }
 
-// joint window geometry: the single-batch choice (G = 1) over the summed terms of each channel
-// joint window geometry: the single-batch choice (G = 1) over the summed terms of each channel of the largest bucket set,
-// then one bucket set per params class with proofs (G = sets; T stays every term of the mix)
-static MsmGeom mix_geom(u32 N, u32 T, u32 right_terms, u32 left_terms, u32 sets) {
+// joint window geometry: the choice for `groups` fold groups of N / groups proofs (one group: the single-batch choice) over the
+// terms of each channel of the largest bucket set per group, then one bucket set per (group, params class with proofs)
+// (G = sets; T stays every term of the mix)
+static MsmGeom mix_geom(u32 N, u32 T, u32 right_terms, u32 left_terms, u32 sets, u32 groups) {
   MsmGeom g{};
   g.n = N;  // (picks the chunk size and bucket lanes as for a single batch of N proofs; the mixed kernels map terms through the segments)
   g.G = 1;
   g.N = N;
   g.T = T;
-  choose_windows(g, right_terms, left_terms, N, 1, 0);
+  choose_windows(g, right_terms, left_terms, (u32)(((u64)N + groups - 1) / groups), groups, 0);
   g.G = sets;
   return g;
 }
@@ -3284,7 +3381,7 @@ static int ensure_mix_lines(h2v_mix* mx, const MsmGeom& q) {
 
 static std::vector<h2v_ctx*> mix_active(const h2v_mix* mx) {
   std::vector<h2v_ctx*> v;
-  for (u32 sg : mx->seg_member) v.push_back(mx->m[sg]);
+  for (u32 mi : mx->active) v.push_back(mx->m[mi]);
   return v;
 }
 
@@ -3302,9 +3399,16 @@ static int mix_enqueue(h2v_mix* mx, int mode, h2v_ctx** fail) {
   const bool timed = !ctx->use_graphs;  // direct launches: the lead's events time the joint stages (h2v_last_timings)
   if (timed) CKC(cudaEventRecord(ctx->ev[0], s));
   CKC(cudaEventRecord(mx->ev_fork, s));
-  for (u32 sg = 0; sg < mx->seg_member.size(); sg++) {
-    const u32 mi = mx->seg_member[sg];
+  // fold coefficients of every group, written into the members' arrays: on the lead's auxiliary stream while the proofs are
+  // parsed (every member's d_r holds the r_i of the whole call)
+  CKC(cudaStreamWaitEvent(ctx->stream_aux, mx->ev_fork, 0));
+  KLAUNCH_P(false, k_rlc_scan_groups, mx->groups, RLC_NT, 0, ctx->stream_aux, mx->m[mx->active[0]]->d_r.as<Fr>(), mx->d_grange.as<u32>(),
+            mx->d_seg.as<MixSeg>(), (u32)mx->m.size());
+  CKC(cudaEventRecord(ctx->ev_join, ctx->stream_aux));
+  u32 sh_max = 0;
+  for (u32 mi : mx->active) {
     h2v_ctx* mb = mx->m[mi];
+    sh_max = std::max<u32>(sh_max, mb->hd.n_shared);
     *fail = mb;
     if (mb != ctx) {
       cudaError_t e = cudaStreamWaitEvent(mb->stream, mx->ev_fork, 0);
@@ -3313,8 +3417,7 @@ static int mix_enqueue(h2v_mix* mx, int mode, h2v_ctx** fail) {
         return -2;
       }
     }
-    int rc = enqueue_stages(mb);
-    if (!rc) rc = enqueue_shared_reduce(mb, mb->geom, mb->mb, mb->stream);
+    int rc = enqueue_stages(mb, false);
     if (rc) return rc;
     if (mb != ctx) {
       *fail = ctx;
@@ -3323,9 +3426,11 @@ static int mix_enqueue(h2v_mix* mx, int mode, h2v_ctx** fail) {
     }
   }
   *fail = ctx;
+  CKC(cudaStreamWaitEvent(s, ctx->ev_join, 0));
   if (timed) CKC(cudaEventRecord(ctx->ev[3], s));  // MSM = [3] -> [4], pairing = [4] -> [5]
   {
     NvtxRange nv_("h2v:mix_msm");
+    if (sh_max) KLAUNCH(k_shared_reduce_seg, dim3((u32)mx->segs.size(), sh_max), 256, 0, s, mx->d_seg.as<MixSeg>());
     const MixTerms src{mx->d_seg.as<MixSeg>(), (u32)mx->segs.size()};
     int rc = enqueue_buckets(ctx, g, mx->b, s, TermArrays{}, src, nullptr, 0);
     if (rc) return rc;
@@ -3333,7 +3438,7 @@ static int mix_enqueue(h2v_mix* mx, int mode, h2v_ctx** fail) {
   if (timed) CKC(cudaEventRecord(ctx->ev[4], s));
   if (mode & RUN_PAIRING) {
     NvtxRange nv_("h2v:pairing");
-    int rc = launch_pairing(ctx, g, mx->lines(), mx->b.wsums.as<G1Jac>(), 1, mx->run, mx->sets);
+    int rc = launch_pairing(ctx, g, mx->lines(), mx->b.wsums.as<G1Jac>(), mx->groups, mx->run, mx->sets);
     if (rc) return rc;
   }
   const u32 cb = g.c[0] | g.c[1] << 16, wd = g.W[0] | g.W[1] << 16, npts = g.W[0] + g.W[1];
@@ -3355,7 +3460,7 @@ static int mix_enqueue(h2v_mix* mx, int mode, h2v_ctx** fail) {
     KLAUNCH_P(false, k_wait_verdict, 1, 64, 0, s, cm.d_dyn, cm.window, cm.lay, 1u, vd);
   }
   if (timed) CKC(cudaEventRecord(ctx->ev[5], s));
-  if (mode & RUN_ACCUM)  // one (L, R) per bucket set: its window sums are wsums[set][W0 + W1]
+  if (mode & RUN_ACCUM)  // one (L, R) per bucket set (group-major): its window sums are wsums[set][W0 + W1]
     for (u32 st = 0; st < g.G; st++) {
       FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {g.wbase[0], g.wbase[1]}};
       KLAUNCH(k_fold_accum, 1, 32, 0, s, fa, mx->b.wsums.as<G1Jac>() + (size_t)st * (g.W[0] + g.W[1]), ctx->d_acc_bytes.as<u8>() + 128 * (size_t)st);
@@ -3374,17 +3479,19 @@ static u64 mix_graph_key(const h2v_mix* mx, int mode) {
   const h2v_ctx* lead = mx->m[0];
   const MsmGeom& g = mx->geom;
   mix((mode & RUN_ACCUM) ? 1 : 0);
-  for (u32 sg = 0; sg < mx->seg_member.size(); sg++) {
-    h2v_ctx* mb = mx->m[mx->seg_member[sg]];
+  // (not the split of the members' proofs over the groups: the segment table and the group ranges are device data)
+  mix(mx->groups);
+  for (u32 mi : mx->active) {
+    h2v_ctx* mb = mx->m[mi];
     mix((u64)(size_t)mb);
     mix(graph_key(mb, 0));  // the member's shape, options and buffers (what enqueue_stages and the segment read)
-    mix(mx->segs[sg].cls);  // the class assignment (bucket set of the segment)
+    mix(mx->set_of_class[mx->cls_of[mi]]);  // the class assignment (bucket set of the member)
   }
   for (int ch = 0; ch < 2; ch++) mix((u64)g.c[ch] | (u64)g.W[ch] << 8 | (u64)g.Z[ch] << 16);
   mix((u64)g.T | (u64)g.m << 32);
   mix((u64)g.N | (u64)g.G << 32);
   const DevBuf* bufs[] = {&mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets, &mx->b.wsums,
-                          &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &lead->d_M, &lead->d_gsums, &lead->d_verdict, &lead->d_acc_bytes,
+                          &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_grange, &mx->d_ssum, &lead->d_M, &lead->d_gsums, &lead->d_verdict, &lead->d_acc_bytes,
                           &mx->lines_buf()};
   for (const DevBuf* b : bufs) mix((u64)(size_t)b->p);
   mix(mx->run);
@@ -3478,25 +3585,36 @@ static u32 mix_count_sets(const h2v_mix* mx, const u32* counts) {
   return (u32)std::count(used.begin(), used.end(), true);
 }
 
-// batch_accum in class order from one 128 B (L, R) per bucket set; a class without proofs adds nothing: all-zero bytes
-static void mix_class_accum(const h2v_mix* mx, const u8* acc, u8* batch_accum) {
+// batch_accum in class order from one 128 B (L, R) per bucket set; a class without proofs adds nothing: all-zero bytes.
+// qcounts != null: one group of a grouped batch, whose member counts these are (a class with proofs elsewhere in the call but
+// none in this group is all-zero too)
+static void mix_class_accum(const h2v_mix* mx, const u8* acc, u8* batch_accum, const u32* qcounts = nullptr) {
   for (u32 c = 0; c < mx->set_of_class.size(); c++) {
-    if (mx->set_of_class[c] == ~0u) memset(batch_accum + 128 * (size_t)c, 0, 128);
+    bool has = mx->set_of_class[c] != ~0u;
+    if (has && qcounts) {
+      has = false;
+      for (u32 i = 0; i < mx->m.size(); i++) has |= mx->cls_of[i] == c && qcounts[i] != 0;
+    }
+    if (!has) memset(batch_accum + 128 * (size_t)c, 0, 128);
     else memcpy(batch_accum + 128 * (size_t)c, acc + 128 * (size_t)mx->set_of_class[c], 128);
   }
 }
 
-// Validation and upload of a mixed batch: local[m] proofs of member m, member-major in proofs / offsets, which are proofs
-// [gbase, gbase + sum local) of the member-major concatenation of gcounts[m] proofs (a whole batch: local = gcounts, gbase = 0).
-// The fold coefficients and the bucket sets are those of the global batch.  Window geometry: max_shard = 0 the mix's own choice
-// over its terms, otherwise every rank's common choice for shards of up to max_shard proofs (mix_shard_bound).  Then the
-// segment table, the joint MSM's buffers and the lines.  Everything up to the first upload_impl is host-only.
-static int mix_upload(h2v_mix* mx, const u32* local, const u32* gcounts, u64 gbase, u32 max_shard, const u8* proofs, const u64* proof_off,
+// Validation and upload of a mixed batch of `groups` fold groups: qcounts[q * K + m] proofs of member m in group q, in call
+// order (group-major, member-major inside a group) in proofs / offsets.  They are proofs [gbase, gbase + n) of the member-major
+// concatenation of gcounts[m] proofs (a whole batch: gcounts = the members' totals, gbase = 0; a shard: one group).  The fold
+// coefficients and the bucket sets are those of the global batch.  Window geometry: max_shard = 0 the mix's own choice over its
+// terms, otherwise every rank's common choice for shards of up to max_shard proofs (mix_shard_bound).  Then the segment table,
+// the group ranges, the joint MSM's buffers and the lines.  Everything up to the first upload_impl is host-only.
+static int mix_upload(h2v_mix* mx, u32 groups, const u32* qcounts, const u32* gcounts, u64 gbase, u32 max_shard, const u8* proofs, const u64* proof_off,
                       const u8* instances, const u64* inst_off, const u8* rlc, u64 seed, h2v_ctx** fail) {
   const u32 K = (u32)mx->m.size();
   h2v_ctx* lead = mx->m[0];
   *fail = nullptr;
   u64 N = 0, n = 0;
+  std::vector<u32> local(K, 0);  // the members' totals
+  for (u32 q = 0; q < groups; q++)
+    for (u32 i = 0; i < K; i++) local[i] += qcounts[(size_t)q * K + i];
   for (u32 i = 0; i < K; i++) {
     N += gcounts[i];
     n += local[i];
@@ -3528,15 +3646,15 @@ static int mix_upload(h2v_mix* mx, const u32* local, const u32* gcounts, u64 gba
       mx->err = "member " + std::to_string(i) + " has a pending fold-group or shard-hint option: mixed batches do not combine with them";
       return -1;
     }
-    if (local[i]) terms += (u64)local[i] * (msm_points(c->hd) + msm_mo(c->hd)) + c->hd.n_shared;
+    if (local[i]) terms += (u64)local[i] * (msm_points(c->hd) + msm_mo(c->hd)) + (u64)groups * c->hd.n_shared;
   }
   // term ids carry the sign in bit 31 (k_msm_scatter): the limit of upload_impl, over the whole mix
   if (terms >= (1ull << 31)) {
     mx->err = "mixed batch too large for the 32-bit index space of the MSM (split it into several batches)";
     return -1;
   }
-  // fold randomness, defined over the whole concatenation (c_j = prod_{i > j} r_i for j in [0, N)): explicit scalars, the
-  // mix's key, the test seed, or one key drawn from the OS for this batch; the same key is set on every member
+  // fold randomness, defined over the call indices (c_i = prod_{i' > i in the same group} r_i'): explicit scalars, the mix's
+  // key, the test seed, or one key drawn from the OS for this batch; the same key is set on every member
   RlcKey key{};
   bool keyed = false;
   if (!rlc && mx->has_key) {
@@ -3553,75 +3671,120 @@ static int mix_upload(h2v_mix* mx, const u32* local, const u32* gcounts, u64 gba
   mx->opt_shard_hint = 0;
   mx->ran = false;
   mx->xchg_root = false;
-  mx->counts.assign(local, local + K);
-  // 1. every member's slice as a shard [gbase + off, gbase + off + local) of the global batch of N proofs
-  std::vector<u32> nm(K), Pm(K), Mm(K), Sm(K);
-  u64 off = 0;
+  mx->counts = local;
+  mx->groups = groups;
+  mx->call_base = gbase;
+  mx->active.clear();
+  for (u32 i = 0; i < K; i++)
+    if (local[i]) mx->active.push_back(i);
+  // 1. every member's proofs of all groups, in group order, as one upload whose r_i are those of the whole call
+  std::vector<u32> Pm(K), Mm(K), Sm(K);
+  std::vector<u64> first(groups * (size_t)K);  // position in the call of the first proof of (group, member)
+  {
+    u64 at = 0;
+    for (u32 q = 0; q < groups; q++)
+      for (u32 i = 0; i < K; i++) {
+        first[(size_t)q * K + i] = at;
+        at += qcounts[(size_t)q * K + i];
+      }
+  }
   for (u32 i = 0; i < K; i++) {
     h2v_ctx* c = mx->m[i];
-    nm[i] = local[i];
     Pm[i] = msm_points(c->hd);
     Mm[i] = msm_mo(c->hd);
     Sm[i] = c->hd.n_shared;
     if (!local[i]) continue;
-    std::vector<u64> po(local[i] + 1), io(local[i] + 1);
-    for (u32 j = 0; j <= local[i]; j++) {
-      po[j] = proof_off[off + j] - proof_off[off];
-      io[j] = inst_off[off + j] - inst_off[off];
+    std::vector<u64> po(1, 0), io(1, 0);
+    UploadPieces pcs;
+    for (u32 q = 0; q < groups; q++) {
+      const u32 cnt = qcounts[(size_t)q * K + i];
+      const u64 f = first[(size_t)q * K + i];
+      if (!cnt) continue;
+      for (u32 j = 1; j <= cnt; j++) {
+        po.push_back(po.back() + proof_off[f + j] - proof_off[f + j - 1]);
+        io.push_back(io.back() + inst_off[f + j] - inst_off[f + j - 1]);
+      }
+      pcs.proofs.emplace_back(proofs ? proofs + proof_off[f] : nullptr, proof_off[f + cnt] - proof_off[f]);
+      pcs.instances.emplace_back(instances ? instances + 32 * inst_off[f] : nullptr, 32 * (inst_off[f + cnt] - inst_off[f]));
     }
     if (keyed) {
       c->opt_key = key;
       c->opt_has_key = true;
     }
     *fail = c;
-    int rc = upload_impl(c, local[i], proofs ? proofs + proof_off[off] : nullptr, po.data(), instances ? instances + 32 * inst_off[off] : nullptr,
-                         io.data(), rlc, keyed ? 0 : seed, gbase + off, N);
+    // (one piece: the member's proofs are contiguous in the call and upload_impl copies them directly)
+    int rc = upload_impl(c, local[i], pcs.proofs[0].first, po.data(), pcs.instances[0].first, io.data(), rlc, keyed ? 0 : seed, gbase, N,
+                         pcs.proofs.size() > 1 ? &pcs : nullptr);
     if (rc) return rc;
-    off += local[i];
   }
-  // 2. bucket sets (one per params class with proofs in the global batch, in class order), segment table, joint geometry,
-  // buffers, lines
+  // 2. bucket sets (group-major: one per params class with proofs in the global batch, in class order, per group), segment
+  // table, group ranges, joint geometry, buffers, lines
   mix_assign_sets(mx, gcounts);
-  std::vector<u32> set_of_member(K);
-  for (u32 i = 0; i < K; i++) set_of_member[i] = mx->set_of_class[mx->cls_of[i]];
-  mx->segs.assign(K, MixSeg{});
-  mx->seg_member.assign(K, 0);
+  std::vector<u32> set_of_member(K, 0);
+  for (u32 i = 0; i < K; i++)
+    if (mx->set_of_class[mx->cls_of[i]] != ~0u) set_of_member[i] = mx->set_of_class[mx->cls_of[i]];
+  const u32 nseg = groups * K;
+  mx->segs.assign(nseg, MixSeg{});
   unsigned long long total = 0;
-  const u32 nseg = mix_layout(K, nm.data(), Pm.data(), Mm.data(), Sm.data(), mx->segs.data(), mx->seg_member.data(), &total, set_of_member.data());
-  mx->segs.resize(nseg);
-  mx->seg_member.resize(nseg);
-  std::vector<u64> right_terms(mx->sets), left_terms(mx->sets);  // per bucket set
+  mix_layout_groups(groups, K, qcounts, Pm.data(), Mm.data(), Sm.data(), set_of_member.data(), mx->sets, gbase, mx->segs.data(), &total);
+  u32 sh_all = 0;  // shared bases of one group over the members with proofs
+  std::vector<u32> sh_off(K, 0);
+  for (u32 i : mx->active) {
+    sh_off[i] = sh_all;
+    sh_all += Sm[i];
+  }
+  std::vector<u64> right_terms(mx->sets), left_terms(mx->sets);  // per params class with proofs, over all groups
+  for (u32 i : mx->active) {
+    right_terms[set_of_member[i]] += (u64)local[i] * Pm[i] + (u64)groups * Sm[i];
+    left_terms[set_of_member[i]] += (u64)local[i] * Mm[i];
+  }
+  h2v_ctx* ctx = lead;
+  *fail = lead;
+  CKC(cudaSetDevice(lead->device));
+  CKC(mx->d_ssum.ensure(32 * ((size_t)groups * sh_all + 1)));
   for (u32 sg = 0; sg < nseg; sg++) {
     MixSeg& s = mx->segs[sg];
-    h2v_ctx* c = mx->m[mx->seg_member[sg]];
+    const u32 i = sg % K;
+    if (!local[i]) continue;
+    h2v_ctx* c = mx->m[i];
     s.right = c->d_right.as<Fr>();
     s.left = c->d_left.as<Fr>();
+    s.shared = c->d_shared.as<Fr>();
     s.coef = c->mb.coef.as<Fr>();
-    s.shared_sum = c->mb.shared_sum.as<Fr>();
+    s.shared_sum = mx->d_ssum.as<Fr>() + (size_t)(sg / K) * sh_all + sh_off[i];
     s.pts = c->d_pts.as<G1Affine>();
     s.shared_pts = c->pv().sec<G1Affine>(c->hd.off_shared_pts);
-    right_terms[s.cls] += (u64)s.n * s.P + s.Sh;
-    left_terms[s.cls] += (u64)s.n * s.n_mo;
+  }
+  mx->grange.assign(groups + 1, 0);
+  if (groups == 1) {
+    mx->grange[1] = (u32)N;  // (a shard scans the whole global batch and writes its own range)
+  } else {
+    for (u32 q = 0; q < groups; q++) {
+      u64 nq = 0;
+      for (u32 i = 0; i < K; i++) nq += qcounts[(size_t)q * K + i];
+      mx->grange[q + 1] = mx->grange[q] + (u32)nq;
+    }
   }
   if (max_shard) {  // every rank the same (c, W): the partials add up window-wise
     unsigned long long rb = 0, lb = 0;
     mix_shard_bound(K, Pm.data(), Mm.data(), Sm.data(), gcounts, max_shard, &rb, &lb);
-    mx->geom = mix_geom(max_shard, (u32)total, (u32)std::min(rb, 0xFFFFFFFFull), (u32)std::min(lb, 0xFFFFFFFFull), mx->sets);
+    mx->geom = mix_geom(max_shard, (u32)total, (u32)std::min(rb, 0xFFFFFFFFull), (u32)std::min(lb, 0xFFFFFFFFull), mx->sets, 1);
   } else {
+    // (per group: the largest class's terms over the groups; from the members' totals, so a new split keeps the geometry)
     const u32 big = (u32)(std::max_element(right_terms.begin(), right_terms.end()) - right_terms.begin());
-    mx->geom = mix_geom((u32)N, (u32)total, (u32)right_terms[big], (u32)left_terms[big], mx->sets);
+    mx->geom = mix_geom((u32)N, (u32)total, (u32)((right_terms[big] + groups - 1) / groups), (u32)((left_terms[big] + groups - 1) / groups),
+                        mx->sets * groups, groups);
   }
-  mx->run = mix_line_run(mx->sets, mx->geom.W[0], mx->geom.W[1], line_run(1));
-  h2v_ctx* ctx = lead;
-  *fail = lead;
-  CKC(cudaSetDevice(lead->device));
+  mx->run = mix_line_run(mx->sets, mx->geom.W[0], mx->geom.W[1], line_run(groups));
   CKC(ensure_msm_bufs(mx->geom, mx->b, 0, true));
   CKC(mx->d_seg.ensure(sizeof(MixSeg) * nseg));
   CKC(cudaMemcpyAsync(mx->d_seg.p, mx->segs.data(), sizeof(MixSeg) * nseg, cudaMemcpyHostToDevice, lead->stream));
-  CKC(lead->d_M.ensure(sizeof(E12) * (H2V_ATE_ITERS + MILLER_SEGS)));  // one check of up to 128 pairs
-  CKC(lead->d_gsums.ensure(sizeof(G1Jac) * 128));
-  CKC(lead->d_verdict.ensure(16));
-  CKC(lead->d_acc_bytes.ensure(128 * (size_t)mx->sets));
+  CKC(mx->d_grange.ensure(4 * ((size_t)groups + 1)));
+  CKC(cudaMemcpyAsync(mx->d_grange.p, mx->grange.data(), 4 * ((size_t)groups + 1), cudaMemcpyHostToDevice, lead->stream));
+  CKC(lead->d_M.ensure(sizeof(E12) * (H2V_ATE_ITERS + MILLER_SEGS) * (size_t)groups));  // one check of up to 128 pairs per group
+  CKC(lead->d_gsums.ensure(sizeof(G1Jac) * 128 * (size_t)groups));
+  CKC(lead->d_verdict.ensure(4 * (size_t)groups + 16));
+  CKC(lead->d_acc_bytes.ensure(128 * (size_t)mx->sets * groups));
   if (max_shard) {
     CKC(mx->d_partial.ensure((size_t)H2V_PARTIAL_BYTES * mx->sets));
     CKC(lead->d_wsums_fin.ensure(sizeof(G1Jac) * 128 * (size_t)mx->sets));
@@ -3638,58 +3801,114 @@ static void mix_mark_ran(h2v_mix* mx) {
   mx->ran = true;
 }
 
-// statuses of the upload's proofs, member-major; attribute: every member's proofs are re-checked on their own first
-// (poly/strategy.rs:26-30).  *all_ok = every status is H2V_OK.
-static int mix_statuses(h2v_mix* mx, bool attribute, u8* status, bool* all_ok, h2v_ctx** fail) {
+// statuses of the upload's proofs in call order; attribute: the members' proofs are re-checked on their own first
+// (poly/strategy.rs:26-30), with gverd (one word per group, non-zero = accepted) only those of rejected groups.
+// *all_ok = every status is H2V_OK.
+static int mix_statuses(h2v_mix* mx, bool attribute, const u32* gverd, u8* status, bool* all_ok, h2v_ctx** fail) {
   *all_ok = true;
-  u64 off = 0;
-  for (u32 i = 0; i < mx->m.size(); i++) {
-    const u32 cnt = mx->counts[i];
-    if (!cnt) continue;
+  const u32 K = (u32)mx->m.size();
+  for (u32 i : mx->active) {
     h2v_ctx* c = mx->m[i];
     *fail = c;
-    int rc = attribute ? attribute_impl(c) : 0;
-    if (!rc) rc = download_status(c, status + off);
+    bool attr = attribute;
+    if (attr && gverd) {
+      std::vector<u32> acc(mx->counts[i], 0);
+      bool any_acc = false, any_rej = false;
+      for (u32 q = 0; q < mx->groups; q++) {
+        const MixSeg& sg = mx->segs[(size_t)q * K + i];
+        for (u32 j = 0; j < sg.n; j++) acc[sg.j0 + j] = gverd[q] ? 1u : 0u;
+        if (sg.n) (gverd[q] ? any_acc : any_rej) = true;
+      }
+      attr = any_rej;
+      if (any_rej && any_acc) c->attr_accepted.swap(acc);
+    }
+    int rc = attr ? attribute_impl(c) : 0;
+    if (!rc) rc = download_status(c, nullptr);
     if (rc) return rc;
-    for (u32 j = 0; j < cnt; j++) *all_ok &= status[off + j] == ST_OK;
-    off += cnt;
+    const u32* hs = c->h_status.as<u32>();
+    for (u32 q = 0; q < mx->groups; q++) {
+      const MixSeg& sg = mx->segs[(size_t)q * K + i];
+      u8* out = status + (sg.call0 - mx->call_base);
+      for (u32 j = 0; j < sg.n; j++) {
+        out[j] = (u8)hs[sg.j0 + j];
+        *all_ok &= out[j] == ST_OK;
+      }
+    }
   }
   return 0;
 }
 
-static int mix_verify_impl(h2v_mix* mx, const u32* counts, const u8* proofs, const u64* proof_off, const u8* instances, const u64* inst_off,
-                           const u8* rlc, u64 seed, u8* status, u8* batch_accum, int* verdict, h2v_ctx** fail) {
+// The grouped mixed batch (a plain mix: one group): upload, one launch set with one pairing check per group, statuses, verdicts.
+static int mix_verify_impl(h2v_mix* mx, u32 groups, const u32* counts, const u8* proofs, const u64* proof_off, const u8* instances,
+                           const u64* inst_off, const u8* rlc, u64 seed, u8* status, u8* group_verdicts, u8* batch_accum, int* verdict,
+                           h2v_ctx** fail) {
   h2v_ctx* lead = mx->m[0];
   *fail = nullptr;
   if (!counts || !proof_off || !inst_off || !status || !verdict) {
     mx->err = "null argument";
     return -1;
   }
+  if (groups == 0 || groups > 1024) {
+    mx->err = "a grouped mixed batch takes 1 .. 1024 groups";
+    return -1;
+  }
+  const u32 K = (u32)mx->m.size();
+  std::vector<u32> totals(K, 0);
+  for (u32 q = 0; q < groups; q++) {
+    u64 nq = 0;
+    for (u32 i = 0; i < K; i++) {
+      nq += counts[(size_t)q * K + i];
+      totals[i] += counts[(size_t)q * K + i];  // (wraps only when the call exceeds 2^32 proofs, refused below)
+    }
+    if (nq == 0 && groups > 1) {
+      mx->err = "group " + std::to_string(q) + " has no proofs";
+      return -1;
+    }
+  }
   {
-    int rc = mix_upload(mx, counts, counts, 0, 0, proofs, proof_off, instances, inst_off, rlc, seed, fail);
+    u64 N = 0;
+    for (u32 q = 0; q < groups; q++)
+      for (u32 i = 0; i < K; i++) N += counts[(size_t)q * K + i];
+    if (N == 0 || N > 0xFFFFFFFFull) {
+      mx->err = "a mixed batch needs between 1 and 2^32 - 1 proofs";
+      return -1;
+    }
+  }
+  {
+    int rc = mix_upload(mx, groups, counts, totals.data(), 0, 0, proofs, proof_off, instances, inst_off, rlc, seed, fail);
     if (rc) return rc;
   }
-  // 3. stages + joint MSM + pairing (one graph)
+  // 3. stages + joint MSM + one pairing check per group (one graph)
   {
     int rc = mix_run(mx, RUN_PAIRING | (batch_accum ? RUN_ACCUM : 0), fail);
     if (rc) return rc;
   }
   h2v_ctx* ctx = lead;
   *fail = lead;
-  CKC(lead->h_verd.ensure(16));
-  u32* hv = lead->h_verd.as<u32>();
-  CKC(cudaMemcpyAsync(hv, lead->d_verdict.p, 4, cudaMemcpyDeviceToHost, lead->stream));
-  std::vector<u8> acc(batch_accum ? 128 * (size_t)mx->sets : 0);
+  CKC(lead->h_verd.ensure(4 * (size_t)groups + 16));
+  CKC(cudaMemcpyAsync(lead->h_verd.p, lead->d_verdict.p, 4 * (size_t)groups, cudaMemcpyDeviceToHost, lead->stream));
+  std::vector<u8> acc(batch_accum ? 128 * (size_t)mx->sets * groups : 0);
   if (batch_accum) CKC(cudaMemcpyAsync(acc.data(), lead->d_acc_bytes.p, acc.size(), cudaMemcpyDeviceToHost, lead->stream));
   CKC(ctx_sync(lead));
-  if (batch_accum) mix_class_accum(mx, acc.data(), batch_accum);
-  const bool accepted = hv[0] != 0;
-  // 4. statuses; on a rejected fold every member's proofs are re-checked on their own (poly/strategy.rs:26-30)
+  const std::vector<u32> hv(lead->h_verd.as<u32>(), lead->h_verd.as<u32>() + groups);  // (attribution reuses the lead's staging)
+  if (batch_accum)
+    for (u32 q = 0; q < groups; q++)
+      mix_class_accum(mx, acc.data() + 128 * (size_t)mx->sets * q, batch_accum + 128 * mx->class_rep.size() * q, counts + (size_t)q * K);
+  bool accepted = true;
+  for (u32 v : hv) accepted &= v != 0;
+  // 4. statuses; after a rejected check the proofs of the rejected groups are re-checked on their own (poly/strategy.rs:26-30)
   mix_mark_ran(mx);
   bool all_ok = false;
-  int rc = mix_statuses(mx, !accepted, status, &all_ok, fail);
+  int rc = mix_statuses(mx, !accepted, hv.data(), status, &all_ok, fail);
   if (rc) return rc;
-  *verdict = accepted && all_ok ? 1 : 0;
+  int all = 1;
+  for (u32 q = 0; q < groups; q++) {
+    bool ok = hv[q] != 0;
+    for (u32 i = mx->grange[q]; i < mx->grange[q + 1]; i++) ok &= status[i] == ST_OK;
+    if (group_verdicts) group_verdicts[q] = ok ? 1 : 0;
+    all &= ok ? 1 : 0;
+  }
+  *verdict = all;
   return 0;
 }
 
@@ -3744,7 +3963,7 @@ static int mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members
   mx->ev_join.assign(n_members, nullptr);
   h2v_ctx* l = mx->m[0];
   for (DevBuf* d : {&mx->b.coef, &mx->b.shared_sum, &mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets,
-                    &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_partial})
+                    &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_grange, &mx->d_ssum, &mx->d_partial})
     d->st = &l->stream;
   for (auto& sl : mx->mlines) sl.buf.st = &l->stream;
   cudaError_t e = cudaSetDevice(l->device);
@@ -3776,7 +3995,7 @@ void h2v_mix_destroy(h2v_mix* mx) {
   for (auto& gsl : mx->graphs)
     if (gsl.exec) cudaGraphExecDestroy(gsl.exec);
   for (DevBuf* d : {&mx->b.coef, &mx->b.shared_sum, &mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets,
-                    &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_partial})
+                    &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_grange, &mx->d_ssum, &mx->d_partial})
     d->release();
   for (auto& sl : mx->mlines) sl.buf.release();
   cudaStreamSynchronize(l->stream);  // the stream-ordered frees
@@ -3810,7 +4029,23 @@ int h2v_mix_verify(h2v_mix* mx, const uint32_t* counts, const uint8_t* proofs, c
   NvtxRange nv_("h2v:mix");
   mx->err.clear();
   h2v_ctx* fail = nullptr;
-  const int rc = mix_verify_impl(mx, counts, proofs, proof_off, instances, inst_off, rlc_scalars, seed, status, batch_accum, verdict, &fail);
+  const int rc = mix_verify_impl(mx, 1, counts, proofs, proof_off, instances, inst_off, rlc_scalars, seed, status, nullptr, batch_accum, verdict, &fail);
+  return mix_report(mx, rc, fail);
+}
+
+int h2v_mix_verify_groups(h2v_mix* mx, uint32_t groups, const uint32_t* counts, const uint8_t* proofs, const uint64_t* proof_off,
+                          const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint8_t* status,
+                          uint8_t* group_verdicts, uint8_t* batch_accum, int* verdict) {
+  if (!mx) return -1;
+  NvtxRange nv_("h2v:mix_groups");
+  mx->err.clear();
+  if (mx->opt_shard_hint) {
+    mx->err = "a shard hint is pending (h2v_mix_set_shard_hint): grouped mixed batches are not sharded";
+    return -1;
+  }
+  h2v_ctx* fail = nullptr;
+  const int rc = mix_verify_impl(mx, groups, counts, proofs, proof_off, instances, inst_off, rlc_scalars, seed, status, group_verdicts, batch_accum,
+                                 verdict, &fail);
   return mix_report(mx, rc, fail);
 }
 
@@ -3862,7 +4097,7 @@ static int mix_accumulate_shard_impl(h2v_mix* mx, const uint32_t* global_counts,
     return -1;
   }
   int rc = mix_shard_args(mx, global_counts, global_base, n, proof_off, inst_off, status, local, &max_shard);
-  if (!rc) rc = mix_upload(mx, local.data(), global_counts, global_base, max_shard, proofs, proof_off, instances, inst_off, rlc_scalars, seed, fail);
+  if (!rc) rc = mix_upload(mx, 1, local.data(), global_counts, global_base, max_shard, proofs, proof_off, instances, inst_off, rlc_scalars, seed, fail);
   if (!rc) rc = mix_run(mx, RUN_PARTIAL, fail);
   if (rc) return rc;
   mix_mark_ran(mx);
@@ -3871,7 +4106,7 @@ static int mix_accumulate_shard_impl(h2v_mix* mx, const uint32_t* global_counts,
   CKC(cudaMemcpyAsync(partial, mx->d_partial.p, (size_t)H2V_PARTIAL_BYTES * mx->sets, cudaMemcpyDefault, ctx->stream));
   CKC(ctx_sync(ctx));
   bool all_ok = false;
-  return mix_statuses(mx, false, status, &all_ok, fail);
+  return mix_statuses(mx, false, nullptr, status, &all_ok, fail);
 }
 
 int h2v_mix_accumulate_shard(h2v_mix* mx, const uint32_t* global_counts, uint64_t global_base, uint32_t n, const uint8_t* proofs,
@@ -3940,7 +4175,7 @@ int h2v_mix_attribute_shard(h2v_mix* mx, uint8_t* status) {
   }
   h2v_ctx* fail = nullptr;
   bool all_ok = false;
-  const int rc = mix_statuses(mx, true, status, &all_ok, &fail);  // (before fail is read)
+  const int rc = mix_statuses(mx, true, nullptr, status, &all_ok, &fail);  // (before fail is read)
   return mix_report(mx, rc, fail);
 }
 
@@ -3967,7 +4202,7 @@ static int mix_verify_shard_impl(h2v_mix* mx, const uint32_t* global_counts, uin
               std::to_string(sets) + " bucket sets (h2v_comm_init with max_groups >= the params classes with proofs)";
     return -1;
   }
-  rc = mix_upload(mx, local.data(), global_counts, global_base, max_shard, proofs, proof_off, instances, inst_off, rlc_scalars, seed, fail);
+  rc = mix_upload(mx, 1, local.data(), global_counts, global_base, max_shard, proofs, proof_off, instances, inst_off, rlc_scalars, seed, fail);
   if (rc) return rc;
   *fail = ctx;
   CKC(cudaSetDevice(ctx->device));
@@ -3979,7 +4214,7 @@ static int mix_verify_shard_impl(h2v_mix* mx, const uint32_t* global_counts, uin
   if ((rc = read_verdicts(ctx, &all, true, 1)) != 0) return rc;
   mx->xchg_root = root == cm.lay.rank;
   bool all_ok = false;
-  if ((rc = mix_statuses(mx, !all, status, &all_ok, fail)) != 0) return rc;
+  if ((rc = mix_statuses(mx, !all, nullptr, status, &all_ok, fail)) != 0) return rc;
   *verdict = (int)all;
   return 0;
 }

@@ -2,11 +2,12 @@
 // id to its scalar, its point and its channel; everything after them sees digits and bucket ids only.  Two sources:
 //   single VK   (MsmGeom, msm_point): G fold groups of one plan, each n*P right-channel proof terms, n*n_mo left-channel
 //               terms, Sh shared-base terms
-//   mixed batch (MixSeg table): one segment per member context with proofs, consecutive in term-id space; inside a segment
-//               the terms keep the single-VK order of one fold group, over the member's own arrays.  A one-segment table
-//               therefore maps every term exactly as msm_point / channel_of_term do.  The MsmGeom of a mix has T = every
-//               term of the mix and G = bucket sets: one per params class with proofs (h2v_mix_create_multi_params), 1
-//               otherwise; a segment's terms go to the bucket set of its class (MixSeg::cls).
+//   mixed batch (MixSeg table): one segment per (group, member) of a grouped mix (mix_layout_groups; a plain mix is one
+//               group), consecutive in term-id space; inside a segment the terms keep the single-VK order of one fold group,
+//               over a window [j0, j0 + n) of the member's own arrays (per-proof stride = the member's upload).  A
+//               one-segment table therefore maps every term exactly as msm_point / channel_of_term do.  The MsmGeom of a mix
+//               has T = every term of the mix and G = bucket sets: groups x (params classes with proofs in the call); the
+//               terms of segment (q, m) go to bucket set q * S + (set of m's class) (MixSeg::cls).
 // Compiles on the host too (tests/hostlib/mix_harness.cpp checks the mapping without a GPU).
 #pragma once
 #include "curve.cuh"
@@ -54,16 +55,21 @@ H2V_HD const G1Affine& msm_point(const MsmGeom& g, u32 t, const G1Affine* pts, c
 // ---- mixed batches (h2v_mix): members of different verifying keys in one MSM
 static constexpr u32 MIX_MAX_MEMBERS = 64;
 
-// One member with proofs.  The arrays are the member's own (one fold group: per-proof stride n).
+// The proofs of one member in one group: proofs [j0, j0 + n) of the member's upload (its arrays have per-proof stride
+// `stride`), call indices [call0, call0 + n) of the fold randomness.  Sh = the member's shared bases when it has proofs
+// anywhere in the call (a group without its proofs still carries them, with zero scalars), 0 otherwise.
 struct MixSeg {
   u32 t0, T;            // first term id, terms (n*P + n*n_mo + Sh)
-  u32 n, P, n_mo, Sh;   // the member's proofs and plan shape
-  u32 cls;              // bucket set of the member's params class (0 in a single-params mix)
-  const Fr* right;      // [P][n]     right-channel scalars of the proof points
-  const Fr* left;       // [n_mo][n]  left-channel scalars of the multi-open points
-  const Fr* coef;       // [n]        fold coefficients c_j of the member's slice of the global batch
-  const Fr* shared_sum; // [Sh]       sum_j c_j * shared scalar, canonical (k_shared_reduce)
-  const G1Affine* pts;  // [P][n]     decompressed proof points
+  u32 n, P, n_mo, Sh;   // the segment's proofs and the member's plan shape
+  u32 cls;              // bucket set: group * sets + set of the member's params class
+  u32 j0, stride;       // first proof of the segment in the member's arrays, proofs of the member's upload
+  u32 call0;            // call index of the segment's first proof (r_i, c_i)
+  const Fr* right;      // [P][stride]     right-channel scalars of the proof points
+  const Fr* left;       // [n_mo][stride]  left-channel scalars of the multi-open points
+  const Fr* shared;     // [Sh][stride]    per-proof shared-base scalars
+  Fr* coef;             // [stride]        fold coefficients c_j of the member's proofs (k_rlc_scan_groups)
+  Fr* shared_sum;       // [Sh]            sum over the segment of c_j * shared scalar, canonical (k_shared_reduce_seg)
+  const G1Affine* pts;  // [P][stride]     decompressed proof points
   const G1Affine* shared_pts;  // [Sh] fixed | sigma | G of the member's plan
 };
 
@@ -74,7 +80,7 @@ struct SingleVkTerms {
 struct MixTerms {
   static constexpr bool mixed = true;
   const MixSeg* seg;
-  u32 count;  // 1 .. MIX_MAX_MEMBERS
+  u32 count;  // groups * members (empty segments included)
 };
 
 // Segment table of `members` members with n[m] proofs each (members without proofs get no segment): t0 / T / shape / cls
@@ -82,7 +88,7 @@ struct MixTerms {
 // of member m (null: every segment in set 0).
 inline u32 mix_layout(u32 members, const u32* n, const u32* P, const u32* n_mo, const u32* Sh, MixSeg* seg, u32* member_of, unsigned long long* total,
                       const u32* set = nullptr) {
-  u32 count = 0;
+  u32 count = 0, calls = 0;
   unsigned long long t = 0;
   for (u32 m = 0; m < members; m++) {
     if (!n[m]) continue;
@@ -93,6 +99,9 @@ inline u32 mix_layout(u32 members, const u32* n, const u32* P, const u32* n_mo, 
     s.n_mo = n_mo[m];
     s.Sh = Sh[m];
     s.cls = set ? set[m] : 0;
+    s.stride = s.n;
+    s.call0 = calls;
+    calls += s.n;
     s.T = s.n * s.P + s.n * s.n_mo + s.Sh;
     t += s.T;
     member_of[count] = m;
@@ -100,6 +109,58 @@ inline u32 mix_layout(u32 members, const u32* n, const u32* P, const u32* n_mo, 
   }
   *total = t;
   return count;
+}
+
+// Grouped mixed batches (h2v_mix_verify_groups): groups x members segments, group-major, empty ones included (seg[q * members
+// + m] = member m's counts[q * members + m] proofs of group q).  The call order is group-major, member-major inside a group,
+// starting at call index call_base; a member's upload holds its proofs of every group in group order.  Members with proofs
+// anywhere in the call (sum over q > 0) carry their Sh shared bases in every group, so the term count, and every launch
+// shape, depends on the members' totals and `groups` only, never on the split.  set[m] = bucket set of member m's class
+// among `sets` (read for members with proofs only).  *total = terms of all segments.  groups = 1 maps every term as
+// mix_layout does.
+inline void mix_layout_groups(u32 groups, u32 members, const u32* counts, const u32* P, const u32* n_mo, const u32* Sh, const u32* set, u32 sets,
+                              unsigned long long call_base, MixSeg* seg, unsigned long long* total) {
+  unsigned long long t = 0, call = call_base;
+  for (u32 m = 0; m < members; m++) {  // j0 of group 0 and the member's total (stride)
+    u32 sum = 0;
+    for (u32 q = 0; q < groups; q++) sum += counts[(size_t)q * members + m];
+    for (u32 q = 0; q < groups; q++) seg[(size_t)q * members + m].stride = sum;
+  }
+  for (u32 q = 0; q < groups; q++)
+    for (u32 m = 0; m < members; m++) {
+      MixSeg& s = seg[(size_t)q * members + m];
+      const u32 stride = s.stride;
+      s = MixSeg{};
+      s.stride = stride;
+      s.j0 = q ? seg[(size_t)(q - 1) * members + m].j0 + seg[(size_t)(q - 1) * members + m].n : 0;
+      s.n = counts[(size_t)q * members + m];
+      s.P = P[m];
+      s.n_mo = n_mo[m];
+      s.Sh = stride ? Sh[m] : 0;
+      s.cls = stride ? q * sets + set[m] : q * sets;
+      s.call0 = (u32)call;
+      s.t0 = (u32)t;
+      s.T = s.n * s.P + s.n * s.n_mo + s.Sh;
+      t += s.T;
+      call += s.n;
+    }
+  *total = t;
+}
+
+// Write phase of the ragged-group coefficient scan (k_rlc_scan_groups) for one thread's chunk [lo, hi) of group q's call
+// indices: run = product of the group's r_i above hi; c_i = run * (r_i' for i < i' < hi) goes to [j0 + i - call0] of the
+// member array of the segment holding i (seg = group q's `members` segments, call0 ascending; an index no segment holds, in
+// a shard the other ranks' proofs, is scanned but not written).
+H2V_HD void mix_scan_chunk(const Fr* r, unsigned long long lo, unsigned long long hi, Fr run, const MixSeg* seg, u32 members) {
+  u32 k = 0;  // the last segment with call0 <= i: found once, then walked down as i falls
+  if (hi > lo)
+    while (k + 1 < members && seg[k + 1].call0 <= hi - 1) k++;
+  for (unsigned long long i = hi; i-- > lo;) {
+    while (k > 0 && seg[k].call0 > i) k--;
+    const MixSeg& s = seg[k];
+    if (i >= s.call0 && i < (unsigned long long)s.call0 + s.n) s.coef[s.j0 + (i - s.call0)] = run;
+    run = run * r[i];
+  }
 }
 
 // Sharded mixed batches: a rank owns proofs [base, base + n) of the member-major concatenation of global_counts[members]
@@ -159,15 +220,15 @@ H2V_HD MixTerm mix_term(const MixSeg& s, u32 tl) {
 }
 H2V_HD u32 mix_channel(const MixTerm& m) { return m.kind == 1 ? 1u : 0u; }
 H2V_HD const G1Affine& mix_point(const MixSeg& s, const MixTerm& m) {
-  if (m.kind == 0) return s.pts[(size_t)m.i * s.n + m.j];
-  if (m.kind == 1) return s.pts[(size_t)(s.P - s.n_mo + m.i) * s.n + m.j];
+  if (m.kind == 0) return s.pts[(size_t)m.i * s.stride + s.j0 + m.j];
+  if (m.kind == 1) return s.pts[(size_t)(s.P - s.n_mo + m.i) * s.stride + s.j0 + m.j];
   return s.shared_pts[m.i];
 }
 // the term's scalar, canonical: c_j times the proof's scalar, or the column sum of a shared base (0 for an identity base:
 // an all-zero fixed column)
 H2V_HD Fr mix_scalar(const MixSeg& s, const MixTerm& m) {
-  if (m.kind == 0) return (s.right[(size_t)m.i * s.n + m.j] * s.coef[m.j]).to_canonical();
-  if (m.kind == 1) return (s.left[(size_t)m.i * s.n + m.j] * s.coef[m.j]).to_canonical();
+  if (m.kind == 0) return (s.right[(size_t)m.i * s.stride + s.j0 + m.j] * s.coef[s.j0 + m.j]).to_canonical();
+  if (m.kind == 1) return (s.left[(size_t)m.i * s.stride + s.j0 + m.j] * s.coef[s.j0 + m.j]).to_canonical();
   const G1Affine& sp = s.shared_pts[m.i];
   return (sp.x.is_zero() && sp.y.is_zero()) ? Fr::zero() : s.shared_sum[m.i];
 }

@@ -338,6 +338,35 @@ int h2v_mix_attribute_shard(h2v_mix* mx, uint8_t* status);
 int h2v_mix_verify_shard(h2v_mix* mx, const uint32_t* global_counts, uint64_t global_base, uint32_t n, const uint8_t* proofs, const uint64_t* proof_off,
                          const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint32_t root, uint8_t* status,
                          int* verdict);
+
+/* ---- grouped mixed batches: many independent mixed batches in one launch set, one pairing check and verdict each ------------
+ * `groups` (1 .. 1024) independent batches of the mix's members, each what h2v_mix_verify would take: counts[q * M + m] =
+ * proofs of member m in group q (M = members; 0 allowed), every group with at least one proof, N = sum counts.  proofs /
+ * offsets / instances follow the call order: group 0's member-major concatenation, then group 1's, ...  The r_i are indexed
+ * by call index i in [0, N); group q covers [o_q, o_q + N_q) and proof j of it is folded with c_j = prod_{i in group q, i > j}
+ * r_i: the fold restarts at every group boundary.  rlc_scalars (N x 32 B; group q's slice = what h2v_mix_verify takes for
+ * group q alone), the mix's one-shot key, the test seed and OS entropy (one fresh key per call) follow the precedence of
+ * h2v_mix_verify and expand by call index; aggregation members: one rho per member upload.
+ * Group q passes when prod_p e(L_{q,p}, [s_p]g2_p) e(R_{q,p}, -g2_p) = 1 over the params classes with proofs anywhere in
+ * the call (a class without proofs in group q contributes the identity); the 128-pair budget of the check applies per group.
+ * Every member uploads once (its proofs of all groups, in group order: h2v_batch_set_columns on a member describes them in
+ * that order) and runs its per-proof stages once; the joint bucket MSM has one bucket set per (group, class) and the pairing
+ * kernels one check per group, all in one CUDA graph whose key depends on the members' totals and `groups`, not on the split.
+ *   status          N bytes, call order
+ *   group_verdicts  optional, `groups` bytes: 1 exactly when h2v_mix_verify on group q alone would return verdict 1 (the
+ *                   group's check accepted and every proof of it is H2V_OK)
+ *   batch_accum     optional, groups x classes x 128 B: per group the class layout of h2v_mix_verify (all-zero bytes for a
+ *                   class without proofs in that group)
+ *   verdict         the AND of the group verdicts
+ * After a rejected check only the proofs of the rejected groups are re-checked on their own (poly/strategy.rs:26-30), with
+ * coefficients of their own as in h2v_verify_batch; proofs of accepted groups keep their accumulate-time statuses.
+ * Refused before any device call, text in h2v_mix_last_error(mx), state unchanged (the one-shot key stays set): groups = 0 or
+ * > 1024, a group without proofs, a null counts / proof_off / inst_off / status / verdict, N = 0 or N >= 2^32, more terms
+ * than the 31-bit term ids hold, zero or non-canonical rlc_scalars, a member with a pending fold-group or shard-hint option,
+ * a pending h2v_mix_set_shard_hint.  h2v_mix_verify is this call with groups = 1. */
+int h2v_mix_verify_groups(h2v_mix* mx, uint32_t groups, const uint32_t* counts, const uint8_t* proofs, const uint64_t* proof_off,
+                          const uint8_t* instances, const uint64_t* inst_off, const uint8_t* rlc_scalars, uint64_t seed, uint8_t* status,
+                          uint8_t* group_verdicts, uint8_t* batch_accum, int* verdict);
 int h2v_mix_comm_last_batch_accum(h2v_mix* mx, uint8_t* batch_accum);
 
 /* ---- persistent accumulators: AccumulatorStrategy as a value that lives across calls ------------------------------------
