@@ -1229,6 +1229,24 @@ struct HostBuf {
   }
 };
 
+// One slot of a CUDA-graph LRU (graph_lookup): the instantiated launch set of one key and the kernels it launches
+struct GraphSlot {
+  u64 key = 0, used = 0;
+  u64 kernels = 0;
+  cudaGraphExec_t exec = nullptr;
+};
+
+// LRU of prepared G2 window-line tables, one slot per (pair geometry, params classes) (ensure_lines): a service alternating
+// batch shapes must not rebuild ~5,000 lines on the host at every call
+struct LinesCache {
+  struct Slot {
+    u64 key = ~0ull, used = 0;
+    DevBuf buf;
+  } s[4];
+  int cur = -1;  // a context's cache: the slot of its current batch's geometry
+  u64 clock = 0;
+};
+
 struct h2v_ctx {
   int device = -1;  // -1 until a device was selected (h2v_ctx_destroy then frees host state only)
   cudaStream_t stream = nullptr;
@@ -1262,25 +1280,15 @@ struct h2v_ctx {
   u32 rlc_source = 0;  // of the last upload: 0 caller scalars, 1 test seed, 2 caller key, 3 key drawn from the OS
   bool opt_has_agg_scalar = false;  // next upload of an aggregation context: rho from the caller (h2v_batch_set_agg_scalar)
   Fr opt_agg_scalar{}, h_rho{};     // (Montgomery) the caller's rho; rho of the last upload, source of its copy to d_rho
-  // prepared G2 window lines, one slot per window geometry (small LRU: a service alternating batch shapes on one
-  // context must not rebuild ~5,000 lines on the host at every call)
-  struct LinesSlot {
-    u64 key = ~0ull, used = 0;
-    DevBuf buf;
-  } lines[4];
-  int lines_cur = -1;       // slot of the current geometry
+  LinesCache lines;         // prepared G2 window lines, one slot per window geometry
   u64 lines_builds = 0;     // host rebuilds so far (h2v_ctx_cache_stats)
-  u64 use_clock = 0;        // LRU clock of both caches
   // CUDA graphs: the ~20 kernels of a batch are captured once per (mode, shape, buffers) and replayed with one launch
   bool use_graphs = true;
   bool use_pdl = false;  // programmatic dependent launch between the kernels of a batch (pdl_prologue)
   bool capturing = false;
   bool stages_timed = false;  // ev[1..5] of the last run are valid (direct launches only)
-  struct GraphSlot {
-    u64 key = 0, used = 0;
-    u64 kernels = 0;
-    cudaGraphExec_t exec = nullptr;
-  } graphs[16];             // LRU over (entry point, batch shape, buffers): alternating shapes replay, never recapture
+  GraphSlot graphs[16];     // LRU over (entry point, batch shape, buffers): alternating shapes replay, never recapture
+  u64 graph_clock = 0;
   u64 graph_captures = 0;   // captures so far (h2v_ctx_cache_stats)
   // accumulator of the absorb being enqueued (RUN_ABSORB, h2v_acc_absorb): its (R, L), records and record counter
   struct AbsorbTarget {
@@ -1315,12 +1323,12 @@ struct h2v_ctx {
   // one-shot for the next attribute_impl (a grouped mixed batch): per proof of the upload, non-zero = its group accepted
   // (not re-checked); empty = every proof is looked at
   std::vector<u32> attr_accepted;
-  const G2Line* d_lines() const { return lines_cur >= 0 ? lines[lines_cur].buf.as<G2Line>() : nullptr; }
+  const G2Line* d_lines() const { return lines.cur >= 0 ? lines.s[lines.cur].buf.as<G2Line>() : nullptr; }
   std::vector<DevBuf*> all_bufs() {
     std::vector<DevBuf*> v = {&d_plan, &d_proofs, &d_proof_off, &d_inst, &d_inst_off, &d_ncols, &d_col_len, &d_pts, &d_bad, &d_status, &d_vals, &d_scratch,
                               &d_right, &d_shared, &d_left, &d_rlc_bytes, &d_r, &d_acc_bytes, &d_verdict, &d_partials, &d_pp_prod, &d_pp_lr, &d_pp_bytes,
                               &d_hook, &d_chal, &d_flush, &d_M, &d_partial_out, &d_wsums_fin, &d_sub_pairs, &d_sub_verdict, &d_sub_M, &d_gsums, &d_ptsc, &d_rho,
-                              &d_attr_r, &d_attr_mask, &lines[0].buf, &lines[1].buf, &lines[2].buf, &lines[3].buf};
+                              &d_attr_r, &d_attr_mask, &lines.s[0].buf, &lines.s[1].buf, &lines.s[2].buf, &lines.s[3].buf};
     for (MsmBufs* m : {&mb, &ab})
       for (DevBuf* d : {&m->coef, &m->shared_sum, &m->dig, &m->hist, &m->off, &m->cursor, &m->order, &m->sorted, &m->buckets, &m->wsums, &m->partials_msm, &m->tiles})
         v.push_back(d);
@@ -1501,6 +1509,72 @@ static cudaError_t ctx_sync(h2v_ctx* ctx) {
   return cudaEventSynchronize(ctx->ev_done);
 }
 
+// Graph keys: an FNV-style hash of what a captured launch set depends on (kept in memory only, never persisted)
+struct KeyHash {
+  u64 h = 0xcbf29ce484222325ull;
+  void mix(u64 v) {
+    h ^= v;
+    h *= 0x100000001b3ull;
+    h ^= h >> 29;
+  }
+};
+// the window geometry: c / W / Z per channel, terms and chunk, bucket sets and proofs
+static void hash_geom(KeyHash& k, const MsmGeom& g) {
+  for (int ch = 0; ch < 2; ch++) k.mix((u64)g.c[ch] | (u64)g.W[ch] << 8 | (u64)g.Z[ch] << 16);
+  k.mix((u64)g.T | (u64)g.m << 32);
+  k.mix((u64)g.G | (u64)g.N << 32);
+}
+
+// The CUDA-graph LRU of a launch set: *out = the slot of `key`, captured from enqueue() on stream s (which may fork onto other
+// streams) and instantiated on a miss.  During a capture every context of ctxs[0, n_ctxs) is marked capturing (no stage
+// events) and gets its launch counter back afterwards: the slot counts the captured kernels, which the caller credits at each
+// replay.  ctxs[0] reports the errors and counts the capture.
+template <size_t N, class Enqueue>
+static int graph_lookup(GraphSlot (&slots)[N], u64& clock, u64 key, h2v_ctx* const* ctxs, size_t n_ctxs, cudaStream_t s, Enqueue&& enqueue,
+                        GraphSlot** out) {
+  h2v_ctx* ctx = ctxs[0];
+  clock++;
+  GraphSlot* hit = nullptr;
+  GraphSlot* victim = &slots[0];
+  for (GraphSlot& sl : slots) {
+    if (sl.exec && sl.key == key) hit = &sl;
+    if (!sl.exec ? victim->exec != nullptr : (victim->exec && sl.used < victim->used)) victim = &sl;
+  }
+  GraphSlot& gs = hit ? *hit : *victim;
+  gs.used = clock;
+  *out = &gs;
+  if (hit) return 0;
+  trace(ctx, "graph capture begins");
+  if (gs.exec) cudaGraphExecDestroy(gs.exec);
+  gs.exec = nullptr;
+  gs.key = 0;
+  std::vector<u64> before(n_ctxs);
+  for (size_t i = 0; i < n_ctxs; i++) before[i] = ctxs[i]->launches;
+  CKC(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+  for (size_t i = 0; i < n_ctxs; i++) ctxs[i]->capturing = true;
+  const int rc = enqueue();
+  for (size_t i = 0; i < n_ctxs; i++) ctxs[i]->capturing = false;
+  cudaGraph_t graph = nullptr;
+  const cudaError_t ce = cudaStreamEndCapture(s, &graph);
+  gs.kernels = 0;
+  for (size_t i = 0; i < n_ctxs; i++) {
+    gs.kernels += ctxs[i]->launches - before[i];
+    ctxs[i]->launches = before[i];
+  }
+  if (rc) {
+    if (graph) cudaGraphDestroy(graph);
+    return rc;
+  }
+  CKC(ce);
+  const cudaError_t ie = cudaGraphInstantiate(&gs.exec, graph, prio_mode() ? cudaGraphInstantiateFlagUseNodePriority : 0);
+  cudaGraphDestroy(graph);
+  CKC(ie);
+  gs.key = key;
+  ctx->graph_captures++;
+  trace(ctx, "graph instantiated");
+  return 0;
+}
+
 // Window size per channel.  Thanks to the scalar lift k'' = k + z*r every window is uniformly filled, so
 // the choice is a pure work trade-off: bucket additions (11 MM) against bucket reduction (2 x 16 MM
 // per bucket plus the per-chunk offset multiplication), with a floor on the per-bucket serial chain.
@@ -1610,43 +1684,49 @@ static MsmGeom pair_geom_run(const MsmGeom& g, u32 run) {
 static MsmGeom pair_geom(const MsmGeom& g, u32 groups) { return pair_geom_run(g, line_run(groups)); }
 static u64 lines_key_of(const MsmGeom& g) { return (u64)g.c[0] | (u64)g.W[0] << 12 | (u64)g.c[1] << 24 | (u64)g.W[1] << 36; }
 
-// Prepared Miller lines of [2^(c w)] Q for the current window geometry (host: G2Prepared-style
-// preparation, once per geometry; the last few geometries stay cached in the context).
-static int ensure_lines(h2v_ctx* ctx, const MsmGeom& g, int* slot_out) {
-  const u64 key = lines_key_of(g);
-  ctx->use_clock++;
+// The slot of lc that holds the prepared Miller lines of [2^(c w)] Q for pair geometry q, one table per params class of
+// `classes`, concatenated in that order.  key names q and the classes.  A miss prepares them on the host (G2Prepared-style),
+// uploads them on ctx's stream and counts a build in ctx->lines_builds; slot `pinned` (-1: none) is never evicted.
+static int ensure_lines(h2v_ctx* ctx, LinesCache& lc, u64 key, const MsmGeom& q, const std::vector<const PlanInfo*>& classes, int pinned, int* slot_out) {
+  lc.clock++;
   int victim = -1;
   for (int i = 0; i < 4; i++) {
-    if (ctx->lines[i].key == key) {
-      ctx->lines[i].used = ctx->use_clock;
+    if (lc.s[i].key == key) {
+      lc.s[i].used = lc.clock;
       *slot_out = i;
       return 0;
     }
-    if (i == ctx->lines_cur && slot_out != &ctx->lines_cur) continue;  // never evict the batch's own geometry for an auxiliary one
-    if (victim < 0 || ctx->lines[i].used < ctx->lines[victim].used) victim = i;
+    if (i == pinned) continue;
+    if (victim < 0 || lc.s[i].used < lc.s[victim].used) victim = i;
   }
-  if (g.W[0] + g.W[1] > 128) {
+  if (classes.size() * (q.W[0] + q.W[1]) > 128) {
     ctx->err = "window geometry exceeds 128 (channel, window) pairs";
     return -1;
   }
-  std::vector<u8> tab;
-  build_window_lines(ctx->info, g.c[0], g.W[0], g.c[1], g.W[1], tab);
-  h2v_ctx::LinesSlot& sl = ctx->lines[victim];
+  std::vector<u8> tab, one;
+  for (const PlanInfo* info : classes) {
+    build_window_lines(*info, q.c[0], q.W[0], q.c[1], q.W[1], one);
+    tab.insert(tab.end(), one.begin(), one.end());
+  }
+  LinesCache::Slot& sl = lc.s[victim];
   CKC(ctx_sync(ctx));  // the victim's lines may still be read by queued work
   sl.key = ~0ull;
   CKC(sl.buf.ensure(tab.size()));
-  CKC(ctx->d_M.ensure(sizeof(E12) * (H2V_ATE_ITERS + MILLER_SEGS)));
-  CKC(ctx->d_wsums_fin.ensure(sizeof(G1Jac) * 128));
-  CKC(ctx->d_partial_out.ensure(H2V_PARTIAL_BYTES));
   CKC(cudaMemcpyAsync(sl.buf.p, tab.data(), tab.size(), cudaMemcpyHostToDevice, ctx->stream));
   CKC(ctx_sync(ctx));
   sl.key = key;
-  sl.used = ctx->use_clock;
+  sl.used = lc.clock;
   *slot_out = victim;
   ctx->lines_builds++;
   return 0;
 }
-static int ensure_lines(h2v_ctx* ctx, u32 groups) { return ensure_lines(ctx, pair_geom(ctx->geom, groups), &ctx->lines_cur); }
+// lines of pair geometry q from ctx's own params and cache; an auxiliary geometry (slot_out not the batch's own slot) never
+// evicts the batch's geometry
+static int ensure_lines(h2v_ctx* ctx, const MsmGeom& q, int* slot_out) {
+  LinesCache& lc = ctx->lines;
+  return ensure_lines(ctx, lc, lines_key_of(q), q, {&ctx->info}, slot_out == &lc.cur ? -1 : lc.cur, slot_out);
+}
+static int ensure_lines(h2v_ctx* ctx, u32 groups) { return ensure_lines(ctx, pair_geom(ctx->geom, groups), &ctx->lines.cur); }
 
 // the batch pairing check over `wsums` (W0 + W1 Jacobian window sums per bucket set, window geometry g) -> d_verdict[group].
 // Each of the `groups` checks pairs `sets` consecutive bucket sets (a multi-params mix: one per params class, 1 otherwise)
@@ -1676,7 +1756,6 @@ static int launch_pairing(h2v_ctx* ctx, const MsmGeom& g, const G2Line* lines, c
   }
   return 0;
 }
-static int launch_pairing(h2v_ctx* ctx, const G1Jac* wsums, u32 groups) { return launch_pairing(ctx, ctx->geom, ctx->d_lines(), wsums, groups); }
 
 // Attribution: `count` independent 2-pair checks e(pairs[i][1], [s]G2) e(pairs[i][0], -G2) == 1 (pairs: right | left accumulator,
 // Jacobian) -> verdict[i]; groups for which sk says "skip" keep their verdict word.  M: E12[count][H2V_ATE_ITERS] scratch.
@@ -2432,8 +2511,70 @@ static int enqueue_stages(h2v_ctx* ctx, bool own_coef = true) {
   return 0;
 }
 
-static int enqueue_batch(h2v_ctx* ctx, int mode) {
+// k_fold_accum over `count` consecutive bucket sets of window sums (geometry g): one 128 B affine (L, R) per set at out
+static int enqueue_fold_accum(h2v_ctx* ctx, const MsmGeom& g, const G1Jac* wsums, u32 count, u8* out, bool pdl) {
+  const FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {0, g.W[0]}};
+  for (u32 st = 0; st < count; st++)
+    KLAUNCH_P(pdl, k_fold_accum, 1, 32, 0, ctx->stream, fa, wsums + (size_t)st * (g.W[0] + g.W[1]), out + 128 * (size_t)st);
+  return 0;
+}
+
+// What follows the MSM in a launch set: its window sums and how they are checked (enqueue_tail)
+struct TailArgs {
+  MsmGeom g;              // window geometry; g.G bucket sets
+  G1Jac* wsums;           // [g.G][W0 + W1] window sums of the MSM
+  const G2Line* lines;    // prepared lines of the pair geometry, one table per bucket set of a check
+  u32 checks, sets, run;  // pairing checks, bucket sets per check, window-combination run (0 = line_run(checks))
+  u8* partial;            // RUN_PARTIAL: one H2V_PARTIAL_BYTES blob per bucket set
+};
+// The kernels of a launch set after its MSM, on ctx's stream (ctx: the context, or the lead of a mixed batch), by the RUN_*
+// mode bits: pairing checks -> d_verdict, packed partials, the device-side exchange over ctx's channel, the absorb into
+// ctx->absorb (a context's own batch: its r_i and coefficients), the folded (L, R) of every bucket set -> d_acc_bytes.
+// Stage events ev[4..6] unless capturing.
+static int enqueue_tail(h2v_ctx* ctx, int mode, const TailArgs& t) {
   cudaStream_t s = ctx->stream;
+  const MsmGeom& g = t.g;
+  const u32 cb = g.c[0] | g.c[1] << 16, wd = g.W[0] | g.W[1] << 16, npts = g.W[0] + g.W[1];
+  if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[4], s));
+  if (mode & RUN_PAIRING) {
+    NvtxRange nv_("h2v:pairing");
+    int prc = launch_pairing(ctx, g, t.lines, t.wsums, t.checks, t.run, t.sets);
+    if (prc) return prc;
+  }
+  if (mode & RUN_PARTIAL) KLAUNCH(k_pack_partial, dim3(8, g.G), 256, 0, s, cb, wd, npts, t.wsums, t.partial);
+  if (mode & RUN_XCHG) {
+    NvtxRange nv_("h2v:exchange");
+    // The one exchange step of a sharded batch, device side (exchange.cuh): partials (one blob per bucket set) -> the root's
+    // window over NVLink; root: wait for all ranks, sum in place, pairing checks, verdicts -> every rank's window; every rank:
+    // wait for them.
+    h2v_ctx::Comm& cm = ctx->comm;
+    u32* vd = ctx->d_verdict.as<u32>();
+    CKC(cudaMemsetAsync(vd + t.checks, 0, 8, s));  // error words of this launch set
+    KLAUNCH(k_pack_partial_x, g.G, 256, 0, s, cb, wd, npts, t.wsums, cm.d_dyn, cm.d_peers, cm.lay, cm.d_done);
+    if (mode & RUN_ROOT) {
+      KLAUNCH_P(false, k_sum_partials, g.G, 128, 0, s, cm.lay.world, cb, wd, npts, cm.window + cm.lay.partials_off(), (size_t)cm.lay.max_groups * H2V_PARTIAL_BYTES,
+                ctx->d_wsums_fin.as<G1Jac>(), vd + t.checks, cm.d_dyn, (const u64*)(cm.window + cm.lay.arrive_off()));
+      int prc = launch_pairing(ctx, g, t.lines, ctx->d_wsums_fin.as<G1Jac>(), t.checks, t.run, t.sets);
+      if (prc) return prc;
+      KLAUNCH_P(false, k_bcast_verdict, 1, 256, 0, s, cm.d_dyn, cm.d_peers, cm.lay, t.checks, vd, vd + t.checks);
+    }
+    KLAUNCH_P(false, k_wait_verdict, 1, 64, 0, s, cm.d_dyn, cm.window, cm.lay, t.checks, vd);
+  }
+  if (mode & RUN_ABSORB) {
+    const AccGeom ag{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}};
+    const h2v_ctx::AbsorbTarget& at = ctx->absorb;
+    KLAUNCH(k_acc_absorb, 1, 32 * cdiv(4 * acc_items(ag), 32), 0, s, ag, t.wsums, ctx->d_r.as<Fr>(), ctx->mb.coef.as<Fr>(), at.acc, at.records, at.count, at.cap);
+  }
+  if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[5], s));
+  if (mode & RUN_ACCUM) {
+    int arc = enqueue_fold_accum(ctx, g, t.wsums, g.G, ctx->d_acc_bytes.as<u8>(), ctx->use_pdl);
+    if (arc) return arc;
+  }
+  if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[6], s));
+  return 0;
+}
+
+static int enqueue_batch(h2v_ctx* ctx, int mode) {
   const MsmGeom& g = ctx->geom;
   if ((mode & RUN_ACCUM) && g.G != 1) {
     ctx->err = "the folded accumulator hook is defined for a single fold group";
@@ -2445,85 +2586,37 @@ static int enqueue_batch(h2v_ctx* ctx, int mode) {
   }
   {
     NvtxRange nv_("h2v:msm");
-    int mrc = enqueue_msm(ctx, g, ctx->mb, s, nullptr, 0);
+    int mrc = enqueue_msm(ctx, g, ctx->mb, ctx->stream, nullptr, 0);
     if (mrc) return mrc;
   }
-  if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[4], s));
-  if (mode & RUN_PAIRING) {
-    NvtxRange nv_("h2v:pairing");
-    int prc = launch_pairing(ctx, ctx->mb.wsums.as<G1Jac>(), g.G);
-    if (prc) return prc;
-  }
-  if (mode & RUN_PARTIAL) {
-    KLAUNCH(k_pack_partial, dim3(8, g.G), 256, 0, s, g.c[0] | g.c[1] << 16, g.W[0] | g.W[1] << 16, g.W[0] + g.W[1], ctx->mb.wsums.as<G1Jac>(), ctx->d_partial_out.as<u8>());
-  }
-  if (mode & RUN_XCHG) {
-    NvtxRange nv_("h2v:exchange");
-    // The one exchange step of a sharded batch, device side (exchange.cuh): partials -> the root's window over NVLink;
-    // root: wait for all ranks, sum in place, pairing checks, verdicts -> every rank's window; every rank: wait for them.
-    h2v_ctx::Comm& cm = ctx->comm;
-    const u32 cb = g.c[0] | g.c[1] << 16, wd = g.W[0] | g.W[1] << 16, npts = g.W[0] + g.W[1];
-    u32* vd = ctx->d_verdict.as<u32>();
-    CKC(cudaMemsetAsync(vd + g.G, 0, 8, s));  // error words of this launch set
-    KLAUNCH(k_pack_partial_x, g.G, 256, 0, s, cb, wd, npts, ctx->mb.wsums.as<G1Jac>(), cm.d_dyn, cm.d_peers, cm.lay, cm.d_done);
-    if (mode & RUN_ROOT) {
-      KLAUNCH_P(false, k_sum_partials, g.G, 128, 0, s, cm.lay.world, cb, wd, npts, cm.window + cm.lay.partials_off(), (size_t)cm.lay.max_groups * H2V_PARTIAL_BYTES,
-                ctx->d_wsums_fin.as<G1Jac>(), vd + g.G, cm.d_dyn, (const u64*)(cm.window + cm.lay.arrive_off()));
-      int prc = launch_pairing(ctx, ctx->d_wsums_fin.as<G1Jac>(), g.G);
-      if (prc) return prc;
-      KLAUNCH_P(false, k_bcast_verdict, 1, 256, 0, s, cm.d_dyn, cm.d_peers, cm.lay, g.G, vd, vd + g.G);
-    }
-    KLAUNCH_P(false, k_wait_verdict, 1, 64, 0, s, cm.d_dyn, cm.window, cm.lay, g.G, vd);
-  }
-  if (mode & RUN_ABSORB) {
-    const AccGeom ag{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}};
-    const h2v_ctx::AbsorbTarget& at = ctx->absorb;
-    KLAUNCH(k_acc_absorb, 1, 32 * cdiv(4 * acc_items(ag), 32), 0, s, ag, ctx->mb.wsums.as<G1Jac>(), ctx->d_r.as<Fr>(), ctx->mb.coef.as<Fr>(), at.acc, at.records,
-            at.count, at.cap);
-  }
-  if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[5], s));
-  if (mode & RUN_ACCUM) {
-    FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {g.wbase[0], g.wbase[1]}};
-    KLAUNCH(k_fold_accum, 1, 32, 0, s, fa, ctx->mb.wsums.as<G1Jac>(), ctx->d_acc_bytes.as<u8>());
-  }
-  if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[6], s));
-  return 0;
+  return enqueue_tail(ctx, mode, TailArgs{g, ctx->mb.wsums.as<G1Jac>(), ctx->d_lines(), g.G, 1, 0, ctx->d_partial_out.as<u8>()});
 }
 
-
 static u64 graph_key(const h2v_ctx* ctx, int mode) {
-  u64 h = 0xcbf29ce484222325ull;
-  auto mix = [&h](u64 v) {
-    h ^= v;
-    h *= 0x100000001b3ull;
-    h ^= h >> 29;
-  };
-  const MsmGeom& g = ctx->geom;
-  mix((u64)mode);
-  mix(ctx->n);
-  mix(ctx->gcount);
-  mix(ctx->gbase);
-  mix(ctx->scratch_rows);
-  mix((u64)ctx->has_ncols | (u64)ctx->has_col_len << 1);
-  for (int ch = 0; ch < 2; ch++) mix((u64)g.c[ch] | (u64)g.W[ch] << 8 | (u64)g.Z[ch] << 16);
-  mix((u64)g.T | (u64)g.m << 32);
-  mix((u64)g.G | (u64)g.N << 32);
+  KeyHash k;
+  k.mix((u64)mode);
+  k.mix(ctx->n);
+  k.mix(ctx->gcount);
+  k.mix(ctx->gbase);
+  k.mix(ctx->scratch_rows);
+  k.mix((u64)ctx->has_ncols | (u64)ctx->has_col_len << 1);
+  hash_geom(k, ctx->geom);
   const DevBuf* bufs[] = {&ctx->d_plan, &ctx->d_proofs, &ctx->d_proof_off, &ctx->d_inst, &ctx->d_inst_off, &ctx->d_ncols, &ctx->d_col_len,
                           &ctx->d_pts, &ctx->d_bad, &ctx->d_status, &ctx->d_vals, &ctx->d_scratch, &ctx->d_right, &ctx->d_shared, &ctx->d_left,
                           &ctx->d_r, &ctx->mb.coef, &ctx->mb.shared_sum, &ctx->mb.dig, &ctx->mb.hist, &ctx->mb.off, &ctx->mb.cursor, &ctx->mb.order,
                           &ctx->mb.sorted, &ctx->mb.buckets, &ctx->mb.wsums, &ctx->d_acc_bytes, &ctx->d_verdict, &ctx->mb.partials_msm,
                           &ctx->d_M, &ctx->d_partial_out, &ctx->mb.tiles, &ctx->d_wsums_fin, &ctx->d_ptsc};
-  for (const DevBuf* b : bufs) mix((u64)(size_t)b->p);
-  mix((u64)(size_t)ctx->d_lines());
-  mix((u64)(size_t)ctx->d_gsums.p | (u64)line_run(ctx->geom.G ? ctx->geom.G : 1) << 56);
-  mix((u64)(size_t)ctx->comm.window);
-  if (ctx->hd.n_carry) mix((u64)(size_t)ctx->d_rho.p);
+  for (const DevBuf* b : bufs) k.mix((u64)(size_t)b->p);
+  k.mix((u64)(size_t)ctx->d_lines());
+  k.mix((u64)(size_t)ctx->d_gsums.p | (u64)line_run(ctx->geom.G ? ctx->geom.G : 1) << 56);
+  k.mix((u64)(size_t)ctx->comm.window);
+  if (ctx->hd.n_carry) k.mix((u64)(size_t)ctx->d_rho.p);
   if (mode & RUN_ABSORB) {
-    mix((u64)(size_t)ctx->absorb.acc);
-    mix((u64)(size_t)ctx->absorb.records);
-    mix((u64)(size_t)ctx->absorb.count | (u64)ctx->absorb.cap << 48);
+    k.mix((u64)(size_t)ctx->absorb.acc);
+    k.mix((u64)(size_t)ctx->absorb.records);
+    k.mix((u64)(size_t)ctx->absorb.count | (u64)ctx->absorb.cap << 48);
   }
-  return h | 1;
+  return k.h | 1;
 }
 
 // Every kernel of the batch on the context's stream: replay of the captured graph (one launch) or, with graphs
@@ -2536,53 +2629,17 @@ static int run_impl(h2v_ctx* ctx, int mode) {
   if (!ctx->use_graphs) {
     int rc = enqueue_batch(ctx, mode);
     if (rc) return rc;
-    ctx->stages_timed = true;
-    ctx->verdicts_on_device = (mode & RUN_PAIRING) != 0;
-    ctx->ran = true;
-    return 0;
+  } else {
+    GraphSlot* gs = nullptr;
+    int rc = graph_lookup(ctx->graphs, ctx->graph_clock, graph_key(ctx, mode), &ctx, 1, s, [&] { return enqueue_batch(ctx, mode); }, &gs);
+    if (rc) return rc;
+    CKC(cudaEventRecord(ctx->ev[0], s));
+    CKC(cudaGraphLaunch(gs->exec, s));
+    CKC(cudaEventRecord(ctx->ev[6], s));
+    trace(ctx, "graph launched");
+    ctx->launches += gs->kernels;
   }
-  const u64 key = graph_key(ctx, mode);
-  ctx->use_clock++;
-  h2v_ctx::GraphSlot* hit = nullptr;
-  h2v_ctx::GraphSlot* victim = &ctx->graphs[0];
-  for (auto& sl : ctx->graphs) {
-    if (sl.exec && sl.key == key) hit = &sl;
-    if (!sl.exec ? victim->exec != nullptr : (victim->exec && sl.used < victim->used)) victim = &sl;
-  }
-  h2v_ctx::GraphSlot& gs = hit ? *hit : *victim;
-  gs.used = ctx->use_clock;
-  if (!hit) {
-    trace(ctx, "graph capture begins");
-    if (gs.exec) cudaGraphExecDestroy(gs.exec);
-    gs.exec = nullptr;
-    gs.key = 0;
-    const u64 before = ctx->launches;
-    CKC(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    ctx->capturing = true;
-    const int rc = enqueue_batch(ctx, mode);
-    ctx->capturing = false;
-    cudaGraph_t graph = nullptr;
-    const cudaError_t ce = cudaStreamEndCapture(s, &graph);
-    gs.kernels = ctx->launches - before;
-    ctx->launches = before;
-    if (rc) {
-      if (graph) cudaGraphDestroy(graph);
-      return rc;
-    }
-    CKC(ce);
-    const cudaError_t ie = cudaGraphInstantiate(&gs.exec, graph, prio_mode() ? cudaGraphInstantiateFlagUseNodePriority : 0);
-    cudaGraphDestroy(graph);
-    CKC(ie);
-    gs.key = key;
-    ctx->graph_captures++;
-    trace(ctx, "graph instantiated");
-  }
-  CKC(cudaEventRecord(ctx->ev[0], s));
-  CKC(cudaGraphLaunch(gs.exec, s));
-  CKC(cudaEventRecord(ctx->ev[6], s));
-  trace(ctx, "graph launched");
-  ctx->launches += gs.kernels;
-  ctx->stages_timed = false;
+  ctx->stages_timed = !ctx->use_graphs;
   ctx->verdicts_on_device = (mode & RUN_PAIRING) != 0;
   ctx->ran = true;
   return 0;
@@ -2648,7 +2705,7 @@ static int attribute_impl(h2v_ctx* ctx) {
     int lrc = ensure_lines(ctx, unit, &unit_slot);  // lines of -G2 (pair 0, right) and [s]G2 (pair 1, left)
     if (lrc) return lrc;
   }
-  const G2Line* unit_lines = ctx->lines[unit_slot].buf.as<G2Line>();
+  const G2Line* unit_lines = ctx->lines.s[unit_slot].buf.as<G2Line>();
   CKC(ctx->d_sub_M.ensure(sizeof(E12) * H2V_ATE_ITERS * (size_t)CHUNK));
   CKC(ctx->d_pp_lr.ensure(sizeof(G1Jac) * (size_t)2 * CHUNK));
   CKC(ctx->d_pp_prod.ensure(sizeof(G1Jac) * (size_t)CHUNK * nbases));
@@ -2849,11 +2906,7 @@ static int sum_and_pair(h2v_ctx* ctx, const MsmGeom& g, const G2Line* lines, u32
   if (prc) return prc;
   if (batch_accum) {
     CKC(ctx->d_acc_bytes.ensure(128 * (size_t)sets));
-    FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {0, g.W[0]}};
-    for (u32 st = 0; st < sets; st++) {
-      k_fold_accum<<<1, 32, 0, s>>>(fa, ctx->d_wsums_fin.as<G1Jac>() + (size_t)st * npts, ctx->d_acc_bytes.as<u8>() + 128 * (size_t)st);
-      LAUNCH_CHECK();
-    }
+    if ((prc = enqueue_fold_accum(ctx, g, ctx->d_wsums_fin.as<G1Jac>(), sets, ctx->d_acc_bytes.as<u8>(), false)) != 0) return prc;
     CKC(cudaMemcpyAsync(batch_accum, ctx->d_acc_bytes.p, 128 * (size_t)sets, cudaMemcpyDeviceToHost, s));
   }
   CKC(ctx->h_verd.ensure(4 * (size_t)(groups + 2)));
@@ -2879,14 +2932,14 @@ static int finalize_impl(h2v_ctx* ctx, u32 n_partials, u32 groups, const u8* par
   int rc = device_partials(ctx, partials, (size_t)H2V_PARTIAL_BYTES * n_partials * groups, &d_parts);
   if (rc) return rc;
   if (ctx->n == 0 && (rc = partial_geom(ctx, d_parts, ctx->geom)) != 0) return rc;  // a context that has not processed a shard itself
-  const int lines_of_batch = ctx->lines_cur;  // the resident batch of this context keeps its own line geometry (restored below)
+  const int lines_of_batch = ctx->lines.cur;  // the resident batch of this context keeps its own line geometry (restored below)
   {
     int lrc = ensure_lines(ctx, groups);
     if (lrc) return lrc;
   }
   u32 all = 0;
   rc = sum_and_pair(ctx, ctx->geom, ctx->d_lines(), 0, n_partials, groups, 1, d_parts, batch_accum, group_verdicts, &all);
-  if (lines_of_batch >= 0 && ctx->n) ctx->lines_cur = lines_of_batch;
+  if (lines_of_batch >= 0 && ctx->n) ctx->lines.cur = lines_of_batch;
   if (rc) return rc;
   if (verdict) *verdict = (int)all;
   return 0;
@@ -3068,10 +3121,8 @@ int h2v_verify_shard(h2v_ctx* ctx, uint32_t n, const uint8_t* proofs, const uint
 int h2v_comm_last_batch_accum(h2v_ctx* ctx, uint8_t* batch_accum) {
   if (!ctx || !batch_accum || !ctx->comm.ready || ctx->geom.G != 1) return -1;
   CKC(cudaSetDevice(ctx->device));
-  const MsmGeom& g = ctx->geom;
-  FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {0, g.W[0]}};
-  k_fold_accum<<<1, 32, 0, ctx->stream>>>(fa, ctx->d_wsums_fin.as<G1Jac>(), ctx->d_acc_bytes.as<u8>());
-  LAUNCH_CHECK();
+  const int rc = enqueue_fold_accum(ctx, ctx->geom, ctx->d_wsums_fin.as<G1Jac>(), 1, ctx->d_acc_bytes.as<u8>(), false);
+  if (rc) return rc;
   CKC(cudaMemcpyAsync(batch_accum, ctx->d_acc_bytes.p, 128, cudaMemcpyDeviceToHost, ctx->stream));
   CKC(ctx_sync(ctx));
   return 0;
@@ -3289,9 +3340,9 @@ struct h2v_mix {
   u64 call_base = 0;           // call index of the upload's first proof (a shard: its global base)
   std::vector<u32> grange;     // call-index range of every group: [grange[q], grange[q + 1])
   MsmGeom geom{};
-  int lines_slot = -1;  // the lead's prepared lines of the joint geometry (single-params mix)
-  h2v_ctx::GraphSlot graphs[8];  // LRU over (member shapes, buffers), as for a context
-  u64 use_clock = 0;
+  int lines_slot = -1;  // slot of the lines of the joint geometry: in mlines (multi-params mix) or the lead's cache
+  GraphSlot graphs[8];  // LRU over (member shapes, buffers), as for a context
+  u64 graph_clock = 0;
   // params classes: members whose params agree on (g, g2, s_g2), numbered by first appearance (one class unless multi)
   bool multi = false;
   std::vector<u32> cls_of;     // per member
@@ -3299,19 +3350,16 @@ struct h2v_mix {
   // current batch: bucket set of each class (~0u: no proofs), bucket sets, run length of the window combination
   std::vector<u32> set_of_class;
   u32 sets = 1, run = 0;
-  // multi-params mix: line tables of (pair geometry, classes with proofs), set-major; an LRU of its own, so that the lead's
+  // multi-params mix: line tables of (pair geometry, classes with proofs), set-major; a cache of its own, so that the lead's
   // cache (keyed by geometry alone) never holds a multi-class table
-  h2v_ctx::LinesSlot mlines[4];
-  int mlines_cur = -1;
-  u64 mlines_clock = 0;
+  LinesCache mlines;
   // sharded mixed batches (h2v_mix_accumulate_shard / h2v_mix_verify_shard)
   DevBuf d_partial;          // this rank's partials: one H2V_PARTIAL_BYTES blob per bucket set (RUN_PARTIAL)
   u32 opt_shard_hint = 0;    // one-shot: window geometry for shards of up to this many proofs (h2v_mix_set_shard_hint)
   std::vector<u32> counts;   // proofs per member of the batch / shard last uploaded
   bool ran = false;          // a launch set ran on that upload (h2v_mix_attribute_shard)
   bool xchg_root = false;    // the last launch set went through the exchange with this rank as its root
-  const G2Line* lines() const { return multi ? mlines[mlines_cur].buf.as<G2Line>() : m[0]->lines[lines_slot].buf.as<G2Line>(); }
-  const DevBuf& lines_buf() const { return multi ? mlines[mlines_cur].buf : m[0]->lines[lines_slot].buf; }
+  const G2Line* lines() const { return (multi ? mlines : m[0]->lines).s[lines_slot].buf.as<G2Line>(); }
 };
 
 static const G1Affine& plan_g(const h2v_ctx* c) {  // params.g: the last shared base of every plan
@@ -3339,44 +3387,21 @@ static MsmGeom mix_geom(u32 N, u32 T, u32 right_terms, u32 left_terms, u32 sets,
   return g;
 }
 
-// The multi-params line table of the current batch: build_window_lines over each class with proofs (its (q_right, q_left)),
-// concatenated in class order, for the pair geometry q; cached in the mix under (geometry, classes with proofs).
-static int ensure_mix_lines(h2v_mix* mx, const MsmGeom& q) {
-  h2v_ctx* ctx = mx->m[0];
+extern "C++" {  // (inside the extern "C" block of the ABI: the mix's overloads of ensure_lines and graph_key)
+// The lines of the current batch's pair geometry q -> mx->lines_slot.  A single-params mix uses the lead's lines and cache.  A
+// multi-params mix uses one table per class with proofs (its (q_right, q_left)), in class order, cached in the mix under
+// (geometry, classes with proofs).
+static int ensure_lines(h2v_mix* mx, const MsmGeom& q) {
+  h2v_ctx* lead = mx->m[0];
+  if (!mx->multi) return ensure_lines(lead, q, &mx->lines_slot);
   u64 key = lines_key_of(q);
+  std::vector<const PlanInfo*> classes;
   for (u32 c = 0; c < mx->set_of_class.size(); c++)
-    if (mx->set_of_class[c] != ~0u) key |= 1ull << (48 + c);
-  mx->mlines_clock++;
-  int victim = 0;
-  for (int i = 0; i < 4; i++) {
-    if (mx->mlines[i].key == key) {
-      mx->mlines[i].used = mx->mlines_clock;
-      mx->mlines_cur = i;
-      return 0;
+    if (mx->set_of_class[c] != ~0u) {
+      key |= 1ull << (48 + c);
+      classes.push_back(&mx->m[mx->class_rep[c]]->info);
     }
-    if (mx->mlines[i].used < mx->mlines[victim].used) victim = i;
-  }
-  if (mx->sets * (q.W[0] + q.W[1]) > 128) {
-    ctx->err = "window geometry exceeds 128 (channel, window) pairs";
-    return -1;
-  }
-  std::vector<u8> tab, one;
-  for (u32 c = 0; c < mx->set_of_class.size(); c++) {
-    if (mx->set_of_class[c] == ~0u) continue;
-    build_window_lines(mx->m[mx->class_rep[c]]->info, q.c[0], q.W[0], q.c[1], q.W[1], one);
-    tab.insert(tab.end(), one.begin(), one.end());
-  }
-  h2v_ctx::LinesSlot& sl = mx->mlines[victim];
-  CKC(ctx_sync(ctx));  // the victim's lines may still be read by queued work
-  sl.key = ~0ull;
-  CKC(sl.buf.ensure(tab.size()));
-  CKC(cudaMemcpyAsync(sl.buf.p, tab.data(), tab.size(), cudaMemcpyHostToDevice, ctx->stream));
-  CKC(ctx_sync(ctx));
-  sl.key = key;
-  sl.used = mx->mlines_clock;
-  mx->mlines_cur = victim;
-  ctx->lines_builds++;
-  return 0;
+  return ensure_lines(lead, mx->mlines, key, q, classes, -1, &mx->lines_slot);
 }
 
 static std::vector<h2v_ctx*> mix_active(const h2v_mix* mx) {
@@ -3386,7 +3411,7 @@ static std::vector<h2v_ctx*> mix_active(const h2v_mix* mx) {
 }
 
 // Every kernel of a mixed batch: the members' stages forked onto their own streams, the joint MSM on the lead's stream, then,
-// by the RUN_* mode bits of enqueue_batch: RUN_PAIRING the pairing check over every bucket set -> the lead's d_verdict[0];
+// by the RUN_* mode bits (enqueue_tail on the lead): RUN_PAIRING the pairing check over every bucket set -> the lead's d_verdict[0];
 // RUN_ACCUM (with RUN_PAIRING) one folded (L, R) per bucket set; RUN_PARTIAL one partial per bucket set -> mx->d_partial
 // (sharded mixes); RUN_XCHG (+ RUN_ROOT) the device-side exchange over the lead's channel, the root's summed window sums in
 // the lead's d_wsums_fin.  *fail = the context whose call failed.
@@ -3396,8 +3421,8 @@ static int mix_enqueue(h2v_mix* mx, int mode, h2v_ctx** fail) {
   cudaStream_t s = ctx->stream;
   const MsmGeom& g = mx->geom;
   CKC(cudaMemsetAsync(mx->b.hist.p, 0, 4 * ((size_t)g.nb() * g.G + 2 * SIZE_BINS), s));
-  const bool timed = !ctx->use_graphs;  // direct launches: the lead's events time the joint stages (h2v_last_timings)
-  if (timed) CKC(cudaEventRecord(ctx->ev[0], s));
+  // (direct launches: the lead's events time the joint stages, h2v_last_timings)
+  if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[0], s));
   CKC(cudaEventRecord(mx->ev_fork, s));
   // fold coefficients of every group, written into the members' arrays: on the lead's auxiliary stream while the proofs are
   // parsed (every member's d_r holds the r_i of the whole call)
@@ -3427,7 +3452,7 @@ static int mix_enqueue(h2v_mix* mx, int mode, h2v_ctx** fail) {
   }
   *fail = ctx;
   CKC(cudaStreamWaitEvent(s, ctx->ev_join, 0));
-  if (timed) CKC(cudaEventRecord(ctx->ev[3], s));  // MSM = [3] -> [4], pairing = [4] -> [5]
+  if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[3], s));  // MSM = [3] -> [4], pairing = [4] -> [5]
   {
     NvtxRange nv_("h2v:mix_msm");
     if (sh_max) KLAUNCH(k_shared_reduce_seg, dim3((u32)mx->segs.size(), sh_max), 256, 0, s, mx->d_seg.as<MixSeg>());
@@ -3435,78 +3460,41 @@ static int mix_enqueue(h2v_mix* mx, int mode, h2v_ctx** fail) {
     int rc = enqueue_buckets(ctx, g, mx->b, s, TermArrays{}, src, nullptr, 0);
     if (rc) return rc;
   }
-  if (timed) CKC(cudaEventRecord(ctx->ev[4], s));
-  if (mode & RUN_PAIRING) {
-    NvtxRange nv_("h2v:pairing");
-    int rc = launch_pairing(ctx, g, mx->lines(), mx->b.wsums.as<G1Jac>(), mx->groups, mx->run, mx->sets);
-    if (rc) return rc;
-  }
-  const u32 cb = g.c[0] | g.c[1] << 16, wd = g.W[0] | g.W[1] << 16, npts = g.W[0] + g.W[1];
-  if (mode & RUN_PARTIAL) KLAUNCH(k_pack_partial, dim3(8, g.G), 256, 0, s, cb, wd, npts, mx->b.wsums.as<G1Jac>(), mx->d_partial.as<u8>());
-  if (mode & RUN_XCHG) {
-    NvtxRange nv_("h2v:exchange");
-    // as enqueue_batch's exchange step, with one blob per bucket set and ONE check over all sets on the root
-    h2v_ctx::Comm& cm = ctx->comm;
-    u32* vd = ctx->d_verdict.as<u32>();
-    CKC(cudaMemsetAsync(vd + 1, 0, 8, s));  // error words of this launch set
-    KLAUNCH(k_pack_partial_x, g.G, 256, 0, s, cb, wd, npts, mx->b.wsums.as<G1Jac>(), cm.d_dyn, cm.d_peers, cm.lay, cm.d_done);
-    if (mode & RUN_ROOT) {
-      KLAUNCH_P(false, k_sum_partials, g.G, 128, 0, s, cm.lay.world, cb, wd, npts, cm.window + cm.lay.partials_off(), (size_t)cm.lay.max_groups * H2V_PARTIAL_BYTES,
-                ctx->d_wsums_fin.as<G1Jac>(), vd + 1, cm.d_dyn, (const u64*)(cm.window + cm.lay.arrive_off()));
-      int prc = launch_pairing(ctx, g, mx->lines(), ctx->d_wsums_fin.as<G1Jac>(), 1, mx->run, mx->sets);
-      if (prc) return prc;
-      KLAUNCH_P(false, k_bcast_verdict, 1, 256, 0, s, cm.d_dyn, cm.d_peers, cm.lay, 1u, vd, vd + 1);
-    }
-    KLAUNCH_P(false, k_wait_verdict, 1, 64, 0, s, cm.d_dyn, cm.window, cm.lay, 1u, vd);
-  }
-  if (timed) CKC(cudaEventRecord(ctx->ev[5], s));
-  if (mode & RUN_ACCUM)  // one (L, R) per bucket set (group-major): its window sums are wsums[set][W0 + W1]
-    for (u32 st = 0; st < g.G; st++) {
-      FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {g.wbase[0], g.wbase[1]}};
-      KLAUNCH(k_fold_accum, 1, 32, 0, s, fa, mx->b.wsums.as<G1Jac>() + (size_t)st * (g.W[0] + g.W[1]), ctx->d_acc_bytes.as<u8>() + 128 * (size_t)st);
-    }
-  if (timed) CKC(cudaEventRecord(ctx->ev[6], s));
-  return 0;
+  // one check per group over its bucket sets; a sharded mix (one group) exchanges one blob per bucket set
+  return enqueue_tail(ctx, mode, TailArgs{g, mx->b.wsums.as<G1Jac>(), mx->lines(), mx->groups, mx->sets, mx->run, mx->d_partial.as<u8>()});
 }
 
-static u64 mix_graph_key(const h2v_mix* mx, int mode) {
-  u64 h = 0xcbf29ce484222325ull;
-  auto mix = [&h](u64 v) {
-    h ^= v;
-    h *= 0x100000001b3ull;
-    h ^= h >> 29;
-  };
+static u64 graph_key(const h2v_mix* mx, int mode) {
+  KeyHash k;
   const h2v_ctx* lead = mx->m[0];
-  const MsmGeom& g = mx->geom;
-  mix((mode & RUN_ACCUM) ? 1 : 0);
+  k.mix((mode & RUN_ACCUM) ? 1 : 0);
   // (not the split of the members' proofs over the groups: the segment table and the group ranges are device data)
-  mix(mx->groups);
+  k.mix(mx->groups);
   for (u32 mi : mx->active) {
     h2v_ctx* mb = mx->m[mi];
-    mix((u64)(size_t)mb);
-    mix(graph_key(mb, 0));  // the member's shape, options and buffers (what enqueue_stages and the segment read)
-    mix(mx->set_of_class[mx->cls_of[mi]]);  // the class assignment (bucket set of the member)
+    k.mix((u64)(size_t)mb);
+    k.mix(graph_key(mb, 0));  // the member's shape, options and buffers (what enqueue_stages and the segment read)
+    k.mix(mx->set_of_class[mx->cls_of[mi]]);  // the class assignment (bucket set of the member)
   }
-  for (int ch = 0; ch < 2; ch++) mix((u64)g.c[ch] | (u64)g.W[ch] << 8 | (u64)g.Z[ch] << 16);
-  mix((u64)g.T | (u64)g.m << 32);
-  mix((u64)g.N | (u64)g.G << 32);
+  hash_geom(k, mx->geom);
   const DevBuf* bufs[] = {&mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets, &mx->b.wsums,
-                          &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_grange, &mx->d_ssum, &lead->d_M, &lead->d_gsums, &lead->d_verdict, &lead->d_acc_bytes,
-                          &mx->lines_buf()};
-  for (const DevBuf* b : bufs) mix((u64)(size_t)b->p);
-  mix(mx->run);
+                          &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_grange, &mx->d_ssum, &lead->d_M, &lead->d_gsums, &lead->d_verdict, &lead->d_acc_bytes};
+  for (const DevBuf* b : bufs) k.mix((u64)(size_t)b->p);
+  k.mix((u64)(size_t)mx->lines());
+  k.mix(mx->run);
   if (mode & (RUN_PARTIAL | RUN_XCHG)) {  // sharded launch sets: the mode (root or not), the partial buffers and the lead's channel
     const h2v_ctx::Comm& cm = lead->comm;
-    mix((u64)mode);
-    mix((u64)(size_t)mx->d_partial.p);
-    mix((u64)(size_t)lead->d_wsums_fin.p);
-    mix((u64)(size_t)cm.window);
-    mix((u64)(size_t)cm.d_peers ^ (u64)(size_t)cm.d_dyn << 1 ^ (u64)(size_t)cm.d_done << 2);
-    mix((u64)cm.lay.rank | (u64)cm.lay.world << 32);
-    mix(cm.lay.max_groups);
+    k.mix((u64)mode);
+    k.mix((u64)(size_t)mx->d_partial.p);
+    k.mix((u64)(size_t)lead->d_wsums_fin.p);
+    k.mix((u64)(size_t)cm.window);
+    k.mix((u64)(size_t)cm.d_peers ^ (u64)(size_t)cm.d_dyn << 1 ^ (u64)(size_t)cm.d_done << 2);
+    k.mix((u64)cm.lay.rank | (u64)cm.lay.world << 32);
+    k.mix(cm.lay.max_groups);
   }
-  return h | 1;
+  return k.h | 1;
 }
+}  // extern "C++"
 
 // the launch set on the lead's stream: graph replay (capture on a miss) or, with the lead's graphs off, direct launches
 static int mix_run(h2v_mix* mx, int mode, h2v_ctx** fail) {
@@ -3514,57 +3502,20 @@ static int mix_run(h2v_mix* mx, int mode, h2v_ctx** fail) {
   *fail = lead;
   h2v_ctx* ctx = lead;
   cudaStream_t s = lead->stream;
-  const std::vector<h2v_ctx*> act = mix_active(mx);
   // the members' uploads were queued on their own streams: the launch set (forked from the lead's stream) follows them
-  for (h2v_ctx* mb : act) {
-    if (mb == lead) continue;
-    const u32 mi = (u32)(std::find(mx->m.begin(), mx->m.end(), mb) - mx->m.begin());
-    CKC(cudaEventRecord(mx->ev_join[mi], mb->stream));
+  for (u32 mi : mx->active) {
+    if (mi == 0) continue;
+    CKC(cudaEventRecord(mx->ev_join[mi], mx->m[mi]->stream));
     CKC(cudaStreamWaitEvent(s, mx->ev_join[mi], 0));
   }
   lead->stages_timed = !lead->use_graphs;
   if (!lead->use_graphs) return mix_enqueue(mx, mode, fail);
-  const u64 key = mix_graph_key(mx, mode);
-  mx->use_clock++;
-  h2v_ctx::GraphSlot* hit = nullptr;
-  h2v_ctx::GraphSlot* victim = &mx->graphs[0];
-  for (auto& sl : mx->graphs) {
-    if (sl.exec && sl.key == key) hit = &sl;
-    if (!sl.exec ? victim->exec != nullptr : (victim->exec && sl.used < victim->used)) victim = &sl;
-  }
-  h2v_ctx::GraphSlot& gs = hit ? *hit : *victim;
-  gs.used = mx->use_clock;
-  if (!hit) {
-    if (gs.exec) cudaGraphExecDestroy(gs.exec);
-    gs.exec = nullptr;
-    gs.key = 0;
-    std::vector<u64> before;
-    for (h2v_ctx* c : mx->m) before.push_back(c->launches);
-    CKC(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-    for (h2v_ctx* mb : act) mb->capturing = true;
-    const int rc = mix_enqueue(mx, mode, fail);
-    for (h2v_ctx* mb : act) mb->capturing = false;
-    cudaGraph_t graph = nullptr;
-    const cudaError_t ce = cudaStreamEndCapture(s, &graph);
-    gs.kernels = 0;
-    for (size_t i = 0; i < mx->m.size(); i++) {
-      gs.kernels += mx->m[i]->launches - before[i];
-      mx->m[i]->launches = before[i];
-    }
-    if (rc) {
-      if (graph) cudaGraphDestroy(graph);
-      return rc;
-    }
-    *fail = lead;
-    CKC(ce);
-    const cudaError_t ie = cudaGraphInstantiate(&gs.exec, graph, 0);
-    cudaGraphDestroy(graph);
-    CKC(ie);
-    gs.key = key;
-    lead->graph_captures++;
-  }
-  CKC(cudaGraphLaunch(gs.exec, s));
-  lead->launches += gs.kernels;
+  // (every member is marked capturing, the lead too when it has no proofs: mix_enqueue records the lead's events)
+  GraphSlot* gs = nullptr;
+  int rc = graph_lookup(mx->graphs, mx->graph_clock, graph_key(mx, mode), mx->m.data(), mx->m.size(), s, [&] { return mix_enqueue(mx, mode, fail); }, &gs);
+  if (rc) return rc;
+  CKC(cudaGraphLaunch(gs->exec, s));
+  lead->launches += gs->kernels;
   return 0;
 }
 
@@ -3789,8 +3740,7 @@ static int mix_upload(h2v_mix* mx, u32 groups, const u32* qcounts, const u32* gc
     CKC(mx->d_partial.ensure((size_t)H2V_PARTIAL_BYTES * mx->sets));
     CKC(lead->d_wsums_fin.ensure(sizeof(G1Jac) * 128 * (size_t)mx->sets));
   }
-  const MsmGeom q = pair_geom_run(mx->geom, mx->run);
-  return mx->multi ? ensure_mix_lines(mx, q) : ensure_lines(lead, q, &mx->lines_slot);
+  return ensure_lines(mx, pair_geom_run(mx->geom, mx->run));
 }
 
 static void mix_mark_ran(h2v_mix* mx) {
@@ -3965,7 +3915,7 @@ static int mix_create(h2v_mix** out, h2v_ctx* const* members, uint32_t n_members
   for (DevBuf* d : {&mx->b.coef, &mx->b.shared_sum, &mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets,
                     &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_grange, &mx->d_ssum, &mx->d_partial})
     d->st = &l->stream;
-  for (auto& sl : mx->mlines) sl.buf.st = &l->stream;
+  for (auto& sl : mx->mlines.s) sl.buf.st = &l->stream;
   cudaError_t e = cudaSetDevice(l->device);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&mx->ev_fork, cudaEventDisableTiming);
   for (u32 i = 0; i < n_members && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&mx->ev_join[i], cudaEventDisableTiming);
@@ -3997,7 +3947,7 @@ void h2v_mix_destroy(h2v_mix* mx) {
   for (DevBuf* d : {&mx->b.coef, &mx->b.shared_sum, &mx->b.dig, &mx->b.hist, &mx->b.off, &mx->b.cursor, &mx->b.order, &mx->b.sorted, &mx->b.buckets,
                     &mx->b.wsums, &mx->b.partials_msm, &mx->b.tiles, &mx->d_seg, &mx->d_grange, &mx->d_ssum, &mx->d_partial})
     d->release();
-  for (auto& sl : mx->mlines) sl.buf.release();
+  for (auto& sl : mx->mlines.s) sl.buf.release();
   cudaStreamSynchronize(l->stream);  // the stream-ordered frees
   if (mx->ev_fork) cudaEventDestroy(mx->ev_fork);
   for (cudaEvent_t ev : mx->ev_join)
@@ -4145,9 +4095,7 @@ static int mix_finalize_impl(h2v_mix* mx, const uint32_t* global_counts, uint32_
   if (!rc) rc = partial_geom(ctx, d_parts, g);  // the geometry every rank packed with (k_sum_partials flags a rank that did not)
   if (rc) return rc;
   mx->run = mix_line_run(mx->sets, g.W[0], g.W[1], line_run(1));
-  const MsmGeom q = pair_geom_run(g, mx->run);
-  rc = mx->multi ? ensure_mix_lines(mx, q) : ensure_lines(ctx, q, &mx->lines_slot);
-  if (rc) return rc;
+  if ((rc = ensure_lines(mx, pair_geom_run(g, mx->run))) != 0) return rc;
   std::vector<u8> acc(batch_accum ? 128 * (size_t)mx->sets : 0);
   u32 all = 0;
   rc = sum_and_pair(ctx, g, mx->lines(), mx->run, n_partials, 1, mx->sets, d_parts, batch_accum ? acc.data() : nullptr, nullptr, &all);
@@ -4237,15 +4185,11 @@ static int mix_comm_accum_impl(h2v_mix* mx, uint8_t* batch_accum) {
     return -1;
   }
   h2v_ctx* ctx = mx->m[0];
-  const MsmGeom& g = mx->geom;
-  const u32 npts = g.W[0] + g.W[1];
   std::vector<u8> acc(128 * (size_t)mx->sets);
   CKC(cudaSetDevice(ctx->device));
-  FoldArgs fa{{g.W[0], g.W[1]}, {g.c[0], g.c[1]}, {0, g.W[0]}};
-  for (u32 st = 0; st < mx->sets; st++) {  // the root's summed window sums of every bucket set (lead's d_wsums_fin)
-    k_fold_accum<<<1, 32, 0, ctx->stream>>>(fa, ctx->d_wsums_fin.as<G1Jac>() + (size_t)st * npts, ctx->d_acc_bytes.as<u8>() + 128 * (size_t)st);
-    LAUNCH_CHECK();
-  }
+  // the root's summed window sums of every bucket set (lead's d_wsums_fin)
+  const int rc = enqueue_fold_accum(ctx, mx->geom, ctx->d_wsums_fin.as<G1Jac>(), mx->sets, ctx->d_acc_bytes.as<u8>(), false);
+  if (rc) return rc;
   CKC(cudaMemcpyAsync(acc.data(), ctx->d_acc_bytes.p, acc.size(), cudaMemcpyDeviceToHost, ctx->stream));
   CKC(ctx_sync(ctx));
   mix_class_accum(mx, acc.data(), batch_accum);
@@ -4528,7 +4472,7 @@ int h2v_acc_finalize(h2v_acc* a, int* verdict, uint8_t* absorb_verdicts, uint32_
   int unit_slot = -1;
   int rc = ensure_lines(ctx, unit, &unit_slot);  // lines of -G2 (pair 0, right) and [s]G2 (pair 1, left)
   if (rc) return acc_fail(a, "anchor", ctx, rc);
-  const G2Line* unit_lines = ctx->lines[unit_slot].buf.as<G2Line>();
+  const G2Line* unit_lines = ctx->lines.s[unit_slot].buf.as<G2Line>();
   const PairSkip none{nullptr, nullptr, 1, 0};
   u32* hv = a->h_buf.as<u32>();
   CKA(cudaStreamWaitEvent(s, a->ev, 0));
