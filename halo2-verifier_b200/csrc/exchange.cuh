@@ -71,6 +71,9 @@ __device__ __forceinline__ bool spin_until_ge(const u64* p, u64 want, u64 timeou
   }
 }
 
+// (The header of a partial carries its window bits and window count, not whether the windows came from a GLV split: the
+// window sums of a split scalar keep their meaning, sum_w 2^(c w) S_w = sum k P, and every rank derives the same geometry
+// from the same batch shape, so partials of equal (c, W) add up either way.)
 // Packs the window sums of fold group blockIdx.x into a partial (32-byte header + 128 Jacobian slots) and stores it
 // into slot [rank][group] of the ROOT's window (peer memory over NVLink; the root's own window when rank == root);
 // the last block to finish publishes this rank's sequence number there.  16-byte stores.

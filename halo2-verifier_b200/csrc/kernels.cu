@@ -97,10 +97,20 @@ __global__ void k_init(PlanView pv, u32 n, const u64* inst_off, const u32* ncols
   status[j] = st;
 }
 
-__global__ void __launch_bounds__(128) k_decompress(PlanView pv, u32 n, const u8* proofs, const u64* proof_off, G1Affine* pts, u32* ptsc, u32* bad, u32 blk_off, u32 blk_total) {
+// phi != null (a lifted GLV geometry, phi_rows): also phi(P) = (beta x, y) of every point into phi (the layout of pts), and
+// every shared base b into pts[msm_points * n + b] with its phi into phi[msm_points * n + b]
+__global__ void __launch_bounds__(128) k_decompress(PlanView pv, u32 n, const u8* proofs, const u64* proof_off, G1Affine* pts, G1Affine* phi, u32* ptsc, u32* bad,
+                                                    u32 blk_off, u32 blk_total) {
   pdl_prologue();
   TlScope tl_(1, pts);
   const PlanHeader& hd = pv.h();
+  if (phi)
+    for (u32 i = (blk_off + blockIdx.x) * blockDim.x + threadIdx.x; i < hd.n_shared; i += blk_total * blockDim.x) {
+      G1Affine q = pv.sec<G1Affine>(hd.off_shared_pts)[i];
+      pts[(size_t)msm_points(hd) * n + i] = q;
+      q.x = Fq::mul_c(q.x, glv_beta());
+      phi[(size_t)msm_points(hd) * n + i] = q;
+    }
   // grid-stride: the grid may be capped below the work (wide_grid) so that this multiplier-bound kernel leaves block
   // slots on every SM to the latency-bound kernels of the other contexts in flight
   for (u32 t = (blk_off + blockIdx.x) * blockDim.x + threadIdx.x; t < n * hd.n_points; t += blk_total * blockDim.x) {
@@ -117,6 +127,10 @@ __global__ void __launch_bounds__(128) k_decompress(PlanView pv, u32 n, const u8
       atomicMin(&bad[j], pv.sec<u32>(hd.off_pt_item)[slot]);
     }
     pts[t] = p;
+    if (phi) {
+      p.x = Fq::mul_c(p.x, glv_beta());
+      phi[t] = p;
+    }
     if (ptsc) {
       uint4* o = (uint4*)(ptsc + 16 * (size_t)t);
       o[0] = make_uint4(canon[0].l[0], canon[0].l[1], canon[0].l[2], canon[0].l[3]);
@@ -199,7 +213,7 @@ __global__ void __launch_bounds__(64, MINB) k_scalar(PlanView pv, u32 n, const u
 // stages found (the precedence of the instance check, lib.rs:51-55) and all its scalars are zeroed.  An identity point gets
 // scalar 0 (the MSM kernels take every affine point as a curve point).
 __global__ void __launch_bounds__(128) k_agg(PlanView pv, u32 n, const u8* inst, const u64* inst_off, const u32* col_len, const Fr* rho,
-                                             G1Affine* pts, Fr* right, Fr* shared, Fr* left, u32* status) {
+                                             G1Affine* pts, G1Affine* phi, Fr* right, Fr* shared, Fr* left, u32* status) {
   pdl_prologue();
   const u32 j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= n) return;
@@ -245,6 +259,10 @@ __global__ void __launch_bounds__(128) k_agg(PlanView pv, u32 n, const u8* inst,
     a.x = ok ? p[q].x : Fq::zero();
     a.y = ok ? p[q].y : Fq::zero();
     pts[(size_t)(P0 + q) * n + j] = a;
+    if (phi) {  // (as in k_decompress)
+      a.x = Fq::mul_c(a.x, glv_beta());
+      phi[(size_t)(P0 + q) * n + j] = a;
+    }
   }
   right[(size_t)P0 * n + j] = live && !id[0] ? r : Fr::zero();
   right[(size_t)(P0 + 1) * n + j] = Fr::zero();
@@ -434,6 +452,13 @@ __global__ void __launch_bounds__(128) k_msm_digits(MsmGeom g, const Fr* right, 
     return;
   }
   if (g.glv) {  // k = k1 + k2 lambda: row 2 t of P, row 2 t + 1 of phi(P)
+    if (g.Z2[ch]) {  // lifted halves, k = a - b lambda (glv_lift)
+      u32 a[5], b[5];
+      glv_lift_term(k.l, t, g.Z[ch], g.Z2[ch], a, b);
+      msm_emit_digits<5>(g, ch, grp, a, false, dig + (size_t)(2 * t) * g.Wmax, hist);
+      msm_emit_digits<5>(g, ch, grp, b, true, dig + (size_t)(2 * t + 1) * g.Wmax, hist);
+      return;
+    }
     GlvHalf h1, h2;
     glv_decompose(k.l, h1, h2);
     msm_emit_digits<5>(g, ch, grp, h1.l, h1.neg, dig + (size_t)(2 * t) * g.Wmax, hist);
@@ -628,8 +653,10 @@ __device__ __forceinline__ G1Jac shfl_down_jac(const G1Jac& p, u32 delta) {
   return r;
 }
 
-// GLV = true (attribution sub-batches): entry 2 t + 1 stands for phi(P_t) = (beta x, y); few, long buckets (56 entries with 4-bit
-// windows), so GLV_BUCKET_LANES lanes share a bucket (entries e0 + q, e0 + q + LANES, ...) and add their partial sums with shuffles
+// GLV = true: entry 2 t + 1 stands for phi(P_t) = (beta x, y).  LANES > 1 (attribution sub-batches): few, long buckets (56 entries
+// with 4-bit windows), so GLV_BUCKET_LANES lanes share a bucket (entries e0 + q, e0 + q + LANES, ...), add their partial sums with
+// shuffles and multiply x by beta themselves.  LANES = 1 (lifted GLV geometry of launch sets): many buckets, one lane each, phi(P)
+// read from the phi rows after the points (one multiplication per point when they are written instead of one per entry)
 #ifndef GLV_BUCKET_LANES
 #define GLV_BUCKET_LANES 2
 #endif
@@ -676,14 +703,21 @@ __global__ void __launch_bounds__(128) k_msm_bucket_sum(MsmGeom g, u32 nb, const
       if (live && q == 0) buckets[b] = acc;
     }
   } else {
-    static_assert(!GLV, "the GLV variant shares its buckets between lanes");
     for (u32 t = (blk_off + blockIdx.x) * blockDim.x + threadIdx.x; t < nb; t += blk_total * blockDim.x) {  // grid-stride, see k_decompress
       const u32 b = order[t];
       G1Jac acc = G1Jac::identity();
       const u32 e0 = off[b], e1 = off[b + 1];
       for (u32 e = e0; e < e1; e++) {
         const u32 ent = sorted[e];
-        acc = g1_add_mixed(acc, term_point(g, ent & 0x7FFFFFFFu, pts, shared_pts, src), (ent >> 31) != 0);
+        if constexpr (GLV) {  // a lifted GLV geometry (launch sets): entry 2 t + 1 reads the precomputed phi(P_t)
+          static_assert(!Src::mixed, "mixed batches have no GLV split");
+          const u32 row = ent & 0x7FFFFFFFu;
+          const G1Affine* p = &msm_point(g, row >> 1, pts, shared_pts);  // (shared_pts: the copy after the points, phi_rows)
+          if (row & 1) p += (size_t)g.P * g.N + g.Sh;
+          acc = g1_add_mixed(acc, *p, (ent >> 31) != 0);
+        } else {
+          acc = g1_add_mixed(acc, term_point(g, ent & 0x7FFFFFFFu, pts, shared_pts, src), (ent >> 31) != 0);
+        }
       }
       buckets[b] = acc;
     }
@@ -1518,9 +1552,9 @@ struct KeyHash {
     h ^= h >> 29;
   }
 };
-// the window geometry: c / W / Z per channel, terms and chunk, bucket sets and proofs
+// the window geometry: c / W / Z / Z2 per channel and the GLV split, terms and chunk, bucket sets and proofs
 static void hash_geom(KeyHash& k, const MsmGeom& g) {
-  for (int ch = 0; ch < 2; ch++) k.mix((u64)g.c[ch] | (u64)g.W[ch] << 8 | (u64)g.Z[ch] << 16);
+  for (int ch = 0; ch < 2; ch++) k.mix((u64)g.c[ch] | (u64)g.W[ch] << 8 | (u64)g.Z[ch] << 16 | (u64)g.Z2[ch] << 40 | (u64)g.glv << 63);
   k.mix((u64)g.T | (u64)g.m << 32);
   k.mix((u64)g.G | (u64)g.N << 32);
 }
@@ -1575,29 +1609,36 @@ static int graph_lookup(GraphSlot (&slots)[N], u64& clock, u64 key, h2v_ctx* con
   return 0;
 }
 
+// Windows of a lifted GLV geometry: W c >= 131, so that 2^(W c - 1) >= 2^130 leaves room for at least 7 lattice lifts of
+// each half (glv_lift_ranges); with the bare minimum of 130 bits the top window of c = 13 stays 4x the mean load.
+static u32 glv_windows(u32 c) { return (131 + c - 1) / c; }
+
 // Window size per channel.  Thanks to the scalar lift k'' = k + z*r every window is uniformly filled, so
 // the choice is a pure work trade-off: bucket additions (11 MM) against bucket reduction (2 x 16 MM
 // per bucket plus the per-chunk offset multiplication), with a floor on the per-bucket serial chain.
 // chain_weight: 1 = throughput (several fold groups share the launches: total work decides), 2 = latency (a single
 // batch: the longest bucket chain is on the critical path).  Measured, 4096 VM proofs: c = 11 -> 5.91 M proofs/s and
 // 3.08 ms alone, c = 12 -> 5.80 M and 2.92 ms.
-static double choose_window(u32 terms, u32& c_out, u32& W_out, double chain_floor, double chain_weight) {
-  double best = 1e300, best_chain = 0;
+// Returns the modelled time; chain_out = the chosen window's bucket chain.  glv: the terms are split into two lifted GLV halves
+// (glv_lift): twice the entries per window, glv_windows(c) windows.
+static double choose_window(u32 terms, bool glv, double chain_floor, double chain_weight, u32& c_out, u32& W_out, double& chain_out) {
+  double best = 1e300;
   for (u32 c = 4; c <= 15; c++) {
-    const u32 W = (255 + c - 1) / c;
+    const u32 W = glv ? glv_windows(c) : (255 + c - 1) / c;
     const double B = (double)(1u << (c - 1));
-    const double work = (double)W * ((double)terms * 11.0 + B * 150.0);  // per bucket: measured (window sweep on B200), not just 2 additions
-    const double chain = ((double)terms / B + 1.0) * 11.0;  // dependent MM per bucket thread
+    const double e = glv ? 2.0 * terms : (double)terms;  // entries per window
+    const double work = (double)W * (e * 11.0 + B * 150.0);  // per bucket: measured (window sweep on B200), not just 2 additions
+    const double chain = (e / B + 1.0) * 11.0;  // dependent MM per bucket thread
     // both channels share the bucket kernels: only a chain longer than the other channel's costs latency
     const double t = work / 10e9 + std::max(0.0, chain - chain_floor) * 0.4e-6 * chain_weight;
     if (t < best) {
       best = t;
-      best_chain = chain;
+      chain_out = chain;
       c_out = c;
       W_out = W;
     }
   }
-  return best_chain;
+  return best;
 }
 
 // Z = floor(2^(W*c-1) / r): k + z*r < 2^(W*c-1) for z < Z, so the top signed digit never carries out.
@@ -1611,12 +1652,27 @@ static u32 lift_range(u32 c, u32 W) {
 // n_geom >= n: the window geometry is chosen as for a batch of n_geom proofs (sharded batches: every
 // rank must use the same windows so that partial window sums add up, see h2v_batch_set_shard_hint)
 // window fields of g for right_terms / left_terms terms per channel and fold group (the batch size n_geom picks the chunk)
-static void choose_windows(MsmGeom& g, u32 right_terms, u32 left_terms, u32 n_geom, u32 groups, u32 force_c) {
+static void choose_windows(MsmGeom& g, u32 right_terms, u32 left_terms, u32 n_geom, u32 groups, u32 force_c, bool glv_ok = false) {
   const double cw = groups > 1 ? 1.0 : 2.0;
-  const double chain_right = choose_window(right_terms, g.c[0], g.W[0], 0.0, cw);
-  choose_window(left_terms, g.c[1], g.W[1], chain_right, cw);
+  double chain;
+  double cost = choose_window(right_terms, false, 0.0, cw, g.c[0], g.W[0], chain);
+  cost += choose_window(left_terms, false, chain, cw, g.c[1], g.W[1], chain);
   const char* f0 = getenv("H2V_MSM_WINDOW_RIGHT");
   const char* f1 = getenv("H2V_MSM_WINDOW_LEFT");
+  const char* fg = getenv("H2V_MSM_GLV");
+  g.glv = 0;
+  if (glv_ok && !force_c && !f0 && !f1) {
+    u32 c[2], W[2];
+    double gcost = choose_window(right_terms, true, 0.0, cw, c[0], W[0], chain);
+    gcost += choose_window(left_terms, true, chain, cw, c[1], W[1], chain);
+    if (fg ? atoi(fg) == 1 : groups > 1 && gcost < cost) {
+      g.glv = 1;
+      for (int ch = 0; ch < 2; ch++) {
+        g.c[ch] = c[ch];
+        g.W[ch] = W[ch];
+      }
+    }
+  }
   for (int ch = 0; ch < 2; ch++) {
     const char* f = ch == 0 ? f0 : f1;
     if (force_c) {  // attribution sub-batches: both channels with the same window size (one reduction chunk per window),
@@ -1627,7 +1683,9 @@ static void choose_windows(MsmGeom& g, u32 right_terms, u32 left_terms, u32 n_ge
       g.W[ch] = (255 + g.c[ch] - 1) / g.c[ch];
     }
     g.B[ch] = 1u << (g.c[ch] - 1);
-    g.Z[ch] = force_c ? 1u : lift_range(g.c[ch], g.W[ch]);
+    g.Z2[ch] = 0;
+    if (g.glv) glv_lift_ranges(g.c[ch], g.W[ch], g.Z[ch], g.Z2[ch]);
+    else g.Z[ch] = force_c ? 1u : lift_range(g.c[ch], g.W[ch]);
   }
   g.wbase[0] = 0;
   g.wbase[1] = g.W[0];
@@ -1642,7 +1700,7 @@ static void choose_windows(MsmGeom& g, u32 right_terms, u32 left_terms, u32 n_ge
     const int m = atoi(fm);
     if (m == 2 || m == 4 || m == 8) g.m = (u32)m;
   }
-  g.glv = force_c ? 1u : 0u;
+  if (force_c) g.glv = 1;
   if (force_c) g.m = g.B[0];  // the whole window is one chunk: its weighted sum IS the window sum (enqueue_msm skips the second step)
 }
 static MsmGeom choose_geom(u32 n, const PlanHeader& hd, u32 n_geom, u32 groups = 1, u32 force_c = 0) {
@@ -1655,7 +1713,8 @@ static MsmGeom choose_geom(u32 n, const PlanHeader& hd, u32 n_geom, u32 groups =
   g.Sh = hd.n_shared;
   g.T = n * g.P + n * g.n_mo + hd.n_shared;
   if (n_geom < n) n_geom = n;
-  choose_windows(g, n_geom * g.P + hd.n_shared, n_geom * g.n_mo, n_geom, groups, force_c);
+  // (a GLV split doubles the term ids: 2 G T must stay inside the 31 bits of a bucket entry, k_msm_scatter)
+  choose_windows(g, n_geom * g.P + hd.n_shared, n_geom * g.n_mo, n_geom, groups, force_c, 2ull * g.T * groups < (1ull << 31));
   return g;
 }
 
@@ -1829,6 +1888,7 @@ static cudaError_t preload_kernels() {
   H2V_PRELOAD((k_msm_bucket_sum<false, 2, SingleVkTerms>));
   H2V_PRELOAD((k_msm_bucket_sum<false, 4, SingleVkTerms>));
   H2V_PRELOAD((k_msm_bucket_sum<true, GLV_BUCKET_LANES, SingleVkTerms>));
+  H2V_PRELOAD((k_msm_bucket_sum<true, 1, SingleVkTerms>));
   H2V_PRELOAD((k_msm_bucket_sum<false, 1, MixTerms>));
   H2V_PRELOAD((k_msm_bucket_sum<false, 2, MixTerms>));
   H2V_PRELOAD((k_msm_bucket_sum<false, 4, MixTerms>));
@@ -2209,11 +2269,12 @@ static int enqueue_buckets(h2v_ctx* ctx, const MsmGeom& g, h2v_ctx::MsmBufs& B, 
     // lanes per bucket: 1 for launch sets of several fold groups (throughput: no shuffle additions), 2 for a single batch and
     // for the attribution sub-batches (their bucket chains are latency)
     static const int lanes_env = getenv("H2V_BUCKET_LANES") ? atoi(getenv("H2V_BUCKET_LANES")) : 0;
-    const u32 lanes = g.glv ? GLV_BUCKET_LANES : (lanes_env ? (u32)lanes_env : (g.G == 1 && g.n <= 8192 ? 2u : 1u));
+    // (a lifted GLV geometry: one lane per bucket, as for the plain launch sets it replaces)
+    const u32 lanes = g.lifted() ? 1u : g.glv ? GLV_BUCKET_LANES : (lanes_env ? (u32)lanes_env : (g.G == 1 && g.n <= 8192 ? 2u : 1u));
     void (*kern)(MsmGeom, u32, const u32*, const u32*, const u32*, const G1Affine*, const G1Affine*, G1Jac*, u32, u32, Src);
     kern = lanes == 2 ? k_msm_bucket_sum<false, 2, Src> : lanes == 4 ? k_msm_bucket_sum<false, 4, Src> : k_msm_bucket_sum<false, 1, Src>;
     if constexpr (!Src::mixed)  // (a mixed batch has no GLV split)
-      if (g.glv) kern = k_msm_bucket_sum<true, GLV_BUCKET_LANES, Src>;
+      if (g.glv) kern = g.lifted() ? k_msm_bucket_sum<true, 1, Src> : k_msm_bucket_sum<true, GLV_BUCKET_LANES, Src>;
     const u32 total = wide_grid((u64)(lanes == 2 || lanes == 4 || g.glv ? lanes : 1u) * nb, 0), K = std::min(wide_split(), total), per = cdiv(total, K);
     for (u32 off = 0; off < total; off += per)
       KLAUNCH(kern, std::min(per, total - off), 128, 0, s, g, nb, B.off.as<u32>(), B.order.as<u32>(), B.sorted.as<u32>(), ta.pts, ta.shared_pts,
@@ -2238,8 +2299,8 @@ static int enqueue_msm(h2v_ctx* ctx, const MsmGeom& g, h2v_ctx::MsmBufs& B, cuda
   int rc = enqueue_shared_reduce(ctx, g, B, s);
   if (rc) return rc;
   PlanView pv = ctx->pv();
-  const TermArrays ta{ctx->d_right.as<Fr>(), ctx->d_left.as<Fr>(), B.coef.as<Fr>(), B.shared_sum.as<Fr>(), ctx->d_pts.as<G1Affine>(),
-                      pv.sec<G1Affine>(ctx->hd.off_shared_pts)};
+  const G1Affine* shared_pts = g.lifted() ? ctx->d_pts.as<G1Affine>() + (size_t)g.P * g.N : pv.sec<G1Affine>(ctx->hd.off_shared_pts);  // (phi_rows)
+  const TermArrays ta{ctx->d_right.as<Fr>(), ctx->d_left.as<Fr>(), B.coef.as<Fr>(), B.shared_sum.as<Fr>(), ctx->d_pts.as<G1Affine>(), shared_pts};
   return enqueue_buckets(ctx, g, B, s, ta, SingleVkTerms{}, parent_verdict, parent_size);
 }
 
@@ -2259,6 +2320,14 @@ static cudaError_t ensure_msm_bufs(const MsmGeom& g, h2v_ctx::MsmBufs& B, u32 n_
   if ((e = B.buckets.ensure(sizeof(G1Jac) * nb)) != cudaSuccess) return e;
   if ((e = B.wsums.ensure(sizeof(G1Jac) * (size_t)(g.W[0] + g.W[1]) * g.G)) != cudaSuccess) return e;
   return B.partials_msm.ensure(sizeof(G1Jac) * (nb / g.m));
+}
+
+// phi(P) rows of a lifted GLV geometry (k_decompress, k_agg write them; k_msm_bucket_sum<true, 1> reads them).  d_pts holds
+// [points: msm_points * N | shared bases: n_shared | phi of the points | phi of the shared bases], so that phi of the base at
+// d_pts[i] is d_pts[i + D], D = msm_points * N + n_shared, for proof points and shared bases alike: the MSM of a lifted
+// geometry reads its shared bases from the copy.  Returns d_pts + D, null for other geometries.
+static G1Affine* phi_rows(h2v_ctx* ctx) {
+  return ctx->geom.lifted() ? ctx->d_pts.as<G1Affine>() + (size_t)ctx->geom.P * ctx->geom.N + ctx->geom.Sh : nullptr;
 }
 
 // Host ranges that make up a batch's proof bytes and instance bytes, in order (a member of a grouped mixed batch: its proofs
@@ -2337,7 +2406,8 @@ static int upload_impl(h2v_ctx* ctx, u32 n, const u8* proofs, const u64* proof_o
   CKC(ctx->d_proof_off.ensure(8 * (size_t)(n + 1)));
   CKC(ctx->d_inst.ensure(32 * iscal + 64));
   CKC(ctx->d_inst_off.ensure(8 * (size_t)(n + 1)));
-  CKC(ctx->d_pts.ensure(sizeof(G1Affine) * (size_t)n * msm_points(hd)));
+  // (a lifted GLV geometry: a copy of the shared bases and the phi rows after the points, phi_rows)
+  CKC(ctx->d_pts.ensure(sizeof(G1Affine) * ((size_t)n * msm_points(hd) + (g.lifted() ? (size_t)n * msm_points(hd) + 2 * hd.n_shared : 0))));
   if (hd.hash == HASH_BLAKE2B) CKC(ctx->d_ptsc.ensure(64 * (size_t)n * hd.n_points));
   CKC(ctx->d_bad.ensure(4 * (size_t)n));
   CKC(ctx->d_status.ensure(4 * (size_t)n));
@@ -2469,7 +2539,7 @@ static int enqueue_stages(h2v_ctx* ctx, bool own_coef = true) {
     const u32 total = wide_grid((u64)n * hd.n_points, 0), K = std::min(wide_split(), total), per = cdiv(total, K);
     for (u32 off = 0; off < total; off += per)
       KLAUNCH(k_decompress, std::min(per, total - off), 128, 0, s, pv, n, ctx->d_proofs.as<u8>(), ctx->d_proof_off.as<u64>(), ctx->d_pts.as<G1Affine>(),
-              use_quad ? ctx->d_ptsc.as<u32>() : nullptr, ctx->d_bad.as<u32>(), off, total);
+              phi_rows(ctx), use_quad ? ctx->d_ptsc.as<u32>() : nullptr, ctx->d_bad.as<u32>(), off, total);
   }
   nvtxRangePop();
   if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[1], s));
@@ -2503,7 +2573,7 @@ static int enqueue_stages(h2v_ctx* ctx, bool own_coef = true) {
   }
   if (hd.n_carry)
     KLAUNCH(k_agg, cdiv(n, 128), 128, 0, s, pv, n, ctx->d_inst.as<u8>(), ctx->d_inst_off.as<u64>(), ctx->has_col_len ? ctx->d_col_len.as<u32>() : nullptr,
-            ctx->d_rho.as<Fr>(), ctx->d_pts.as<G1Affine>(), ctx->d_right.as<Fr>(), ctx->d_shared.as<Fr>(), ctx->d_left.as<Fr>(), ctx->d_status.as<u32>());
+            ctx->d_rho.as<Fr>(), ctx->d_pts.as<G1Affine>(), phi_rows(ctx), ctx->d_right.as<Fr>(), ctx->d_shared.as<Fr>(), ctx->d_left.as<Fr>(), ctx->d_status.as<u32>());
   nvtxRangePop();
   set_launch_class('N');
   if (!ctx->capturing) CKC(cudaEventRecord(ctx->ev[3], s));
@@ -3257,6 +3327,11 @@ int h2v_last_msm_geometry(const h2v_ctx* ctx, uint32_t* out4) {
   out4[2] = ctx->geom.T;
   out4[3] = ctx->geom.nb();
   return 0;
+}
+
+int h2v_last_msm_glv(const h2v_ctx* ctx) {
+  if (!ctx) return -1;
+  return ctx->geom.lifted() ? 1 : 0;
 }
 
 int h2v_selftest_field(int device, uint32_t count, uint64_t seed) {

@@ -34,8 +34,11 @@ struct MsmGeom {
   u32 Z[2];  // scalar lift range: k'' = k + z*r, z in [0, Z), keeps every window (also the top one) uniformly filled
   u32 Wmax;  // row stride of the digit table
   u32 m;     // buckets per reduction chunk
-  u32 glv;   // 1: every term is split into its two GLV halves (glv.cuh), rows / entries 2 t + half; windows cover 130 bits
+  u32 glv;   // 1: every term is split into its two GLV halves (glv.cuh), rows / entries 2 t + half; windows cover 130 bits or more
              // (the attribution sub-batches: half the windows -> half the doublings of their explicit window combination)
+  u32 Z2[2]; // lattice-lift range z' of a lifted GLV geometry (glv_lift), 0 = halves unlifted (attribution).  A lifted geometry
+             // reads phi(P) from the phi rows that follow the points (phi_rows)
+  H2V_HOST_DEVICE bool lifted() const { return glv && Z2[0]; }
   H2V_HOST_DEVICE u32 nb() const { return W[0] * B[0] + W[1] * B[1]; }
   H2V_HOST_DEVICE u32 channel_of_term(u32 tl) const { return (tl >= n * P && tl < n * P + n * n_mo) ? 1u : 0u; }  // tl = term inside its group
 };

@@ -461,6 +461,9 @@ int h2v_debug_timeline_stop(int device, void* out, uint32_t capacity, uint32_t* 
 int h2v_ctx_work_model(const h2v_ctx* ctx, uint32_t instance_rows, double* out4);
 /* MSM geometry of the last run: out[0] window bits, [1] windows, [2] terms, [3] buckets */
 int h2v_last_msm_geometry(const h2v_ctx* ctx, uint32_t* out4);
+/* GLV split of the last run's MSM: 1 when every scalar was split as k = a - b lambda into lifted half-length digit rows
+ * (window geometry of h2v_last_msm_geometry then covers ~131 bits), 0 for plain windows */
+int h2v_last_msm_glv(const h2v_ctx* ctx);
 
 /* ---- device self tests (used by tests/ only) ---------------------------------------------------
  * Runs the PTX field multiplication against the portable one on `count` pseudo-random and edge
